@@ -26,6 +26,8 @@ ABI_SYMBOLS = [
     "dctc_carver_image", "dctc_carver_resize_width", "dctc_carver_enlarge_width", "dctc_carver_set_incremental", "dctc_carver_rebuild_count", "dctc_pixel_energy",
     "dctc_energy_minmax_dev", "dctc_energy_image_dev", "dctc_carver_energy_image", "dctc_preview_energy",
     "dctc_carver_set_dump_vmaps", "dctc_carver_vmap", "dctc_carver_paint_seams",
+    "dctc_carver_batch_create", "dctc_carver_batch_destroy", "dctc_carver_batch_load", "dctc_carver_batch_resize_width",
+    "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy", "dctc_carver_batch_vmap",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -109,6 +111,14 @@ def lib():
         "dctc_carver_set_dump_vmaps": (i32, [vp, i32]),
         "dctc_carver_vmap": (i32, [vp, vp, vp]),
         "dctc_carver_paint_seams": (i32, [vp, vp, i32, C.c_size_t]),
+        "dctc_carver_batch_create": (i32, [vp, i32, i32, i32, i32, i32, C.POINTER(vp)]),
+        "dctc_carver_batch_destroy": (None, [vp]),
+        "dctc_carver_batch_load": (i32, [vp, vp, sz, sz]),
+        "dctc_carver_batch_resize_width": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_width": (i32, [vp]),
+        "dctc_carver_batch_images": (i32, [vp, vp]),
+        "dctc_carver_batch_energy": (i32, [vp, vp]),
+        "dctc_carver_batch_vmap": (i32, [vp, vp, vp]),
         "dctc_pixel_energy": (f32, [i32, i32, i32, i32, vp, vp]),
         "dctc_synth_fill_dev": (i32, [vp, vp, i32, sz, i32, i32, i32, sz, u32, i32, i32, i32]),
         "dctc_synth_byte": (C.c_uint8, [u32, u32, u32, u32, u32, i32]),
@@ -442,6 +452,77 @@ class Context:
         a, b, c = C.c_double(), C.c_double(), C.c_double()
         _check(lib().dctc_pcie_probe(self._h, nbytes, iters, C.byref(a), C.byref(b), C.byref(c)), "dctc_pcie_probe")
         return {"h2d_gbs": a.value, "d2h_gbs": b.value, "bidir_gbs_per_dir": c.value}
+
+
+class CarverBatch:
+    """n equally sized frames retargeted together by one device seam loop (dctc_carver_batch_*): every phase of the loop
+    is one launch for all frames, and each frame gets exactly what a single carver session on the same context gives
+    it.  imgs: uint8 [n, h, w] or [n, h, w, ch].  Uses the context's operator and kernel selection at construction."""
+
+    def __init__(self, ctx, imgs, dump_vmaps=False):
+        imgs = np.asarray(imgs)
+        if imgs.dtype != np.uint8:
+            raise TypeError("frames must be uint8")
+        if imgs.ndim == 3:
+            imgs = imgs[..., None]
+        if imgs.ndim != 4:
+            raise ValueError("frames must be [n, h, w] or [n, h, w, ch]")
+        imgs = np.ascontiguousarray(imgs)
+        self.ctx = ctx
+        self.n, self.h, self.w0, self.ch = imgs.shape
+        self._b = C.c_void_p()
+        _check(lib().dctc_carver_batch_create(ctx.handle, self.n, self.w0, self.h, self.ch, int(bool(dump_vmaps)),
+                                              C.byref(self._b)), "dctc_carver_batch_create")
+        try:
+            _check(lib().dctc_carver_batch_load(self._b, _ptr(imgs), self.h * self.w0 * self.ch, self.w0 * self.ch),
+                   "dctc_carver_batch_load")
+        except Exception:
+            self.close()
+            raise
+
+    @property
+    def handle(self):
+        return self._b
+
+    @property
+    def width(self):
+        return int(lib().dctc_carver_batch_width(self._b))
+
+    def resize_width(self, n_seams):
+        """Removes n_seams vertical seams from every frame; returns int32 [n, n_seams, h], the removed columns in the
+        coordinates of each frame at the time of removal."""
+        seams = np.empty((self.n, n_seams, self.h), np.int32)
+        _check(lib().dctc_carver_batch_resize_width(self._b, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_batch_resize_width")
+        return seams
+
+    def images(self):
+        out = np.empty((self.n, self.h, self.width, self.ch), np.uint8)
+        _check(lib().dctc_carver_batch_images(self._b, _ptr(out)), "dctc_carver_batch_images")
+        return out
+
+    def energy(self):
+        out = np.empty((self.n, self.h, self.width), np.float32)
+        _check(lib().dctc_carver_batch_energy(self._b, _ptr(out)), "dctc_carver_batch_energy")
+        return out
+
+    def vmap(self):
+        """(visibility maps int32 [n, h, w0], depth): removal order per original pixel, 0 = never removed."""
+        out = np.empty((self.n, self.h, self.w0), np.int32)
+        depth = C.c_int(0)
+        _check(lib().dctc_carver_batch_vmap(self._b, _ptr(out), C.byref(depth)), "dctc_carver_batch_vmap")
+        return out, depth.value
+
+    def close(self):
+        if self._b:
+            lib().dctc_carver_batch_destroy(self._b)
+            self._b = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
 
 def band_plan(h, world, rank, blocksize):

@@ -23,10 +23,12 @@ struct DctcK1Args {
     float w_edges, w_textures;  // edges/255, textures/255 (luma is kept in 0..255 units inside the kernels)
     // band mode (K2, per-seam incremental update): when seam != nullptr only the pixels of row y with
     //   x in [min_{|y'-y|<=band_r} seam[y'] - band_r, max_{|y'-y|<=band_r} seam[y'] + band_r - 1] /\ [0, w-1]
-    // are produced (liblqr update_emap), and also copied to band_vals[y*band_stride + x - xmin(y)].
+    // are produced (liblqr update_emap), and also copied to band_vals[y*band_stride + x - xmin(y)].  Batch launches:
+    // frame z reads its seam at seam + z * seam_frame_stride (band_vals is then left null).
     const int* seam;
     float* band_vals;
     int band_r, band_stride;
+    int seam_frame_stride;
     // preview operator (dct_energy_preview_rows, src/render.c:31-60): window offsets -(C-1) .. b-C with C = (b-1)/2
     // (src/dct.h:8-9), BT.601 byte luminance (src/render.h:5), first transform index walks y (tile kernel only)
     int preview;

@@ -41,9 +41,10 @@ __global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Ar
     int tx0 = blockIdx.x * TW;
     __shared__ int s_xmin[TH], s_xmax[TH], s_x0;
     if (a.seam) {  // band mode: the tile row starts at the leftmost band pixel of its rows
+        const int* seam = a.seam + (size_t) blockIdx.z * a.seam_frame_stride;
         if (tid < TH) {
             int lo = a.w, hi = -1;
-            if (ty0 + tid < a.h) dctc_band_limits(a.seam, ty0 + tid, a.h, a.w, a.band_r, &lo, &hi);
+            if (ty0 + tid < a.h) dctc_band_limits(seam, ty0 + tid, a.h, a.w, a.band_r, &lo, &hi);
             s_xmin[tid] = lo;
             s_xmax[tid] = hi;
         }

@@ -10,6 +10,7 @@
 #include <cstdlib>
 #include <type_traits>
 #include <cstring>
+#include <new>
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
 
@@ -24,20 +25,23 @@ int dctc_run_k1(dctc_context* ctx, DctcK1Args& a, int n_frames, cudaStream_t str
 // One CTA per row: shift image bytes and energy floats right of the seam one pixel to the left.
 // Chunks are processed left to right; the barrier between a chunk's loads and its stores also orders them
 // after the previous chunk's loads, so the one-element overlap between neighbouring chunks is safe.
+// Batch sessions: blockIdx.y = frame, whose planes start img_fs bytes / en_fs, m_fs floats after the previous frame's
+// and whose seam is seam[h * frame ...] (h = gridDim.x).
 template <int NT, int K>
 __global__ void __launch_bounds__(NT) dctc_carve_rows_kernel(uint8_t* __restrict__ img, size_t pitch, int channels,
                                                              float* __restrict__ en, size_t en_pitch,
                                                              const int* __restrict__ seam, int w_old,
-                                                             float* __restrict__ mplane, size_t m_pitch)
+                                                             float* __restrict__ mplane, size_t m_pitch,
+                                                             size_t img_fs, size_t en_fs, size_t m_fs)
 {
     DCTC_PDL_PROLOGUE();
-    const int y = blockIdx.x;
-    const int s = seam[y];
-    uint8_t* row = img + (size_t) y * pitch;
-    float* erow = en + (size_t) y * en_pitch;
+    const int y = blockIdx.x, z = blockIdx.y;
+    const int s = seam[(size_t) z * gridDim.x + y];
+    uint8_t* row = img + z * img_fs + (size_t) y * pitch;
+    float* erow = en + z * en_fs + (size_t) y * en_pitch;
     // cumulative map of the seam DP (liblqr keeps it per pixel, so it moves with the pixels): dst x in [s, w_old-1)
     if (mplane) {
-        float* mrow = mplane + (size_t) y * m_pitch;
+        float* mrow = mplane + z * m_fs + (size_t) y * m_pitch;
         for (int base = s; base < w_old - 1; base += NT * K) {
             float v[K];
 #pragma unroll
@@ -257,15 +261,20 @@ __device__ __forceinline__ void dp_unroll(F&& f)
 
 // DP_P float4 groups per lane: strip = 128 * DP_P columns, 128 * DP_P - 2 * DP_R of them published.
 // DP_SR: rows per staged chunk of the bulk-copy variant (32 when two stages per warp fit, else 16), 0 = register ring.
+// One cluster per frame: blockIdx.y = frame of a batch session, whose energy / cumulative planes start en_fs / m_fs
+// floats after the previous frame's, whose seam is seam[h * frame ...], its log seam_log[log_fs * frame ...] and its
+// last-row column xlast[frame].  The tensor map is 3-D (columns, rows, frames) with a box depth of one frame.
 template <int DP_P, int DP_SR>
 __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dctc_seam_dp_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                                     float* __restrict__ mplane, size_t m_pitch,
                                                                     int* __restrict__ seam, int* __restrict__ seam_log,
                                                                     int* __restrict__ run_flag, int nst,
                                                                     const __grid_constant__ CUtensorMap tmap, int use_tmap,
-                                                                    int* __restrict__ xlast)
+                                                                    int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs)
 {
     DCTC_PDL_PROLOGUE();
+    // (the frame's seam, log and xlast offsets are applied after the row loop, so they occupy no registers in it)
+    en += blockIdx.y * en_fs;
     // fallback of the incremental update (dctc_seam_incr_kernel): runs only when that kernel asked for a rebuild
     if (run_flag && *run_flag == 0) return;       // uniform over the cluster, before any cluster barrier
     if (run_flag && blockIdx.x == 0 && threadIdx.x == 0) atomicAdd(run_flag + 1, 1);   // rebuilds since the session was loaded
@@ -319,6 +328,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
     const float* en_g[DP_P];
 #pragma unroll
     for (int g = 0; g < DP_P; g++) en_g[g] = en + (ld_ok[g] ? c0 + 4 * g : 0);
+    float* const mframe = mplane + blockIdx.y * m_fs;
     const int hm1 = h - 1;
 
     // TMA staging of this warp's strip: columns [cs, cs + STRIP) clipped to the row, DP_R rows per stage
@@ -330,12 +340,12 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
     auto issue_chunk = [&](int ch, int st) {   // rows 1 + ch * DP_SR .. (clamped to h - 1) -> stage st = ch % nst
         const uint32_t bar = dp_smem_u32(&ebar[tid >> 5][st]);
         if (use_tmap) {
-            // one 2-D tensor copy (box = STRIP columns x DP_SR rows; columns left of the image and rows below it are
-            // zero-filled by the TMA unit) instead of DP_SR row copies, which the hardware issues one elected lane at a time
+            // one tensor copy (box = STRIP columns x DP_SR rows x 1 frame; columns left of the image and rows below it
+            // are zero-filled by the TMA unit, never read from the next frame) instead of DP_SR row copies, which the hardware issues one elected lane at a time
             if (lane == 0) {
                 asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t) (SRD * STRIP * 4)) : "memory");
-                asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                             ::"r"(dp_smem_u32(estage + (size_t) st * SRD * STRIP)), "l"(&tmap), "r"(cs), "r"(1 + ch * SRD), "r"(bar) : "memory");
+                asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+                             ::"r"(dp_smem_u32(estage + (size_t) st * SRD * STRIP)), "l"(&tmap), "r"(cs), "r"(1 + ch * SRD), "r"(blockIdx.y), "r"(bar) : "memory");
             }
             __syncwarp();
             return;
@@ -374,7 +384,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
     for (int g = 0; g < DP_P; g++) {
         cur[g] = __ldg(reinterpret_cast<const float4*>(en_g[g]));
         const int x = c0 + 4 * g;
-        if (central && ld_ok[g]) *reinterpret_cast<float4*>(mplane + x) = cur[g];
+        if (central && ld_ok[g]) *reinterpret_cast<float4*>(mframe + x) = cur[g];
         patch(cur[g], inf_mask[g]);
         if (!TMA) {
 #pragma unroll
@@ -390,7 +400,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
     // energies are read with immediate offsets from a shared-space base register, cells outside the image are made
     // +inf once per chunk in the staged copy (inf + min = inf, no per-row patch), the cumulative plane is written
     // through one running pointer, and whole blocks run without per-row bounds checks.
-    float* mptr = mplane + m_pitch + c0;             // this lane's first cell of row y
+    float* mptr = mframe + m_pitch + c0;             // this lane's first cell of row y
     unsigned any_mask = 0;
 #pragma unroll
     for (int g = 0; g < DP_P; g++) any_mask |= inf_mask[g];
@@ -570,6 +580,10 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         dp_cluster_sync();   // release/acquire at cluster scope: also orders every CTA's global writes of the cumulative plane
     }
     if (rank == 0 && tid < 32) {
+        const int fz = blockIdx.y;
+        seam += (size_t) fz * h;
+        if (seam_log) seam_log += fz * log_fs;
+        if (xlast) xlast += fz;
         bv = INF;
         bi = 0x7fffffff;
         for (int i = tid; i < nwarps; i += 32) {   // strips in ascending column order: strict < keeps the leftmost
@@ -587,7 +601,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             // parallel back-track: the jump and trace kernels below take over from the seam's last-row column
             if (lane == 0) { *xlast = bi; seam[h - 1] = bi; if (seam_log) seam_log[h - 1] = bi; }
         } else {
-            dp_backtrack(mplane, m_pitch, w, h, bi, seam, seam_log, win, lane);   // serial walk by warp 0 of CTA 0
+            dp_backtrack(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane);   // serial walk by warp 0 of CTA 0
         }
 #ifdef DCTC_SYNC_DEBUG
         if (tid == 0) {
@@ -611,14 +625,18 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
 // into shared memory first), then walks its 32 rows like dp_backtrack does.  ~100 dependent steps instead of h.
 constexpr int JB = 32;
 
+// Batch sessions: blockIdx.z = frame (planes m_fs floats / j_fs bytes apart).
 __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
-                                                             int8_t* __restrict__ jump, size_t j_pitch, int strips)
+                                                             int8_t* __restrict__ jump, size_t j_pitch, int strips,
+                                                             size_t m_fs, size_t j_fs)
 {
     DCTC_PDL_PROLOGUE();
     const int lane = threadIdx.x & 31;
     const int strip = blockIdx.x * 4 + (threadIdx.x >> 5);
     if (strip >= strips) return;
     const int k = blockIdx.y;
+    mplane += blockIdx.z * m_fs;
+    jump += blockIdx.z * j_fs;
     const int yb = h - 1 - JB * k;                    // bottom row of the block
     const int yt = max(yb - JB, 0);                   // top row
     const int steps = yb - yt;
@@ -669,18 +687,24 @@ __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __rest
 constexpr int TR_WIN = 72;                            // walk window: columns x-34 .. x+37 around the block's bottom column
 constexpr int TR_THREADS = 256;
 
+// Batch sessions: blockIdx.y = frame (planes m_fs floats / j_fs bytes apart, seam[h * frame ...],
+// seam_log[log_fs * frame ...], xlast[frame]).
 __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
                                                               const int8_t* __restrict__ jump, size_t j_pitch,
                                                               const int* __restrict__ xlast, int* __restrict__ seam,
-                                                              int* __restrict__ seam_log)
+                                                              int* __restrict__ seam_log, size_t m_fs, size_t j_fs, size_t log_fs)
 {
     extern __shared__ __align__(16) unsigned char tr_smem[];
     __shared__ __align__(16) float win[JB][TR_WIN + 8];
     __shared__ int xb_s;
     DCTC_PDL_PROLOGUE();
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int k = blockIdx.x;
-    const int x0 = *xlast;
+    const int k = blockIdx.x, fz = blockIdx.y;
+    mplane += fz * m_fs;
+    jump += fz * j_fs;
+    seam += (size_t) fz * h;
+    if (seam_log) seam_log += fz * log_fs;
+    const int x0 = xlast[fz];
     // Cone of block j: its bottom column can be x0 - 32 j .. x0 + 32 j.  The entries are staged as aligned 16-byte
     // chunks (at most 4 j + 3 per row, at byte offset 32 j^2 + 16 j of the cone buffer); warp w takes the rows
     // j = w, w + 8, ... and issues all chunks of a row before it stores any of them, so the loads of a row (and of the
@@ -960,15 +984,17 @@ __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restr
 
 // ---- visibility map + seam display (SURVEY section 8f rank 4) ---------------------------------------------------
 // liblqr's update_vsmap: the pixel removed from row y by the k-th seam is original column raw[y][s]; its entry of the
-// visibility map becomes k (1-based).  raw is compacted over the seam like the image (one CTA per row).
+// visibility map becomes k (1-based).  raw is compacted over the seam like the image (one CTA per row).  Batch sessions:
+// blockIdx.y = frame, whose maps follow the previous frame's (w0 x h ints each) and whose seam is seam[h * frame ...].
 __global__ void __launch_bounds__(256) dctc_vs_update_kernel(int* __restrict__ raw, int* __restrict__ vs, int w0,
                                                              const int* __restrict__ seam, int w_old, int order)
 {
     DCTC_PDL_PROLOGUE();
     const int y = blockIdx.x;
-    int* rrow = raw + (size_t) y * w0;
-    const int s = seam[y];
-    if (threadIdx.x == 0) vs[(size_t) y * w0 + rrow[s]] = order;
+    const size_t f0 = (size_t) blockIdx.y * gridDim.x;       // first row of this frame
+    int* rrow = raw + (f0 + y) * w0;
+    const int s = seam[f0 + y];
+    if (threadIdx.x == 0) vs[(f0 + y) * w0 + rrow[s]] = order;
     for (int base = s; base < w_old - 1; base += 256 * 4) {
         int v[4];
 #pragma unroll
@@ -1133,6 +1159,97 @@ static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h,
     return DCTC_OK;
 }
 
+// Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
+// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map.  The single-frame session and the
+// batch session share it, so both run the same kernel variant for the same width.
+using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*, size_t, size_t, size_t);
+struct DpPlan {
+    dp_fn dp = nullptr;
+    int wpc = 0, nst = 0, use_tmap = 0;
+    size_t smem = 0;
+    CUtensorMap tmap;
+};
+
+static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, DpPlan& p)
+{
+    // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
+    const int cap = DP_CL * DP_MAXW;
+    int P = wcur <= cap * (128 - 2 * DP_R) ? 1 : wcur <= cap * (256 - 2 * DP_R) ? 2 : 4;
+    if (const char* ep = getenv("DCTC_DP_P")) {   // timing experiments: wider strips than the width needs
+        const int want = atoi(ep);
+        if ((want == 2 || want == 4) && want > P) P = want;
+    }
+    const int wout = 128 * P - 2 * DP_R;
+    const int strips = (wcur + wout - 1) / wout;
+    const int wpc = (strips + DP_CL - 1) / DP_CL;
+    // energies staged by bulk async copies when at least two stages (DP_SR rows each) per warp fit into shared memory
+    // (the kernel also has ~38 KB of static shared memory: back-track windows, reduction scratch, mbarriers)
+    const size_t xrow_smem = sizeof(float) * 2 * (size_t) wpc * wout;
+    int nst = 0, sr = 0;
+    if (!getenv("DCTC_DP_NO_TMA")) {
+        const size_t row_smem = sizeof(float) * ((size_t) wpc * 128 * P);      // one staged row of every warp
+        const size_t budget = 180 * 1024 - xrow_smem;
+        if (2 * 32 * row_smem <= budget) { sr = 32; nst = 2; }                 // whole 32-row blocks, two in flight
+        else {
+            sr = 16;
+            for (nst = DP_NST_MAX; nst >= 2 && (size_t) nst * 16 * row_smem > budget; nst--) {}
+            if (nst < 2) { sr = 0; nst = 0; }
+        }
+    }
+    p.wpc = wpc;
+    p.nst = nst;
+    p.smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
+    static const dp_fn table[3][3] = {{dctc_seam_dp_kernel<1, 0>, dctc_seam_dp_kernel<1, 16>, dctc_seam_dp_kernel<1, 32>},
+                                      {dctc_seam_dp_kernel<2, 0>, dctc_seam_dp_kernel<2, 16>, dctc_seam_dp_kernel<2, 32>},
+                                      {dctc_seam_dp_kernel<4, 0>, dctc_seam_dp_kernel<4, 16>, dctc_seam_dp_kernel<4, 32>}};
+    p.dp = table[P == 1 ? 0 : P == 2 ? 1 : 2][sr / 16];
+    // tensor map of the energy planes for the staged variant (strips of up to 256 columns: the TMA box limit); frames
+    // are its third dimension, so that a box never reaches into the next frame's rows
+    memset(&p.tmap, 0, sizeof(p.tmap));
+    p.use_tmap = 0;
+    if (sr > 0 && 128 * P <= 256 && !getenv("DCTC_DP_NO_TENSORMAP")) {
+        typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+        void* fp = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qres) == cudaSuccess && fp &&
+            qres == cudaDriverEntryPointSuccess) {
+            const cuuint64_t gdim[3] = {(cuuint64_t) en_pitch, (cuuint64_t) h, (cuuint64_t) n_frames};
+            const cuuint64_t gstr[2] = {(cuuint64_t) en_pitch * sizeof(float), (cuuint64_t) en_pitch * h * sizeof(float)};
+            const cuuint32_t box[3] = {(cuuint32_t) (128 * P), (cuuint32_t) sr, 1};
+            const cuuint32_t estr[3] = {1, 1, 1};
+            if (((encode_fn) fp)(&p.tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*) en, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                                 CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
+                p.use_tmap = 1;
+        } else {
+            (void) cudaGetLastError();
+        }
+    }
+    // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
+    return cudaFuncSetAttribute(p.dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
+}
+
+// Back-track plan for frames of h rows.  The parallel back-track (jump + trace kernels) needs the jump plane and a cone
+// of jump entries in shared memory that grows with the square of the number of 32-row blocks; very tall frames keep the
+// serial walk of the DP kernel.
+struct BtPlan {
+    int nb;             // 32-row blocks
+    size_t cone_smem;   // trace kernel's dynamic shared memory
+    size_t j_pitch;     // bytes per row of the jump plane (nb rows per frame)
+    bool par;           // parallel back-track
+};
+
+static BtPlan bt_plan(int h, size_t m_pitch)
+{
+    BtPlan b;
+    b.nb = (h - 1 + JB - 1) / JB;
+    b.cone_smem = b.nb > 0 ? (size_t) 32 * (b.nb - 1) * (b.nb - 1) + 16 * (size_t) (b.nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
+    b.j_pitch = (m_pitch + 15) & ~(size_t) 15;    // jump rows start 16-byte aligned (staged in 16-byte chunks)
+    b.par = b.nb > 0 && b.cone_smem <= 200 * 1024 && !getenv("DCTC_SERIAL_BACKTRACK");
+    return b;
+}
+
 extern "C" {
 
 int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
@@ -1190,7 +1307,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpyAsync(ctx->c_seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
     dctc_carve_rows_kernel<256, 4><<<h, 256, 0, ctx->stream>>>(ctx->c_img, ctx->c_pitch, ctx->c_ch, ctx->c_en,
-                                                               ctx->c_en_pitch, ctx->c_seam, w_old, nullptr, 0);
+                                                               ctx->c_en_pitch, ctx->c_seam, w_old, nullptr, 0, 0, 0, 0);
     CK(ctx, cudaGetLastError());
     ctx->launches++;
     ctx->c_w = w_old - 1;
@@ -1253,62 +1370,12 @@ int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
         CK(ctx, cudaMalloc((void**) &ctx->c_seam_log, sizeof(int) * (size_t) n_seams * h));
         ctx->c_seam_log_cap = (size_t) n_seams * h;
     }
-    // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
-    const int wcur = ctx->c_w;
-    const int cap = DP_CL * DP_MAXW;
-    int P = wcur <= cap * (128 - 2 * DP_R) ? 1 : wcur <= cap * (256 - 2 * DP_R) ? 2 : 4;
-    if (const char* ep = getenv("DCTC_DP_P")) {   // timing experiments: wider strips than the width needs
-        const int want = atoi(ep);
-        if ((want == 2 || want == 4) && want > P) P = want;
-    }
-    const int wout = 128 * P - 2 * DP_R;
-    const int strips = (wcur + wout - 1) / wout;
-    const int wpc = (strips + DP_CL - 1) / DP_CL;
-    // energies staged by bulk async copies when at least two stages (DP_SR rows each) per warp fit into shared memory
-    // (the kernel also has ~38 KB of static shared memory: back-track windows, reduction scratch, mbarriers)
-    const size_t xrow_smem = sizeof(float) * 2 * (size_t) wpc * wout;
-    int nst = 0, sr = 0;
-    if (!getenv("DCTC_DP_NO_TMA")) {
-        const size_t row_smem = sizeof(float) * ((size_t) wpc * 128 * P);      // one staged row of every warp
-        const size_t budget = 180 * 1024 - xrow_smem;
-        if (2 * 32 * row_smem <= budget) { sr = 32; nst = 2; }                 // whole 32-row blocks, two in flight
-        else {
-            sr = 16;
-            for (nst = DP_NST_MAX; nst >= 2 && (size_t) nst * 16 * row_smem > budget; nst--) {}
-            if (nst < 2) { sr = 0; nst = 0; }
-        }
-    }
-    const size_t dp_smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
-    using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*);
-    static const dp_fn table[3][3] = {{dctc_seam_dp_kernel<1, 0>, dctc_seam_dp_kernel<1, 16>, dctc_seam_dp_kernel<1, 32>},
-                                      {dctc_seam_dp_kernel<2, 0>, dctc_seam_dp_kernel<2, 16>, dctc_seam_dp_kernel<2, 32>},
-                                      {dctc_seam_dp_kernel<4, 0>, dctc_seam_dp_kernel<4, 16>, dctc_seam_dp_kernel<4, 32>}};
-    const dp_fn dp = table[P == 1 ? 0 : P == 2 ? 1 : 2][sr / 16];
-    // tensor map of the energy plane for the staged variant (strips of up to 256 columns: the TMA box limit)
-    CUtensorMap tmap;
-    memset(&tmap, 0, sizeof(tmap));
-    int use_tmap = 0;
-    if (sr > 0 && 128 * P <= 256 && !getenv("DCTC_DP_NO_TENSORMAP")) {
-        typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-        void* fp = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qres) == cudaSuccess && fp &&
-            qres == cudaDriverEntryPointSuccess) {
-            const cuuint64_t gdim[2] = {(cuuint64_t) ctx->c_en_pitch, (cuuint64_t) h};
-            const cuuint64_t gstr[1] = {(cuuint64_t) ctx->c_en_pitch * sizeof(float)};
-            const cuuint32_t box[2] = {(cuuint32_t) (128 * P), (cuuint32_t) sr};
-            const cuuint32_t estr[2] = {1, 1};
-            if (((encode_fn) fp)(&tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, ctx->c_en, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                 CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
-                use_tmap = 1;
-        } else {
-            (void) cudaGetLastError();
-        }
-    }
-    // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
-    CK(ctx, cudaFuncSetAttribute(dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (dp_smem > 1024 ? dp_smem : 1024)));
+    DpPlan plan;
+    CK(ctx, dp_plan(ctx->c_w, h, ctx->c_en, ctx->c_en_pitch, 1, plan));
+    const dp_fn dp = plan.dp;
+    const int wpc = plan.wpc, nst = plan.nst, use_tmap = plan.use_tmap;
+    const size_t dp_smem = plan.smem;
+    const CUtensorMap& tmap = plan.tmap;
     // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
     const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
     const bool incr_ok = ctx->c_incremental && incr_smem <= 160 * 1024;
@@ -1318,12 +1385,10 @@ int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
         CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 8));
         CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 8, ctx->stream));
     }
-    // parallel back-track (jump + trace kernels): needs the jump plane and a cone of jump entries in shared memory that
-    // grows with the square of the number of 32-row blocks; very tall images keep the serial walk of the DP kernel
-    const int nb = (h - 1 + JB - 1) / JB;
-    const size_t cone_smem = nb > 0 ? (size_t) 32 * (nb - 1) * (nb - 1) + 16 * (size_t) (nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
-    const size_t j_pitch = (m_pitch + 15) & ~(size_t) 15;    // jump rows start 16-byte aligned (staged in 16-byte chunks)
-    const bool par_bt = nb > 0 && cone_smem <= 200 * 1024 && !getenv("DCTC_SERIAL_BACKTRACK");
+    const BtPlan bt = bt_plan(h, m_pitch);
+    const int nb = bt.nb;
+    const size_t cone_smem = bt.cone_smem, j_pitch = bt.j_pitch;
+    const bool par_bt = bt.par;
     int* const xlast = par_bt ? ctx->c_band + 4 : nullptr;
     if (par_bt) {
         if (!ctx->c_dir) CK(ctx, cudaMalloc((void**) &ctx->c_dir, (size_t) nb * j_pitch));
@@ -1338,20 +1403,21 @@ int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
             // update_mmap + build_vpath: walk the changed cells only; the full rebuild below runs only if the walk gave up
             dctc_seam_incr_kernel<<<1, 32, incr_smem, ctx->stream>>>(ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch, r,
                                                                      ctx->c_seam, log_s, ctx->c_band);
-            dp<<<DP_CL, wpc * 32, dp_smem, ctx->stream>>>(ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch, ctx->c_seam, log_s, ctx->c_band, nst, tmap, use_tmap, nullptr);
+            dp<<<DP_CL, wpc * 32, dp_smem, ctx->stream>>>(ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch, ctx->c_seam, log_s, ctx->c_band, nst, tmap, use_tmap, nullptr,
+                                                          (size_t) 0, (size_t) 0, (size_t) 0);
             ctx->launches++;
         } else {
             // build_mmap, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per block
             // (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor drains and
             // blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
             CK(ctx, dctc_launch_pdl(dp, dim3(DP_CL), dim3(wpc * 32), dp_smem, ctx->stream, pdl, ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch,
-                                    ctx->c_seam, log_s, (int*) nullptr, nst, tmap, use_tmap, xlast));
+                                    ctx->c_seam, log_s, (int*) nullptr, nst, tmap, use_tmap, xlast, 0, 0, 0));
             if (par_bt) {
                 const int js = (w_old + 63) / 64;
                 CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, nb), dim3(128), 0, ctx->stream, pdl, ctx->c_m, m_pitch, w_old, h,
-                                        ctx->c_dir, j_pitch, js));
+                                        ctx->c_dir, j_pitch, js, 0, 0));
                 CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(nb), dim3(TR_THREADS), cone_smem, ctx->stream, pdl, ctx->c_m, m_pitch, w_old, h,
-                                        ctx->c_dir, j_pitch, xlast, ctx->c_seam, log_s));
+                                        ctx->c_dir, j_pitch, xlast, ctx->c_seam, log_s, 0, 0, 0));
                 ctx->launches += 2;
             }
         }
@@ -1365,7 +1431,7 @@ int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
         }
         // carve: compact image and energy rows over the seam
         CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h), dim3(256), 0, ctx->stream, pdl, ctx->c_img, ctx->c_pitch, ctx->c_ch, ctx->c_en,
-                                ctx->c_en_pitch, ctx->c_seam, w_old, incr_ok ? ctx->c_m : (float*) nullptr, m_pitch));
+                                ctx->c_en_pitch, ctx->c_seam, w_old, incr_ok ? ctx->c_m : (float*) nullptr, m_pitch, 0, 0, 0));
         CK(ctx, cudaGetLastError());
         ctx->launches += 2;
         ctx->c_w = w_old - 1;
@@ -1517,6 +1583,274 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
         ctx->mirror_valid = true;
     }
     return ctx->h_mirror[(size_t) y * w + x];
+}
+
+}  // extern "C"
+
+// ---- batch session: n equally sized frames through one device seam loop ---------------------------------------------
+// The kernels of the loop above take the frame from a spare grid dimension, so one launch per phase serves every frame
+// and each frame's seam DP runs on its own cluster of DP_CL CTAs (a single 1080p frame keeps 8 of 148 SMs busy).  The
+// session owns its device buffers and never touches the context's single-frame session; it uses the context's device,
+// stream and launch counter, and the operator / kernel selection the context had when the frames were loaded.
+// Per frame: image, energy plane, cumulative plane and jump plane (frame f of each at f * its frame stride), h seam
+// columns, one last-row column slot, and the visibility maps when requested.  The cumulative map is always rebuilt.
+struct dctc_carver_batch {
+    dctc_context* ctx = nullptr;
+    int n = 0, w0 = 0, w = 0, h = 0, ch = 0;
+    bool dump_vmaps = false, loaded = false;
+    int blocksize = 8, kernel = DCTC_KERNEL_AUTO;   // the context's operator and kernel selection at load time
+    float edges = 0.5f, textures = 0.5f;
+    size_t pitch = 0, img_fs = 0;       // image: bytes per row, per frame
+    size_t en_pitch = 0, m_pitch = 0;   // energy / cumulative planes: floats per row (frames pitch * h floats apart)
+    uint8_t* img = nullptr;
+    float* en = nullptr;
+    float* m = nullptr;
+    int8_t* dir = nullptr;              // jump planes of the parallel back-track
+    size_t dir_fs = 0;
+    int* seam = nullptr;                // n * h: the seam each frame is removing
+    int* xlast = nullptr;               // n: last-row column of each frame's seam
+    int* seam_log = nullptr;            // n * n_seams * h of the current dctc_carver_batch_resize_width call, frame-major
+    size_t seam_log_cap = 0;
+    int* raw = nullptr;                 // n * w0 * h: original column of every current pixel
+    int* vs = nullptr;                  // n * w0 * h: removal order of every original pixel
+    int depth = 0;
+};
+
+namespace {
+
+// dctc_run_k1 reads the operator from the context: swap the batch's in for the duration of a call
+struct BatchParams {
+    dctc_context* ctx;
+    int blocksize, kernel;
+    float edges, textures;
+    BatchParams(dctc_carver_batch* b)
+        : ctx(b->ctx), blocksize(b->ctx->blocksize), kernel(b->ctx->kernel), edges(b->ctx->edges), textures(b->ctx->textures)
+    {
+        ctx->blocksize = b->blocksize; ctx->kernel = b->kernel; ctx->edges = b->edges; ctx->textures = b->textures;
+    }
+    ~BatchParams() { ctx->blocksize = blocksize; ctx->kernel = kernel; ctx->edges = edges; ctx->textures = textures; }
+};
+
+void batch_free(dctc_carver_batch* b)
+{
+    cudaFree(b->img); cudaFree(b->en); cudaFree(b->m); cudaFree(b->dir); cudaFree(b->seam); cudaFree(b->xlast);
+    cudaFree(b->seam_log); cudaFree(b->raw); cudaFree(b->vs);
+}
+
+int batch_alloc(dctc_carver_batch* b)
+{
+    dctc_context* ctx = b->ctx;
+    const size_t n = (size_t) b->n, h = (size_t) b->h;
+    CK(ctx, cudaMalloc((void**) &b->img, b->img_fs * n));
+    CK(ctx, cudaMalloc((void**) &b->en, sizeof(float) * b->en_pitch * h * n));
+    CK(ctx, cudaMemsetAsync(b->en, 0, sizeof(float) * b->en_pitch * h * n, ctx->stream));
+    CK(ctx, cudaMalloc((void**) &b->m, sizeof(float) * b->m_pitch * h * n));
+    CK(ctx, cudaMemsetAsync(b->m, 0, sizeof(float) * b->m_pitch * h * n, ctx->stream));
+    CK(ctx, cudaMalloc((void**) &b->seam, sizeof(int) * h * n));
+    CK(ctx, cudaMalloc((void**) &b->xlast, sizeof(int) * n));
+    CK(ctx, cudaMemsetAsync(b->xlast, 0, sizeof(int) * n, ctx->stream));
+    if (b->dump_vmaps) {
+        CK(ctx, cudaMalloc((void**) &b->raw, sizeof(int) * (size_t) b->w0 * h * n));
+        CK(ctx, cudaMalloc((void**) &b->vs, sizeof(int) * (size_t) b->w0 * h * n));
+    }
+    const BtPlan bt = bt_plan(b->h, b->m_pitch);
+    b->dir_fs = (size_t) bt.nb * bt.j_pitch;
+    if (bt.par) CK(ctx, cudaMalloc((void**) &b->dir, b->dir_fs * n));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+// full energy map of every frame in one K1 launch (the FP32 kernels of the single session: see carver_full_energy)
+int batch_full_energy(dctc_carver_batch* b)
+{
+    dctc_context* ctx = b->ctx;
+    DctcK1Args a;
+    memset(&a, 0, sizeof(a));
+    a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = b->h; a.channels = b->ch;
+    a.out = b->en; a.out_pitch = b->en_pitch;
+    a.frame_stride = b->img_fs; a.out_frame_stride = b->en_pitch * b->h;
+    if (ctx->kernel == DCTC_KERNEL_AUTO || ctx->kernel == DCTC_KERNEL_TC_SPLIT || ctx->kernel == DCTC_KERNEL_FP32_STREAM) ctx->kernel = DCTC_KERNEL_FP32_MARCH;
+    return dctc_run_k1(ctx, a, b->n, ctx->stream);   // (the caller's BatchParams restores the kernel selection)
+}
+
+}  // namespace
+
+extern "C" {
+
+int dctc_carver_batch_create(dctc_context* ctx, int n_frames, int w, int h, int channels, int dump_vmaps, dctc_carver_batch** batch)
+{
+    if (!ctx || !batch) return DCTC_ERR_INVALID;
+    *batch = nullptr;
+    if (n_frames <= 0 || w <= 0 || h <= 0 || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
+    if (n_frames > 65535) return DCTC_ERR_UNSUPPORTED;   // the frame is a grid dimension of every launch
+    CK(ctx, cudaSetDevice(ctx->device));
+    dctc_carver_batch* b = new (std::nothrow) dctc_carver_batch;
+    if (!b) return DCTC_ERR_NOMEM;
+    b->ctx = ctx;
+    b->n = n_frames; b->w0 = b->w = w; b->h = h; b->ch = channels;
+    b->dump_vmaps = dump_vmaps != 0;
+    b->pitch = ((size_t) w * channels + 15) & ~(size_t) 15;
+    b->img_fs = b->pitch * h;
+    b->en_pitch = ((size_t) w + 3) & ~(size_t) 3;
+    b->m_pitch = b->en_pitch < (size_t) DP_WIN ? (size_t) DP_WIN : b->en_pitch;   // back-track windows stay inside
+    const int rc = batch_alloc(b);
+    if (rc) {
+        batch_free(b);
+        delete b;
+        return rc;
+    }
+    *batch = b;
+    return DCTC_OK;
+}
+
+void dctc_carver_batch_destroy(dctc_carver_batch* b)
+{
+    if (!b) return;
+    if (cudaSetDevice(b->ctx->device) == cudaSuccess) cudaStreamSynchronize(b->ctx->stream);
+    batch_free(b);
+    delete b;
+}
+
+int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t frame_stride, size_t pitch)
+{
+    if (!b || !imgs) return DCTC_ERR_INVALID;
+    const size_t row = (size_t) b->w0 * b->ch;
+    if (pitch < row || (b->n > 1 && frame_stride < pitch * b->h)) return DCTC_ERR_INVALID;
+    dctc_context* ctx = b->ctx;
+    const int bs = ctx->blocksize;
+    if (!(bs == 2 || bs == 4 || bs == 8 || bs == 16)) return DCTC_ERR_BLOCKSIZE;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    b->loaded = false;
+    b->blocksize = ctx->blocksize; b->kernel = ctx->kernel; b->edges = ctx->edges; b->textures = ctx->textures;
+    b->w = b->w0;
+    for (int f = 0; f < b->n; f++)
+        CK(ctx, cudaMemcpy2DAsync(b->img + (size_t) f * b->img_fs, b->pitch, imgs + (size_t) f * frame_stride, pitch, row, b->h,
+                                  cudaMemcpyDefault, ctx->stream));
+    if (b->dump_vmaps) {
+        const size_t nv = (size_t) b->w0 * b->h * b->n;
+        CK(ctx, cudaMemsetAsync(b->vs, 0, sizeof(int) * nv, ctx->stream));
+        dctc_iota_rows_kernel<<<(unsigned) ((nv + 255) / 256), 256, 0, ctx->stream>>>(b->raw, b->w0, b->h * b->n);
+        CK(ctx, cudaGetLastError());
+        ctx->launches++;
+        b->depth = 0;
+    }
+    int rc;
+    {
+        BatchParams scope(b);
+        rc = batch_full_energy(b);
+    }
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    b->loaded = true;
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? b->w : 0; }
+
+int dctc_carver_batch_resize_width(dctc_carver_batch* b, int n_seams, int* seams_out)
+{
+    if (!b || n_seams < 0) return DCTC_ERR_INVALID;
+    if (!b->loaded) return DCTC_ERR_STATE;
+    if (n_seams == 0) return DCTC_OK;
+    if (n_seams >= b->w) return DCTC_ERR_STATE;
+    if (b->w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
+    dctc_context* ctx = b->ctx;
+    const int n = b->n, h = b->h;
+    CK(ctx, cudaSetDevice(ctx->device));
+    BatchParams scope(b);
+    const int r = ctx->blocksize / 2, bs = band_stride(ctx);
+    const size_t log_fs = (size_t) n_seams * h;
+    if (b->seam_log_cap < log_fs * n) {
+        cudaFree(b->seam_log);
+        b->seam_log = nullptr; b->seam_log_cap = 0;
+        CK(ctx, cudaMalloc((void**) &b->seam_log, sizeof(int) * log_fs * n));
+        b->seam_log_cap = log_fs * n;
+    }
+    const size_t en_fs = b->en_pitch * h, m_fs = b->m_pitch * h;
+    DpPlan plan;
+    CK(ctx, dp_plan(b->w, h, b->en, b->en_pitch, n, plan));
+    BtPlan bt = bt_plan(h, b->m_pitch);
+    bt.par = bt.par && b->dir;
+    if (bt.par && bt.cone_smem > 40 * 1024)
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+    int* const xlast = bt.par ? b->xlast : nullptr;
+    const bool pdl = !getenv("DCTC_NO_PDL");
+    for (int s = 0; s < n_seams; s++) {
+        const int w_old = b->w;
+        int* log_s = b->seam_log + (size_t) s * h;
+        // build_mmap + build_vpath, one cluster per frame, then the jump maps and traces of all frames
+        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl, b->en, b->en_pitch, w_old, h,
+                                b->m, b->m_pitch, b->seam, log_s, (int*) nullptr, plan.nst, plan.tmap, plan.use_tmap, xlast, en_fs, m_fs, log_fs));
+        if (bt.par) {
+            const int js = (w_old + 63) / 64;
+            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, b->m, b->m_pitch,
+                                    w_old, h, b->dir, bt.j_pitch, js, m_fs, b->dir_fs));
+            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, b->m, b->m_pitch,
+                                    w_old, h, b->dir, bt.j_pitch, b->xlast, b->seam, log_s, m_fs, b->dir_fs, log_fs));
+            ctx->launches += 2;
+        }
+        if (b->dump_vmaps) {   // update_vsmap
+            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->raw, b->vs, b->w0, b->seam, w_old,
+                                    ++b->depth));
+            ctx->launches++;
+        }
+        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->img, b->pitch, b->ch, b->en,
+                                b->en_pitch, b->seam, w_old, (float*) nullptr, b->m_pitch, b->img_fs, en_fs, (size_t) 0));
+        ctx->launches += 2;
+        b->w = w_old - 1;
+        // update_emap: band K1 around every frame's removed seam (the band values are not read back)
+        DctcK1Args a;
+        memset(&a, 0, sizeof(a));
+        a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = h; a.channels = b->ch;
+        a.out = b->en; a.out_pitch = b->en_pitch;
+        a.frame_stride = b->img_fs; a.out_frame_stride = en_fs;
+        a.seam = b->seam; a.seam_frame_stride = h; a.band_r = r; a.band_stride = bs;
+        a.pdl = pdl ? 1 : 0;
+        const int rc = dctc_run_k1(ctx, a, n, ctx->stream);
+        if (rc) return rc;
+    }
+    if (seams_out)
+        CK(ctx, cudaMemcpyAsync(seams_out, b->seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
+{
+    if (!b || !out) return DCTC_ERR_INVALID;
+    if (!b->loaded) return DCTC_ERR_STATE;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t rb = (size_t) b->w * b->ch;   // frames are pitch * h bytes apart: n * h rows of one pitch
+    CK(ctx, cudaMemcpy2DAsync(out, rb, b->img, b->pitch, rb, (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
+{
+    if (!b || !out) return DCTC_ERR_INVALID;
+    if (!b->loaded) return DCTC_ERR_STATE;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    CK(ctx, cudaMemcpy2DAsync(out, sizeof(float) * b->w, b->en, sizeof(float) * b->en_pitch, sizeof(float) * b->w,
+                              (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
+{
+    if (!b) return DCTC_ERR_INVALID;
+    if (!b->loaded || !b->dump_vmaps) return DCTC_ERR_STATE;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (vmap_out)
+        CK(ctx, cudaMemcpyAsync(vmap_out, b->vs, sizeof(int) * (size_t) b->w0 * b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    if (depth_out) *depth_out = b->depth;
+    return DCTC_OK;
 }
 
 }  // extern "C"

@@ -184,6 +184,36 @@ int dctc_carver_vmap(dctc_context *ctx, int *vmap_out, int *depth_out);
  * x < w-1, y < h-1 becomes (0, (guchar)(255.0 * vis / depth), 0); painted on the device. */
 int dctc_carver_paint_seams(dctc_context *ctx, uint8_t *img, int channels, size_t pitch_bytes);
 
+/* ---- K2 batch: n equally sized frames through one device seam loop -----------------------------------------
+ * A batch session, owned by the caller and tied to one context (destroy it before the context).  It has its own
+ * device buffers and never touches the context's single-frame session.  Every phase of the seam loop is one launch
+ * for all frames, and every frame's seam DP runs on its own cluster, so frames retarget side by side.  Each frame
+ * gets exactly the seams, image, energy map and visibility map that dctc_carver_load + dctc_carver_resize_width
+ * give it on its own.  The cumulative map is always rebuilt (no incremental mode).
+ * Errors: DCTC_ERR_INVALID for NULL pointers, n_frames <= 0, a channel count outside 1..4, a pitch or frame stride
+ * that is too small; DCTC_ERR_STATE for a resize before a load or n_seams >= the current width; DCTC_ERR_UNSUPPORTED
+ * for widths the device seam DP does not cover (as dctc_carver_resize_width) and n_frames > 65535. */
+typedef struct dctc_carver_batch dctc_carver_batch;
+/* n_frames frames of w x h, channels 1..4; uses the context's device, stream, blocksize / edges / textures and kernel
+ * selection as they are at load time.  dump_vmaps: also keep a visibility map per frame. */
+int dctc_carver_batch_create(dctc_context *ctx, int n_frames, int w, int h, int channels, int dump_vmaps,
+                             dctc_carver_batch **batch);
+void dctc_carver_batch_destroy(dctc_carver_batch *batch);
+/* host frames (frame_stride_bytes apart, rows pitch_bytes apart) -> device, full energy map of every frame (one K1
+ * batch launch).  A load restarts the session at the original width w. */
+int dctc_carver_batch_load(dctc_carver_batch *batch, const uint8_t *imgs, size_t frame_stride_bytes, size_t pitch_bytes);
+/* removes n_seams vertical seams from every frame; seams_out (may be NULL): n_frames * n_seams * h ints, frame-major,
+ * in the coordinates at removal time (the layout dctc_carver_resize_width uses, per frame) */
+int dctc_carver_batch_resize_width(dctc_carver_batch *batch, int n_seams, int *seams_out);
+/* current width of every frame */
+int dctc_carver_batch_width(const dctc_carver_batch *batch);
+/* current images (n_frames * h * w * channels, pitch w * channels) / energy maps (n_frames * h * w floats) */
+int dctc_carver_batch_images(dctc_carver_batch *batch, uint8_t *out);
+int dctc_carver_batch_energy(dctc_carver_batch *batch, float *out);
+/* visibility map of every frame over the loaded width w0 (n_frames * h * w0 ints) and the common depth; needs
+ * dump_vmaps at create time */
+int dctc_carver_batch_vmap(dctc_carver_batch *batch, int *vmap_out, int *depth_out);
+
 /* ---- K3: energy-image export ------------------------------------------------------------------------------
  * Replaces lqr_carver_get_energy_image(carver, buf, orientation, LQR_COLDEPTH_8I, LQR_GREY_IMAGE) as called at
  * src/render.c:191 (the plug-in's "output energy" option, src/render.c:175-202): e -> 1/(1+1/e) (= e/(1+e)),
