@@ -27,7 +27,8 @@ ABI_SYMBOLS = [
     "dctc_energy_minmax_dev", "dctc_energy_image_dev", "dctc_carver_energy_image", "dctc_preview_energy",
     "dctc_carver_set_dump_vmaps", "dctc_carver_vmap", "dctc_carver_paint_seams",
     "dctc_carver_batch_create", "dctc_carver_batch_destroy", "dctc_carver_batch_load", "dctc_carver_batch_resize_width",
-    "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy", "dctc_carver_batch_vmap",
+    "dctc_carver_batch_enlarge_width", "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy",
+    "dctc_carver_batch_vmap",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -115,6 +116,7 @@ def lib():
         "dctc_carver_batch_destroy": (None, [vp]),
         "dctc_carver_batch_load": (i32, [vp, vp, sz, sz]),
         "dctc_carver_batch_resize_width": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_enlarge_width": (i32, [vp, i32, vp]),
         "dctc_carver_batch_width": (i32, [vp]),
         "dctc_carver_batch_images": (i32, [vp, vp]),
         "dctc_carver_batch_energy": (i32, [vp, vp]),
@@ -457,9 +459,23 @@ class Context:
 class CarverBatch:
     """n equally sized frames retargeted together by one device seam loop (dctc_carver_batch_*): every phase of the loop
     is one launch for all frames, and each frame gets exactly what a single carver session on the same context gives
-    it.  imgs: uint8 [n, h, w] or [n, h, w, ch].  Uses the context's operator and kernel selection at construction."""
+    it.  imgs: uint8 [n, h, w] or [n, h, w, ch].  Uses the context's operator and kernel selection at load time."""
 
     def __init__(self, ctx, imgs, dump_vmaps=False):
+        imgs = self._frames(imgs)
+        self.ctx = ctx
+        self.n, self.h, self.w0, self.ch = imgs.shape
+        self._b = C.c_void_p()
+        _check(lib().dctc_carver_batch_create(ctx.handle, self.n, self.w0, self.h, self.ch, int(bool(dump_vmaps)),
+                                              C.byref(self._b)), "dctc_carver_batch_create")
+        try:
+            self.load(imgs)
+        except Exception:
+            self.close()
+            raise
+
+    @staticmethod
+    def _frames(imgs):
         imgs = np.asarray(imgs)
         if imgs.dtype != np.uint8:
             raise TypeError("frames must be uint8")
@@ -467,18 +483,15 @@ class CarverBatch:
             imgs = imgs[..., None]
         if imgs.ndim != 4:
             raise ValueError("frames must be [n, h, w] or [n, h, w, ch]")
-        imgs = np.ascontiguousarray(imgs)
-        self.ctx = ctx
-        self.n, self.h, self.w0, self.ch = imgs.shape
-        self._b = C.c_void_p()
-        _check(lib().dctc_carver_batch_create(ctx.handle, self.n, self.w0, self.h, self.ch, int(bool(dump_vmaps)),
-                                              C.byref(self._b)), "dctc_carver_batch_create")
-        try:
-            _check(lib().dctc_carver_batch_load(self._b, _ptr(imgs), self.h * self.w0 * self.ch, self.w0 * self.ch),
-                   "dctc_carver_batch_load")
-        except Exception:
-            self.close()
-            raise
+        return np.ascontiguousarray(imgs)
+
+    def load(self, imgs):
+        """Loads new frames of the batch's shape and restarts it at the original width (also after enlarge_width)."""
+        imgs = self._frames(imgs)
+        if imgs.shape != (self.n, self.h, self.w0, self.ch):
+            raise ValueError("frames must have the batch's shape %s" % ((self.n, self.h, self.w0, self.ch),))
+        _check(lib().dctc_carver_batch_load(self._b, _ptr(imgs), self.h * self.w0 * self.ch, self.w0 * self.ch),
+               "dctc_carver_batch_load")
 
     @property
     def handle(self):
@@ -494,6 +507,15 @@ class CarverBatch:
         seams = np.empty((self.n, n_seams, self.h), np.int32)
         _check(lib().dctc_carver_batch_resize_width(self._b, int(n_seams), _ptr(seams) if n_seams else None),
                "dctc_carver_batch_resize_width")
+        return seams
+
+    def enlarge_width(self, n_seams):
+        """lqr_carver_resize to a larger width for every frame: returns int32 [n, n_seams, h], the seams a shrink by
+        n_seams would remove (as resize_width), every pixel of which is then doubled.  The frames become w0 + n_seams
+        wide; vmap() keeps the start frames' maps.  No further resize until the next load()."""
+        seams = np.empty((self.n, n_seams, self.h), np.int32)
+        _check(lib().dctc_carver_batch_enlarge_width(self._b, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_batch_enlarge_width")
         return seams
 
     def images(self):

@@ -1035,16 +1035,18 @@ __global__ void __launch_bounds__(256) dctc_paint_seams_kernel(uint8_t* __restri
 // liblqr's lqr_carver_inflate [from memory: PARITY UNPINNED]: every pixel the first n seams went through is doubled;
 // the new pixel sits on its left and holds the integer mean (a + b) / 2 of the pixel and its left neighbour in the
 // original row (a copy in column 0).  One CTA per row: block-wide prefix sum of the "seam pixel" flags gives every
-// original pixel its output column.
+// original pixel its output column.  Batch sessions: blockIdx.y = frame, whose source image, visibility map and output
+// image start orig_fs bytes, vs_fs ints and out_fs bytes after the previous frame's.
 __global__ void __launch_bounds__(256) dctc_inflate_rows_kernel(const uint8_t* __restrict__ orig, size_t pitch, int channels, int w0,
-                                                                const int* __restrict__ vs, int n, uint8_t* __restrict__ out, size_t out_pitch)
+                                                                const int* __restrict__ vs, int n, uint8_t* __restrict__ out, size_t out_pitch,
+                                                                size_t orig_fs, size_t vs_fs, size_t out_fs)
 {
     __shared__ int wsum[8];
     __shared__ int running;
-    const int y = blockIdx.x, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const uint8_t* src = orig + (size_t) y * pitch;
-    uint8_t* dst = out + (size_t) y * out_pitch;
-    const int* vrow = vs + (size_t) y * w0;
+    const int y = blockIdx.x, z = blockIdx.y, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const uint8_t* src = orig + z * orig_fs + (size_t) y * pitch;
+    uint8_t* dst = out + z * out_fs + (size_t) y * out_pitch;
+    const int* vrow = vs + z * vs_fs + (size_t) y * w0;
     if (tid == 0) running = 0;
     __syncthreads();
     for (int base = 0; base < w0; base += 256) {
@@ -1483,7 +1485,7 @@ int dctc_carver_enlarge_width(dctc_context* ctx, int n_seams, int* seams_out)
         ctx->c_dump_vmaps = dump_saved;
     }
     if (rc == DCTC_OK) {
-        dctc_inflate_rows_kernel<<<h, 256, 0, ctx->stream>>>(d_orig, p0, ch, w0, ctx->c_vs, n_seams, d_new, p1);
+        dctc_inflate_rows_kernel<<<h, 256, 0, ctx->stream>>>(d_orig, p0, ch, w0, ctx->c_vs, n_seams, d_new, p1, 0, 0, 0);
         e = cudaGetLastError();
         ctx->launches++;
         if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
@@ -1612,8 +1614,18 @@ struct dctc_carver_batch {
     int* seam_log = nullptr;            // n * n_seams * h of the current dctc_carver_batch_resize_width call, frame-major
     size_t seam_log_cap = 0;
     int* raw = nullptr;                 // n * w0 * h: original column of every current pixel
-    int* vs = nullptr;                  // n * w0 * h: removal order of every original pixel
+    int* vs = nullptr;                  // n * w0 * h: removal order of every original pixel (without dump_vmaps: the
+                                        // enlarge's, allocated by the first enlarge)
     int depth = 0;
+    // dctc_carver_batch_enlarge_width: a copy of the start frames (frames img_fs bytes apart) and the enlarged frames
+    // (wide_w = w0 + n_seams wide, frames wide_pitch * h bytes / wide_en_pitch * h floats apart).  Allocated by the first
+    // enlarge and kept for the next (the enlarged planes are reallocated when n_seams changes), freed by the destroy.
+    bool enlarged = false;              // the current frames are the enlarged ones
+    uint8_t* start_img = nullptr;
+    uint8_t* wide_img = nullptr;
+    float* wide_en = nullptr;
+    int wide_w = 0;
+    size_t wide_pitch = 0, wide_en_pitch = 0;
 };
 
 namespace {
@@ -1635,6 +1647,7 @@ void batch_free(dctc_carver_batch* b)
 {
     cudaFree(b->img); cudaFree(b->en); cudaFree(b->m); cudaFree(b->dir); cudaFree(b->seam); cudaFree(b->xlast);
     cudaFree(b->seam_log); cudaFree(b->raw); cudaFree(b->vs);
+    cudaFree(b->start_img); cudaFree(b->wide_img); cudaFree(b->wide_en);
 }
 
 int batch_alloc(dctc_carver_batch* b)
@@ -1660,17 +1673,133 @@ int batch_alloc(dctc_carver_batch* b)
     return DCTC_OK;
 }
 
-// full energy map of every frame in one K1 launch (the FP32 kernels of the single session: see carver_full_energy)
-int batch_full_energy(dctc_carver_batch* b)
+// full energy map of every frame of w x h pixels (images at img, energy planes at en, frames h rows apart) in one K1
+// launch (the FP32 kernels of the single session: see carver_full_energy)
+int batch_full_energy(dctc_carver_batch* b, const uint8_t* img, size_t pitch, int w, float* en, size_t en_pitch)
 {
     dctc_context* ctx = b->ctx;
     DctcK1Args a;
     memset(&a, 0, sizeof(a));
-    a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = b->h; a.channels = b->ch;
-    a.out = b->en; a.out_pitch = b->en_pitch;
-    a.frame_stride = b->img_fs; a.out_frame_stride = b->en_pitch * b->h;
+    a.img = img; a.pitch = pitch; a.w = w; a.h = b->h; a.channels = b->ch;
+    a.out = en; a.out_pitch = en_pitch;
+    a.frame_stride = pitch * b->h; a.out_frame_stride = en_pitch * b->h;
     if (ctx->kernel == DCTC_KERNEL_AUTO || ctx->kernel == DCTC_KERNEL_TC_SPLIT || ctx->kernel == DCTC_KERNEL_FP32_STREAM) ctx->kernel = DCTC_KERNEL_FP32_MARCH;
     return dctc_run_k1(ctx, a, b->n, ctx->stream);   // (the caller's BatchParams restores the kernel selection)
+}
+
+// empty visibility maps (w0 * h ints per frame) and the identity column map raw[frame][y][x] = x
+int batch_vmaps_reset(dctc_carver_batch* b, int* raw, int* vs)
+{
+    dctc_context* ctx = b->ctx;
+    const size_t nv = (size_t) b->w0 * b->h * b->n;
+    CK(ctx, cudaMemsetAsync(vs, 0, sizeof(int) * nv, ctx->stream));
+    dctc_iota_rows_kernel<<<(unsigned) ((nv + 255) / 256), 256, 0, ctx->stream>>>(raw, b->w0, b->h * b->n);
+    CK(ctx, cudaGetLastError());
+    ctx->launches++;
+    b->depth = 0;
+    return DCTC_OK;
+}
+
+// The device seam loop of every frame: removes n_seams seams from the images and energy planes (b->w shrinks by n_seams)
+// and, when raw / vs are given (maps as batch_vmaps_reset leaves them), records each removed pixel's order in vs.  The
+// caller has checked the width and holds a BatchParams scope.
+int batch_seam_loop(dctc_carver_batch* b, int n_seams, int* seams_out, int* raw, int* vs)
+{
+    dctc_context* ctx = b->ctx;
+    const int n = b->n, h = b->h;
+    const int r = ctx->blocksize / 2, bs = band_stride(ctx);
+    const size_t log_fs = (size_t) n_seams * h;
+    if (b->seam_log_cap < log_fs * n) {
+        cudaFree(b->seam_log);
+        b->seam_log = nullptr; b->seam_log_cap = 0;
+        CK(ctx, cudaMalloc((void**) &b->seam_log, sizeof(int) * log_fs * n));
+        b->seam_log_cap = log_fs * n;
+    }
+    const size_t en_fs = b->en_pitch * h, m_fs = b->m_pitch * h;
+    DpPlan plan;
+    CK(ctx, dp_plan(b->w, h, b->en, b->en_pitch, n, plan));
+    BtPlan bt = bt_plan(h, b->m_pitch);
+    bt.par = bt.par && b->dir;
+    if (bt.par && bt.cone_smem > 40 * 1024)
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+    int* const xlast = bt.par ? b->xlast : nullptr;
+    const bool pdl = !getenv("DCTC_NO_PDL");
+    for (int s = 0; s < n_seams; s++) {
+        const int w_old = b->w;
+        int* log_s = b->seam_log + (size_t) s * h;
+        // build_mmap + build_vpath, one cluster per frame, then the jump maps and traces of all frames
+        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl, b->en, b->en_pitch, w_old, h,
+                                b->m, b->m_pitch, b->seam, log_s, (int*) nullptr, plan.nst, plan.tmap, plan.use_tmap, xlast, en_fs, m_fs, log_fs));
+        if (bt.par) {
+            const int js = (w_old + 63) / 64;
+            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, b->m, b->m_pitch,
+                                    w_old, h, b->dir, bt.j_pitch, js, m_fs, b->dir_fs));
+            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, b->m, b->m_pitch,
+                                    w_old, h, b->dir, bt.j_pitch, b->xlast, b->seam, log_s, m_fs, b->dir_fs, log_fs));
+            ctx->launches += 2;
+        }
+        if (vs) {   // update_vsmap
+            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, raw, vs, b->w0, b->seam, w_old,
+                                    ++b->depth));
+            ctx->launches++;
+        }
+        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->img, b->pitch, b->ch, b->en,
+                                b->en_pitch, b->seam, w_old, (float*) nullptr, b->m_pitch, b->img_fs, en_fs, (size_t) 0));
+        ctx->launches += 2;
+        b->w = w_old - 1;
+        // update_emap: band K1 around every frame's removed seam (the band values are not read back)
+        DctcK1Args a;
+        memset(&a, 0, sizeof(a));
+        a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = h; a.channels = b->ch;
+        a.out = b->en; a.out_pitch = b->en_pitch;
+        a.frame_stride = b->img_fs; a.out_frame_stride = en_fs;
+        a.seam = b->seam; a.seam_frame_stride = h; a.band_r = r; a.band_stride = bs;
+        a.pdl = pdl ? 1 : 0;
+        const int rc = dctc_run_k1(ctx, a, n, ctx->stream);
+        if (rc) return rc;
+    }
+    if (seams_out)
+        CK(ctx, cudaMemcpyAsync(seams_out, b->seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+// Device work of dctc_carver_batch_enlarge_width: the start frames are copied to start_img, the seam loop runs on the
+// batch's planes with visibility maps, the inflate kernel writes the enlarged frames and K1 their full energy maps.
+int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
+{
+    dctc_context* ctx = b->ctx;
+    const size_t n = (size_t) b->n, h = (size_t) b->h, nv = (size_t) b->w0 * h * n;
+    const int w1 = b->w0 + n_seams;
+    if (!b->start_img) CK(ctx, cudaMalloc((void**) &b->start_img, b->img_fs * n));
+    if (!b->raw) CK(ctx, cudaMalloc((void**) &b->raw, sizeof(int) * nv));
+    if (!b->vs) CK(ctx, cudaMalloc((void**) &b->vs, sizeof(int) * nv));
+    if (b->wide_w != w1) {
+        cudaFree(b->wide_img); cudaFree(b->wide_en);
+        b->wide_img = nullptr; b->wide_en = nullptr; b->wide_w = 0;
+        b->wide_pitch = ((size_t) w1 * b->ch + 15) & ~(size_t) 15;
+        b->wide_en_pitch = ((size_t) w1 + 3) & ~(size_t) 3;
+        CK(ctx, cudaMalloc((void**) &b->wide_img, b->wide_pitch * h * n));
+        CK(ctx, cudaMalloc((void**) &b->wide_en, sizeof(float) * b->wide_en_pitch * h * n));
+        b->wide_w = w1;
+    }
+    CK(ctx, cudaMemcpyAsync(b->start_img, b->img, b->img_fs * n, cudaMemcpyDeviceToDevice, ctx->stream));
+    if (!b->dump_vmaps) {   // (a batch with dump_vmaps had its maps reset by the load, and no seam was removed since)
+        const int rc = batch_vmaps_reset(b, b->raw, b->vs);
+        if (rc) return rc;
+    }
+    BatchParams scope(b);
+    int rc = batch_seam_loop(b, n_seams, seams_out, b->raw, b->vs);
+    if (rc) return rc;
+    // every pixel of those seams doubled, all frames in one launch
+    dctc_inflate_rows_kernel<<<dim3(b->h, b->n), 256, 0, ctx->stream>>>(b->start_img, b->pitch, b->ch, b->w0, b->vs, n_seams, b->wide_img,
+                                                                        b->wide_pitch, b->img_fs, (size_t) b->w0 * h, b->wide_pitch * h);
+    CK(ctx, cudaGetLastError());
+    ctx->launches++;
+    rc = batch_full_energy(b, b->wide_img, b->wide_pitch, w1, b->wide_en, b->wide_en_pitch);
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
 }
 
 }  // namespace
@@ -1722,23 +1851,17 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = false;
+    b->enlarged = false;
     b->blocksize = ctx->blocksize; b->kernel = ctx->kernel; b->edges = ctx->edges; b->textures = ctx->textures;
     b->w = b->w0;
     for (int f = 0; f < b->n; f++)
         CK(ctx, cudaMemcpy2DAsync(b->img + (size_t) f * b->img_fs, b->pitch, imgs + (size_t) f * frame_stride, pitch, row, b->h,
                                   cudaMemcpyDefault, ctx->stream));
-    if (b->dump_vmaps) {
-        const size_t nv = (size_t) b->w0 * b->h * b->n;
-        CK(ctx, cudaMemsetAsync(b->vs, 0, sizeof(int) * nv, ctx->stream));
-        dctc_iota_rows_kernel<<<(unsigned) ((nv + 255) / 256), 256, 0, ctx->stream>>>(b->raw, b->w0, b->h * b->n);
-        CK(ctx, cudaGetLastError());
-        ctx->launches++;
-        b->depth = 0;
-    }
-    int rc;
+    int rc = b->dump_vmaps ? batch_vmaps_reset(b, b->raw, b->vs) : DCTC_OK;
+    if (rc) return rc;
     {
         BatchParams scope(b);
-        rc = batch_full_energy(b);
+        rc = batch_full_energy(b, b->img, b->pitch, b->w, b->en, b->en_pitch);
     }
     if (rc) return rc;
     CK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1751,68 +1874,33 @@ int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? b->w : 0; }
 int dctc_carver_batch_resize_width(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!b->loaded) return DCTC_ERR_STATE;
+    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
     if (n_seams >= b->w) return DCTC_ERR_STATE;
     if (b->w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
     dctc_context* ctx = b->ctx;
-    const int n = b->n, h = b->h;
     CK(ctx, cudaSetDevice(ctx->device));
     BatchParams scope(b);
-    const int r = ctx->blocksize / 2, bs = band_stride(ctx);
-    const size_t log_fs = (size_t) n_seams * h;
-    if (b->seam_log_cap < log_fs * n) {
-        cudaFree(b->seam_log);
-        b->seam_log = nullptr; b->seam_log_cap = 0;
-        CK(ctx, cudaMalloc((void**) &b->seam_log, sizeof(int) * log_fs * n));
-        b->seam_log_cap = log_fs * n;
-    }
-    const size_t en_fs = b->en_pitch * h, m_fs = b->m_pitch * h;
-    DpPlan plan;
-    CK(ctx, dp_plan(b->w, h, b->en, b->en_pitch, n, plan));
-    BtPlan bt = bt_plan(h, b->m_pitch);
-    bt.par = bt.par && b->dir;
-    if (bt.par && bt.cone_smem > 40 * 1024)
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
-    int* const xlast = bt.par ? b->xlast : nullptr;
-    const bool pdl = !getenv("DCTC_NO_PDL");
-    for (int s = 0; s < n_seams; s++) {
-        const int w_old = b->w;
-        int* log_s = b->seam_log + (size_t) s * h;
-        // build_mmap + build_vpath, one cluster per frame, then the jump maps and traces of all frames
-        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl, b->en, b->en_pitch, w_old, h,
-                                b->m, b->m_pitch, b->seam, log_s, (int*) nullptr, plan.nst, plan.tmap, plan.use_tmap, xlast, en_fs, m_fs, log_fs));
-        if (bt.par) {
-            const int js = (w_old + 63) / 64;
-            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, b->m, b->m_pitch,
-                                    w_old, h, b->dir, bt.j_pitch, js, m_fs, b->dir_fs));
-            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, b->m, b->m_pitch,
-                                    w_old, h, b->dir, bt.j_pitch, b->xlast, b->seam, log_s, m_fs, b->dir_fs, log_fs));
-            ctx->launches += 2;
-        }
-        if (b->dump_vmaps) {   // update_vsmap
-            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->raw, b->vs, b->w0, b->seam, w_old,
-                                    ++b->depth));
-            ctx->launches++;
-        }
-        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->img, b->pitch, b->ch, b->en,
-                                b->en_pitch, b->seam, w_old, (float*) nullptr, b->m_pitch, b->img_fs, en_fs, (size_t) 0));
-        ctx->launches += 2;
-        b->w = w_old - 1;
-        // update_emap: band K1 around every frame's removed seam (the band values are not read back)
-        DctcK1Args a;
-        memset(&a, 0, sizeof(a));
-        a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = h; a.channels = b->ch;
-        a.out = b->en; a.out_pitch = b->en_pitch;
-        a.frame_stride = b->img_fs; a.out_frame_stride = en_fs;
-        a.seam = b->seam; a.seam_frame_stride = h; a.band_r = r; a.band_stride = bs;
-        a.pdl = pdl ? 1 : 0;
-        const int rc = dctc_run_k1(ctx, a, n, ctx->stream);
-        if (rc) return rc;
-    }
-    if (seams_out)
-        CK(ctx, cudaMemcpyAsync(seams_out, b->seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return batch_seam_loop(b, n_seams, seams_out, b->dump_vmaps ? b->raw : nullptr, b->dump_vmaps ? b->vs : nullptr);
+}
+
+int dctc_carver_batch_enlarge_width(dctc_carver_batch* b, int n_seams, int* seams_out)
+{
+    if (!b || n_seams < 0) return DCTC_ERR_INVALID;
+    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
+    if (n_seams == 0) return DCTC_OK;
+    if (n_seams >= b->w || b->w != b->w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
+    if (b->w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    // the seam loop carves the loaded frames in place: until every frame is enlarged the batch is not loaded, so that a
+    // failure leaves it unloaded rather than half-updated
+    b->loaded = false;
+    const int rc = batch_enlarge(b, n_seams, seams_out);
+    if (rc) return rc;
+    b->w = b->w0 + n_seams;
+    b->enlarged = true;
+    b->loaded = true;
     return DCTC_OK;
 }
 
@@ -1823,7 +1911,9 @@ int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
     dctc_context* ctx = b->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
     const size_t rb = (size_t) b->w * b->ch;   // frames are pitch * h bytes apart: n * h rows of one pitch
-    CK(ctx, cudaMemcpy2DAsync(out, rb, b->img, b->pitch, rb, (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
+    const uint8_t* img = b->enlarged ? b->wide_img : b->img;
+    const size_t pitch = b->enlarged ? b->wide_pitch : b->pitch;
+    CK(ctx, cudaMemcpy2DAsync(out, rb, img, pitch, rb, (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
 }
@@ -1834,7 +1924,9 @@ int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
     if (!b->loaded) return DCTC_ERR_STATE;
     dctc_context* ctx = b->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
-    CK(ctx, cudaMemcpy2DAsync(out, sizeof(float) * b->w, b->en, sizeof(float) * b->en_pitch, sizeof(float) * b->w,
+    const float* en = b->enlarged ? b->wide_en : b->en;
+    const size_t en_pitch = b->enlarged ? b->wide_en_pitch : b->en_pitch;
+    CK(ctx, cudaMemcpy2DAsync(out, sizeof(float) * b->w, en, sizeof(float) * en_pitch, sizeof(float) * b->w,
                               (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;

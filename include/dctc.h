@@ -189,10 +189,12 @@ int dctc_carver_paint_seams(dctc_context *ctx, uint8_t *img, int channels, size_
  * device buffers and never touches the context's single-frame session.  Every phase of the seam loop is one launch
  * for all frames, and every frame's seam DP runs on its own cluster, so frames retarget side by side.  Each frame
  * gets exactly the seams, image, energy map and visibility map that dctc_carver_load + dctc_carver_resize_width
- * give it on its own.  The cumulative map is always rebuilt (no incremental mode).
+ * give it on its own, and dctc_carver_batch_enlarge_width gives every frame what dctc_carver_enlarge_width gives it.
+ * The cumulative map is always rebuilt: incremental mode and height retargeting are not batched.
  * Errors: DCTC_ERR_INVALID for NULL pointers, n_frames <= 0, a channel count outside 1..4, a pitch or frame stride
- * that is too small; DCTC_ERR_STATE for a resize before a load or n_seams >= the current width; DCTC_ERR_UNSUPPORTED
- * for widths the device seam DP does not cover (as dctc_carver_resize_width) and n_frames > 65535. */
+ * that is too small; DCTC_ERR_STATE for a resize before a load, after an enlarge or with n_seams >= the current width;
+ * DCTC_ERR_UNSUPPORTED for widths the device seam DP does not cover (as dctc_carver_resize_width) and
+ * n_frames > 65535. */
 typedef struct dctc_carver_batch dctc_carver_batch;
 /* n_frames frames of w x h, channels 1..4; uses the context's device, stream, blocksize / edges / textures and kernel
  * selection as they are at load time.  dump_vmaps: also keep a visibility map per frame. */
@@ -200,11 +202,26 @@ int dctc_carver_batch_create(dctc_context *ctx, int n_frames, int w, int h, int 
                              dctc_carver_batch **batch);
 void dctc_carver_batch_destroy(dctc_carver_batch *batch);
 /* host frames (frame_stride_bytes apart, rows pitch_bytes apart) -> device, full energy map of every frame (one K1
- * batch launch).  A load restarts the session at the original width w. */
+ * batch launch).  A load restarts the session at the original width w, also after an enlarge. */
 int dctc_carver_batch_load(dctc_carver_batch *batch, const uint8_t *imgs, size_t frame_stride_bytes, size_t pitch_bytes);
 /* removes n_seams vertical seams from every frame; seams_out (may be NULL): n_frames * n_seams * h ints, frame-major,
  * in the coordinates at removal time (the layout dctc_carver_resize_width uses, per frame) */
 int dctc_carver_batch_resize_width(dctc_carver_batch *batch, int n_seams, int *seams_out);
+/* lqr_carver_resize to a larger width for every frame (the single session's dctc_carver_enlarge_width, per frame):
+ * the n_seams seams a shrink would remove (seams_out as dctc_carver_batch_resize_width), then every pixel of those
+ * seams is doubled.  Frames become w0 + n_seams wide; _images / _energy / _width reflect the enlarged frames (the energy
+ * is the full map of the enlarged frame); _vmap (needs dump_vmaps) returns the start frames' maps over w0, depth
+ * n_seams.  Each frame gets exactly the seams, enlarged image, energy map and start-frame visibility map that
+ * dctc_carver_load + dctc_carver_enlarge_width give it alone on the same context.  A batch created without dump_vmaps
+ * enlarges too (the removal order then lives in buffers the first enlarge allocates).
+ * n_seams == 0: DCTC_OK, nothing happens.  DCTC_ERR_INVALID: NULL batch, n_seams < 0.  DCTC_ERR_STATE: not loaded, not
+ * at the loaded width (a resize ran since the load), n_seams >= w.  DCTC_ERR_UNSUPPORTED: frames wider than the
+ * device seam DP covers (checked before any work: the batch stays loaded).
+ * After an enlarge, _resize_width and _enlarge_width return DCTC_ERR_STATE until the next dctc_carver_batch_load,
+ * which restarts the batch at w x h.  A CUDA failure during the enlarge leaves the batch unloaded (DCTC_ERR_STATE until
+ * the next load).  The buffers an enlarge allocates (a copy of the start frames, the enlarged frames, the removal
+ * order) are reused by the next enlarge (the enlarged frames' when n_seams is the same) and freed by the destroy. */
+int dctc_carver_batch_enlarge_width(dctc_carver_batch *batch, int n_seams, int *seams_out);
 /* current width of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
 /* current images (n_frames * h * w * channels, pitch w * channels) / energy maps (n_frames * h * w floats) */
