@@ -122,14 +122,14 @@ int dctc_set_params(dctc_context* ctx, const DctcEnergyParameters* p)
     if (!ctx || !p) return DCTC_ERR_INVALID;
     if (!valid_blocksize(p->blocksize)) return DCTC_ERR_BLOCKSIZE;
     if (!(std::isfinite(p->edges) && std::isfinite(p->textures))) return DCTC_ERR_INVALID;
-    const bool changed = ctx->edges != p->edges || ctx->textures != p->textures || ctx->blocksize != p->blocksize;
-    ctx->edges = p->edges;
-    ctx->textures = p->textures;
-    ctx->blocksize = p->blocksize;
+    const bool changed = ctx->op.edges != p->edges || ctx->op.textures != p->textures || ctx->op.blocksize != p->blocksize;
+    ctx->op.edges = p->edges;
+    ctx->op.textures = p->textures;
+    ctx->op.blocksize = p->blocksize;
     ctx->mirror_valid = false;
     // a loaded carver session keeps its map in step with the operator (band radius, weights), like liblqr, whose
     // lqr_carver_set_energy_function (src/render.c:314-315) invalidates the energy map
-    if (changed && ctx->c_img) return dctc_carver_params_changed(ctx);
+    if (changed && ctx->carver) return dctc_carver_params_changed(ctx);
     return DCTC_OK;
 }
 
@@ -137,7 +137,7 @@ int dctc_set_kernel(dctc_context* ctx, int kernel)
 {
     if (!ctx) return DCTC_ERR_INVALID;
     if (kernel < DCTC_KERNEL_AUTO || kernel > DCTC_KERNEL_FP32_STREAM) return DCTC_ERR_INVALID;
-    ctx->kernel = kernel;
+    ctx->op.kernel = kernel;
     return DCTC_OK;
 }
 
@@ -149,21 +149,17 @@ unsigned long long dctc_launch_count(const dctc_context* ctx) { return ctx ? ctx
 
 // ---- K1 dispatch ------------------------------------------------------------------------------------------
 
-static void fill_weights(const dctc_context* ctx, DctcK1Args& a)
+// The context supplies the device, the tensor-core counters and the launch counter; op the operator and kernel selection.
+int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream)
 {
     // E = max|T| * weight; the kernels keep luma in 0..255 units, so the 1/255 of liblqr's reader folds in here.
-    a.w_edges = (float) ((double) ctx->edges / 255.0);
-    a.w_textures = (float) ((double) ctx->textures / 255.0);
-}
-
-int dctc_run_k1(dctc_context* ctx, DctcK1Args& a, int n_frames, cudaStream_t stream)
-{
-    fill_weights(ctx, a);
-    const bool uniform = ctx->edges == ctx->textures;
-    int kernel = ctx->kernel;
+    a.w_edges = (float) ((double) op.edges / 255.0);
+    a.w_textures = (float) ((double) op.textures / 255.0);
+    const bool uniform = op.edges == op.textures;
+    int kernel = op.kernel;
     // band mode (per-seam update) always runs in the tile kernel; block size 8 full maps default to the tensor-core
     // kernel (which hands configurations outside its fast path to the FP32 march kernel)
-    if (a.seam || ctx->blocksize != 8) {
+    if (a.seam || op.blocksize != 8) {
         kernel = DCTC_KERNEL_FP32_TILE;   // block sizes 2, 4, 16 pick their fast path below
     } else if (kernel == DCTC_KERNEL_AUTO) {
         kernel = DCTC_KERNEL_TC_SPLIT;
@@ -176,14 +172,14 @@ int dctc_run_k1(dctc_context* ctx, DctcK1Args& a, int n_frames, cudaStream_t str
         // block sizes 2 and 4 (HBM-bound): full maps stream through the register-march kernel unless the tile kernel was
         // asked for explicitly; both produce bit-identical maps
         e = cudaErrorNotSupported;
-        if ((ctx->kernel == DCTC_KERNEL_AUTO || ctx->kernel == DCTC_KERNEL_FP32_STREAM) && !a.seam && !a.preview &&
-            (ctx->blocksize == 2 || ctx->blocksize == 4))
-            e = dctc_launch_k1_small(a, ctx->blocksize, n_frames, uniform, ctx->sm_count, stream);
+        if ((op.kernel == DCTC_KERNEL_AUTO || op.kernel == DCTC_KERNEL_FP32_STREAM) && !a.seam && !a.preview &&
+            (op.blocksize == 2 || op.blocksize == 4))
+            e = dctc_launch_k1_small(a, op.blocksize, n_frames, uniform, ctx->sm_count, stream);
         // block size 16 (compute-bound): full maps run their y-pass on the tensor cores unless the FP32 tile kernel was
         // asked for explicitly (or the configuration is outside the tensor-core fast path)
-        if (ctx->kernel != DCTC_KERNEL_FP32_TILE && ctx->kernel != DCTC_KERNEL_FP32_MARCH && !a.seam && !a.preview && ctx->blocksize == 16)
+        if (op.kernel != DCTC_KERNEL_FP32_TILE && op.kernel != DCTC_KERNEL_FP32_MARCH && !a.seam && !a.preview && op.blocksize == 16)
             e = dctc_launch_k1_tc16(a, n_frames, uniform, ctx->tc_counters + (ctx->tc_next++ % DCTC_TC_COUNTERS), ctx->sm_count, stream);
-        if (e == cudaErrorNotSupported) e = dctc_launch_k1_tile(a, ctx->blocksize, n_frames, uniform, stream);
+        if (e == cudaErrorNotSupported) e = dctc_launch_k1_tile(a, op.blocksize, n_frames, uniform, stream);
         break;
     case DCTC_KERNEL_FP32_MARCH: e = dctc_launch_k1_march8(a, n_frames, uniform, stream); break;
     case DCTC_KERNEL_TC_SPLIT:
@@ -240,7 +236,7 @@ int dctc_energy_batch_dev(dctc_context* ctx, const uint8_t* d_imgs, int n_frames
     int rc = check_image(w, h, channels, pitch);
     if (rc) return rc;
     if (out_pitch < (size_t) w) return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     // grid.z carries the frame index: split very large batches
     for (int f0 = 0; f0 < n_frames; f0 += 32768) {
@@ -250,7 +246,7 @@ int dctc_energy_batch_dev(dctc_context* ctx, const uint8_t* d_imgs, int n_frames
                    out_pitch);
         a.frame_stride = frame_stride;
         a.out_frame_stride = out_frame_stride;
-        rc = dctc_run_k1(ctx, a, nf, ctx->stream);
+        rc = dctc_run_k1(ctx, ctx->op, a, nf, ctx->stream);
         if (rc) return rc;
     }
     if (sync) CK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -276,14 +272,14 @@ int dctc_energy_band_dev_at(dctc_context* ctx, const uint8_t* d_band, int w, int
     if ((top_rows > 0 && (!d_top || top_pitch < (size_t) w * channels)) ||
         (bot_rows > 0 && (!d_bot || bot_pitch < (size_t) w * channels)))
         return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     DctcK1Args a;
     plain_args(a, d_band, w, band_rows, channels, pitch, d_out, out_pitch);
     a.top = d_top; a.top_rows = d_top ? top_rows : 0; a.top_pitch = top_pitch;
     a.bot = d_bot; a.bot_rows = d_bot ? bot_rows : 0; a.bot_pitch = bot_pitch;
     a.row_origin = band_y0;
-    rc = dctc_run_k1(ctx, a, 1, ctx->stream);
+    rc = dctc_run_k1(ctx, ctx->op, a, 1, ctx->stream);
     if (rc) return rc;
     if (sync) CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
@@ -303,7 +299,7 @@ int dctc_energy_batch(dctc_context* ctx, const uint8_t* imgs, int n_frames, size
     int rc = check_image(w, h, channels, pitch);
     if (rc) return rc;
     if (n_frames > 1 && (frame_stride < pitch * (size_t) h || out_frame_stride < (size_t) w * h)) return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     const size_t row_bytes = (size_t) w * channels;
     const size_t d_pitch = (row_bytes + 15) & ~(size_t) 15;
@@ -326,7 +322,7 @@ int dctc_energy_batch(dctc_context* ctx, const uint8_t* imgs, int n_frames, size
         if (f >= DCTC_SLOTS) CK(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_out[s], 0));  // slot output drained
         DctcK1Args a;
         plain_args(a, ctx->d_in[s], w, h, channels, d_pitch, ctx->d_out[s], (size_t) w);
-        rc = dctc_run_k1(ctx, a, 1, ctx->stream);
+        rc = dctc_run_k1(ctx, ctx->op, a, 1, ctx->stream);
         if (rc) return rc;
         CK(ctx, cudaEventRecord(ctx->ev_k[s], ctx->stream));
         CK(ctx, cudaStreamWaitEvent(ctx->s_out, ctx->ev_k[s], 0));

@@ -11,6 +11,7 @@
 #include <type_traits>
 #include <cstring>
 #include <new>
+#include <utility>
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
 
@@ -19,8 +20,6 @@
         cudaError_t e_ = (call);                                  \
         if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
     } while (0)
-
-int dctc_run_k1(dctc_context* ctx, DctcK1Args& a, int n_frames, cudaStream_t stream);
 
 // One CTA per row: shift image bytes and energy floats right of the seam one pixel to the left.
 // Chunks are processed left to right; the barrier between a chunk's loads and its stores also orders them
@@ -1079,91 +1078,116 @@ __global__ void __launch_bounds__(256) dctc_inflate_rows_kernel(const uint8_t* _
     }
 }
 
-void dctc_carver_release(dctc_context* ctx)
+// ---- carver sessions: host side -------------------------------------------------------------------------------------
+// Both sessions keep their device state in a CarverFrames (dctc_launch.h): the context's single session one frame, a
+// batch session n equally sized frames.  The kernels above take the frame from a spare grid dimension, so one launch per
+// phase serves every frame and each frame's seam DP runs on its own cluster of DP_CL CTAs; a frame gets exactly the
+// seams, image, energy plane and visibility map whatever the number of frames around it.
+
+constexpr int DP_MAX_W = DP_CL * DP_MAXW * (512 - 2 * DP_R);   // widest frame the seam DP's strips cover
+
+// Geometry of n frames of w x h pixels: image rows 16-byte aligned, energy rows a multiple of 4 floats, cumulative rows
+// at least one back-track window (DP_WIN floats) wide, so that the windows stay inside the plane.
+static void frames_init(CarverFrames& f, int n, int w, int h, int ch)
 {
-    if (ctx->c_img) cudaFree(ctx->c_img);
-    if (ctx->c_en) cudaFree(ctx->c_en);
-    if (ctx->c_m) cudaFree(ctx->c_m);
-    if (ctx->c_dir) cudaFree(ctx->c_dir);
-    if (ctx->c_seam_log) cudaFree(ctx->c_seam_log);
-    if (ctx->c_raw) cudaFree(ctx->c_raw);
-    if (ctx->c_vs) cudaFree(ctx->c_vs);
-    if (ctx->c_seam) cudaFree(ctx->c_seam);
-    if (ctx->c_band) cudaFree(ctx->c_band);
-    if (ctx->c_band_vals) cudaFree(ctx->c_band_vals);
-    if (ctx->h_mirror) cudaFreeHost(ctx->h_mirror);
-    if (ctx->h_band) cudaFreeHost(ctx->h_band);
-    ctx->c_img = nullptr; ctx->c_en = nullptr; ctx->c_m = nullptr; ctx->c_dir = nullptr; ctx->c_seam_log = nullptr; ctx->c_seam_log_cap = 0; ctx->c_raw = nullptr; ctx->c_vs = nullptr; ctx->c_vs_depth = 0; ctx->c_vs_w = 0; ctx->c_seam = nullptr; ctx->c_band = nullptr;
-    ctx->c_band_vals = nullptr; ctx->h_mirror = nullptr; ctx->h_band = nullptr;
-    ctx->c_w0 = ctx->c_w = ctx->c_h = ctx->c_ch = 0;
-    ctx->c_m_valid = false;
-    ctx->c_pitch = 0;
-    ctx->c_en_pitch = 0;
-    ctx->mirror_valid = false;
+    f.n = n; f.w0 = f.w = w; f.h = h; f.ch = ch;
+    f.pitch = ((size_t) w * ch + 15) & ~(size_t) 15;
+    f.img_fs = f.pitch * h;
+    f.en_pitch = ((size_t) w + 3) & ~(size_t) 3;
+    f.m_pitch = f.en_pitch < (size_t) DP_WIN ? (size_t) DP_WIN : f.en_pitch;
 }
 
-static void carver_args(const dctc_context* ctx, DctcK1Args& a)
+static void frames_free(CarverFrames& f)
 {
-    memset(&a, 0, sizeof(a));
-    a.img = ctx->c_img; a.pitch = ctx->c_pitch; a.w = ctx->c_w; a.h = ctx->c_h; a.channels = ctx->c_ch;
-    a.out = ctx->c_en; a.out_pitch = ctx->c_en_pitch;
+    cudaFree(f.img); cudaFree(f.en); cudaFree(f.m); cudaFree(f.dir); cudaFree(f.seam); cudaFree(f.xlast);
+    cudaFree(f.seam_log); cudaFree(f.raw); cudaFree(f.vs);
+    f = CarverFrames();
 }
 
-static int band_stride(const dctc_context* ctx) { return 4 * (ctx->blocksize / 2); }
-
-// Full energy map of the session's current image.  A carver session keeps one arithmetic for the whole seam loop: the
-// per-seam band updates run in the FP32 tile kernel, so full maps use the bit-identical FP32 march kernel rather than
-// the tensor-core kernel (liblqr: update_emap must reproduce what build_emap would give on the carved image).
-static int carver_full_energy(dctc_context* ctx)
+// Images, energy planes and seams; the seam loop adds its planes on first use (frames_loop_buffers), visibility maps are
+// added by frames_vmaps.
+static int frames_alloc(dctc_context* ctx, CarverFrames& f)
 {
-    DctcK1Args a;
-    carver_args(ctx, a);
-    const int saved_kernel = ctx->kernel;
-    if (ctx->kernel == DCTC_KERNEL_AUTO || ctx->kernel == DCTC_KERNEL_TC_SPLIT || ctx->kernel == DCTC_KERNEL_FP32_STREAM) ctx->kernel = DCTC_KERNEL_FP32_MARCH;
-    const int rc = dctc_run_k1(ctx, a, 1, ctx->stream);
-    ctx->kernel = saved_kernel;
-    return rc;
-}
-
-// dctc_set_params with a session loaded (liblqr: lqr_carver_set_energy_function invalidates the energy map): the
-// resident map is rebuilt with the new operator and the cumulative plane of the seam DP is dropped.
-int dctc_carver_params_changed(dctc_context* ctx)
-{
-    if (!ctx->c_img) return DCTC_OK;
-    CK(ctx, cudaSetDevice(ctx->device));
-    ctx->mirror_valid = false;
-    ctx->c_m_valid = false;
-    const int rc = carver_full_energy(ctx);
-    if (rc) return rc;
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    const size_t n = (size_t) f.n, h = (size_t) f.h;
+    CK(ctx, cudaMalloc((void**) &f.img, f.img_fs * n));
+    CK(ctx, cudaMalloc((void**) &f.en, sizeof(float) * f.en_pitch * h * n));
+    CK(ctx, cudaMemsetAsync(f.en, 0, sizeof(float) * f.en_pitch * h * n, ctx->stream));
+    CK(ctx, cudaMalloc((void**) &f.seam, sizeof(int) * h * n));
+    CK(ctx, cudaMalloc((void**) &f.xlast, sizeof(int) * n));
+    CK(ctx, cudaMemsetAsync(f.xlast, 0, sizeof(int) * n, ctx->stream));
     return DCTC_OK;
 }
 
-static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
+// Empty visibility maps (w0 x h ints per frame) and the identity column map raw[frame][y][x] = x.  Maps are allocated when
+// the frames have no raw map (a visibility map kept from before a single-session enlarge belongs to the narrower start
+// frame and is replaced).
+static int frames_vmaps(dctc_context* ctx, CarverFrames& f)
 {
-    // img may be host or device memory (cudaMemcpyDefault: the enlarge path reloads the session from a device buffer)
-    ctx->c_w0 = ctx->c_w = w; ctx->c_h = h; ctx->c_ch = channels;
-    ctx->c_pitch = ((size_t) w * channels + 15) & ~(size_t) 15;
-    const size_t npx = (size_t) w * h;
-    ctx->c_en_pitch = ((size_t) w + 3) & ~(size_t) 3;
-    CK(ctx, cudaMalloc((void**) &ctx->c_img, ctx->c_pitch * h));
-    CK(ctx, cudaMalloc((void**) &ctx->c_en, sizeof(float) * ctx->c_en_pitch * h));
-    CK(ctx, cudaMemsetAsync(ctx->c_en, 0, sizeof(float) * ctx->c_en_pitch * h, ctx->stream));
-    CK(ctx, cudaMalloc((void**) &ctx->c_seam, sizeof(int) * h));
-    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * 32));
-    CK(ctx, cudaMallocHost((void**) &ctx->h_mirror, sizeof(float) * npx));
-    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * 32 + sizeof(int) * h));
-    CK(ctx, cudaMemcpy2DAsync(ctx->c_img, ctx->c_pitch, img, pitch, (size_t) w * channels, h, cudaMemcpyDefault,
-                              ctx->stream));
-    int rc = carver_full_energy(ctx);
-    if (rc) return rc;
+    const size_t nv = (size_t) f.w0 * f.h * f.n;
+    if (!f.raw) {
+        cudaFree(f.vs);
+        f.vs = nullptr;
+        CK(ctx, cudaMalloc((void**) &f.vs, sizeof(int) * nv));
+        CK(ctx, cudaMalloc((void**) &f.raw, sizeof(int) * nv));
+    }
+    CK(ctx, cudaMemsetAsync(f.vs, 0, sizeof(int) * nv, ctx->stream));
+    dctc_iota_rows_kernel<<<(unsigned) ((nv + 255) / 256), 256, 0, ctx->stream>>>(f.raw, f.w0, f.h * f.n);
+    CK(ctx, cudaGetLastError());
+    ctx->launches++;
+    f.depth = 0;
+    f.vs_w = f.w0;
+    return DCTC_OK;
+}
+
+// A carver session keeps one arithmetic for the whole seam loop: the per-seam band updates run in the FP32 tile kernel, so
+// full maps use the bit-identical FP32 march kernel rather than the tensor-core kernel (liblqr: update_emap must reproduce
+// what build_emap would give on the carved image).
+static DctcK1Op carver_op(DctcK1Op op)
+{
+    if (op.kernel == DCTC_KERNEL_AUTO || op.kernel == DCTC_KERNEL_TC_SPLIT || op.kernel == DCTC_KERNEL_FP32_STREAM)
+        op.kernel = DCTC_KERNEL_FP32_MARCH;
+    return op;
+}
+
+// K1 over the frames' current images into their energy planes; with a seam (h per frame), band mode around it with the
+// operator's band radius
+static DctcK1Args frames_k1_args(const CarverFrames& f, const DctcK1Op& op, const int* seam)
+{
+    DctcK1Args a;
+    memset(&a, 0, sizeof(a));
+    a.img = f.img; a.pitch = f.pitch; a.w = f.w; a.h = f.h; a.channels = f.ch;
+    a.out = f.en; a.out_pitch = f.en_pitch;
+    a.frame_stride = f.img_fs; a.out_frame_stride = f.en_pitch * f.h;
+    if (seam) {
+        a.seam = seam; a.seam_frame_stride = f.h;
+        a.band_r = op.blocksize / 2; a.band_stride = 4 * (op.blocksize / 2);
+    }
+    return a;
+}
+
+static int frames_full_energy(dctc_context* ctx, const CarverFrames& f, const DctcK1Op& op)
+{
+    DctcK1Args a = frames_k1_args(f, op, nullptr);
+    return dctc_run_k1(ctx, op, a, f.n, ctx->stream);
+}
+
+// Images (w * ch bytes per row), energy planes (w floats per row) and visibility maps (vs_w ints per row) of all frames,
+// n * h rows each, to the host
+static int frames_download(dctc_context* ctx, const CarverFrames& f, uint8_t* img, float* en, int* vs)
+{
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t rows = (size_t) f.h * f.n, rb = (size_t) f.w * f.ch;   // frames are h rows apart in every plane
+    if (img) CK(ctx, cudaMemcpy2DAsync(img, rb, f.img, f.pitch, rb, rows, cudaMemcpyDeviceToHost, ctx->stream));
+    if (en)
+        CK(ctx, cudaMemcpy2DAsync(en, sizeof(float) * f.w, f.en, sizeof(float) * f.en_pitch, sizeof(float) * f.w, rows,
+                                  cudaMemcpyDeviceToHost, ctx->stream));
+    if (vs) CK(ctx, cudaMemcpyAsync(vs, f.vs, sizeof(int) * f.vs_w * rows, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
 }
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
-// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map.  The single-frame session and the
-// batch session share it, so both run the same kernel variant for the same width.
+// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map.
 using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*, size_t, size_t, size_t);
 struct DpPlan {
     dp_fn dp = nullptr;
@@ -1252,13 +1276,190 @@ static BtPlan bt_plan(int h, size_t m_pitch)
     return b;
 }
 
+// Planes of the seam loop, allocated by its first call: cumulative planes, jump planes (parallel back-track only) and a
+// seam log of log_fs ints per frame.
+static int frames_loop_buffers(dctc_context* ctx, CarverFrames& f, const BtPlan& bt, size_t log_fs)
+{
+    const size_t n = (size_t) f.n;
+    if (!f.m) {
+        CK(ctx, cudaMalloc((void**) &f.m, sizeof(float) * f.m_pitch * f.h * n));
+        CK(ctx, cudaMemsetAsync(f.m, 0, sizeof(float) * f.m_pitch * f.h * n, ctx->stream));
+    }
+    if (bt.par && !f.dir) {
+        f.dir_fs = (size_t) bt.nb * bt.j_pitch;
+        CK(ctx, cudaMalloc((void**) &f.dir, f.dir_fs * n));
+    }
+    if (f.seam_log_cap < log_fs * n) {
+        cudaFree(f.seam_log);
+        f.seam_log = nullptr; f.seam_log_cap = 0;
+        CK(ctx, cudaMalloc((void**) &f.seam_log, sizeof(int) * log_fs * n));
+        f.seam_log_cap = log_fs * n;
+    }
+    return DCTC_OK;
+}
+
+// The device seam loop of every frame: removes n_seams seams from the images and energy planes (f.w shrinks by n_seams).
+// Per seam: build_mmap + build_vpath (seam DP, then jump + trace or the DP's serial walk), update_vsmap when vmaps (maps
+// as frames_vmaps leaves them), the carve, and update_emap (band K1 around each removed seam).  The caller has checked the
+// width.
+// incr_valid, single session only: the incremental cumulative map of dctc_carver_set_incremental (its flag buffer is
+// ctx->c_band); *incr_valid says whether f.m holds the map of the image before the last removal, compacted over that seam.
+// The walk then replaces DP + jump + trace, the DP only runs when the walk gave up, and the carve also compacts f.m.
+static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, bool vmaps,
+                     bool* incr_valid)
+{
+    const int n = f.n, h = f.h;
+    const size_t log_fs = (size_t) n_seams * h, en_fs = f.en_pitch * h, m_fs = f.m_pitch * h;
+    const BtPlan bt = bt_plan(h, f.m_pitch);
+    int rc = frames_loop_buffers(ctx, f, bt, log_fs);
+    if (rc) return rc;
+    DpPlan plan;
+    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, plan));
+    if (bt.par && bt.cone_smem > 40 * 1024)
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+    int* const xlast = bt.par ? f.xlast : nullptr;
+    // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
+    const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
+    const bool incr = incr_valid && n == 1 && incr_smem <= 160 * 1024;
+    if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_incr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
+        if (!ctx->c_band) {
+            CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 4));
+            CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 4, ctx->stream));
+        }
+    }
+    const bool pdl = !getenv("DCTC_NO_PDL");
+    for (int s = 0; s < n_seams; s++) {
+        const int w_old = f.w;
+        int* log_s = f.seam_log + (size_t) s * h;
+        const bool walk = incr && *incr_valid;
+        if (walk) {
+            // update_mmap + build_vpath: walk the changed cells only; the DP below rebuilds the map only if the walk gave up
+            dctc_seam_incr_kernel<<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2,
+                                                                     f.seam, log_s, ctx->c_band);
+            CK(ctx, cudaGetLastError());
+            ctx->launches++;
+        }
+        // build_mmap, one cluster per frame, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per
+        // block and frame (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor
+        // drains and blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
+        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl && !walk, f.en, f.en_pitch, w_old,
+                                h, f.m, f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
+                                plan.use_tmap, walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs));
+        if (bt.par && !walk) {
+            const int js = (w_old + 63) / 64;
+            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, f.m, f.m_pitch,
+                                    w_old, h, f.dir, bt.j_pitch, js, m_fs, f.dir_fs));
+            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, f.m, f.m_pitch,
+                                    w_old, h, f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs));
+            ctx->launches += 2;
+        }
+#ifdef DCTC_SYNC_DEBUG
+        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: dp kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
+#endif
+        if (vmaps) {   // update_vsmap
+            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, f.raw, f.vs, f.w0, f.seam, w_old,
+                                    ++f.depth));
+            ctx->launches++;
+        }
+        // carve: compact image and energy rows (and the cumulative rows of the incremental map) over the seam
+        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, f.img, f.pitch, f.ch, f.en,
+                                f.en_pitch, f.seam, w_old, incr ? f.m : (float*) nullptr, f.m_pitch, f.img_fs, en_fs, m_fs));
+        ctx->launches += 2;
+        f.w = w_old - 1;
+        if (incr_valid) *incr_valid = incr;   // the plane now holds the map of the image before this removal, moved with the pixels
+#ifdef DCTC_SYNC_DEBUG
+        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: carve kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
+#endif
+        // update_emap: K1 in band mode around every frame's removed seam
+        DctcK1Args a = frames_k1_args(f, op, f.seam);
+        a.pdl = pdl ? 1 : 0;
+        rc = dctc_run_k1(ctx, op, a, n, ctx->stream);
+        if (rc) return rc;
+#ifdef DCTC_SYNC_DEBUG
+        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: band kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
+#endif
+    }
+    if (seams_out)
+        CK(ctx, cudaMemcpyAsync(seams_out, f.seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+// Enlarge core of both sessions (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): the start
+// frames are copied to start_img, the seam loop removes n_seams seams and records their order in the visibility maps (as
+// frames_vmaps leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images
+// (w0 + n_seams wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
+static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, bool* incr_valid,
+                          uint8_t* start_img, CarverFrames& wide)
+{
+    CK(ctx, cudaMemcpyAsync(start_img, f.img, f.img_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream));
+    int rc = seam_loop(ctx, f, op, n_seams, seams_out, true, incr_valid);
+    if (rc) return rc;
+    dctc_inflate_rows_kernel<<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(start_img, f.pitch, f.ch, f.w0, f.vs, n_seams, wide.img, wide.pitch,
+                                                                      f.img_fs, (size_t) f.w0 * f.h, wide.img_fs);
+    CK(ctx, cudaGetLastError());
+    ctx->launches++;
+    rc = frames_full_energy(ctx, wide, op);
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+// ---- single session (the context's) --------------------------------------------------------------------------------
+
+void dctc_carver_release(dctc_context* ctx)
+{
+    if (ctx->carver) {
+        frames_free(*ctx->carver);
+        delete ctx->carver;
+        ctx->carver = nullptr;
+    }
+    cudaFree(ctx->c_band); cudaFree(ctx->c_band_vals);
+    cudaFreeHost(ctx->h_mirror); cudaFreeHost(ctx->h_band);
+    ctx->c_band = nullptr; ctx->c_band_vals = nullptr; ctx->h_mirror = nullptr; ctx->h_band = nullptr;
+    ctx->c_m_valid = false;
+    ctx->mirror_valid = false;
+}
+
+// dctc_set_params with a session loaded (liblqr: lqr_carver_set_energy_function invalidates the energy map): the
+// resident map is rebuilt with the new operator and the cumulative plane of the seam DP is dropped.
+int dctc_carver_params_changed(dctc_context* ctx)
+{
+    if (!ctx->carver) return DCTC_OK;
+    CK(ctx, cudaSetDevice(ctx->device));
+    ctx->mirror_valid = false;
+    ctx->c_m_valid = false;
+    const int rc = frames_full_energy(ctx, *ctx->carver, carver_op(ctx->op));
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
+{
+    CarverFrames* f = new (std::nothrow) CarverFrames;
+    if (!f) return DCTC_ERR_NOMEM;
+    ctx->carver = f;
+    frames_init(*f, 1, w, h, channels);
+    int rc = frames_alloc(ctx, *f);
+    if (rc) return rc;
+    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * 32));
+    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * 32 + sizeof(int) * h));
+    CK(ctx, cudaMemcpy2DAsync(f->img, f->pitch, img, pitch, (size_t) w * channels, h, cudaMemcpyDefault, ctx->stream));
+    rc = frames_full_energy(ctx, *f, carver_op(ctx->op));
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
 extern "C" {
 
 int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
 {
     if (!ctx || !img || w <= 0 || h <= 0 || channels < 1 || channels > 4 || pitch < (size_t) w * channels)
         return DCTC_ERR_INVALID;
-    const int b = ctx->blocksize;
+    const int b = ctx->op.blocksize;
     if (!(b == 2 || b == 4 || b == 8 || b == 16)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -1269,36 +1470,30 @@ int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int ch
     return rc;
 }
 
-int dctc_carver_width(const dctc_context* ctx) { return ctx ? ctx->c_w : 0; }
-int dctc_carver_height(const dctc_context* ctx) { return ctx ? ctx->c_h : 0; }
+int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? ctx->carver->w : 0; }
+int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? ctx->carver->h : 0; }
 
 int dctc_carver_energy(dctc_context* ctx, float* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->c_img) return DCTC_ERR_STATE;
-    CK(ctx, cudaSetDevice(ctx->device));
-    CK(ctx, cudaMemcpy2DAsync(out, sizeof(float) * ctx->c_w, ctx->c_en, sizeof(float) * ctx->c_en_pitch,
-                              sizeof(float) * ctx->c_w, ctx->c_h, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    if (!ctx->carver) return DCTC_ERR_STATE;
+    return frames_download(ctx, *ctx->carver, nullptr, out, nullptr);
 }
 
 int dctc_carver_image(dctc_context* ctx, uint8_t* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->c_img) return DCTC_ERR_STATE;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const size_t rb = (size_t) ctx->c_w * ctx->c_ch;
-    CK(ctx, cudaMemcpy2DAsync(out, rb, ctx->c_img, ctx->c_pitch, rb, ctx->c_h, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    if (!ctx->carver) return DCTC_ERR_STATE;
+    return frames_download(ctx, *ctx->carver, out, nullptr, nullptr);
 }
 
 int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out, int* xmin, int* xmax)
 {
     if (!ctx || !seam_x) return DCTC_ERR_INVALID;
-    if (!ctx->c_img || ctx->c_w <= 1) return DCTC_ERR_STATE;
-    const int h = ctx->c_h, w_old = ctx->c_w, r = ctx->blocksize / 2, bs = band_stride(ctx);
+    CarverFrames* f = ctx->carver;
+    if (!f || f->w <= 1) return DCTC_ERR_STATE;
+    const DctcK1Op op = carver_op(ctx->op);
+    const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
     int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * 32);
     for (int y = 0; y < h; y++) {
         if (seam_x[y] < 0 || seam_x[y] >= w_old) return DCTC_ERR_STATE;
@@ -1307,18 +1502,17 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
         h_seam[y] = seam_x[y];
     }
     CK(ctx, cudaSetDevice(ctx->device));
-    CK(ctx, cudaMemcpyAsync(ctx->c_seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
-    dctc_carve_rows_kernel<256, 4><<<h, 256, 0, ctx->stream>>>(ctx->c_img, ctx->c_pitch, ctx->c_ch, ctx->c_en,
-                                                               ctx->c_en_pitch, ctx->c_seam, w_old, nullptr, 0, 0, 0, 0);
+    CK(ctx, cudaMemcpyAsync(f->seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
+    dctc_carve_rows_kernel<256, 4><<<h, 256, 0, ctx->stream>>>(f->img, f->pitch, f->ch, f->en, f->en_pitch, f->seam, w_old, nullptr,
+                                                               0, 0, 0, 0);
     CK(ctx, cudaGetLastError());
     ctx->launches++;
-    ctx->c_w = w_old - 1;
+    f->w = w_old - 1;
     ctx->mirror_valid = false;
     ctx->c_m_valid = false;     // the host picked this seam: the device's cumulative plane no longer matches
-    DctcK1Args a;
-    carver_args(ctx, a);
-    a.seam = ctx->c_seam; a.band_r = r; a.band_vals = ctx->c_band_vals; a.band_stride = bs;
-    int rc = dctc_run_k1(ctx, a, 1, ctx->stream);
+    DctcK1Args a = frames_k1_args(*f, op, f->seam);
+    a.band_vals = ctx->c_band_vals;
+    int rc = dctc_run_k1(ctx, op, a, 1, ctx->stream);
     if (rc) return rc;
     if (band_out) {
         CK(ctx, cudaMemcpyAsync(ctx->h_band, ctx->c_band_vals, sizeof(float) * (size_t) h * bs, cudaMemcpyDeviceToHost,
@@ -1328,7 +1522,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     size_t k = 0;
     for (int y = 0; y < h; y++) {
         int lo, hi;
-        dctc_band_limits(h_seam, y, h, ctx->c_w, r, &lo, &hi);
+        dctc_band_limits(h_seam, y, h, f->w, r, &lo, &hi);
         if (xmin) xmin[y] = lo;
         if (xmax) xmax[y] = hi;
         if (band_out && hi >= lo) {
@@ -1342,169 +1536,65 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
 int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
 {
     if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!ctx->c_img) return DCTC_ERR_STATE;
+    CarverFrames* f = ctx->carver;
+    if (!f) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= ctx->c_w) return DCTC_ERR_STATE;
-    const int h = ctx->c_h, r = ctx->blocksize / 2, bs = band_stride(ctx);
-    if (ctx->c_w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
+    if (n_seams >= f->w) return DCTC_ERR_STATE;
+    if (f->w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
     CK(ctx, cudaSetDevice(ctx->device));
-    if (ctx->c_dump_vmaps && !ctx->c_raw) {
-        if (ctx->c_w != ctx->c_w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
-        const size_t n = (size_t) ctx->c_w0 * h;
-        CK(ctx, cudaMalloc((void**) &ctx->c_raw, sizeof(int) * n));
-        CK(ctx, cudaMalloc((void**) &ctx->c_vs, sizeof(int) * n));
-        CK(ctx, cudaMemsetAsync(ctx->c_vs, 0, sizeof(int) * n, ctx->stream));
-        dctc_iota_rows_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, ctx->stream>>>(ctx->c_raw, ctx->c_w0, h);
-        CK(ctx, cudaGetLastError());
-        ctx->launches++;
-        ctx->c_vs_depth = 0;
-        ctx->c_vs_w = ctx->c_w0;
-    }
-    // cumulative-map plane, rows padded so that the back-track windows (DP_WIN floats) stay inside
-    const size_t m_pitch = ctx->c_en_pitch < (size_t) DP_WIN ? (size_t) DP_WIN : ctx->c_en_pitch;
-    if (!ctx->c_m) {
-        CK(ctx, cudaMalloc((void**) &ctx->c_m, sizeof(float) * m_pitch * (size_t) h));
-        CK(ctx, cudaMemsetAsync(ctx->c_m, 0, sizeof(float) * m_pitch * (size_t) h, ctx->stream));
-    }
-    if (ctx->c_seam_log_cap < (size_t) n_seams * h) {
-        if (ctx->c_seam_log) cudaFree(ctx->c_seam_log);
-        ctx->c_seam_log = nullptr; ctx->c_seam_log_cap = 0;
-        CK(ctx, cudaMalloc((void**) &ctx->c_seam_log, sizeof(int) * (size_t) n_seams * h));
-        ctx->c_seam_log_cap = (size_t) n_seams * h;
-    }
-    DpPlan plan;
-    CK(ctx, dp_plan(ctx->c_w, h, ctx->c_en, ctx->c_en_pitch, 1, plan));
-    const dp_fn dp = plan.dp;
-    const int wpc = plan.wpc, nst = plan.nst, use_tmap = plan.use_tmap;
-    const size_t dp_smem = plan.smem;
-    const CUtensorMap& tmap = plan.tmap;
-    // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
-    const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
-    const bool incr_ok = ctx->c_incremental && incr_smem <= 160 * 1024;
-    if (incr_ok)   // dynamic + static shared memory can exceed the 48 KB default
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_incr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
-    if (!ctx->c_band) {
-        CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 8));
-        CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 8, ctx->stream));
-    }
-    const BtPlan bt = bt_plan(h, m_pitch);
-    const int nb = bt.nb;
-    const size_t cone_smem = bt.cone_smem, j_pitch = bt.j_pitch;
-    const bool par_bt = bt.par;
-    int* const xlast = par_bt ? ctx->c_band + 4 : nullptr;
-    if (par_bt) {
-        if (!ctx->c_dir) CK(ctx, cudaMalloc((void**) &ctx->c_dir, (size_t) nb * j_pitch));
-        if (cone_smem > 40 * 1024)
-            CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) cone_smem));
-    }
-    const bool pdl = !getenv("DCTC_NO_PDL");
-    for (int s = 0; s < n_seams; s++) {
-        const int w_old = ctx->c_w;
-        int* log_s = ctx->c_seam_log + (size_t) s * h;
-        if (ctx->c_m_valid && incr_ok) {
-            // update_mmap + build_vpath: walk the changed cells only; the full rebuild below runs only if the walk gave up
-            dctc_seam_incr_kernel<<<1, 32, incr_smem, ctx->stream>>>(ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch, r,
-                                                                     ctx->c_seam, log_s, ctx->c_band);
-            dp<<<DP_CL, wpc * 32, dp_smem, ctx->stream>>>(ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch, ctx->c_seam, log_s, ctx->c_band, nst, tmap, use_tmap, nullptr,
-                                                          (size_t) 0, (size_t) 0, (size_t) 0);
-            ctx->launches++;
-        } else {
-            // build_mmap, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per block
-            // (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor drains and
-            // blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
-            CK(ctx, dctc_launch_pdl(dp, dim3(DP_CL), dim3(wpc * 32), dp_smem, ctx->stream, pdl, ctx->c_en, ctx->c_en_pitch, w_old, h, ctx->c_m, m_pitch,
-                                    ctx->c_seam, log_s, (int*) nullptr, nst, tmap, use_tmap, xlast, 0, 0, 0));
-            if (par_bt) {
-                const int js = (w_old + 63) / 64;
-                CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, nb), dim3(128), 0, ctx->stream, pdl, ctx->c_m, m_pitch, w_old, h,
-                                        ctx->c_dir, j_pitch, js, 0, 0));
-                CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(nb), dim3(TR_THREADS), cone_smem, ctx->stream, pdl, ctx->c_m, m_pitch, w_old, h,
-                                        ctx->c_dir, j_pitch, xlast, ctx->c_seam, log_s, 0, 0, 0));
-                ctx->launches += 2;
-            }
-        }
-#ifdef DCTC_SYNC_DEBUG
-        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: dp kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
-#endif
-        if (ctx->c_dump_vmaps) {   // update_vsmap
-            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h), dim3(256), 0, ctx->stream, pdl, ctx->c_raw, ctx->c_vs, ctx->c_vs_w, ctx->c_seam, w_old,
-                                    ++ctx->c_vs_depth));
-            ctx->launches++;
-        }
-        // carve: compact image and energy rows over the seam
-        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h), dim3(256), 0, ctx->stream, pdl, ctx->c_img, ctx->c_pitch, ctx->c_ch, ctx->c_en,
-                                ctx->c_en_pitch, ctx->c_seam, w_old, incr_ok ? ctx->c_m : (float*) nullptr, m_pitch, 0, 0, 0));
-        CK(ctx, cudaGetLastError());
-        ctx->launches += 2;
-        ctx->c_w = w_old - 1;
-        ctx->c_m_valid = incr_ok;   // the plane now holds the map of the image before this removal, moved with the pixels
-        // update_emap: K1 in band mode around the removed seam
-        DctcK1Args a;
-        carver_args(ctx, a);
-        a.seam = ctx->c_seam; a.band_r = r; a.band_vals = ctx->c_band_vals; a.band_stride = bs;
-        a.pdl = pdl ? 1 : 0;
-#ifdef DCTC_SYNC_DEBUG
-        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: carve kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
-#endif
-        int rc = dctc_run_k1(ctx, a, 1, ctx->stream);
+    if (ctx->c_dump_vmaps && !f->raw) {
+        if (f->w != f->w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
+        const int rc = frames_vmaps(ctx, *f);
         if (rc) return rc;
-#ifdef DCTC_SYNC_DEBUG
-        { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: band kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
-#endif
     }
     ctx->mirror_valid = false;
-    if (seams_out)
-        CK(ctx, cudaMemcpyAsync(seams_out, ctx->c_seam_log, sizeof(int) * (size_t) n_seams * h, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    if (!ctx->c_incremental) ctx->c_m_valid = false;
+    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_dump_vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
 }
 
-// lqr_carver_resize to a LARGER width (seams_number > 0, src/render.c:357-363): the n seams a shrink would remove,
-// then the inflate kernel; the session continues on the enlarged image (energy map rebuilt), the visibility map of the
-// start frame stays readable through dctc_carver_vmap.
+// lqr_carver_resize to a LARGER width: frames_enlarge, after which the session continues on the enlarged frame (its w0
+// is the new width, its energy map the one frames_enlarge computed); the visibility map of the start frame stays readable
+// through dctc_carver_vmap and dctc_carver_paint_seams.  A failure leaves the session unloaded.
 int dctc_carver_enlarge_width(dctc_context* ctx, int n_seams, int* seams_out)
 {
     if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!ctx->c_img) return DCTC_ERR_STATE;
+    CarverFrames* f = ctx->carver;
+    if (!f) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= ctx->c_w || ctx->c_w != ctx->c_w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded frame
-    const int w0 = ctx->c_w, h = ctx->c_h, ch = ctx->c_ch, w1 = w0 + n_seams;
+    if (n_seams >= f->w || f->w != f->w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded frame
+    if (f->w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
     CK(ctx, cudaSetDevice(ctx->device));
-    uint8_t* d_orig = nullptr;
-    uint8_t* d_new = nullptr;
-    const size_t p0 = ctx->c_pitch, p1 = ((size_t) w1 * ch + 15) & ~(size_t) 15;
-    CK(ctx, cudaMalloc((void**) &d_orig, p0 * h));
-    cudaError_t e = cudaMalloc((void**) &d_new, p1 * h);
-    if (e != cudaSuccess) { cudaFree(d_orig); return dctc_fail_cuda(ctx, e); }
-    e = cudaMemcpyAsync(d_orig, ctx->c_img, p0 * h, cudaMemcpyDeviceToDevice, ctx->stream);
-    int rc = e == cudaSuccess ? DCTC_OK : dctc_fail_cuda(ctx, e);
-    const bool dump_saved = ctx->c_dump_vmaps;
+    CarverFrames* wide = new (std::nothrow) CarverFrames;
+    if (!wide) return DCTC_ERR_NOMEM;
+    uint8_t* start = nullptr;
+    frames_init(*wide, 1, f->w0 + n_seams, f->h, f->ch);
+    int rc = frames_alloc(ctx, *wide);
+    if (rc == DCTC_OK) rc = frames_vmaps(ctx, *f);
     if (rc == DCTC_OK) {
-        ctx->c_dump_vmaps = true;                      // the seams' order per original pixel drives the pixel synthesis
-        rc = dctc_carver_resize_width(ctx, n_seams, seams_out);
-        ctx->c_dump_vmaps = dump_saved;
-    }
-    if (rc == DCTC_OK) {
-        dctc_inflate_rows_kernel<<<h, 256, 0, ctx->stream>>>(d_orig, p0, ch, w0, ctx->c_vs, n_seams, d_new, p1, 0, 0, 0);
-        e = cudaGetLastError();
-        ctx->launches++;
-        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        const cudaError_t e = cudaMalloc((void**) &start, f->img_fs);
         if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
     }
-    if (rc == DCTC_OK) {
-        // continue the session on the enlarged image; keep the visibility map of the start frame
-        int* vs = ctx->c_vs;
-        const int depth = ctx->c_vs_depth, vs_w = ctx->c_vs_w;
-        ctx->c_vs = nullptr;
+    if (rc == DCTC_OK)
+        rc = frames_enlarge(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_incremental ? &ctx->c_m_valid : nullptr, start, *wide);
+    cudaFree(start);
+    if (rc) {
+        frames_free(*wide);
+        delete wide;
         dctc_carver_release(ctx);
-        rc = carver_load_impl(ctx, d_new, w1, h, ch, p1);
-        if (rc != DCTC_OK) dctc_carver_release(ctx);
-        if (rc == DCTC_OK) { ctx->c_vs = vs; ctx->c_vs_depth = depth; ctx->c_vs_w = vs_w; }
-        else cudaFree(vs);
+        return rc;
     }
-    cudaFree(d_orig);
-    cudaFree(d_new);
-    return rc;
+    std::swap(wide->vs, f->vs);
+    wide->depth = f->depth;
+    wide->vs_w = f->vs_w;
+    frames_free(*f);
+    delete f;
+    ctx->carver = wide;
+    // as after a load: no cumulative map, no host mirror (the frame is wider), rebuild count from zero
+    cudaFree(ctx->c_band); cudaFreeHost(ctx->h_mirror);
+    ctx->c_band = nullptr; ctx->h_mirror = nullptr;
+    ctx->c_m_valid = false;
+    ctx->mirror_valid = false;
+    return DCTC_OK;
 }
 
 int dctc_carver_set_incremental(dctc_context* ctx, int on)
@@ -1516,7 +1606,7 @@ int dctc_carver_set_incremental(dctc_context* ctx, int on)
 
 int dctc_carver_rebuild_count(dctc_context* ctx)
 {
-    if (!ctx || !ctx->c_img) return -1;
+    if (!ctx || !ctx->carver) return -1;
     if (!ctx->c_band) return 0;
     int v[4] = {0, 0, 0, 0};
     if (cudaSetDevice(ctx->device) != cudaSuccess) return -1;
@@ -1538,20 +1628,19 @@ int dctc_carver_set_dump_vmaps(dctc_context* ctx, int on)
 int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
 {
     if (!ctx) return DCTC_ERR_INVALID;
-    if (!ctx->c_img || !ctx->c_vs) return DCTC_ERR_STATE;
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (vmap_out)
-        CK(ctx, cudaMemcpyAsync(vmap_out, ctx->c_vs, sizeof(int) * (size_t) ctx->c_vs_w * ctx->c_h, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    if (depth_out) *depth_out = ctx->c_vs_depth;
-    return DCTC_OK;
+    const CarverFrames* f = ctx->carver;
+    if (!f || !f->vs) return DCTC_ERR_STATE;
+    const int rc = frames_download(ctx, *f, nullptr, nullptr, vmap_out);
+    if (rc == DCTC_OK && depth_out) *depth_out = f->depth;
+    return rc;
 }
 
 int dctc_carver_paint_seams(dctc_context* ctx, uint8_t* img, int channels, size_t pitch)
 {
     if (!ctx || !img || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
-    if (!ctx->c_img || !ctx->c_vs || ctx->c_vs_depth <= 0) return DCTC_ERR_STATE;
-    const int w = ctx->c_vs_w, h = ctx->c_h;
+    const CarverFrames* f = ctx->carver;
+    if (!f || !f->vs || f->depth <= 0) return DCTC_ERR_STATE;
+    const int w = f->vs_w, h = f->h;
     if (pitch < (size_t) w * channels) return DCTC_ERR_INVALID;
     CK(ctx, cudaSetDevice(ctx->device));
     uint8_t* d = nullptr;
@@ -1559,7 +1648,7 @@ int dctc_carver_paint_seams(dctc_context* ctx, uint8_t* img, int channels, size_
     CK(ctx, cudaMalloc((void**) &d, dp * h));
     cudaError_t e = cudaMemcpy2DAsync(d, dp, img, pitch, (size_t) w * channels, h, cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) {
-        dctc_paint_seams_kernel<<<dim3((w + 255) / 256, h), 256, 0, ctx->stream>>>(d, dp, channels, w, h, ctx->c_vs, ctx->c_vs_depth);
+        dctc_paint_seams_kernel<<<dim3((w + 255) / 256, h), 256, 0, ctx->stream>>>(d, dp, channels, w, h, f->vs, f->depth);
         e = cudaGetLastError();
         ctx->launches++;
     }
@@ -1576,11 +1665,16 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
     (void) rw;
     DctcCarverEnergyParams* p = (DctcCarverEnergyParams*) extra_data;
     dctc_context* ctx = p ? p->gpu : nullptr;
-    if (!ctx || !ctx->c_img || w != ctx->c_w || h != ctx->c_h || x < 0 || y < 0 || x >= w || y >= h) {
+    if (!ctx || !ctx->carver || w != ctx->carver->w || h != ctx->carver->h || x < 0 || y < 0 || x >= w || y >= h) {
         if (ctx) ctx->last_cuda = 0;
         return __builtin_nanf("");
     }
     if (!ctx->mirror_valid) {
+        // (sized at the first use: the session only gets narrower until the next load or enlarge, which free it)
+        if (!ctx->h_mirror) {
+            const cudaError_t e = cudaMallocHost((void**) &ctx->h_mirror, sizeof(float) * (size_t) w * h);
+            if (e != cudaSuccess) { ctx->h_mirror = nullptr; dctc_fail_cuda(ctx, e); return __builtin_nanf(""); }
+        }
         if (dctc_carver_energy(ctx, ctx->h_mirror) != DCTC_OK) return __builtin_nanf("");
         ctx->mirror_valid = true;
     }
@@ -1590,216 +1684,54 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
 }  // extern "C"
 
 // ---- batch session: n equally sized frames through one device seam loop ---------------------------------------------
-// The kernels of the loop above take the frame from a spare grid dimension, so one launch per phase serves every frame
-// and each frame's seam DP runs on its own cluster of DP_CL CTAs (a single 1080p frame keeps 8 of 148 SMs busy).  The
-// session owns its device buffers and never touches the context's single-frame session; it uses the context's device,
-// stream and launch counter, and the operator / kernel selection the context had when the frames were loaded.
-// Per frame: image, energy plane, cumulative plane and jump plane (frame f of each at f * its frame stride), h seam
-// columns, one last-row column slot, and the visibility maps when requested.  The cumulative map is always rebuilt.
+// The batch owns its frames and never touches the context's single session; it uses the context's device, stream and
+// launch counter, and the operator / kernel selection the context had when the frames were loaded.  The cumulative map is
+// always rebuilt (incremental mode is a single-session option).
 struct dctc_carver_batch {
     dctc_context* ctx = nullptr;
-    int n = 0, w0 = 0, w = 0, h = 0, ch = 0;
+    CarverFrames f;
+    DctcK1Op op;                        // the context's operator at load time, with the carver's kernel rule (carver_op)
     bool dump_vmaps = false, loaded = false;
-    int blocksize = 8, kernel = DCTC_KERNEL_AUTO;   // the context's operator and kernel selection at load time
-    float edges = 0.5f, textures = 0.5f;
-    size_t pitch = 0, img_fs = 0;       // image: bytes per row, per frame
-    size_t en_pitch = 0, m_pitch = 0;   // energy / cumulative planes: floats per row (frames pitch * h floats apart)
-    uint8_t* img = nullptr;
-    float* en = nullptr;
-    float* m = nullptr;
-    int8_t* dir = nullptr;              // jump planes of the parallel back-track
-    size_t dir_fs = 0;
-    int* seam = nullptr;                // n * h: the seam each frame is removing
-    int* xlast = nullptr;               // n: last-row column of each frame's seam
-    int* seam_log = nullptr;            // n * n_seams * h of the current dctc_carver_batch_resize_width call, frame-major
-    size_t seam_log_cap = 0;
-    int* raw = nullptr;                 // n * w0 * h: original column of every current pixel
-    int* vs = nullptr;                  // n * w0 * h: removal order of every original pixel (without dump_vmaps: the
-                                        // enlarge's, allocated by the first enlarge)
-    int depth = 0;
-    // dctc_carver_batch_enlarge_width: a copy of the start frames (frames img_fs bytes apart) and the enlarged frames
-    // (wide_w = w0 + n_seams wide, frames wide_pitch * h bytes / wide_en_pitch * h floats apart).  Allocated by the first
-    // enlarge and kept for the next (the enlarged planes are reallocated when n_seams changes), freed by the destroy.
+    // dctc_carver_batch_enlarge_width: a copy of the start frames and the enlarged frames (images and energy planes).
+    // Allocated by the first enlarge and kept for the next (the enlarged frames are reallocated when n_seams changes),
+    // freed by the destroy.
     bool enlarged = false;              // the current frames are the enlarged ones
     uint8_t* start_img = nullptr;
-    uint8_t* wide_img = nullptr;
-    float* wide_en = nullptr;
-    int wide_w = 0;
-    size_t wide_pitch = 0, wide_en_pitch = 0;
+    CarverFrames wide;
 };
 
 namespace {
 
-// dctc_run_k1 reads the operator from the context: swap the batch's in for the duration of a call
-struct BatchParams {
-    dctc_context* ctx;
-    int blocksize, kernel;
-    float edges, textures;
-    BatchParams(dctc_carver_batch* b)
-        : ctx(b->ctx), blocksize(b->ctx->blocksize), kernel(b->ctx->kernel), edges(b->ctx->edges), textures(b->ctx->textures)
-    {
-        ctx->blocksize = b->blocksize; ctx->kernel = b->kernel; ctx->edges = b->edges; ctx->textures = b->textures;
-    }
-    ~BatchParams() { ctx->blocksize = blocksize; ctx->kernel = kernel; ctx->edges = edges; ctx->textures = textures; }
-};
+const CarverFrames& batch_frames(const dctc_carver_batch* b) { return b->enlarged ? b->wide : b->f; }
 
 void batch_free(dctc_carver_batch* b)
 {
-    cudaFree(b->img); cudaFree(b->en); cudaFree(b->m); cudaFree(b->dir); cudaFree(b->seam); cudaFree(b->xlast);
-    cudaFree(b->seam_log); cudaFree(b->raw); cudaFree(b->vs);
-    cudaFree(b->start_img); cudaFree(b->wide_img); cudaFree(b->wide_en);
+    frames_free(b->f);
+    frames_free(b->wide);
+    cudaFree(b->start_img);
 }
 
-int batch_alloc(dctc_carver_batch* b)
-{
-    dctc_context* ctx = b->ctx;
-    const size_t n = (size_t) b->n, h = (size_t) b->h;
-    CK(ctx, cudaMalloc((void**) &b->img, b->img_fs * n));
-    CK(ctx, cudaMalloc((void**) &b->en, sizeof(float) * b->en_pitch * h * n));
-    CK(ctx, cudaMemsetAsync(b->en, 0, sizeof(float) * b->en_pitch * h * n, ctx->stream));
-    CK(ctx, cudaMalloc((void**) &b->m, sizeof(float) * b->m_pitch * h * n));
-    CK(ctx, cudaMemsetAsync(b->m, 0, sizeof(float) * b->m_pitch * h * n, ctx->stream));
-    CK(ctx, cudaMalloc((void**) &b->seam, sizeof(int) * h * n));
-    CK(ctx, cudaMalloc((void**) &b->xlast, sizeof(int) * n));
-    CK(ctx, cudaMemsetAsync(b->xlast, 0, sizeof(int) * n, ctx->stream));
-    if (b->dump_vmaps) {
-        CK(ctx, cudaMalloc((void**) &b->raw, sizeof(int) * (size_t) b->w0 * h * n));
-        CK(ctx, cudaMalloc((void**) &b->vs, sizeof(int) * (size_t) b->w0 * h * n));
-    }
-    const BtPlan bt = bt_plan(b->h, b->m_pitch);
-    b->dir_fs = (size_t) bt.nb * bt.j_pitch;
-    if (bt.par) CK(ctx, cudaMalloc((void**) &b->dir, b->dir_fs * n));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
-}
-
-// full energy map of every frame of w x h pixels (images at img, energy planes at en, frames h rows apart) in one K1
-// launch (the FP32 kernels of the single session: see carver_full_energy)
-int batch_full_energy(dctc_carver_batch* b, const uint8_t* img, size_t pitch, int w, float* en, size_t en_pitch)
-{
-    dctc_context* ctx = b->ctx;
-    DctcK1Args a;
-    memset(&a, 0, sizeof(a));
-    a.img = img; a.pitch = pitch; a.w = w; a.h = b->h; a.channels = b->ch;
-    a.out = en; a.out_pitch = en_pitch;
-    a.frame_stride = pitch * b->h; a.out_frame_stride = en_pitch * b->h;
-    if (ctx->kernel == DCTC_KERNEL_AUTO || ctx->kernel == DCTC_KERNEL_TC_SPLIT || ctx->kernel == DCTC_KERNEL_FP32_STREAM) ctx->kernel = DCTC_KERNEL_FP32_MARCH;
-    return dctc_run_k1(ctx, a, b->n, ctx->stream);   // (the caller's BatchParams restores the kernel selection)
-}
-
-// empty visibility maps (w0 * h ints per frame) and the identity column map raw[frame][y][x] = x
-int batch_vmaps_reset(dctc_carver_batch* b, int* raw, int* vs)
-{
-    dctc_context* ctx = b->ctx;
-    const size_t nv = (size_t) b->w0 * b->h * b->n;
-    CK(ctx, cudaMemsetAsync(vs, 0, sizeof(int) * nv, ctx->stream));
-    dctc_iota_rows_kernel<<<(unsigned) ((nv + 255) / 256), 256, 0, ctx->stream>>>(raw, b->w0, b->h * b->n);
-    CK(ctx, cudaGetLastError());
-    ctx->launches++;
-    b->depth = 0;
-    return DCTC_OK;
-}
-
-// The device seam loop of every frame: removes n_seams seams from the images and energy planes (b->w shrinks by n_seams)
-// and, when raw / vs are given (maps as batch_vmaps_reset leaves them), records each removed pixel's order in vs.  The
-// caller has checked the width and holds a BatchParams scope.
-int batch_seam_loop(dctc_carver_batch* b, int n_seams, int* seams_out, int* raw, int* vs)
-{
-    dctc_context* ctx = b->ctx;
-    const int n = b->n, h = b->h;
-    const int r = ctx->blocksize / 2, bs = band_stride(ctx);
-    const size_t log_fs = (size_t) n_seams * h;
-    if (b->seam_log_cap < log_fs * n) {
-        cudaFree(b->seam_log);
-        b->seam_log = nullptr; b->seam_log_cap = 0;
-        CK(ctx, cudaMalloc((void**) &b->seam_log, sizeof(int) * log_fs * n));
-        b->seam_log_cap = log_fs * n;
-    }
-    const size_t en_fs = b->en_pitch * h, m_fs = b->m_pitch * h;
-    DpPlan plan;
-    CK(ctx, dp_plan(b->w, h, b->en, b->en_pitch, n, plan));
-    BtPlan bt = bt_plan(h, b->m_pitch);
-    bt.par = bt.par && b->dir;
-    if (bt.par && bt.cone_smem > 40 * 1024)
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
-    int* const xlast = bt.par ? b->xlast : nullptr;
-    const bool pdl = !getenv("DCTC_NO_PDL");
-    for (int s = 0; s < n_seams; s++) {
-        const int w_old = b->w;
-        int* log_s = b->seam_log + (size_t) s * h;
-        // build_mmap + build_vpath, one cluster per frame, then the jump maps and traces of all frames
-        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl, b->en, b->en_pitch, w_old, h,
-                                b->m, b->m_pitch, b->seam, log_s, (int*) nullptr, plan.nst, plan.tmap, plan.use_tmap, xlast, en_fs, m_fs, log_fs));
-        if (bt.par) {
-            const int js = (w_old + 63) / 64;
-            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, b->m, b->m_pitch,
-                                    w_old, h, b->dir, bt.j_pitch, js, m_fs, b->dir_fs));
-            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, b->m, b->m_pitch,
-                                    w_old, h, b->dir, bt.j_pitch, b->xlast, b->seam, log_s, m_fs, b->dir_fs, log_fs));
-            ctx->launches += 2;
-        }
-        if (vs) {   // update_vsmap
-            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, raw, vs, b->w0, b->seam, w_old,
-                                    ++b->depth));
-            ctx->launches++;
-        }
-        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, b->img, b->pitch, b->ch, b->en,
-                                b->en_pitch, b->seam, w_old, (float*) nullptr, b->m_pitch, b->img_fs, en_fs, (size_t) 0));
-        ctx->launches += 2;
-        b->w = w_old - 1;
-        // update_emap: band K1 around every frame's removed seam (the band values are not read back)
-        DctcK1Args a;
-        memset(&a, 0, sizeof(a));
-        a.img = b->img; a.pitch = b->pitch; a.w = b->w; a.h = h; a.channels = b->ch;
-        a.out = b->en; a.out_pitch = b->en_pitch;
-        a.frame_stride = b->img_fs; a.out_frame_stride = en_fs;
-        a.seam = b->seam; a.seam_frame_stride = h; a.band_r = r; a.band_stride = bs;
-        a.pdl = pdl ? 1 : 0;
-        const int rc = dctc_run_k1(ctx, a, n, ctx->stream);
-        if (rc) return rc;
-    }
-    if (seams_out)
-        CK(ctx, cudaMemcpyAsync(seams_out, b->seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
-}
-
-// Device work of dctc_carver_batch_enlarge_width: the start frames are copied to start_img, the seam loop runs on the
-// batch's planes with visibility maps, the inflate kernel writes the enlarged frames and K1 their full energy maps.
+// Device work of dctc_carver_batch_enlarge_width
 int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
     dctc_context* ctx = b->ctx;
-    const size_t n = (size_t) b->n, h = (size_t) b->h, nv = (size_t) b->w0 * h * n;
-    const int w1 = b->w0 + n_seams;
-    if (!b->start_img) CK(ctx, cudaMalloc((void**) &b->start_img, b->img_fs * n));
-    if (!b->raw) CK(ctx, cudaMalloc((void**) &b->raw, sizeof(int) * nv));
-    if (!b->vs) CK(ctx, cudaMalloc((void**) &b->vs, sizeof(int) * nv));
-    if (b->wide_w != w1) {
-        cudaFree(b->wide_img); cudaFree(b->wide_en);
-        b->wide_img = nullptr; b->wide_en = nullptr; b->wide_w = 0;
-        b->wide_pitch = ((size_t) w1 * b->ch + 15) & ~(size_t) 15;
-        b->wide_en_pitch = ((size_t) w1 + 3) & ~(size_t) 3;
-        CK(ctx, cudaMalloc((void**) &b->wide_img, b->wide_pitch * h * n));
-        CK(ctx, cudaMalloc((void**) &b->wide_en, sizeof(float) * b->wide_en_pitch * h * n));
-        b->wide_w = w1;
+    CarverFrames& f = b->f;
+    const int w1 = f.w0 + n_seams;
+    if (!b->start_img) CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
+    if (b->wide.w0 != w1) {
+        frames_free(b->wide);
+        frames_init(b->wide, f.n, w1, f.h, f.ch);
+        const int rc = frames_alloc(ctx, b->wide);
+        if (rc) {
+            frames_free(b->wide);
+            return rc;
+        }
     }
-    CK(ctx, cudaMemcpyAsync(b->start_img, b->img, b->img_fs * n, cudaMemcpyDeviceToDevice, ctx->stream));
     if (!b->dump_vmaps) {   // (a batch with dump_vmaps had its maps reset by the load, and no seam was removed since)
-        const int rc = batch_vmaps_reset(b, b->raw, b->vs);
+        const int rc = frames_vmaps(ctx, f);
         if (rc) return rc;
     }
-    BatchParams scope(b);
-    int rc = batch_seam_loop(b, n_seams, seams_out, b->raw, b->vs);
-    if (rc) return rc;
-    // every pixel of those seams doubled, all frames in one launch
-    dctc_inflate_rows_kernel<<<dim3(b->h, b->n), 256, 0, ctx->stream>>>(b->start_img, b->pitch, b->ch, b->w0, b->vs, n_seams, b->wide_img,
-                                                                        b->wide_pitch, b->img_fs, (size_t) b->w0 * h, b->wide_pitch * h);
-    CK(ctx, cudaGetLastError());
-    ctx->launches++;
-    rc = batch_full_energy(b, b->wide_img, b->wide_pitch, w1, b->wide_en, b->wide_en_pitch);
-    if (rc) return rc;
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    return frames_enlarge(ctx, f, b->op, n_seams, seams_out, nullptr, b->start_img, b->wide);
 }
 
 }  // namespace
@@ -1816,13 +1748,13 @@ int dctc_carver_batch_create(dctc_context* ctx, int n_frames, int w, int h, int 
     dctc_carver_batch* b = new (std::nothrow) dctc_carver_batch;
     if (!b) return DCTC_ERR_NOMEM;
     b->ctx = ctx;
-    b->n = n_frames; b->w0 = b->w = w; b->h = h; b->ch = channels;
     b->dump_vmaps = dump_vmaps != 0;
-    b->pitch = ((size_t) w * channels + 15) & ~(size_t) 15;
-    b->img_fs = b->pitch * h;
-    b->en_pitch = ((size_t) w + 3) & ~(size_t) 3;
-    b->m_pitch = b->en_pitch < (size_t) DP_WIN ? (size_t) DP_WIN : b->en_pitch;   // back-track windows stay inside
-    const int rc = batch_alloc(b);
+    frames_init(b->f, n_frames, w, h, channels);
+    int rc = frames_alloc(ctx, b->f);
+    if (rc == DCTC_OK) {
+        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+    }
     if (rc) {
         batch_free(b);
         delete b;
@@ -1843,45 +1775,41 @@ void dctc_carver_batch_destroy(dctc_carver_batch* b)
 int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t frame_stride, size_t pitch)
 {
     if (!b || !imgs) return DCTC_ERR_INVALID;
-    const size_t row = (size_t) b->w0 * b->ch;
-    if (pitch < row || (b->n > 1 && frame_stride < pitch * b->h)) return DCTC_ERR_INVALID;
+    CarverFrames& f = b->f;
+    const size_t row = (size_t) f.w0 * f.ch;
+    if (pitch < row || (f.n > 1 && frame_stride < pitch * f.h)) return DCTC_ERR_INVALID;
     dctc_context* ctx = b->ctx;
-    const int bs = ctx->blocksize;
+    const int bs = ctx->op.blocksize;
     if (!(bs == 2 || bs == 4 || bs == 8 || bs == 16)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = false;
     b->enlarged = false;
-    b->blocksize = ctx->blocksize; b->kernel = ctx->kernel; b->edges = ctx->edges; b->textures = ctx->textures;
-    b->w = b->w0;
-    for (int f = 0; f < b->n; f++)
-        CK(ctx, cudaMemcpy2DAsync(b->img + (size_t) f * b->img_fs, b->pitch, imgs + (size_t) f * frame_stride, pitch, row, b->h,
+    b->op = carver_op(ctx->op);
+    f.w = f.w0;
+    for (int i = 0; i < f.n; i++)
+        CK(ctx, cudaMemcpy2DAsync(f.img + (size_t) i * f.img_fs, f.pitch, imgs + (size_t) i * frame_stride, pitch, row, f.h,
                                   cudaMemcpyDefault, ctx->stream));
-    int rc = b->dump_vmaps ? batch_vmaps_reset(b, b->raw, b->vs) : DCTC_OK;
-    if (rc) return rc;
-    {
-        BatchParams scope(b);
-        rc = batch_full_energy(b, b->img, b->pitch, b->w, b->en, b->en_pitch);
-    }
+    int rc = b->dump_vmaps ? frames_vmaps(ctx, f) : DCTC_OK;
+    if (rc == DCTC_OK) rc = frames_full_energy(ctx, f, b->op);
     if (rc) return rc;
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = true;
     return DCTC_OK;
 }
 
-int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? b->w : 0; }
+int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? batch_frames(b).w : 0; }
 
 int dctc_carver_batch_resize_width(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
     if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= b->w) return DCTC_ERR_STATE;
-    if (b->w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
+    if (n_seams >= b->f.w) return DCTC_ERR_STATE;
+    if (b->f.w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
     dctc_context* ctx = b->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
-    BatchParams scope(b);
-    return batch_seam_loop(b, n_seams, seams_out, b->dump_vmaps ? b->raw : nullptr, b->dump_vmaps ? b->vs : nullptr);
+    return seam_loop(ctx, b->f, b->op, n_seams, seams_out, b->dump_vmaps, nullptr);
 }
 
 int dctc_carver_batch_enlarge_width(dctc_carver_batch* b, int n_seams, int* seams_out)
@@ -1889,8 +1817,8 @@ int dctc_carver_batch_enlarge_width(dctc_carver_batch* b, int n_seams, int* seam
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
     if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= b->w || b->w != b->w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
-    if (b->w > DP_CL * DP_MAXW * (512 - 2 * DP_R)) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
+    if (n_seams >= b->f.w || b->f.w != b->f.w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
+    if (b->f.w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
     dctc_context* ctx = b->ctx;
     CK(ctx, cudaSetDevice(ctx->device));
     // the seam loop carves the loaded frames in place: until every frame is enlarged the batch is not loaded, so that a
@@ -1898,7 +1826,6 @@ int dctc_carver_batch_enlarge_width(dctc_carver_batch* b, int n_seams, int* seam
     b->loaded = false;
     const int rc = batch_enlarge(b, n_seams, seams_out);
     if (rc) return rc;
-    b->w = b->w0 + n_seams;
     b->enlarged = true;
     b->loaded = true;
     return DCTC_OK;
@@ -1908,41 +1835,23 @@ int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
     if (!b->loaded) return DCTC_ERR_STATE;
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const size_t rb = (size_t) b->w * b->ch;   // frames are pitch * h bytes apart: n * h rows of one pitch
-    const uint8_t* img = b->enlarged ? b->wide_img : b->img;
-    const size_t pitch = b->enlarged ? b->wide_pitch : b->pitch;
-    CK(ctx, cudaMemcpy2DAsync(out, rb, img, pitch, rb, (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    return frames_download(b->ctx, batch_frames(b), out, nullptr, nullptr);
 }
 
 int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
     if (!b->loaded) return DCTC_ERR_STATE;
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    const float* en = b->enlarged ? b->wide_en : b->en;
-    const size_t en_pitch = b->enlarged ? b->wide_en_pitch : b->en_pitch;
-    CK(ctx, cudaMemcpy2DAsync(out, sizeof(float) * b->w, en, sizeof(float) * en_pitch, sizeof(float) * b->w,
-                              (size_t) b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
+    return frames_download(b->ctx, batch_frames(b), nullptr, out, nullptr);
 }
 
 int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
 {
     if (!b) return DCTC_ERR_INVALID;
     if (!b->loaded || !b->dump_vmaps) return DCTC_ERR_STATE;
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (vmap_out)
-        CK(ctx, cudaMemcpyAsync(vmap_out, b->vs, sizeof(int) * (size_t) b->w0 * b->h * b->n, cudaMemcpyDeviceToHost, ctx->stream));
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    if (depth_out) *depth_out = b->depth;
-    return DCTC_OK;
+    const int rc = frames_download(b->ctx, b->f, nullptr, nullptr, vmap_out);
+    if (rc == DCTC_OK && depth_out) *depth_out = b->f.depth;
+    return rc;
 }
 
 }  // extern "C"

@@ -142,9 +142,10 @@ int dctc_energy_image_dev(dctc_context* ctx, const float* d_en, size_t en_pitch,
 int dctc_carver_energy_image(dctc_context* ctx, uint8_t* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->c_img) return DCTC_ERR_STATE;
+    const CarverFrames* f = ctx->carver;
+    if (!f) return DCTC_ERR_STATE;
     CK(ctx, cudaSetDevice(ctx->device));
-    const int w = ctx->c_w, h = ctx->c_h;
+    const int w = f->w, h = f->h;
     const size_t need = (size_t) w * h;
     if (ctx->k3_img_cap < need) {
         if (ctx->k3_img) cudaFree(ctx->k3_img);
@@ -152,7 +153,7 @@ int dctc_carver_energy_image(dctc_context* ctx, uint8_t* out)
         CK(ctx, cudaMalloc((void**) &ctx->k3_img, need));
         ctx->k3_img_cap = need;
     }
-    int rc = dctc_energy_image_dev(ctx, ctx->c_en, ctx->c_en_pitch, w, h, nullptr, ctx->k3_img, (size_t) w, 0);
+    int rc = dctc_energy_image_dev(ctx, f->en, f->en_pitch, w, h, nullptr, ctx->k3_img, (size_t) w, 0);
     if (rc) return rc;
     CK(ctx, cudaMemcpyAsync(out, ctx->k3_img, need, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
@@ -213,14 +214,12 @@ __global__ void __launch_bounds__(256) dctc_preview_normalize_kernel(const float
 
 }  // namespace
 
-int dctc_run_k1(dctc_context* ctx, DctcK1Args& a, int n_frames, cudaStream_t stream);
-
 extern "C" int dctc_preview_energy(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch,
                                    float* energy_out, uint8_t* image_out)
 {
     if (!ctx || !img || w <= 0 || h <= 0 || pitch < (size_t) w * channels) return DCTC_ERR_INVALID;
     if (!(channels == 1 || channels == 3 || channels == 4)) return DCTC_ERR_INVALID;   // convert_row_to_luminance, src/render.c:62-79
-    const int b = ctx->blocksize;
+    const int b = ctx->op.blocksize;
     if (!(b == 2 || b == 4 || b == 8 || b == 16)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     int rc = ensure_lohi(ctx);
@@ -239,8 +238,8 @@ extern "C" int dctc_preview_energy(dctc_context* ctx, const uint8_t* img, int w,
         a.out = d_en; a.out_pitch = (size_t) w;
         a.preview = 1;
         // the preview operator works on 0..255 luminance bytes and applies the weights as they are (no 1/255)
-        a.w_edges = ctx->edges; a.w_textures = ctx->textures;
-        e = dctc_launch_k1_tile(a, b, 1, ctx->edges == ctx->textures, ctx->stream);
+        a.w_edges = ctx->op.edges; a.w_textures = ctx->op.textures;
+        e = dctc_launch_k1_tile(a, b, 1, ctx->op.edges == ctx->op.textures, ctx->stream);
         if (e == cudaSuccess) ctx->launches++;
     }
     if (e == cudaSuccess && energy_out)

@@ -49,6 +49,38 @@ cudaError_t dctc_launch_synth(uint8_t* d_img, int n_frames, size_t frame_stride,
 constexpr int DCTC_SLOTS = 4;   // device staging slots of the host-buffer batch call (H2D, kernel and D2H of different frames overlap)
 constexpr int DCTC_TC_COUNTERS = 64;
 
+// The energy operator and the K1 kernel selection of a K1 launch (dctc_run_k1)
+struct DctcK1Op {
+    float edges = 0.5f, textures = 0.5f;  // defaults src/main.c:30-33
+    int blocksize = 8;
+    int kernel = DCTC_KERNEL_AUTO;
+};
+
+// Device state of a carver session: n frames of w x h pixels (w0 x h when loaded), frame f of every plane at f times the
+// plane's frame stride.  The context's single session is one of these with n = 1, a batch session (dctc_carver_batch)
+// holds one with n frames; both run the same seam loop over it (dctc_k2_carver.cu).
+struct CarverFrames {
+    int n = 0, w0 = 0, w = 0, h = 0, ch = 0;
+    size_t pitch = 0, img_fs = 0;       // image: bytes per row, per frame
+    size_t en_pitch = 0, m_pitch = 0;   // energy / cumulative planes: floats per row (multiple of 4: 16-byte aligned rows;
+                                        // m_pitch >= DP_WIN), frames pitch * h floats apart
+    uint8_t* img = nullptr;             // compacted in place per seam
+    float* en = nullptr;
+    float* m = nullptr;                 // cumulative map of the seam DP (rebuilt per seam, read back by the back-track)
+    int8_t* dir = nullptr;              // jump planes of the parallel back-track: per 32-row block and bottom column, the
+    size_t dir_fs = 0;                  // path's column offset at the block top
+    int* seam = nullptr;                // n * h: the seam each frame is removing
+    int* xlast = nullptr;               // n: last-row column of each frame's seam
+    int* seam_log = nullptr;            // n * n_seams * h of the current seam loop, frame-major
+    size_t seam_log_cap = 0;
+    // visibility maps (lqr_carver_set_dump_vmaps, src/render.c:374): raw = original column of every current pixel,
+    // vs = removal order of every original pixel (0 = never removed); vs_w x h ints per frame, only when requested
+    int* raw = nullptr;
+    int* vs = nullptr;
+    int depth = 0;
+    int vs_w = 0;                       // width of the frame the maps belong to (w0 when they were reset)
+};
+
 struct dctc_context {
     int device = 0;
     cudaStream_t stream = nullptr;      // compute
@@ -56,9 +88,7 @@ struct dctc_context {
     cudaStream_t s_out = nullptr;       // D2H
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr;
     cudaEvent_t ev_in[DCTC_SLOTS] = {}, ev_k[DCTC_SLOTS] = {}, ev_out[DCTC_SLOTS] = {};
-    float edges = 0.5f, textures = 0.5f;  // defaults src/main.c:30-33
-    int blocksize = 8;
-    int kernel = DCTC_KERNEL_AUTO;
+    DctcK1Op op;                        // dctc_set_params, dctc_set_kernel
     int last_cuda = 0;
     unsigned long long launches = 0;
     int sm_count = 0;
@@ -68,30 +98,15 @@ struct dctc_context {
     uint8_t* d_in[DCTC_SLOTS] = {};
     float* d_out[DCTC_SLOTS] = {};
     size_t d_in_cap[DCTC_SLOTS] = {}, d_out_cap[DCTC_SLOTS] = {};
-    // carver session (K2)
-    uint8_t* c_img = nullptr;      // device image, pitch c_pitch, compacted in place per seam
-    float* c_en = nullptr;         // device energy, pitch c_en_pitch floats (multiple of 4: 16-byte aligned rows)
-    size_t c_en_pitch = 0;
-    float* c_m = nullptr;          // cumulative map of the device seam DP (rebuilt per seam, read back by the back-track)
-    int8_t* c_dir = nullptr;       // jump plane of the parallel back-track: per 32-row block and bottom column, the path's column offset at the block top
-    int* c_seam_log = nullptr;     // seams of dctc_carver_resize_width, n_seams * h
-    size_t c_seam_log_cap = 0;
-    // visibility map (lqr_carver_set_dump_vmaps, src/render.c:374): raw = original column of every current pixel,
-    // vs = removal order of every original pixel (0 = never removed); both w0 x h ints, only when requested
-    int* c_raw = nullptr;
-    int* c_vs = nullptr;
-    int c_vs_depth = 0;
-    int c_vs_w = 0;                // width of the frame the visibility map belongs to (the session's width when it was requested)
-    bool c_dump_vmaps = false;
-    int* c_seam = nullptr;         // h entries
-    int* c_band = nullptr;         // c_band[0]: 'rebuild the cumulative map from scratch' flag of the incremental seam DP; c_band[4]: last-row column of the current seam (device)
+    // carver session (K2): one frame, null when nothing is loaded; the single-session-only state follows
+    CarverFrames* carver = nullptr;
+    bool c_dump_vmaps = false;     // record the visibility map in the next seam loops (lqr_carver_set_dump_vmaps)
+    int* c_band = nullptr;         // c_band[0]: 'rebuild the cumulative map from scratch' flag of the incremental seam DP, c_band[1]: rebuilds (device)
     bool c_incremental = false;    // device seam loop: update the cumulative map incrementally (dctc_carver_set_incremental)
     bool c_m_valid = false;        // the cumulative plane holds the map of the image before the last removal, compacted over that seam
-    float* c_band_vals = nullptr;  // packed band values
-    float* h_mirror = nullptr;     // host mirror of the energy map (pinned)
-    int* h_band = nullptr;         // pinned 2*h
-    int c_w0 = 0, c_w = 0, c_h = 0, c_ch = 0;
-    size_t c_pitch = 0;
+    float* c_band_vals = nullptr;  // packed band values of dctc_carve_and_update
+    float* h_mirror = nullptr;     // host mirror of the energy map for dctc_pixel_energy (pinned, allocated by its first use)
+    int* h_band = nullptr;         // pinned: band values and seam of dctc_carve_and_update
     bool mirror_valid = false;
     // K3 energy-image export
     unsigned int* k3_lohi = nullptr;   // device (min, max) of the compressed energies, as float bit patterns
@@ -100,5 +115,6 @@ struct dctc_context {
 };
 
 int dctc_fail_cuda(dctc_context* ctx, cudaError_t e);
+int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream);
 void dctc_carver_release(dctc_context* ctx);
 int dctc_carver_params_changed(dctc_context* ctx);   // rebuilds the resident energy map of a loaded carver session

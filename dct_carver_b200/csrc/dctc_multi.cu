@@ -123,7 +123,7 @@ static size_t band_pitch(int w, int ch) { return ((size_t) w * ch + 15) & ~(size
 static int band_alloc(DctcBand& b, dctc_context* ctx, int w, int h, int ch, int rank, int world)
 {
     b.ctx = ctx; b.w = w; b.h = h; b.ch = ch;
-    int rc = dctc_band_plan(h, world, rank, ctx->blocksize, &b.y0, &b.rows, &b.top_need, &b.bot_need);
+    int rc = dctc_band_plan(h, world, rank, ctx->op.blocksize, &b.y0, &b.rows, &b.top_need, &b.bot_need);
     if (rc) return rc;
     b.pitch = band_pitch(w, ch);
     CK(ctx, cudaSetDevice(ctx->device));
