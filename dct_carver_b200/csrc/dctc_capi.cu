@@ -5,12 +5,7 @@
 #include <new>
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
-
-#define CK(ctx, call)                                             \
-    do {                                                          \
-        cudaError_t e_ = (call);                                  \
-        if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
-    } while (0)
+#include "dctc_k1_select.h"
 
 int dctc_fail_cuda(dctc_context* ctx, cudaError_t e)
 {
@@ -19,8 +14,6 @@ int dctc_fail_cuda(dctc_context* ctx, cudaError_t e)
     if (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver) return DCTC_ERR_NO_DEVICE;
     return DCTC_ERR_CUDA;
 }
-
-static bool valid_blocksize(int b) { return b == 2 || b == 4 || b == 8 || b == 16; }
 
 static int check_image(int w, int h, int channels, size_t pitch)
 {
@@ -120,7 +113,7 @@ void dctc_destroy(dctc_context* ctx)
 int dctc_set_params(dctc_context* ctx, const DctcEnergyParameters* p)
 {
     if (!ctx || !p) return DCTC_ERR_INVALID;
-    if (!valid_blocksize(p->blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(p->blocksize)) return DCTC_ERR_BLOCKSIZE;
     if (!(std::isfinite(p->edges) && std::isfinite(p->textures))) return DCTC_ERR_INVALID;
     const bool changed = ctx->op.edges != p->edges || ctx->op.textures != p->textures || ctx->op.blocksize != p->blocksize;
     ctx->op.edges = p->edges;
@@ -149,6 +142,13 @@ unsigned long long dctc_launch_count(const dctc_context* ctx) { return ctx ? ctx
 
 // ---- K1 dispatch ------------------------------------------------------------------------------------------
 
+bool dctc_k1_fast_layout(const DctcK1Args& a)
+{
+    auto aligned16 = [](const void* p, size_t pitch) { return (((uintptr_t) p | pitch) & 15) == 0; };
+    return (a.channels == 3 || a.channels == 1) && aligned16(a.img, a.pitch) && (a.frame_stride & 15) == 0 &&
+           (!a.top || aligned16(a.top, a.top_pitch)) && (!a.bot || aligned16(a.bot, a.bot_pitch));
+}
+
 // The context supplies the device, the tensor-core counters and the launch counter; op the operator and kernel selection.
 int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream)
 {
@@ -156,39 +156,15 @@ int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_fram
     a.w_edges = (float) ((double) op.edges / 255.0);
     a.w_textures = (float) ((double) op.textures / 255.0);
     const bool uniform = op.edges == op.textures;
-    int kernel = op.kernel;
-    // band mode (per-seam update) always runs in the tile kernel; block size 8 full maps default to the tensor-core
-    // kernel (which hands configurations outside its fast path to the FP32 march kernel)
-    if (a.seam || op.blocksize != 8) {
-        kernel = DCTC_KERNEL_FP32_TILE;   // block sizes 2, 4, 16 pick their fast path below
-    } else if (kernel == DCTC_KERNEL_AUTO) {
-        kernel = DCTC_KERNEL_TC_SPLIT;
-    } else if (kernel == DCTC_KERNEL_FP32_STREAM) {
-        kernel = DCTC_KERNEL_FP32_MARCH;  // block size 8 has no streaming kernel: its register-march kernel
-    }
-    cudaError_t e;
-    switch (kernel) {
-    case DCTC_KERNEL_FP32_TILE:
-        // block sizes 2 and 4 (HBM-bound): full maps stream through the register-march kernel unless the tile kernel was
-        // asked for explicitly; both produce bit-identical maps
-        e = cudaErrorNotSupported;
-        if ((op.kernel == DCTC_KERNEL_AUTO || op.kernel == DCTC_KERNEL_FP32_STREAM) && !a.seam && !a.preview &&
-            (op.blocksize == 2 || op.blocksize == 4))
-            e = dctc_launch_k1_small(a, op.blocksize, n_frames, uniform, ctx->sm_count, stream);
-        // block size 16 (compute-bound): full maps run their y-pass on the tensor cores unless the FP32 tile kernel was
-        // asked for explicitly (or the configuration is outside the tensor-core fast path)
-        if (op.kernel != DCTC_KERNEL_FP32_TILE && op.kernel != DCTC_KERNEL_FP32_MARCH && !a.seam && !a.preview && op.blocksize == 16)
-            e = dctc_launch_k1_tc16(a, n_frames, uniform, ctx->tc_counters + (ctx->tc_next++ % DCTC_TC_COUNTERS), ctx->sm_count, stream);
-        if (e == cudaErrorNotSupported) e = dctc_launch_k1_tile(a, op.blocksize, n_frames, uniform, stream);
-        break;
-    case DCTC_KERNEL_FP32_MARCH: e = dctc_launch_k1_march8(a, n_frames, uniform, stream); break;
-    case DCTC_KERNEL_TC_SPLIT:
-        // every launch takes its own work-item counter, so launches in flight on different streams never share one
-        e = dctc_launch_k1_tc8(a, n_frames, uniform, ctx->tc_counters + (ctx->tc_next++ % DCTC_TC_COUNTERS), ctx->sm_count, stream);
-        // outside the tensor-core fast path (channel count / alignment): same operator on the FP32 march kernel
-        if (e == cudaErrorNotSupported) e = dctc_launch_k1_march8(a, n_frames, uniform, stream);
-        break;
-    default: return DCTC_ERR_UNSUPPORTED;
+    // every tensor-core launch takes its own work-item counter, so launches in flight on different streams never share one
+    auto counter = [ctx] { return ctx->tc_counters + (ctx->tc_next++ % DCTC_TC_COUNTERS); };
+    cudaError_t e = cudaSuccess;
+    switch (dctc_k1_select(op.kernel, op.blocksize, a.seam != nullptr, a.preview != 0, dctc_k1_fast_layout(a))) {
+    case DctcK1Variant::Tile: e = dctc_launch_k1_tile(a, op.blocksize, n_frames, uniform, stream); break;
+    case DctcK1Variant::Small: e = dctc_launch_k1_small(a, op.blocksize, n_frames, uniform, ctx->sm_count, stream); break;
+    case DctcK1Variant::March8: e = dctc_launch_k1_march8(a, n_frames, uniform, stream); break;
+    case DctcK1Variant::Tc8: e = dctc_launch_k1_tc8(a, n_frames, uniform, counter(), ctx->sm_count, stream); break;
+    case DctcK1Variant::Tc16: e = dctc_launch_k1_tc16(a, n_frames, uniform, counter(), ctx->sm_count, stream); break;
     }
     if (e != cudaSuccess) return dctc_fail_cuda(ctx, e);
     ctx->launches++;
@@ -236,7 +212,7 @@ int dctc_energy_batch_dev(dctc_context* ctx, const uint8_t* d_imgs, int n_frames
     int rc = check_image(w, h, channels, pitch);
     if (rc) return rc;
     if (out_pitch < (size_t) w) return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     // grid.z carries the frame index: split very large batches
     for (int f0 = 0; f0 < n_frames; f0 += 32768) {
@@ -272,7 +248,7 @@ int dctc_energy_band_dev_at(dctc_context* ctx, const uint8_t* d_band, int w, int
     if ((top_rows > 0 && (!d_top || top_pitch < (size_t) w * channels)) ||
         (bot_rows > 0 && (!d_bot || bot_pitch < (size_t) w * channels)))
         return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     DctcK1Args a;
     plain_args(a, d_band, w, band_rows, channels, pitch, d_out, out_pitch);
@@ -299,7 +275,7 @@ int dctc_energy_batch(dctc_context* ctx, const uint8_t* imgs, int n_frames, size
     int rc = check_image(w, h, channels, pitch);
     if (rc) return rc;
     if (n_frames > 1 && (frame_stride < pitch * (size_t) h || out_frame_stride < (size_t) w * h)) return DCTC_ERR_INVALID;
-    if (!valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     const size_t row_bytes = (size_t) w * channels;
     const size_t d_pitch = (row_bytes + 15) & ~(size_t) 15;

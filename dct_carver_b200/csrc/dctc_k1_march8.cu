@@ -282,10 +282,10 @@ __global__ void __launch_bounds__(MW, 4) dctc_k1_march8_kernel(const DctcK1Args 
 
 }  // namespace
 
+// Full maps (no band / preview mode) in any layout
 cudaError_t dctc_launch_k1_march8(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
-    if (a.seam) return cudaErrorInvalidValue;  // band mode lives in the tile kernel
     const int strips = (a.w + MW - 1) / MW;
     // segment height: long segments amortise the 7-row prologue, short ones fill the machine for small inputs
     int seg = 128;
@@ -293,14 +293,9 @@ cudaError_t dctc_launch_k1_march8(const DctcK1Args& a, int n_frames, bool unifor
     const int segs = (a.h + seg - 1) / seg;
     if (segs > 65535 || n_frames > 65535) return cudaErrorInvalidConfiguration;
     dim3 grid(strips, segs, n_frames), block(MW);
-    // fast path: rows readable for `pitch` bytes, all row pointers 16-byte aligned
-    auto aligned16 = [](const void* p, size_t pitch) { return (((uintptr_t) p | pitch) & 15) == 0; };
-    const bool fast = (a.channels == 3 || a.channels == 1) && aligned16(a.img, a.pitch) && (a.frame_stride & 15) == 0 &&
-                      (!a.top || aligned16(a.top, a.top_pitch)) && (!a.bot || aligned16(a.bot, a.bot_pitch));
-#define DCTC_MARCH_LAUNCH(U, C) dctc_k1_march8_kernel<U, C><<<grid, block, 0, stream>>>(a, seg)
-    if (fast && a.channels == 3) { if (uniform) DCTC_MARCH_LAUNCH(true, 3); else DCTC_MARCH_LAUNCH(false, 3); }
-    else if (fast) { if (uniform) DCTC_MARCH_LAUNCH(true, 1); else DCTC_MARCH_LAUNCH(false, 1); }
-    else { if (uniform) DCTC_MARCH_LAUNCH(true, 0); else DCTC_MARCH_LAUNCH(false, 0); }
-#undef DCTC_MARCH_LAUNCH
-    return cudaGetLastError();
+    // C = 3 / 1 in the fast layout (rows readable for `pitch` bytes, all row pointers 16-byte aligned), else generic C = 0
+    return dctc_dispatch<3, 1, 0>(uniform, dctc_k1_fast_layout(a) ? a.channels : 0, [&](auto U, auto C) {
+        dctc_k1_march8_kernel<U, C><<<grid, block, 0, stream>>>(a, seg);
+        return cudaGetLastError();
+    });
 }

@@ -418,28 +418,17 @@ cudaError_t launch_small(const DctcK1Args& a, int n_frames, bool uniform, int sm
     // 64-bit stores need 8-byte aligned output rows
     const int vec_ok = (((uintptr_t) a.out & 7) == 0 && (a.out_pitch & 1) == 0 && (a.out_frame_stride & 1) == 0) ? 1 : 0;
     dim3 grid(strips, segs, n_frames), block(NT);
-#define DCTC_SMALL_LAUNCH(U, C)                                                                                        \
-    do {                                                                                                               \
-        cudaError_t el = dctc_launch_pdl(dctc_k1_small_kernel<B, U, C>, grid, block, 0, stream, true, a, seg, vec_ok); \
-        if (el != cudaSuccess) return el;                                                                              \
-    } while (0)
-    if (a.channels == 3) { if (uniform) DCTC_SMALL_LAUNCH(true, 3); else DCTC_SMALL_LAUNCH(false, 3); }
-    else { if (uniform) DCTC_SMALL_LAUNCH(true, 1); else DCTC_SMALL_LAUNCH(false, 1); }
-#undef DCTC_SMALL_LAUNCH
-    return cudaGetLastError();
+    const cudaError_t e = dctc_dispatch<3, 1>(uniform, a.channels, [&](auto U, auto C) {
+        return dctc_launch_pdl(dctc_k1_small_kernel<B, U, C>, grid, block, 0, stream, true, a, seg, vec_ok);
+    });
+    return e != cudaSuccess ? e : cudaGetLastError();
 }
 
 }  // namespace
 
-// Returns cudaErrorNotSupported when the configuration is outside this kernel's fast path (the caller then uses the
-// tile kernel): needs block size 2 or 4, 1 or 3 channels, 16-byte aligned row pointers / pitches, no band / preview mode.
+// Block size 2 or 4, full maps (no band / preview mode) in the fast layout (dctc_k1_fast_layout)
 cudaError_t dctc_launch_k1_small(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, int sm_count, cudaStream_t stream)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
-    if (a.seam || a.preview || (blocksize != 2 && blocksize != 4)) return cudaErrorNotSupported;
-    auto aligned16 = [](const void* p, size_t pitch) { return (((uintptr_t) p | pitch) & 15) == 0; };
-    const bool fast = (a.channels == 3 || a.channels == 1) && aligned16(a.img, a.pitch) && (a.frame_stride & 15) == 0 &&
-                      (!a.top || aligned16(a.top, a.top_pitch)) && (!a.bot || aligned16(a.bot, a.bot_pitch));
-    if (!fast) return cudaErrorNotSupported;
     return blocksize == 2 ? launch_small<2>(a, n_frames, uniform, sm_count, stream) : launch_small<4>(a, n_frames, uniform, sm_count, stream);
 }

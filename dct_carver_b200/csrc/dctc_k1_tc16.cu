@@ -572,15 +572,10 @@ __global__ void __launch_bounds__(NTHREADS, 1) dctc_k1_tc16_kernel(const DctcK1A
 
 }  // namespace
 
-// Returns cudaErrorNotSupported when the configuration is outside this kernel's fast path (the caller then uses the
-// FP32 tile kernel): needs 1 or 3 channels, 16-byte aligned rows, no band-mode (per-seam) / preview request.
+// Full maps (no band / preview mode) in the fast layout (dctc_k1_fast_layout); `counter` as for dctc_launch_k1_tc8.
 cudaError_t dctc_launch_k1_tc16(const DctcK1Args& a, int n_frames, bool uniform, int* counter, int sm_count, cudaStream_t stream)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
-    auto aligned16 = [](const void* p, size_t pitch) { return (((uintptr_t) p | pitch) & 15) == 0; };
-    const bool fast = !a.seam && !a.preview && (a.channels == 3 || a.channels == 1) && aligned16(a.img, a.pitch) &&
-                      (a.frame_stride & 15) == 0 && (!a.top || aligned16(a.top, a.top_pitch)) && (!a.bot || aligned16(a.bot, a.bot_pitch));
-    if (!fast || !counter) return cudaErrorNotSupported;
     const int strips = (a.w + PW - 1) / PW;
     const int phase = a.row_origin & 15;
     const int rows = a.h + phase;
@@ -605,15 +600,11 @@ cudaError_t dctc_launch_k1_tc16(const DctcK1Args& a, int n_frames, bool uniform,
     if (items > 0x7fffffffLL) return cudaErrorInvalidConfiguration;
     const int grid = (int) (items < ctas ? items : ctas);
     const int smem = (int) sizeof(Tc16Smem);
-#define DCTC16_LAUNCH(U, C)                                                                                            \
-    do {                                                                                                               \
-        cudaError_t ea = cudaFuncSetAttribute(dctc_k1_tc16_kernel<U, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem); \
-        if (ea != cudaSuccess) return ea;                                                                              \
-        ea = dctc_launch_pdl(dctc_k1_tc16_kernel<U, C>, dim3(grid), dim3(NTHREADS), (size_t) smem, stream, true, a, seg, strips, segs, (int) items, phase, counter); \
-        if (ea != cudaSuccess) return ea;                                                                              \
-    } while (0)
-    if (a.channels == 3) { if (uniform) DCTC16_LAUNCH(true, 3); else DCTC16_LAUNCH(false, 3); }
-    else { if (uniform) DCTC16_LAUNCH(true, 1); else DCTC16_LAUNCH(false, 1); }
-#undef DCTC16_LAUNCH
-    return cudaGetLastError();
+    const cudaError_t e = dctc_dispatch<3, 1>(uniform, a.channels, [&](auto U, auto C) {
+        const cudaError_t ea = cudaFuncSetAttribute(dctc_k1_tc16_kernel<U, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+        if (ea != cudaSuccess) return ea;
+        return dctc_launch_pdl(dctc_k1_tc16_kernel<U, C>, dim3(grid), dim3(NTHREADS), (size_t) smem, stream, true, a, seg, strips, segs,
+                               (int) items, phase, counter);
+    });
+    return e != cudaSuccess ? e : cudaGetLastError();
 }

@@ -28,7 +28,6 @@
 // Per pixel the CUDA cores execute ~120 instructions instead of the ~264 of the FP32 march kernel; the tensor pipe
 // does 24 M128 K16 MMAs per 1024 pixels (16 with N = 64: 36.3 clk each measured, profiles/r01_tcgen05_probe2.txt; 8 with
 // N = 48).  The operands of a group are announced in two halves (k1 = 0..3, 4..7).
-#include <cuda.h>       // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint, no libcuda link)
 #include <cuda_fp16.h>
 #include <cstdio>
 #include <cstring>
@@ -756,18 +755,12 @@ __global__ void __launch_bounds__(NTHREADS, 2) dctc_k1_tc8_kernel(const DctcK1Ar
 
 }  // namespace
 
-// Returns cudaErrorNotSupported when the configuration is outside this kernel's fast path (the caller then uses
-// the FP32 march kernel): needs 1 or 3 channels and 16-byte aligned row pointers / pitches.
+// Full maps (no band / preview mode) in the fast layout (dctc_k1_fast_layout).
 // `counter` is a device int owned by the context (work-item counter of the persistent kernel), zero before the launch;
 // the kernel leaves it at zero again.
 cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, int* counter, int sm_count, cudaStream_t stream)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
-    if (a.seam) return cudaErrorInvalidValue;  // band mode lives in the tile kernel
-    auto aligned16 = [](const void* p, size_t pitch) { return (((uintptr_t) p | pitch) & 15) == 0; };
-    const bool fast = (a.channels == 3 || a.channels == 1) && aligned16(a.img, a.pitch) && (a.frame_stride & 15) == 0 &&
-                      (!a.top || aligned16(a.top, a.top_pitch)) && (!a.bot || aligned16(a.bot, a.bot_pitch));
-    if (!fast || !counter) return cudaErrorNotSupported;
     const int strips = (a.w + MW - 1) / MW;
     // Segment height.  An item of S rows costs S/8 + 2 steps (two prologue groups); the 2 x sm_count resident CTAs take
     // items from a counter, so a launch lasts about ceil(items / CTAs) x (S/8 + 2) steps when the items are few, and
@@ -816,19 +809,7 @@ cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, 
     memset(&tmap, 0, sizeof(tmap));
     int use_tmap = 0;
     {
-        typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-        // looked up once (thread-safe static initialisation: dctc_multi_* launches from one host thread per device)
-        static const encode_fn encode = []() -> encode_fn {
-            void* fp = nullptr;
-            cudaDriverEntryPointQueryResult qres;
-            if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qres) == cudaSuccess && fp &&
-                qres == cudaDriverEntryPointSuccess)
-                return (encode_fn) fp;
-            (void) cudaGetLastError();
-            return nullptr;
-        }();
+        const DctcTensorMapEncodeFn encode = dctc_tensor_map_encoder();
         const size_t fstride = n_frames > 1 ? a.frame_stride : a.pitch * (size_t) a.h;
         const int row = a.channels == 3 ? RawGeom<3>::ROW : RawGeom<1>::ROW;
         if (encode && a.h >= 8 && !getenv("DCTC_TC_NO_TENSORMAP") && (fstride & 15) == 0 && fstride >= a.pitch && a.pitch < (1ull << 40) &&
@@ -842,15 +823,11 @@ cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, 
                 use_tmap = 1;
         }
     }
-#define DCTC_TC_LAUNCH(U, C)                                                                                           \
-    do {                                                                                                               \
-        cudaError_t ea = cudaFuncSetAttribute(dctc_k1_tc8_kernel<U, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, PAD_SMEM); \
-        if (ea != cudaSuccess) return ea;                                                                              \
-        ea = dctc_launch_pdl(dctc_k1_tc8_kernel<U, C>, dim3(grid), dim3(NTHREADS), PAD_SMEM, stream, true, a, seg, strips, segs, (int) items, counter, tmap, use_tmap); \
-        if (ea != cudaSuccess) return ea;                                                                              \
-    } while (0)
-    if (a.channels == 3) { if (uniform) DCTC_TC_LAUNCH(true, 3); else DCTC_TC_LAUNCH(false, 3); }
-    else { if (uniform) DCTC_TC_LAUNCH(true, 1); else DCTC_TC_LAUNCH(false, 1); }
-#undef DCTC_TC_LAUNCH
-    return cudaGetLastError();
+    const cudaError_t e = dctc_dispatch<3, 1>(uniform, a.channels, [&](auto U, auto C) {
+        const cudaError_t ea = cudaFuncSetAttribute(dctc_k1_tc8_kernel<U, C>, cudaFuncAttributeMaxDynamicSharedMemorySize, PAD_SMEM);
+        if (ea != cudaSuccess) return ea;
+        return dctc_launch_pdl(dctc_k1_tc8_kernel<U, C>, dim3(grid), dim3(NTHREADS), PAD_SMEM, stream, true, a, seg, strips, segs,
+                               (int) items, counter, tmap, use_tmap);
+    });
+    return e != cudaSuccess ? e : cudaGetLastError();
 }

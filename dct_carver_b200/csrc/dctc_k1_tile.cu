@@ -147,19 +147,13 @@ static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, 
     // band mode: a tile row spans at most (TH-1) + 4*band_r + 1 columns (seam drift over TH+2r rows plus 2r)
     const int span = a.seam ? (TH + 4 * a.band_r) : a.w;
     dim3 grid((span + TW - 1) / TW, (a.h + TH - 1) / TH, n_frames), block(TW * TH / P);
-    cudaError_t e;
-    if (uniform) {
-        e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+    return dctc_dispatch<0>(uniform, 0, [&](auto U, auto) {   // one kernel for every channel count
+        const cudaError_t e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
         if (e != cudaSuccess) return e;
-        if (a.pdl) return dctc_launch_pdl(dctc_k1_tile_kernel<B, TW, TH, P, true>, grid, block, smem, stream, true, a);
-        dctc_k1_tile_kernel<B, TW, TH, P, true><<<grid, block, smem, stream>>>(a);
-    } else {
-        e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
-        if (e != cudaSuccess) return e;
-        if (a.pdl) return dctc_launch_pdl(dctc_k1_tile_kernel<B, TW, TH, P, false>, grid, block, smem, stream, true, a);
-        dctc_k1_tile_kernel<B, TW, TH, P, false><<<grid, block, smem, stream>>>(a);
-    }
-    return cudaGetLastError();
+        if (a.pdl) return dctc_launch_pdl(dctc_k1_tile_kernel<B, TW, TH, P, U>, grid, block, smem, stream, true, a);
+        dctc_k1_tile_kernel<B, TW, TH, P, U><<<grid, block, smem, stream>>>(a);
+        return cudaGetLastError();
+    });
 }
 
 cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream)

@@ -5,7 +5,6 @@
 // within +-radius of the seam (radius = blocksize/2, registered at src/render.c:314-315).  Here the image and the
 // energy plane stay resident in HBM; one kernel compacts both over the seam, then the K1 tile kernel runs in band
 // mode over just the touched pixels, with arithmetic identical to a full recompute (bit-identical results).
-#include <cuda.h>      // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint, no libcuda link)
 #include <cstdio>
 #include <cstdlib>
 #include <type_traits>
@@ -14,12 +13,6 @@
 #include <utility>
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
-
-#define CK(ctx, call)                                             \
-    do {                                                          \
-        cudaError_t e_ = (call);                                  \
-        if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
-    } while (0)
 
 // One CTA per row: shift image bytes and energy floats right of the seam one pixel to the left.
 // Chunks are processed left to right; the barrier between a chunk's loads and its stores also orders them
@@ -1233,24 +1226,15 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
     // are its third dimension, so that a box never reaches into the next frame's rows
     memset(&p.tmap, 0, sizeof(p.tmap));
     p.use_tmap = 0;
-    if (sr > 0 && 128 * P <= 256 && !getenv("DCTC_DP_NO_TENSORMAP")) {
-        typedef CUresult (*encode_fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                      const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                      CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-        void* fp = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qres) == cudaSuccess && fp &&
-            qres == cudaDriverEntryPointSuccess) {
-            const cuuint64_t gdim[3] = {(cuuint64_t) en_pitch, (cuuint64_t) h, (cuuint64_t) n_frames};
-            const cuuint64_t gstr[2] = {(cuuint64_t) en_pitch * sizeof(float), (cuuint64_t) en_pitch * h * sizeof(float)};
-            const cuuint32_t box[3] = {(cuuint32_t) (128 * P), (cuuint32_t) sr, 1};
-            const cuuint32_t estr[3] = {1, 1, 1};
-            if (((encode_fn) fp)(&p.tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*) en, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                 CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
-                p.use_tmap = 1;
-        } else {
-            (void) cudaGetLastError();
-        }
+    const DctcTensorMapEncodeFn encode = dctc_tensor_map_encoder();
+    if (encode && sr > 0 && 128 * P <= 256 && !getenv("DCTC_DP_NO_TENSORMAP")) {
+        const cuuint64_t gdim[3] = {(cuuint64_t) en_pitch, (cuuint64_t) h, (cuuint64_t) n_frames};
+        const cuuint64_t gstr[2] = {(cuuint64_t) en_pitch * sizeof(float), (cuuint64_t) en_pitch * h * sizeof(float)};
+        const cuuint32_t box[3] = {(cuuint32_t) (128 * P), (cuuint32_t) sr, 1};
+        const cuuint32_t estr[3] = {1, 1, 1};
+        if (encode(&p.tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*) en, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
+            p.use_tmap = 1;
     }
     // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
     return cudaFuncSetAttribute(p.dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
@@ -1460,7 +1444,7 @@ int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int ch
     if (!ctx || !img || w <= 0 || h <= 0 || channels < 1 || channels > 4 || pitch < (size_t) w * channels)
         return DCTC_ERR_INVALID;
     const int b = ctx->op.blocksize;
-    if (!(b == 2 || b == 4 || b == 8 || b == 16)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(b)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     dctc_carver_release(ctx);
@@ -1780,7 +1764,7 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     if (pitch < row || (f.n > 1 && frame_stride < pitch * f.h)) return DCTC_ERR_INVALID;
     dctc_context* ctx = b->ctx;
     const int bs = ctx->op.blocksize;
-    if (!(bs == 2 || bs == 4 || bs == 8 || bs == 16)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(bs)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = false;

@@ -13,12 +13,6 @@
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
 
-#define CK(ctx, call)                                             \
-    do {                                                          \
-        cudaError_t e_ = (call);                                  \
-        if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
-    } while (0)
-
 namespace {
 
 // e >= 0 -> 1 / (1 + 1/e), IEEE divisions (1/0 = inf, 1/inf = 0): the same two roundings as the host carver
@@ -220,7 +214,7 @@ extern "C" int dctc_preview_energy(dctc_context* ctx, const uint8_t* img, int w,
     if (!ctx || !img || w <= 0 || h <= 0 || pitch < (size_t) w * channels) return DCTC_ERR_INVALID;
     if (!(channels == 1 || channels == 3 || channels == 4)) return DCTC_ERR_INVALID;   // convert_row_to_luminance, src/render.c:62-79
     const int b = ctx->op.blocksize;
-    if (!(b == 2 || b == 4 || b == 8 || b == 16)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(b)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     int rc = ensure_lohi(ctx);
     if (rc) return rc;

@@ -1,11 +1,52 @@
 // Internal: kernel launchers and the context layout shared by the C-ABI translation units.
 #pragma once
+#include <cuda.h>       // CUtensorMap (types only: the encoder is fetched with cudaGetDriverEntryPoint, no libcuda link)
 #include <cuda_runtime.h>
 #include <cstddef>
 #include <cstdint>
+#include <type_traits>
 #include "../../include/dctc.h"
 
 struct DctcK1Args;
+
+#define CK(ctx, call)                                             \
+    do {                                                          \
+        cudaError_t e_ = (call);                                  \
+        if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
+    } while (0)
+
+inline bool dctc_valid_blocksize(int b) { return b == 2 || b == 4 || b == 8 || b == 16; }
+
+// Runs f(std::integral_constant<bool, uniform>, std::integral_constant<int, C>) for the first C of the list equal to c
+// (the last C when none is): one kernel instantiation per (uniform, C) pair, picked at run time.
+template <int C, int... Cs, typename F>
+static inline cudaError_t dctc_dispatch(bool uniform, int c, F&& f)
+{
+    if constexpr (sizeof...(Cs) > 0)
+        if (c != C) return dctc_dispatch<Cs...>(uniform, c, f);
+    if (uniform) return f(std::true_type(), std::integral_constant<int, C>());
+    return f(std::false_type(), std::integral_constant<int, C>());
+}
+
+typedef CUresult (*DctcTensorMapEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                          const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                          CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+// The driver's tensor-map encoder, or null when the driver has none.  Looked up once (thread-safe static initialisation:
+// dctc_multi_* launches from one host thread per device).
+inline DctcTensorMapEncodeFn dctc_tensor_map_encoder()
+{
+    static const DctcTensorMapEncodeFn encode = []() -> DctcTensorMapEncodeFn {
+        void* fp = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fp, cudaEnableDefault, &qres) == cudaSuccess && fp &&
+            qres == cudaDriverEntryPointSuccess)
+            return (DctcTensorMapEncodeFn) fp;
+        (void) cudaGetLastError();
+        return nullptr;
+    }();
+    return encode;
+}
 
 // Programmatic dependent launch (the kernels of the device seam loop): a kernel launched with the attribute may be
 // scheduled while its predecessor in the stream is still running; its CTAs then block in DCTC_PDL_PROLOGUE until the
@@ -115,6 +156,10 @@ struct dctc_context {
 };
 
 int dctc_fail_cuda(dctc_context* ctx, cudaError_t e);
+// Launches the one K1 kernel dctc_k1_select picks (dctc_k1_select.h)
 int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream);
+// The layout the Small, Tc8 and Tc16 kernels (and the 1/3-channel variants of the march kernel) read: 1 or 3 channels,
+// image rows, frames and halo rows 16-byte aligned
+bool dctc_k1_fast_layout(const DctcK1Args& a);
 void dctc_carver_release(dctc_context* ctx);
 int dctc_carver_params_changed(dctc_context* ctx);   // rebuilds the resident energy map of a loaded carver session

@@ -29,20 +29,12 @@
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
 
-#define CK(ctx, call)                                             \
-    do {                                                          \
-        cudaError_t e_ = (call);                                  \
-        if (e_ != cudaSuccess) return dctc_fail_cuda((ctx), e_);  \
-    } while (0)
-
-static bool multi_valid_blocksize(int b) { return b == 2 || b == 4 || b == 8 || b == 16; }
-
 // ---- band geometry ----------------------------------------------------------------------------------------------
 
 extern "C" int dctc_band_plan(int h, int world, int rank, int blocksize, int* y0, int* rows, int* top_need, int* bot_need)
 {
     if (h <= 0 || world <= 0 || rank < 0 || rank >= world) return DCTC_ERR_INVALID;
-    if (!multi_valid_blocksize(blocksize)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(blocksize)) return DCTC_ERR_BLOCKSIZE;
     const long long a = (long long) h * rank / world, z = (long long) h * (rank + 1) / world;
     const int tn = rank > 0 ? blocksize / 2 - 1 : 0, bn = rank < world - 1 ? blocksize / 2 : 0;
     if (y0) *y0 = (int) a;
