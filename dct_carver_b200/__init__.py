@@ -23,12 +23,13 @@ ABI_SYMBOLS = [
     "dctc_version", "dctc_device_count", "dctc_stream", "dctc_launch_count",
     "dctc_energy_full", "dctc_energy_full_dev", "dctc_energy_batch_dev", "dctc_energy_band_dev", "dctc_energy_band_dev_at", "dctc_energy_batch",
     "dctc_carver_load", "dctc_carver_width", "dctc_carver_height", "dctc_carver_energy", "dctc_carve_and_update",
-    "dctc_carver_image", "dctc_carver_resize_width", "dctc_carver_enlarge_width", "dctc_carver_set_incremental", "dctc_carver_rebuild_count", "dctc_pixel_energy",
+    "dctc_carver_image", "dctc_carver_resize_width", "dctc_carver_enlarge_width", "dctc_carver_resize_height",
+    "dctc_carver_enlarge_height", "dctc_carver_set_incremental", "dctc_carver_rebuild_count", "dctc_pixel_energy",
     "dctc_energy_minmax_dev", "dctc_energy_image_dev", "dctc_carver_energy_image", "dctc_preview_energy",
     "dctc_carver_set_dump_vmaps", "dctc_carver_vmap", "dctc_carver_paint_seams",
     "dctc_carver_batch_create", "dctc_carver_batch_destroy", "dctc_carver_batch_load", "dctc_carver_batch_resize_width",
     "dctc_carver_batch_enlarge_width", "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy",
-    "dctc_carver_batch_vmap",
+    "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -103,6 +104,8 @@ def lib():
         "dctc_carver_image": (i32, [vp, vp]),
         "dctc_carver_resize_width": (i32, [vp, i32, vp]),
         "dctc_carver_enlarge_width": (i32, [vp, i32, vp]),
+        "dctc_carver_resize_height": (i32, [vp, i32, vp]),
+        "dctc_carver_enlarge_height": (i32, [vp, i32, vp]),
         "dctc_carver_rebuild_count": (i32, [vp]),
         "dctc_carver_set_incremental": (i32, [vp, i32]),
         "dctc_energy_minmax_dev": (i32, [vp, vp, C.c_size_t, i32, i32, vp]),
@@ -118,6 +121,9 @@ def lib():
         "dctc_carver_batch_resize_width": (i32, [vp, i32, vp]),
         "dctc_carver_batch_enlarge_width": (i32, [vp, i32, vp]),
         "dctc_carver_batch_width": (i32, [vp]),
+        "dctc_carver_batch_resize_height": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_enlarge_height": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_height": (i32, [vp]),
         "dctc_carver_batch_images": (i32, [vp, vp]),
         "dctc_carver_batch_energy": (i32, [vp, vp]),
         "dctc_carver_batch_vmap": (i32, [vp, vp, vp]),
@@ -370,6 +376,25 @@ class Context:
                "dctc_carver_enlarge_width")
         return seams
 
+    def carver_resize_height(self, n_seams):
+        """Removes n_seams horizontal seams on the device (lqr_carver_resize(carver, w, h - n_seams)); returns the removed
+        rows, shape (n_seams, w), in the coordinates of the image at the time of removal.  The first seam operation after
+        carver_load fixes the axis: width calls fail until the next load."""
+        w, h = self.carver_size()
+        seams = np.empty((n_seams, w), np.int32)
+        _check(lib().dctc_carver_resize_height(self._h, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_resize_height")
+        return seams
+
+    def carver_enlarge_height(self, n_seams):
+        """lqr_carver_resize to a larger height on the device: returns the n_seams seams (as carver_resize_height does);
+        the session continues on the enlarged image."""
+        w, h = self.carver_size()
+        seams = np.empty((n_seams, w), np.int32)
+        _check(lib().dctc_carver_enlarge_height(self._h, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_enlarge_height")
+        return seams
+
     def carver_set_incremental(self, on):
         """Device seam loop: update the cumulative map incrementally (liblqr's update_mmap) instead of rebuilding it."""
         _check(lib().dctc_carver_set_incremental(self._h, int(bool(on))), "dctc_carver_set_incremental")
@@ -397,7 +422,8 @@ class Context:
         _check(lib().dctc_carver_set_dump_vmaps(self._h, int(on)), "dctc_carver_set_dump_vmaps")
 
     def carver_vmap(self, w0, h):
-        """(visibility map of the original w0 x h pixels, depth): removal order per pixel, 0 = never removed."""
+        """(visibility map of the original w0 x h pixels, depth): removal order per pixel, 0 = never removed (by vertical
+        seams, or by horizontal ones after carver_resize_height / carver_enlarge_height)."""
         out = np.empty((h, w0), np.int32)
         depth = C.c_int(0)
         _check(lib().dctc_carver_vmap(self._h, _ptr(out), C.byref(depth)), "dctc_carver_vmap")
@@ -501,6 +527,10 @@ class CarverBatch:
     def width(self):
         return int(lib().dctc_carver_batch_width(self._b))
 
+    @property
+    def height(self):
+        return int(lib().dctc_carver_batch_height(self._b))
+
     def resize_width(self, n_seams):
         """Removes n_seams vertical seams from every frame; returns int32 [n, n_seams, h], the removed columns in the
         coordinates of each frame at the time of removal."""
@@ -518,18 +548,36 @@ class CarverBatch:
                "dctc_carver_batch_enlarge_width")
         return seams
 
+    def resize_height(self, n_seams):
+        """Removes n_seams horizontal seams from every frame; returns int32 [n, n_seams, w], the removed rows in the
+        coordinates of each frame at the time of removal.  The first seam operation after a load fixes the axis: width
+        calls fail until the next load(), and the other way round."""
+        seams = np.empty((self.n, n_seams, self.width), np.int32)
+        _check(lib().dctc_carver_batch_resize_height(self._b, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_batch_resize_height")
+        return seams
+
+    def enlarge_height(self, n_seams):
+        """lqr_carver_resize to a larger height for every frame (enlarge_width along the other axis): returns int32
+        [n, n_seams, w]; the frames become h + n_seams tall.  No further resize until the next load()."""
+        seams = np.empty((self.n, n_seams, self.width), np.int32)
+        _check(lib().dctc_carver_batch_enlarge_height(self._b, int(n_seams), _ptr(seams) if n_seams else None),
+               "dctc_carver_batch_enlarge_height")
+        return seams
+
     def images(self):
-        out = np.empty((self.n, self.h, self.width, self.ch), np.uint8)
+        out = np.empty((self.n, self.height, self.width, self.ch), np.uint8)
         _check(lib().dctc_carver_batch_images(self._b, _ptr(out)), "dctc_carver_batch_images")
         return out
 
     def energy(self):
-        out = np.empty((self.n, self.h, self.width), np.float32)
+        out = np.empty((self.n, self.height, self.width), np.float32)
         _check(lib().dctc_carver_batch_energy(self._b, _ptr(out)), "dctc_carver_batch_energy")
         return out
 
     def vmap(self):
-        """(visibility maps int32 [n, h, w0], depth): removal order per original pixel, 0 = never removed."""
+        """(visibility maps int32 [n, h, w0], depth): removal order per original pixel, 0 = never removed (by the
+        horizontal seams after resize_height / enlarge_height)."""
         out = np.empty((self.n, self.h, self.w0), np.int32)
         depth = C.c_int(0)
         _check(lib().dctc_carver_batch_vmap(self._b, _ptr(out), C.byref(depth)), "dctc_carver_batch_vmap")

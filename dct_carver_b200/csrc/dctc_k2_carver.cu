@@ -1093,7 +1093,7 @@ static void frames_init(CarverFrames& f, int n, int w, int h, int ch)
 static void frames_free(CarverFrames& f)
 {
     cudaFree(f.img); cudaFree(f.en); cudaFree(f.m); cudaFree(f.dir); cudaFree(f.seam); cudaFree(f.xlast);
-    cudaFree(f.seam_log); cudaFree(f.raw); cudaFree(f.vs);
+    cudaFree(f.seam_log); cudaFree(f.raw); cudaFree(f.vs); cudaFree(f.scratch);
     f = CarverFrames();
 }
 
@@ -1164,19 +1164,73 @@ static int frames_full_energy(dctc_context* ctx, const CarverFrames& f, const Dc
     return dctc_run_k1(ctx, op, a, f.n, ctx->stream);
 }
 
+// ---- the way out: everything the caller sees is in image orientation --------------------------------------------------
+// Transposed frames (a height operation's, frames_transpose) hold the images' transposes; these helpers are the only
+// readers of the flag besides the axis switch.
+
+static int frames_image_w(const CarverFrames& f) { return f.transposed ? f.h : f.w; }
+static int frames_image_h(const CarverFrames& f) { return f.transposed ? f.w : f.h; }
+
+// A plane of every frame in image orientation: cols x rows elements of esize bytes per frame, rows pitch bytes apart,
+// frames rows * pitch bytes apart
+struct Plane {
+    const void* p;
+    size_t pitch;
+    int cols, rows;
+};
+
+// A plane of the frames (cols x f.h elements of esize bytes per frame, rows pitch bytes apart, frames f.h rows apart) in
+// image orientation: the plane itself, or for transposed frames its transpose in the scratch plane (one launch).
+static int frames_oriented(dctc_context* ctx, CarverFrames& f, const void* plane, size_t pitch, int cols, int esize, Plane& out)
+{
+    out = Plane{plane, pitch, cols, f.h};
+    if (!f.transposed) return DCTC_OK;
+    if (!f.scratch) CK(ctx, cudaMalloc(&f.scratch, sizeof(float) * (size_t) f.w0 * f.h * f.n));   // cols <= w0, esize <= 4
+    const size_t spitch = (size_t) esize * f.h;
+    CK(ctx, dctc_launch_transpose(plane, pitch, pitch * f.h, f.scratch, spitch, spitch * cols, cols, f.h, f.n, esize, ctx->stream));
+    ctx->launches++;
+    out = Plane{f.scratch, spitch, f.h, cols};
+    return DCTC_OK;
+}
+
 // Images (w * ch bytes per row), energy planes (w floats per row) and visibility maps (vs_w ints per row) of all frames,
-// n * h rows each, to the host
-static int frames_download(dctc_context* ctx, const CarverFrames& f, uint8_t* img, float* en, int* vs)
+// in image orientation, to the host
+static int frames_download(dctc_context* ctx, CarverFrames& f, uint8_t* img, float* en, int* vs)
 {
     CK(ctx, cudaSetDevice(ctx->device));
-    const size_t rows = (size_t) f.h * f.n, rb = (size_t) f.w * f.ch;   // frames are h rows apart in every plane
-    if (img) CK(ctx, cudaMemcpy2DAsync(img, rb, f.img, f.pitch, rb, rows, cudaMemcpyDeviceToHost, ctx->stream));
-    if (en)
-        CK(ctx, cudaMemcpy2DAsync(en, sizeof(float) * f.w, f.en, sizeof(float) * f.en_pitch, sizeof(float) * f.w, rows,
-                                  cudaMemcpyDeviceToHost, ctx->stream));
-    if (vs) CK(ctx, cudaMemcpyAsync(vs, f.vs, sizeof(int) * f.vs_w * rows, cudaMemcpyDeviceToHost, ctx->stream));
+    struct { void* dst; const void* src; size_t pitch; int cols, esize; } planes[3] = {
+        {img, f.img, f.pitch, f.w, f.ch}, {en, f.en, sizeof(float) * f.en_pitch, f.w, 4}, {vs, f.vs, sizeof(int) * f.vs_w, f.vs_w, 4}};
+    for (const auto& q : planes) {
+        if (!q.dst) continue;
+        Plane p;
+        const int rc = frames_oriented(ctx, f, q.src, q.pitch, q.cols, q.esize, p);
+        if (rc) return rc;
+        const size_t rb = (size_t) p.cols * q.esize;   // frames are p.rows rows apart
+        CK(ctx, cudaMemcpy2DAsync(q.dst, rb, p.p, p.pitch, rb, (size_t) p.rows * f.n, cudaMemcpyDeviceToHost, ctx->stream));
+    }
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
+}
+
+// ---- the axis switch: the first height operation since a load ------------------------------------------------------------
+// liblqr changes the height by transposing the carver (lqr_carver_resize), and so does a carver session: t becomes the
+// transposes of f's frames (one launch), with the full energy maps of the transposed images (one K1 launch with the
+// session's operator, not a transpose of f's maps: the operator's window is not symmetric) and, with vmaps, fresh visibility
+// maps.  The width seam loop then runs on t unchanged.  t is allocated when it has no frames yet (a batch keeps it).
+static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFrames& t, const DctcK1Op& op, bool vmaps)
+{
+    if (!t.img) {
+        frames_init(t, f.n, f.h, f.w, f.ch);
+        t.transposed = true;
+        const int rc = frames_alloc(ctx, t);
+        if (rc) return rc;
+    }
+    t.w = t.w0;
+    CK(ctx, dctc_launch_transpose(f.img, f.pitch, f.img_fs, t.img, t.pitch, t.img_fs, f.w, f.h, f.n, f.ch, ctx->stream));
+    ctx->launches++;
+    int rc = frames_full_energy(ctx, t, op);
+    if (rc == DCTC_OK && vmaps) rc = frames_vmaps(ctx, t);
+    return rc;
 }
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
@@ -1404,6 +1458,7 @@ void dctc_carver_release(dctc_context* ctx)
     ctx->c_band = nullptr; ctx->c_band_vals = nullptr; ctx->h_mirror = nullptr; ctx->h_band = nullptr;
     ctx->c_m_valid = false;
     ctx->mirror_valid = false;
+    ctx->c_axis = DCTC_AXIS_NONE;
 }
 
 // dctc_set_params with a session loaded (liblqr: lqr_carver_set_energy_function invalidates the energy map): the
@@ -1437,6 +1492,116 @@ static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h,
     return DCTC_OK;
 }
 
+int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pitch, int* w, int* h)
+{
+    CarverFrames* f = ctx->carver;
+    Plane p;
+    const int rc = frames_oriented(ctx, *f, f->en, sizeof(float) * f->en_pitch, f->w, sizeof(float), p);
+    if (rc) return rc;
+    *en = (const float*) p.p;
+    *en_pitch = p.pitch / sizeof(float);
+    *w = p.cols;
+    *h = p.rows;
+    return DCTC_OK;
+}
+
+// Checks of a single-session seam operation along `axis` (n_seams > 0, a session loaded): the other axis fixed since the
+// load, n_seams >= the image's extent along the axis, an extent wider than the seam DP covers.  Then the operation fixes
+// the axis, and the first height operation replaces the session's frame by its transpose.  A failed switch leaves the
+// session unloaded.
+static int carver_axis(dctc_context* ctx, int axis, int n_seams)
+{
+    if (ctx->c_axis != DCTC_AXIS_NONE && ctx->c_axis != axis) return DCTC_ERR_STATE;
+    const CarverFrames& f = *ctx->carver;
+    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(f) : frames_image_h(f);
+    if (n_seams >= extent) return DCTC_ERR_STATE;
+    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (axis == DCTC_AXIS_HEIGHT && ctx->c_axis == DCTC_AXIS_NONE) {
+        CarverFrames* t = new (std::nothrow) CarverFrames;
+        if (!t) return DCTC_ERR_NOMEM;
+        const int rc = frames_transpose(ctx, f, *t, carver_op(ctx->op), false);
+        frames_free(*ctx->carver);
+        delete ctx->carver;
+        ctx->carver = t;
+        ctx->mirror_valid = false;
+        ctx->c_m_valid = false;
+        if (rc) {
+            dctc_carver_release(ctx);
+            return rc;
+        }
+    }
+    ctx->c_axis = axis;
+    return DCTC_OK;
+}
+
+// A resize after carver_axis: the seam loop on the session's current frame
+static int carver_resize(dctc_context* ctx, int n_seams, int* seams_out)
+{
+    CarverFrames* f = ctx->carver;
+    if (ctx->c_dump_vmaps && !f->raw) {
+        if (f->w != f->w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
+        const int rc = frames_vmaps(ctx, *f);
+        if (rc) return rc;
+    }
+    ctx->mirror_valid = false;
+    if (!ctx->c_incremental) ctx->c_m_valid = false;
+    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_dump_vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
+}
+
+// An enlarge after carver_axis: frames_enlarge, after which the session continues on the
+// enlarged frame (its w0 is the new width, its energy map the one frames_enlarge computed); the visibility map of the
+// start frame stays readable through dctc_carver_vmap and dctc_carver_paint_seams.  A failure leaves the session unloaded.
+static int carver_enlarge(dctc_context* ctx, int n_seams, int* seams_out)
+{
+    CarverFrames* f = ctx->carver;
+    CarverFrames* wide = new (std::nothrow) CarverFrames;
+    if (!wide) return DCTC_ERR_NOMEM;
+    uint8_t* start = nullptr;
+    frames_init(*wide, 1, f->w0 + n_seams, f->h, f->ch);
+    wide->transposed = f->transposed;
+    int rc = frames_alloc(ctx, *wide);
+    if (rc == DCTC_OK) rc = frames_vmaps(ctx, *f);
+    if (rc == DCTC_OK) {
+        const cudaError_t e = cudaMalloc((void**) &start, f->img_fs);
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+    }
+    if (rc == DCTC_OK)
+        rc = frames_enlarge(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_incremental ? &ctx->c_m_valid : nullptr, start, *wide);
+    cudaFree(start);
+    if (rc) {
+        frames_free(*wide);
+        delete wide;
+        dctc_carver_release(ctx);
+        return rc;
+    }
+    std::swap(wide->vs, f->vs);
+    wide->depth = f->depth;
+    wide->vs_w = f->vs_w;
+    frames_free(*f);
+    delete f;
+    ctx->carver = wide;
+    // as after a load: no cumulative map, no host mirror (the frame is wider), rebuild count from zero
+    cudaFree(ctx->c_band); cudaFreeHost(ctx->h_mirror);
+    ctx->c_band = nullptr; ctx->h_mirror = nullptr;
+    ctx->c_m_valid = false;
+    ctx->mirror_valid = false;
+    return DCTC_OK;
+}
+
+// dctc_carver_resize_width / _height, dctc_carver_enlarge_width / _height
+static int carver_seams(dctc_context* ctx, int axis, bool enlarge, int n_seams, int* seams_out)
+{
+    if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
+    const CarverFrames* f = ctx->carver;
+    if (!f) return DCTC_ERR_STATE;
+    if (n_seams == 0) return DCTC_OK;
+    if (enlarge && f->w != f->w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded (or enlarged) frame
+    const int rc = carver_axis(ctx, axis, n_seams);
+    if (rc) return rc;
+    return enlarge ? carver_enlarge(ctx, n_seams, seams_out) : carver_resize(ctx, n_seams, seams_out);
+}
+
 extern "C" {
 
 int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
@@ -1454,8 +1619,8 @@ int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int ch
     return rc;
 }
 
-int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? ctx->carver->w : 0; }
-int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? ctx->carver->h : 0; }
+int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_w(*ctx->carver) : 0; }
+int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_h(*ctx->carver) : 0; }
 
 int dctc_carver_energy(dctc_context* ctx, float* out)
 {
@@ -1475,7 +1640,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
 {
     if (!ctx || !seam_x) return DCTC_ERR_INVALID;
     CarverFrames* f = ctx->carver;
-    if (!f || f->w <= 1) return DCTC_ERR_STATE;
+    if (!f || f->w <= 1 || ctx->c_axis == DCTC_AXIS_HEIGHT) return DCTC_ERR_STATE;   // vertical seams only
     const DctcK1Op op = carver_op(ctx->op);
     const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
     int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * 32);
@@ -1485,6 +1650,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
         if (y > 0 && (seam_x[y] - seam_x[y - 1] > 1 || seam_x[y - 1] - seam_x[y] > 1)) return DCTC_ERR_INVALID;
         h_seam[y] = seam_x[y];
     }
+    ctx->c_axis = DCTC_AXIS_WIDTH;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpyAsync(f->seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
     dctc_carve_rows_kernel<256, 4><<<h, 256, 0, ctx->stream>>>(f->img, f->pitch, f->ch, f->en, f->en_pitch, f->seam, w_old, nullptr,
@@ -1519,66 +1685,22 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
 
 int dctc_carver_resize_width(dctc_context* ctx, int n_seams, int* seams_out)
 {
-    if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= f->w) return DCTC_ERR_STATE;
-    if (f->w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (ctx->c_dump_vmaps && !f->raw) {
-        if (f->w != f->w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
-        const int rc = frames_vmaps(ctx, *f);
-        if (rc) return rc;
-    }
-    ctx->mirror_valid = false;
-    if (!ctx->c_incremental) ctx->c_m_valid = false;
-    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_dump_vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
+    return carver_seams(ctx, DCTC_AXIS_WIDTH, false, n_seams, seams_out);
 }
 
-// lqr_carver_resize to a LARGER width: frames_enlarge, after which the session continues on the enlarged frame (its w0
-// is the new width, its energy map the one frames_enlarge computed); the visibility map of the start frame stays readable
-// through dctc_carver_vmap and dctc_carver_paint_seams.  A failure leaves the session unloaded.
+int dctc_carver_resize_height(dctc_context* ctx, int n_seams, int* seams_out)
+{
+    return carver_seams(ctx, DCTC_AXIS_HEIGHT, false, n_seams, seams_out);
+}
+
 int dctc_carver_enlarge_width(dctc_context* ctx, int n_seams, int* seams_out)
 {
-    if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= f->w || f->w != f->w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded frame
-    if (f->w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
-    CK(ctx, cudaSetDevice(ctx->device));
-    CarverFrames* wide = new (std::nothrow) CarverFrames;
-    if (!wide) return DCTC_ERR_NOMEM;
-    uint8_t* start = nullptr;
-    frames_init(*wide, 1, f->w0 + n_seams, f->h, f->ch);
-    int rc = frames_alloc(ctx, *wide);
-    if (rc == DCTC_OK) rc = frames_vmaps(ctx, *f);
-    if (rc == DCTC_OK) {
-        const cudaError_t e = cudaMalloc((void**) &start, f->img_fs);
-        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
-    }
-    if (rc == DCTC_OK)
-        rc = frames_enlarge(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_incremental ? &ctx->c_m_valid : nullptr, start, *wide);
-    cudaFree(start);
-    if (rc) {
-        frames_free(*wide);
-        delete wide;
-        dctc_carver_release(ctx);
-        return rc;
-    }
-    std::swap(wide->vs, f->vs);
-    wide->depth = f->depth;
-    wide->vs_w = f->vs_w;
-    frames_free(*f);
-    delete f;
-    ctx->carver = wide;
-    // as after a load: no cumulative map, no host mirror (the frame is wider), rebuild count from zero
-    cudaFree(ctx->c_band); cudaFreeHost(ctx->h_mirror);
-    ctx->c_band = nullptr; ctx->h_mirror = nullptr;
-    ctx->c_m_valid = false;
-    ctx->mirror_valid = false;
-    return DCTC_OK;
+    return carver_seams(ctx, DCTC_AXIS_WIDTH, true, n_seams, seams_out);
+}
+
+int dctc_carver_enlarge_height(dctc_context* ctx, int n_seams, int* seams_out)
+{
+    return carver_seams(ctx, DCTC_AXIS_HEIGHT, true, n_seams, seams_out);
 }
 
 int dctc_carver_set_incremental(dctc_context* ctx, int on)
@@ -1612,7 +1734,7 @@ int dctc_carver_set_dump_vmaps(dctc_context* ctx, int on)
 int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
 {
     if (!ctx) return DCTC_ERR_INVALID;
-    const CarverFrames* f = ctx->carver;
+    CarverFrames* f = ctx->carver;
     if (!f || !f->vs) return DCTC_ERR_STATE;
     const int rc = frames_download(ctx, *f, nullptr, nullptr, vmap_out);
     if (rc == DCTC_OK && depth_out) *depth_out = f->depth;
@@ -1622,17 +1744,20 @@ int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
 int dctc_carver_paint_seams(dctc_context* ctx, uint8_t* img, int channels, size_t pitch)
 {
     if (!ctx || !img || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
-    const CarverFrames* f = ctx->carver;
+    CarverFrames* f = ctx->carver;
     if (!f || !f->vs || f->depth <= 0) return DCTC_ERR_STATE;
-    const int w = f->vs_w, h = f->h;
-    if (pitch < (size_t) w * channels) return DCTC_ERR_INVALID;
     CK(ctx, cudaSetDevice(ctx->device));
+    Plane vs;   // the map in image orientation, row pitch = its width
+    const int rc = frames_oriented(ctx, *f, f->vs, sizeof(int) * f->vs_w, f->vs_w, sizeof(int), vs);
+    if (rc) return rc;
+    const int w = vs.cols, h = vs.rows;
+    if (pitch < (size_t) w * channels) return DCTC_ERR_INVALID;
     uint8_t* d = nullptr;
     const size_t dp = ((size_t) w * channels + 15) & ~(size_t) 15;
     CK(ctx, cudaMalloc((void**) &d, dp * h));
     cudaError_t e = cudaMemcpy2DAsync(d, dp, img, pitch, (size_t) w * channels, h, cudaMemcpyHostToDevice, ctx->stream);
     if (e == cudaSuccess) {
-        dctc_paint_seams_kernel<<<dim3((w + 255) / 256, h), 256, 0, ctx->stream>>>(d, dp, channels, w, h, f->vs, f->depth);
+        dctc_paint_seams_kernel<<<dim3((w + 255) / 256, h), 256, 0, ctx->stream>>>(d, dp, channels, w, h, (const int*) vs.p, f->depth);
         e = cudaGetLastError();
         ctx->launches++;
     }
@@ -1649,7 +1774,7 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
     (void) rw;
     DctcCarverEnergyParams* p = (DctcCarverEnergyParams*) extra_data;
     dctc_context* ctx = p ? p->gpu : nullptr;
-    if (!ctx || !ctx->carver || w != ctx->carver->w || h != ctx->carver->h || x < 0 || y < 0 || x >= w || y >= h) {
+    if (!ctx || !ctx->carver || w != dctc_carver_width(ctx) || h != dctc_carver_height(ctx) || x < 0 || y < 0 || x >= w || y >= h) {
         if (ctx) ctx->last_cuda = 0;
         return __builtin_nanf("");
     }
@@ -1674,35 +1799,72 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
 struct dctc_carver_batch {
     dctc_context* ctx = nullptr;
     CarverFrames f;
+    CarverFrames t;                     // the height operations' frames: transposes of f (the first allocates, destroy frees)
     DctcK1Op op;                        // the context's operator at load time, with the carver's kernel rule (carver_op)
     bool dump_vmaps = false, loaded = false;
-    // dctc_carver_batch_enlarge_width: a copy of the start frames and the enlarged frames (images and energy planes).
-    // Allocated by the first enlarge and kept for the next (the enlarged frames are reallocated when n_seams changes),
-    // freed by the destroy.
+    int axis = DCTC_AXIS_NONE;          // fixed by the first seam operation since the load
+    // dctc_carver_batch_enlarge_width / _height: a copy of the start frames and the enlarged frames (images and energy
+    // planes).  Allocated by the first enlarge and kept for the next (reallocated when their size differs), freed by the
+    // destroy.
     bool enlarged = false;              // the current frames are the enlarged ones
     uint8_t* start_img = nullptr;
+    size_t start_bytes = 0;
     CarverFrames wide;
 };
 
 namespace {
 
-const CarverFrames& batch_frames(const dctc_carver_batch* b) { return b->enlarged ? b->wide : b->f; }
+// the frames the seam operations carve: the loaded ones, or their transposes along the height
+CarverFrames& batch_src(dctc_carver_batch* b) { return b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f; }
+const CarverFrames& batch_frames(const dctc_carver_batch* b)
+{
+    return b->enlarged ? b->wide : b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f;
+}
+CarverFrames& batch_frames(dctc_carver_batch* b) { return const_cast<CarverFrames&>(batch_frames((const dctc_carver_batch*) b)); }
 
 void batch_free(dctc_carver_batch* b)
 {
     frames_free(b->f);
+    frames_free(b->t);
     frames_free(b->wide);
     cudaFree(b->start_img);
 }
 
-// Device work of dctc_carver_batch_enlarge_width
+// Checks of a batch seam operation along `axis` (n_seams > 0, loaded, not enlarged), as carver_axis does them for the
+// single session; the first height operation since the load fills the transposed frames (frames_transpose).  A failed
+// switch leaves the batch unloaded.
+int batch_axis(dctc_carver_batch* b, int axis, int n_seams)
+{
+    if (b->axis != DCTC_AXIS_NONE && b->axis != axis) return DCTC_ERR_STATE;
+    const CarverFrames& f = batch_src(b);
+    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(f) : frames_image_h(f);
+    if (n_seams >= extent) return DCTC_ERR_STATE;
+    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (axis == DCTC_AXIS_HEIGHT && b->axis == DCTC_AXIS_NONE) {
+        b->loaded = false;
+        const int rc = frames_transpose(ctx, b->f, b->t, b->op, b->dump_vmaps);
+        if (rc) return rc;
+        b->loaded = true;
+    }
+    b->axis = axis;
+    return DCTC_OK;
+}
+
+// Device work of dctc_carver_batch_enlarge_width / _height
 int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
     dctc_context* ctx = b->ctx;
-    CarverFrames& f = b->f;
+    CarverFrames& f = batch_src(b);
     const int w1 = f.w0 + n_seams;
-    if (!b->start_img) CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
-    if (b->wide.w0 != w1) {
+    if (b->start_bytes != f.img_fs * f.n) {
+        cudaFree(b->start_img);
+        b->start_img = nullptr; b->start_bytes = 0;
+        CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
+        b->start_bytes = f.img_fs * f.n;
+    }
+    if (b->wide.w0 != w1 || b->wide.h != f.h) {
         frames_free(b->wide);
         frames_init(b->wide, f.n, w1, f.h, f.ch);
         const int rc = frames_alloc(ctx, b->wide);
@@ -1711,11 +1873,31 @@ int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
             return rc;
         }
     }
+    b->wide.transposed = f.transposed;
     if (!b->dump_vmaps) {   // (a batch with dump_vmaps had its maps reset by the load, and no seam was removed since)
         const int rc = frames_vmaps(ctx, f);
         if (rc) return rc;
     }
     return frames_enlarge(ctx, f, b->op, n_seams, seams_out, nullptr, b->start_img, b->wide);
+}
+
+// The batch's resize and enlarge calls.  An enlarge carves the frames in place: until every frame is enlarged the batch is
+// not loaded, so that a failure leaves it unloaded rather than half-updated.
+int batch_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out)
+{
+    if (!b || n_seams < 0) return DCTC_ERR_INVALID;
+    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
+    if (n_seams == 0) return DCTC_OK;
+    if (enlarge && batch_src(b).w != batch_src(b).w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
+    int rc = batch_axis(b, axis, n_seams);
+    if (rc) return rc;
+    if (!enlarge) return seam_loop(b->ctx, batch_src(b), b->op, n_seams, seams_out, b->dump_vmaps, nullptr);
+    b->loaded = false;
+    rc = batch_enlarge(b, n_seams, seams_out);
+    if (rc) return rc;
+    b->enlarged = true;
+    b->loaded = true;
+    return DCTC_OK;
 }
 
 }  // namespace
@@ -1769,6 +1951,7 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = false;
     b->enlarged = false;
+    b->axis = DCTC_AXIS_NONE;
     b->op = carver_op(ctx->op);
     f.w = f.w0;
     for (int i = 0; i < f.n; i++)
@@ -1782,37 +1965,27 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     return DCTC_OK;
 }
 
-int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? batch_frames(b).w : 0; }
+int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? frames_image_w(batch_frames(b)) : 0; }
+int dctc_carver_batch_height(const dctc_carver_batch* b) { return b ? frames_image_h(batch_frames(b)) : 0; }
 
 int dctc_carver_batch_resize_width(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
-    if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= b->f.w) return DCTC_ERR_STATE;
-    if (b->f.w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    return seam_loop(ctx, b->f, b->op, n_seams, seams_out, b->dump_vmaps, nullptr);
+    return batch_seams(b, DCTC_AXIS_WIDTH, false, n_seams, seams_out);
+}
+
+int dctc_carver_batch_resize_height(dctc_carver_batch* b, int n_seams, int* seams_out)
+{
+    return batch_seams(b, DCTC_AXIS_HEIGHT, false, n_seams, seams_out);
 }
 
 int dctc_carver_batch_enlarge_width(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
-    if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (n_seams >= b->f.w || b->f.w != b->f.w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
-    if (b->f.w > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    // the seam loop carves the loaded frames in place: until every frame is enlarged the batch is not loaded, so that a
-    // failure leaves it unloaded rather than half-updated
-    b->loaded = false;
-    const int rc = batch_enlarge(b, n_seams, seams_out);
-    if (rc) return rc;
-    b->enlarged = true;
-    b->loaded = true;
-    return DCTC_OK;
+    return batch_seams(b, DCTC_AXIS_WIDTH, true, n_seams, seams_out);
+}
+
+int dctc_carver_batch_enlarge_height(dctc_carver_batch* b, int n_seams, int* seams_out)
+{
+    return batch_seams(b, DCTC_AXIS_HEIGHT, true, n_seams, seams_out);
 }
 
 int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
@@ -1833,8 +2006,9 @@ int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
 {
     if (!b) return DCTC_ERR_INVALID;
     if (!b->loaded || !b->dump_vmaps) return DCTC_ERR_STATE;
-    const int rc = frames_download(b->ctx, b->f, nullptr, nullptr, vmap_out);
-    if (rc == DCTC_OK && depth_out) *depth_out = b->f.depth;
+    CarverFrames& f = batch_src(b);
+    const int rc = frames_download(b->ctx, f, nullptr, nullptr, vmap_out);
+    if (rc == DCTC_OK && depth_out) *depth_out = f.depth;
     return rc;
 }
 

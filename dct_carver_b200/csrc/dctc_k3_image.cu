@@ -136,10 +136,13 @@ int dctc_energy_image_dev(dctc_context* ctx, const float* d_en, size_t en_pitch,
 int dctc_carver_energy_image(dctc_context* ctx, uint8_t* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    const CarverFrames* f = ctx->carver;
-    if (!f) return DCTC_ERR_STATE;
+    if (!ctx->carver) return DCTC_ERR_STATE;
     CK(ctx, cudaSetDevice(ctx->device));
-    const int w = f->w, h = f->h;
+    const float* en;
+    size_t en_pitch;
+    int w, h;
+    int rc = dctc_carver_energy_plane(ctx, &en, &en_pitch, &w, &h);   // in image orientation
+    if (rc) return rc;
     const size_t need = (size_t) w * h;
     if (ctx->k3_img_cap < need) {
         if (ctx->k3_img) cudaFree(ctx->k3_img);
@@ -147,7 +150,7 @@ int dctc_carver_energy_image(dctc_context* ctx, uint8_t* out)
         CK(ctx, cudaMalloc((void**) &ctx->k3_img, need));
         ctx->k3_img_cap = need;
     }
-    int rc = dctc_energy_image_dev(ctx, f->en, f->en_pitch, w, h, nullptr, ctx->k3_img, (size_t) w, 0);
+    rc = dctc_energy_image_dev(ctx, en, en_pitch, w, h, nullptr, ctx->k3_img, (size_t) w, 0);
     if (rc) return rc;
     CK(ctx, cudaMemcpyAsync(out, ctx->k3_img, need, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));

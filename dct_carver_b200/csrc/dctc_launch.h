@@ -86,6 +86,9 @@ cudaError_t dctc_launch_k1_tc16(const DctcK1Args& a, int n_frames, bool uniform,
 cudaError_t dctc_launch_synth(uint8_t* d_img, int n_frames, size_t frame_stride, int w, int h, int channels,
                               size_t pitch, uint32_t seed, int pattern, int first_frame, int y_offset,
                               cudaStream_t stream);
+// dst[frame][x][y] = src[frame][y][x] over cols x rows elements of esize (1..4) bytes per frame (dctc_transpose.cu)
+cudaError_t dctc_launch_transpose(const void* src, size_t src_pitch, size_t src_fs, void* dst, size_t dst_pitch, size_t dst_fs,
+                                  int cols, int rows, int n_frames, int esize, cudaStream_t stream);
 
 constexpr int DCTC_SLOTS = 4;   // device staging slots of the host-buffer batch call (H2D, kernel and D2H of different frames overlap)
 constexpr int DCTC_TC_COUNTERS = 64;
@@ -100,8 +103,12 @@ struct DctcK1Op {
 // Device state of a carver session: n frames of w x h pixels (w0 x h when loaded), frame f of every plane at f times the
 // plane's frame stride.  The context's single session is one of these with n = 1, a batch session (dctc_carver_batch)
 // holds one with n frames; both run the same seam loop over it (dctc_k2_carver.cu).
+// transposed: the frames are the transposes of the images (a height operation runs the width seam loop on them), so w is
+// the image height and h the image width.  Only the axis switch that fills such frames and the way out to the caller
+// (frames_download, frames_oriented) look at the flag.
 struct CarverFrames {
     int n = 0, w0 = 0, w = 0, h = 0, ch = 0;
+    bool transposed = false;
     size_t pitch = 0, img_fs = 0;       // image: bytes per row, per frame
     size_t en_pitch = 0, m_pitch = 0;   // energy / cumulative planes: floats per row (multiple of 4: 16-byte aligned rows;
                                         // m_pitch >= DP_WIN), frames pitch * h floats apart
@@ -120,7 +127,13 @@ struct CarverFrames {
     int* vs = nullptr;
     int depth = 0;
     int vs_w = 0;                       // width of the frame the maps belong to (w0 when they were reset)
+    void* scratch = nullptr;            // transposed frames: a plane in image orientation on its way out (4 * w0 * h bytes
+                                        // per frame, allocated by the first use)
 };
+
+// The axis a carver session's seam operations work along since its load: the first one fixes it, a call for the other
+// axis returns DCTC_ERR_STATE until the next load
+enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2 };
 
 struct dctc_context {
     int device = 0;
@@ -141,6 +154,7 @@ struct dctc_context {
     size_t d_in_cap[DCTC_SLOTS] = {}, d_out_cap[DCTC_SLOTS] = {};
     // carver session (K2): one frame, null when nothing is loaded; the single-session-only state follows
     CarverFrames* carver = nullptr;
+    int c_axis = 0;                // DCTC_AXIS_* the first seam operation since the load fixed
     bool c_dump_vmaps = false;     // record the visibility map in the next seam loops (lqr_carver_set_dump_vmaps)
     int* c_band = nullptr;         // c_band[0]: 'rebuild the cumulative map from scratch' flag of the incremental seam DP, c_band[1]: rebuilds (device)
     bool c_incremental = false;    // device seam loop: update the cumulative map incrementally (dctc_carver_set_incremental)
@@ -163,3 +177,5 @@ int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_fram
 bool dctc_k1_fast_layout(const DctcK1Args& a);
 void dctc_carver_release(dctc_context* ctx);
 int dctc_carver_params_changed(dctc_context* ctx);   // rebuilds the resident energy map of a loaded carver session
+// The single session's energy plane in image orientation (K3 energy image): device pointer, row pitch in floats, w x h
+int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pitch, int* w, int* h);

@@ -139,7 +139,7 @@ int dctc_energy_batch(dctc_context *ctx, const uint8_t *imgs, int n_frames, size
 
 /* Uploads the image, keeps it device-resident and builds the full map (K1). */
 int dctc_carver_load(dctc_context *ctx, const uint8_t *img, int w, int h, int channels, size_t pitch_bytes);
-/* Current carver width / height. */
+/* Current carver width / height (of the image, also while height operations carve its transpose). */
 int dctc_carver_width(const dctc_context *ctx);
 int dctc_carver_height(const dctc_context *ctx);
 /* Copies the current w*h energy map to the host (row pitch = current width). */
@@ -150,7 +150,8 @@ int dctc_carver_energy(dctc_context *ctx, float *out);
  * On return *xmin / *xmax (h entries each, may be NULL) hold that band and band_out (may be NULL) receives, row
  * by row, the xmax[y]-xmin[y]+1 recomputed values packed back to back (at most 4*(blocksize/2) per row: band_out needs
  * room for h*4*(blocksize/2) floats).  The seam must be connected, |seam_x[y]-seam_x[y-1]| <= 1, as liblqr's are with
- * delta_x = 1 (src/render.c:313); anything else returns DCTC_ERR_INVALID, a column outside [0, w) DCTC_ERR_STATE. */
+ * delta_x = 1 (src/render.c:313); anything else returns DCTC_ERR_INVALID, a column outside [0, w) DCTC_ERR_STATE.
+ * A vertical-seam call: DCTC_ERR_STATE after a height call since the load. */
 int dctc_carve_and_update(dctc_context *ctx, const int *seam_x, float *band_out, int *xmin, int *xmax);
 /* Copies the current (carved) interleaved image back to the host, pitch = w*channels. */
 int dctc_carver_image(dctc_context *ctx, uint8_t *out);
@@ -166,6 +167,22 @@ int dctc_carver_resize_width(dctc_context *ctx, int n_seams, int *seams_out);
  * column 0) [liblqr lqr_carver_inflate, from memory: parity unpinned].  The session continues on the enlarged image
  * (dctc_carver_image / _energy / _width reflect it); dctc_carver_vmap returns the start frame's visibility map. */
 int dctc_carver_enlarge_width(dctc_context *ctx, int n_seams, int *seams_out);
+/* Height retargeting: lqr_carver_resize(carver, w, h -/+ n_seams), the plug-in's PlugInVals.vertically
+ * (src/render.c:357-363).  As liblqr does, the session transposes its image (on the device) and runs the width seam loop
+ * on the transpose, whose energy map is computed afresh with the session's operator.  Every result is what
+ * dctc_carver_load of the transposed image followed by the width call gives, turned back into image orientation.
+ * seams_out (may be NULL): n_seams * w ints, seams_out[s*w + x] = the row removed from column x by seam s, in the
+ * coordinates at removal time.  dctc_carver_width / _height / _image / _energy / _energy_image / _vmap / _paint_seams and
+ * dctc_pixel_energy keep speaking image orientation: the visibility map covers the frame the first height call started
+ * from (row pitch = image width) and holds the order of the horizontal seam that removed each pixel.  (The host carver's
+ * vertically path returns its map transposed.)  Split resizes continue the loop, enlarge continues on the enlarged frame,
+ * incremental mode and dctc_set_params work as for the width.
+ * One axis per load: the first seam operation after dctc_carver_load (resize, enlarge or dctc_carve_and_update) fixes
+ * the axis, and a call along the other axis returns DCTC_ERR_STATE until the next load.  n_seams == 0: DCTC_OK, nothing
+ * happens.  DCTC_ERR_STATE also for n_seams >= the height; DCTC_ERR_UNSUPPORTED for images taller than the device
+ * seam DP covers (the session stays loaded).  A CUDA failure in the first height call leaves the session unloaded. */
+int dctc_carver_resize_height(dctc_context *ctx, int n_seams, int *seams_out);
+int dctc_carver_enlarge_height(dctc_context *ctx, int n_seams, int *seams_out);
 /* Optional: let the device loop update its cumulative map incrementally after each seam, like liblqr's update_mmap
  * (only the cells the removed seam can have changed are recomputed; a row whose changed range gets too wide falls
  * back to the full rebuild).  Same seams bit for bit; off by default because the full rebuild on an 8-CTA cluster is
@@ -189,10 +206,12 @@ int dctc_carver_paint_seams(dctc_context *ctx, uint8_t *img, int channels, size_
  * device buffers and never touches the context's single-frame session.  Every phase of the seam loop is one launch
  * for all frames, and every frame's seam DP runs on its own cluster, so frames retarget side by side.  Each frame
  * gets exactly the seams, image, energy map and visibility map that dctc_carver_load + dctc_carver_resize_width
- * give it on its own, and dctc_carver_batch_enlarge_width gives every frame what dctc_carver_enlarge_width gives it.
- * The cumulative map is always rebuilt: incremental mode and height retargeting are not batched.
+ * give it on its own, and dctc_carver_batch_enlarge_width gives every frame what dctc_carver_enlarge_width gives it;
+ * the _height calls give every frame what the single session's _height calls give it.  The cumulative map is always
+ * rebuilt: incremental mode is not batched.
  * Errors: DCTC_ERR_INVALID for NULL pointers, n_frames <= 0, a channel count outside 1..4, a pitch or frame stride
- * that is too small; DCTC_ERR_STATE for a resize before a load, after an enlarge or with n_seams >= the current width;
+ * that is too small; DCTC_ERR_STATE for a resize before a load, after an enlarge, along the other axis than the first
+ * seam operation since the load, or with n_seams >= the current width (height);
  * DCTC_ERR_UNSUPPORTED for widths the device seam DP does not cover (as dctc_carver_resize_width) and
  * n_frames > 65535. */
 typedef struct dctc_carver_batch dctc_carver_batch;
@@ -222,13 +241,24 @@ int dctc_carver_batch_resize_width(dctc_carver_batch *batch, int n_seams, int *s
  * the next load).  The buffers an enlarge allocates (a copy of the start frames, the enlarged frames, the removal
  * order) are reused by the next enlarge (the enlarged frames' when n_seams is the same) and freed by the destroy. */
 int dctc_carver_batch_enlarge_width(dctc_carver_batch *batch, int n_seams, int *seams_out);
-/* current width of every frame */
+/* Height retargeting of every frame (the single session's dctc_carver_resize_height / _enlarge_height, per frame): the
+ * first height call after a load transposes the frames on the device (one launch) into a transposed frame set the
+ * batch keeps until the destroy, and computes their energy maps (one K1 launch); the width seam loop then runs on them.
+ * seams_out: n_frames * n_seams * w ints, frame-major, seams_out[(f*n_seams + s)*w + x] = the row seam s removed from
+ * column x of frame f.  One axis per load, as for the single session: after a width call the _height calls return
+ * DCTC_ERR_STATE, and the other way round, until the next dctc_carver_batch_load.  _images / _energy / _vmap / _width /
+ * _height speak image orientation; the visibility maps stay n_frames * h * w0 ints.  The enlarge rules of
+ * dctc_carver_batch_enlarge_width apply (its buffers are reallocated when their size differs). */
+int dctc_carver_batch_resize_height(dctc_carver_batch *batch, int n_seams, int *seams_out);
+int dctc_carver_batch_enlarge_height(dctc_carver_batch *batch, int n_seams, int *seams_out);
+/* current width / height of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
+int dctc_carver_batch_height(const dctc_carver_batch *batch);
 /* current images (n_frames * h * w * channels, pitch w * channels) / energy maps (n_frames * h * w floats) */
 int dctc_carver_batch_images(dctc_carver_batch *batch, uint8_t *out);
 int dctc_carver_batch_energy(dctc_carver_batch *batch, float *out);
-/* visibility map of every frame over the loaded width w0 (n_frames * h * w0 ints) and the common depth; needs
- * dump_vmaps at create time */
+/* visibility map of every frame over the loaded size (n_frames * h * w0 ints) and the common depth; needs dump_vmaps
+ * at create time */
 int dctc_carver_batch_vmap(dctc_carver_batch *batch, int *vmap_out, int *depth_out);
 
 /* ---- K3: energy-image export ------------------------------------------------------------------------------
