@@ -30,6 +30,7 @@ ABI_SYMBOLS = [
     "dctc_carver_batch_create", "dctc_carver_batch_destroy", "dctc_carver_batch_load", "dctc_carver_batch_resize_width",
     "dctc_carver_batch_enlarge_width", "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy",
     "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
+    "dctc_resize_plan", "dctc_carver_resize", "dctc_carver_batch_resize",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -53,6 +54,15 @@ class EnergyParameters(C.Structure):
 
 class CarverEnergyParams(C.Structure):
     _fields_ = [("base", EnergyParameters), ("gpu", C.c_void_p)]
+
+
+RESIZE_WIDTH, RESIZE_HEIGHT = 0, 1
+
+
+class ResizePass(C.Structure):
+    """DctcResizePass (include/dctc.h): one pass of a resize plan."""
+    _fields_ = [("axis", C.c_int), ("enlarge", C.c_int), ("n_seams", C.c_int), ("w", C.c_int), ("h", C.c_int),
+                ("seams_offset", C.c_size_t), ("vmap_offset", C.c_size_t)]
 
 
 class DctcError(RuntimeError):
@@ -127,6 +137,9 @@ def lib():
         "dctc_carver_batch_images": (i32, [vp, vp]),
         "dctc_carver_batch_energy": (i32, [vp, vp]),
         "dctc_carver_batch_vmap": (i32, [vp, vp, vp]),
+        "dctc_resize_plan": (i32, [i32, i32, i32, i32, vp, i32]),
+        "dctc_carver_resize": (i32, [vp, i32, i32, vp, vp]),
+        "dctc_carver_batch_resize": (i32, [vp, i32, i32, vp, vp]),
         "dctc_pixel_energy": (f32, [i32, i32, i32, i32, vp, vp]),
         "dctc_synth_fill_dev": (i32, [vp, vp, i32, sz, i32, i32, i32, sz, u32, i32, i32, i32]),
         "dctc_synth_byte": (C.c_uint8, [u32, u32, u32, u32, u32, i32]),
@@ -192,6 +205,46 @@ def _check(status, what):
 
 def _ptr(a):
     return a.ctypes.data_as(C.c_void_p)
+
+
+def resize_plan(w, h, new_w, new_h):
+    """The passes lqr_carver_resize(new_w, new_h) runs from w x h (dctc_resize_plan), in order: dicts with axis ("width"
+    or "height"), enlarge, n_seams, the image size w, h at the start of the pass, and the pass's per-frame offsets (in
+    ints) in the seams and maps buffers of Context.carver_resize / CarverBatch.resize."""
+    n = lib().dctc_resize_plan(w, h, new_w, new_h, None, 0)
+    if n < 0:
+        raise DctcError(n, "dctc_resize_plan")
+    passes = (ResizePass * max(n, 1))()
+    lib().dctc_resize_plan(w, h, new_w, new_h, passes, n)
+    return [dict(axis="width" if p.axis == RESIZE_WIDTH else "height", enlarge=bool(p.enlarge), n_seams=p.n_seams, w=p.w,
+                 h=p.h, seams_offset=p.seams_offset, vmap_offset=p.vmap_offset) for p in passes[:n]]
+
+
+def _resize(fn, handle, w, h, new_w, new_h, vmaps, n_frames):
+    """Runs dctc_carver_resize / dctc_carver_batch_resize (fn) and splits its buffers into one entry per pass: axis,
+    enlarge, seams ([n_frames,] n_seams, len) and, with vmaps, the map ([n_frames,] h, w) of the pass's start frame."""
+    try:
+        plan = resize_plan(w, h, new_w, new_h) if min(w, h, new_w, new_h) > 0 else []
+    except DctcError:
+        plan = []   # the entry point refuses the same sizes and reports its own status
+    lens = [p["h"] if p["axis"] == "width" else p["w"] for p in plan]
+    n_seams = sum(p["n_seams"] * n for p, n in zip(plan, lens))
+    n_maps = sum(p["w"] * p["h"] for p in plan)
+    nf = n_frames or 1
+    seams = np.empty(nf * n_seams, np.int32)
+    maps = np.empty(nf * n_maps, np.int32) if vmaps else None
+    _check(fn(handle, int(new_w), int(new_h), _ptr(seams) if n_seams else None, _ptr(maps) if vmaps and n_maps else None),
+           fn.__name__)
+    lead = (n_frames,) if n_frames else ()
+    out = []
+    for p, n in zip(plan, lens):
+        so, vo = nf * p["seams_offset"], nf * p["vmap_offset"]
+        e = dict(axis=p["axis"], enlarge=p["enlarge"],
+                 seams=seams[so:so + nf * p["n_seams"] * n].reshape(lead + (p["n_seams"], n)))
+        if vmaps:
+            e["vmap"] = maps[vo:vo + nf * p["w"] * p["h"]].reshape(lead + (p["h"], p["w"]))
+        out.append(e)
+    return out
 
 
 def pinned_array(shape, dtype, write_combined=False):
@@ -395,6 +448,14 @@ class Context:
                "dctc_carver_enlarge_height")
         return seams
 
+    def carver_resize(self, new_w, new_h, vmaps=False):
+        """lqr_carver_resize(carver, new_w, new_h) on the device (dctc_carver_resize): the width passes, then the height
+        passes of resize_plan.  Returns one dict per pass: axis, enlarge, seams shaped as the per-axis method returns
+        them and, with vmaps, "vmap", the pass's start-frame visibility map [h, w].  Needs a freshly loaded session;
+        afterwards no seam operation until the next carver_load."""
+        w, h = self.carver_size()
+        return _resize(lib().dctc_carver_resize, self._h, w, h, new_w, new_h, vmaps, None)
+
     def carver_set_incremental(self, on):
         """Device seam loop: update the cumulative map incrementally (liblqr's update_mmap) instead of rebuilding it."""
         _check(lib().dctc_carver_set_incremental(self._h, int(bool(on))), "dctc_carver_set_incremental")
@@ -564,6 +625,12 @@ class CarverBatch:
         _check(lib().dctc_carver_batch_enlarge_height(self._b, int(n_seams), _ptr(seams) if n_seams else None),
                "dctc_carver_batch_enlarge_height")
         return seams
+
+    def resize(self, new_w, new_h, vmaps=False):
+        """Context.carver_resize for every frame (dctc_carver_batch_resize): one dict per pass with seams
+        [n, n_seams, len] and, with vmaps, "vmap" [n, h, w].  Needs a freshly loaded batch; afterwards no seam operation
+        until the next load()."""
+        return _resize(lib().dctc_carver_batch_resize, self._b, self.width, self.height, new_w, new_h, vmaps, self.n)
 
     def images(self):
         out = np.empty((self.n, self.height, self.width, self.ch), np.uint8)

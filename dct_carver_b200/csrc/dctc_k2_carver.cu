@@ -13,6 +13,7 @@
 #include <utility>
 #include "dctc_common.cuh"
 #include "dctc_launch.h"
+#include "dctc_resize_plan.h"
 
 // One CTA per row: shift image bytes and energy floats right of the seam one pixel to the left.
 // Chunks are processed left to right; the barrier between a chunk's loads and its stores also orders them
@@ -1132,6 +1133,13 @@ static int frames_vmaps(dctc_context* ctx, CarverFrames& f)
     return DCTC_OK;
 }
 
+// frames_vmaps unless the maps are as it left them (only the seam loop's map update changes them, and it counts depth)
+static int frames_fresh_vmaps(dctc_context* ctx, CarverFrames& f)
+{
+    if (f.raw && f.depth == 0 && f.vs_w == f.w0 && f.w == f.w0) return DCTC_OK;
+    return frames_vmaps(ctx, f);
+}
+
 // A carver session keeps one arithmetic for the whole seam loop: the per-seam band updates run in the FP32 tile kernel, so
 // full maps use the bit-identical FP32 march kernel rather than the tensor-core kernel (liblqr: update_emap must reproduce
 // what build_emap would give on the carved image).
@@ -1216,10 +1224,13 @@ static int frames_download(dctc_context* ctx, CarverFrames& f, uint8_t* img, flo
 // liblqr changes the height by transposing the carver (lqr_carver_resize), and so does a carver session: t becomes the
 // transposes of f's frames (one launch), with the full energy maps of the transposed images (one K1 launch with the
 // session's operator, not a transpose of f's maps: the operator's window is not symmetric) and, with vmaps, fresh visibility
-// maps.  The width seam loop then runs on t unchanged.  t is allocated when it has no frames yet (a batch keeps it).
+// maps.  The width seam loop then runs on t unchanged.  f may be carved or enlarged (dctc_carver_resize switches the
+// axis on the frame its width passes left).  t is allocated when it has no frames of f's transposed size yet (a batch
+// keeps it).
 static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFrames& t, const DctcK1Op& op, bool vmaps)
 {
-    if (!t.img) {
+    if (!t.img || t.w0 != f.h || t.h != f.w) {
+        frames_free(t);
         frames_init(t, f.n, f.h, f.w, f.ch);
         t.transposed = true;
         const int rc = frames_alloc(ctx, t);
@@ -1505,6 +1516,22 @@ int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pit
     return DCTC_OK;
 }
 
+// The single session's axis switch: its frame is replaced by its transpose (frames_transpose).  A failure leaves the
+// session unloaded.
+static int carver_transpose(dctc_context* ctx)
+{
+    CarverFrames* t = new (std::nothrow) CarverFrames;
+    if (!t) return DCTC_ERR_NOMEM;
+    const int rc = frames_transpose(ctx, *ctx->carver, *t, carver_op(ctx->op), false);
+    frames_free(*ctx->carver);
+    delete ctx->carver;
+    ctx->carver = t;
+    ctx->mirror_valid = false;
+    ctx->c_m_valid = false;
+    if (rc) dctc_carver_release(ctx);
+    return rc;
+}
+
 // Checks of a single-session seam operation along `axis` (n_seams > 0, a session loaded): the other axis fixed since the
 // load, n_seams >= the image's extent along the axis, an extent wider than the seam DP covers.  Then the operation fixes
 // the axis, and the first height operation replaces the session's frame by its transpose.  A failed switch leaves the
@@ -1518,35 +1545,25 @@ static int carver_axis(dctc_context* ctx, int axis, int n_seams)
     if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
     CK(ctx, cudaSetDevice(ctx->device));
     if (axis == DCTC_AXIS_HEIGHT && ctx->c_axis == DCTC_AXIS_NONE) {
-        CarverFrames* t = new (std::nothrow) CarverFrames;
-        if (!t) return DCTC_ERR_NOMEM;
-        const int rc = frames_transpose(ctx, f, *t, carver_op(ctx->op), false);
-        frames_free(*ctx->carver);
-        delete ctx->carver;
-        ctx->carver = t;
-        ctx->mirror_valid = false;
-        ctx->c_m_valid = false;
-        if (rc) {
-            dctc_carver_release(ctx);
-            return rc;
-        }
+        const int rc = carver_transpose(ctx);
+        if (rc) return rc;
     }
     ctx->c_axis = axis;
     return DCTC_OK;
 }
 
-// A resize after carver_axis: the seam loop on the session's current frame
-static int carver_resize(dctc_context* ctx, int n_seams, int* seams_out)
+// A resize after carver_axis: the seam loop on the session's current frame, recording the visibility map when vmaps
+static int carver_resize(dctc_context* ctx, int n_seams, int* seams_out, bool vmaps)
 {
     CarverFrames* f = ctx->carver;
-    if (ctx->c_dump_vmaps && !f->raw) {
+    if (vmaps && !f->raw) {
         if (f->w != f->w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
         const int rc = frames_vmaps(ctx, *f);
         if (rc) return rc;
     }
     ctx->mirror_valid = false;
     if (!ctx->c_incremental) ctx->c_m_valid = false;
-    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_dump_vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
+    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
 }
 
 // An enlarge after carver_axis: frames_enlarge, after which the session continues on the
@@ -1599,7 +1616,36 @@ static int carver_seams(dctc_context* ctx, int axis, bool enlarge, int n_seams, 
     if (enlarge && f->w != f->w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded (or enlarged) frame
     const int rc = carver_axis(ctx, axis, n_seams);
     if (rc) return rc;
-    return enlarge ? carver_enlarge(ctx, n_seams, seams_out) : carver_resize(ctx, n_seams, seams_out);
+    return enlarge ? carver_enlarge(ctx, n_seams, seams_out) : carver_resize(ctx, n_seams, seams_out, ctx->c_dump_vmaps);
+}
+
+// The plan of dctc_carver_resize / dctc_carver_batch_resize from w x h (plan holds DCTC_RESIZE_MAX_PASSES), with every
+// pass's extent along its axis checked against the seam DP's reach before any work
+static int resize_plan(int w, int h, int new_w, int new_h, DctcResizePass* plan, int* n_passes)
+{
+    const int n = dctc_resize_passes(w, h, new_w, new_h, plan, DCTC_RESIZE_MAX_PASSES);
+    if (n < 0) return n;
+    for (int i = 0; i < n; i++)
+        if ((plan[i].axis == DCTC_RESIZE_WIDTH ? plan[i].w : plan[i].h) > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
+    *n_passes = n;
+    return DCTC_OK;
+}
+
+// The passes of dctc_carver_resize on the single session: the per-axis helpers, the axis switch on the current frame,
+// and each pass's map read back before the next pass replaces the frame
+static int carver_passes(dctc_context* ctx, const DctcResizePass* plan, int n, int* seams_out, int* vmaps_out)
+{
+    for (int i = 0; i < n; i++) {
+        const DctcResizePass& p = plan[i];
+        int rc = DCTC_OK;
+        if (p.axis == DCTC_RESIZE_HEIGHT && !ctx->carver->transposed) rc = carver_transpose(ctx);
+        int* seams = seams_out ? seams_out + p.seams_offset : nullptr;
+        if (rc == DCTC_OK)
+            rc = p.enlarge ? carver_enlarge(ctx, p.n_seams, seams) : carver_resize(ctx, p.n_seams, seams, vmaps_out != nullptr);
+        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *ctx->carver, nullptr, nullptr, vmaps_out + p.vmap_offset);
+        if (rc) return rc;
+    }
+    return DCTC_OK;
 }
 
 extern "C" {
@@ -1640,7 +1686,8 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
 {
     if (!ctx || !seam_x) return DCTC_ERR_INVALID;
     CarverFrames* f = ctx->carver;
-    if (!f || f->w <= 1 || ctx->c_axis == DCTC_AXIS_HEIGHT) return DCTC_ERR_STATE;   // vertical seams only
+    if (!f || f->w <= 1 || ctx->c_axis == DCTC_AXIS_HEIGHT || ctx->c_axis == DCTC_AXIS_RESIZED)   // vertical seams only
+        return DCTC_ERR_STATE;
     const DctcK1Op op = carver_op(ctx->op);
     const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
     int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * 32);
@@ -1703,6 +1750,30 @@ int dctc_carver_enlarge_height(dctc_context* ctx, int n_seams, int* seams_out)
     return carver_seams(ctx, DCTC_AXIS_HEIGHT, true, n_seams, seams_out);
 }
 
+int dctc_resize_plan(int w, int h, int new_w, int new_h, DctcResizePass* passes, int max_passes)
+{
+    return dctc_resize_passes(w, h, new_w, new_h, passes, max_passes);
+}
+
+int dctc_carver_resize(dctc_context* ctx, int new_w, int new_h, int* seams_out, int* vmaps_out)
+{
+    if (!ctx || new_w <= 0 || new_h <= 0) return DCTC_ERR_INVALID;
+    const CarverFrames* f = ctx->carver;
+    if (!f || ctx->c_axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
+    DctcResizePass plan[DCTC_RESIZE_MAX_PASSES];
+    int n = 0;
+    int rc = resize_plan(f->w, f->h, new_w, new_h, plan, &n);
+    if (rc || n == 0) return rc;
+    CK(ctx, cudaSetDevice(ctx->device));
+    rc = carver_passes(ctx, plan, n, seams_out, vmaps_out);
+    if (rc) {
+        dctc_carver_release(ctx);
+        return rc;
+    }
+    ctx->c_axis = DCTC_AXIS_RESIZED;
+    return DCTC_OK;
+}
+
 int dctc_carver_set_incremental(dctc_context* ctx, int on)
 {
     if (!ctx) return DCTC_ERR_INVALID;
@@ -1735,7 +1806,7 @@ int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
 {
     if (!ctx) return DCTC_ERR_INVALID;
     CarverFrames* f = ctx->carver;
-    if (!f || !f->vs) return DCTC_ERR_STATE;
+    if (!f || !f->vs || ctx->c_axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // dctc_carver_resize returned its maps
     const int rc = frames_download(ctx, *f, nullptr, nullptr, vmap_out);
     if (rc == DCTC_OK && depth_out) *depth_out = f->depth;
     return rc;
@@ -1745,7 +1816,7 @@ int dctc_carver_paint_seams(dctc_context* ctx, uint8_t* img, int channels, size_
 {
     if (!ctx || !img || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
     CarverFrames* f = ctx->carver;
-    if (!f || !f->vs || f->depth <= 0) return DCTC_ERR_STATE;
+    if (!f || !f->vs || f->depth <= 0 || ctx->c_axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;
     CK(ctx, cudaSetDevice(ctx->device));
     Plane vs;   // the map in image orientation, row pitch = its width
     const int rc = frames_oriented(ctx, *f, f->vs, sizeof(int) * f->vs_w, f->vs_w, sizeof(int), vs);
@@ -1810,6 +1881,11 @@ struct dctc_carver_batch {
     uint8_t* start_img = nullptr;
     size_t start_bytes = 0;
     CarverFrames wide;
+    // dctc_carver_batch_resize: the second enlarged set (consecutive enlarge passes alternate between wide and wide2,
+    // each reading the previous pass's frames; allocated by the first such pair) and the frames the call left (null
+    // until then; no seam operation until the next load)
+    CarverFrames wide2;
+    CarverFrames* resized = nullptr;
 };
 
 namespace {
@@ -1818,6 +1894,7 @@ namespace {
 CarverFrames& batch_src(dctc_carver_batch* b) { return b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f; }
 const CarverFrames& batch_frames(const dctc_carver_batch* b)
 {
+    if (b->resized) return *b->resized;
     return b->enlarged ? b->wide : b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f;
 }
 CarverFrames& batch_frames(dctc_carver_batch* b) { return const_cast<CarverFrames&>(batch_frames((const dctc_carver_batch*) b)); }
@@ -1827,6 +1904,7 @@ void batch_free(dctc_carver_batch* b)
     frames_free(b->f);
     frames_free(b->t);
     frames_free(b->wide);
+    frames_free(b->wide2);
     cudaFree(b->start_img);
 }
 
@@ -1852,11 +1930,11 @@ int batch_axis(dctc_carver_batch* b, int axis, int n_seams)
     return DCTC_OK;
 }
 
-// Device work of dctc_carver_batch_enlarge_width / _height
-int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
+// Device work of dctc_carver_batch_enlarge_width / _height and of an enlarge pass of dctc_carver_batch_resize: f's frames
+// enlarged into wide
+int batch_enlarge(dctc_carver_batch* b, CarverFrames& f, CarverFrames& wide, int n_seams, int* seams_out)
 {
     dctc_context* ctx = b->ctx;
-    CarverFrames& f = batch_src(b);
     const int w1 = f.w0 + n_seams;
     if (b->start_bytes != f.img_fs * f.n) {
         cudaFree(b->start_img);
@@ -1864,21 +1942,21 @@ int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
         CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
         b->start_bytes = f.img_fs * f.n;
     }
-    if (b->wide.w0 != w1 || b->wide.h != f.h) {
-        frames_free(b->wide);
-        frames_init(b->wide, f.n, w1, f.h, f.ch);
-        const int rc = frames_alloc(ctx, b->wide);
+    if (wide.w0 != w1 || wide.h != f.h) {
+        frames_free(wide);
+        frames_init(wide, f.n, w1, f.h, f.ch);
+        const int rc = frames_alloc(ctx, wide);
         if (rc) {
-            frames_free(b->wide);
+            frames_free(wide);
             return rc;
         }
     }
-    b->wide.transposed = f.transposed;
-    if (!b->dump_vmaps) {   // (a batch with dump_vmaps had its maps reset by the load, and no seam was removed since)
-        const int rc = frames_vmaps(ctx, f);
-        if (rc) return rc;
-    }
-    return frames_enlarge(ctx, f, b->op, n_seams, seams_out, nullptr, b->start_img, b->wide);
+    wide.w = wide.w0;   // (a set a previous pass of dctc_carver_batch_resize carved)
+    wide.transposed = f.transposed;
+    // (a batch with dump_vmaps had its maps reset by the load or the axis switch, and no seam was removed since)
+    const int rc = frames_fresh_vmaps(ctx, f);
+    if (rc) return rc;
+    return frames_enlarge(ctx, f, b->op, n_seams, seams_out, nullptr, b->start_img, wide);
 }
 
 // The batch's resize and enlarge calls.  An enlarge carves the frames in place: until every frame is enlarged the batch is
@@ -1886,17 +1964,48 @@ int batch_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out)
 int batch_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out)
 {
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged) return DCTC_ERR_STATE;
+    if (!b->loaded || b->enlarged || b->resized) return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
     if (enlarge && batch_src(b).w != batch_src(b).w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
     int rc = batch_axis(b, axis, n_seams);
     if (rc) return rc;
     if (!enlarge) return seam_loop(b->ctx, batch_src(b), b->op, n_seams, seams_out, b->dump_vmaps, nullptr);
     b->loaded = false;
-    rc = batch_enlarge(b, n_seams, seams_out);
+    rc = batch_enlarge(b, batch_src(b), b->wide, n_seams, seams_out);
     if (rc) return rc;
     b->enlarged = true;
     b->loaded = true;
+    return DCTC_OK;
+}
+
+// The passes of dctc_carver_batch_resize, moving between the batch's frame sets: the loaded frames, their transposes
+// (filled from the current frames at the axis switch) and the two enlarged sets; each pass's maps are read back before
+// the next pass reuses the set they live in.  Maps are recorded when vmaps_out is given, whatever dump_vmaps says.
+int batch_passes(dctc_carver_batch* b, const DctcResizePass* plan, int n, int* seams_out, int* vmaps_out)
+{
+    dctc_context* ctx = b->ctx;
+    const size_t nf = (size_t) b->f.n;
+    CarverFrames* cur = &b->f;
+    for (int i = 0; i < n; i++) {
+        const DctcResizePass& p = plan[i];
+        int rc = DCTC_OK;
+        if (p.axis == DCTC_RESIZE_HEIGHT && !cur->transposed) {
+            rc = frames_transpose(ctx, *cur, b->t, b->op, false);
+            cur = &b->t;
+        }
+        CarverFrames* src = cur;
+        int* seams = seams_out ? seams_out + nf * p.seams_offset : nullptr;
+        if (rc == DCTC_OK && p.enlarge) {
+            cur = cur == &b->wide ? &b->wide2 : &b->wide;
+            rc = batch_enlarge(b, *src, *cur, p.n_seams, seams);
+        } else if (rc == DCTC_OK) {
+            if (vmaps_out) rc = frames_fresh_vmaps(ctx, *src);
+            if (rc == DCTC_OK) rc = seam_loop(ctx, *src, b->op, p.n_seams, seams, vmaps_out != nullptr, nullptr);
+        }
+        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *src, nullptr, nullptr, vmaps_out + nf * p.vmap_offset);
+        if (rc) return rc;
+    }
+    b->resized = cur;
     return DCTC_OK;
 }
 
@@ -1951,6 +2060,7 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = false;
     b->enlarged = false;
+    b->resized = nullptr;
     b->axis = DCTC_AXIS_NONE;
     b->op = carver_op(ctx->op);
     f.w = f.w0;
@@ -1988,6 +2098,23 @@ int dctc_carver_batch_enlarge_height(dctc_carver_batch* b, int n_seams, int* sea
     return batch_seams(b, DCTC_AXIS_HEIGHT, true, n_seams, seams_out);
 }
 
+int dctc_carver_batch_resize(dctc_carver_batch* b, int new_w, int new_h, int* seams_out, int* vmaps_out)
+{
+    if (!b || new_w <= 0 || new_h <= 0) return DCTC_ERR_INVALID;
+    if (!b->loaded || b->enlarged || b->resized || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
+    DctcResizePass plan[DCTC_RESIZE_MAX_PASSES];
+    int n = 0;
+    int rc = resize_plan(b->f.w, b->f.h, new_w, new_h, plan, &n);
+    if (rc || n == 0) return rc;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    b->loaded = false;
+    rc = batch_passes(b, plan, n, seams_out, vmaps_out);
+    if (rc) return rc;
+    b->loaded = true;
+    return DCTC_OK;
+}
+
 int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
@@ -2005,7 +2132,7 @@ int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
 int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
 {
     if (!b) return DCTC_ERR_INVALID;
-    if (!b->loaded || !b->dump_vmaps) return DCTC_ERR_STATE;
+    if (!b->loaded || !b->dump_vmaps || b->resized) return DCTC_ERR_STATE;   // dctc_carver_batch_resize returned its maps
     CarverFrames& f = batch_src(b);
     const int rc = frames_download(b->ctx, f, nullptr, nullptr, vmap_out);
     if (rc == DCTC_OK && depth_out) *depth_out = f.depth;

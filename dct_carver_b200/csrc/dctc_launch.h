@@ -132,8 +132,8 @@ struct CarverFrames {
 };
 
 // The axis a carver session's seam operations work along since its load: the first one fixes it, a call for the other
-// axis returns DCTC_ERR_STATE until the next load
-enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2 };
+// axis returns DCTC_ERR_STATE until the next load.  RESIZED: dctc_carver_resize ran since the load, which fixes both axes.
+enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2, DCTC_AXIS_RESIZED = 3 };
 
 struct dctc_context {
     int device = 0;

@@ -183,6 +183,43 @@ int dctc_carver_enlarge_width(dctc_context *ctx, int n_seams, int *seams_out);
  * seam DP covers (the session stays loaded).  A CUDA failure in the first height call leaves the session unloaded. */
 int dctc_carver_resize_height(dctc_context *ctx, int n_seams, int *seams_out);
 int dctc_carver_enlarge_height(dctc_context *ctx, int n_seams, int *seams_out);
+
+/* Both axes in one call: lqr_carver_resize(carver, new_w, new_h) (src/render.c:377) as a plan of passes.  The width
+ * changes first, then the height.  Along each axis there is either one shrink pass of extent - new_extent seams, or
+ * enlarge passes of min(new_extent - extent, extent - 1) seams each until the target is reached (an enlarge covers
+ * fewer seams than the extent).  The host carver's dctc_lqr_carver_resize follows the same plan. */
+enum { DCTC_RESIZE_WIDTH = 0, DCTC_RESIZE_HEIGHT = 1 };
+typedef struct {
+    int axis;              /* DCTC_RESIZE_WIDTH (vertical seams) or DCTC_RESIZE_HEIGHT (horizontal seams) */
+    int enlarge;           /* 1: the pass inserts n_seams seams, 0: it removes them */
+    int n_seams;
+    int w, h;              /* image size at the start of the pass */
+    size_t seams_offset;   /* ints before this pass's seams in one frame's seams_out block */
+    size_t vmap_offset;    /* ints before this pass's map in one frame's vmaps_out block */
+} DctcResizePass;
+/* Plan of a resize from w x h to new_w x new_h.  Fills the first max_passes passes (passes may be NULL when max_passes
+ * is 0) and returns the number of passes, 0 when nothing changes.  A frame's seams_out needs the last pass's
+ * seams_offset + n_seams * len ints (len = h for a width pass, w for a height pass), its vmaps_out the last pass's
+ * vmap_offset + w * h ints.  DCTC_ERR_INVALID for a non-positive size or max_passes < 0; DCTC_ERR_STATE when a pass
+ * cannot make progress (an extent of 1 cannot grow). */
+int dctc_resize_plan(int w, int h, int new_w, int new_h, DctcResizePass *passes, int max_passes);
+/* Runs the plan on the session's frame, entirely on the device: the width passes as dctc_carver_resize_width /
+ * _enlarge_width run them (an enlarge pass continues on the enlarged frame), then one transpose of the current frame
+ * and one K1 launch on it (the energy rebuild a reload would do), then the height passes as the _height calls run them.
+ * Each pass gives what the per-axis call gives on a session loaded with the image the previous pass left.
+ * seams_out (may be NULL): the passes' seam logs back to back in plan order, pass p at its seams_offset, each in the
+ * layout of the per-axis call (n_seams * h ints for a width pass, n_seams * w for a height pass, coordinates at removal
+ * time).  vmaps_out (may be NULL): one visibility map per pass at its vmap_offset, over the pass's start frame in image
+ * orientation (h * w ints), values 1..n_seams in removal order, 0 = never removed; recorded whenever vmaps_out is given,
+ * whatever dctc_carver_set_dump_vmaps says.  Incremental mode applies to the shrink passes.
+ * Needs a session loaded with no seam operation since the load (DCTC_ERR_STATE otherwise).  new_w == w && new_h == h:
+ * DCTC_OK, nothing happens.  DCTC_ERR_INVALID: new_w <= 0 or new_h <= 0.  DCTC_ERR_STATE also when the plan refuses.
+ * DCTC_ERR_UNSUPPORTED: some pass's extent along its axis is wider than the device seam DP covers (checked on the plan
+ * before any work: the session stays loaded).  Afterwards dctc_carver_width / _height / _image / _energy /
+ * _energy_image, dctc_pixel_energy and dctc_set_params work on the final frame; seam operations, another
+ * dctc_carver_resize, dctc_carver_vmap and dctc_carver_paint_seams return DCTC_ERR_STATE until the next load.  A CUDA
+ * failure leaves the session unloaded. */
+int dctc_carver_resize(dctc_context *ctx, int new_w, int new_h, int *seams_out, int *vmaps_out);
 /* Optional: let the device loop update its cumulative map incrementally after each seam, like liblqr's update_mmap
  * (only the cells the removed seam can have changed are recomputed; a row whose changed range gets too wide falls
  * back to the full rebuild).  Same seams bit for bit; off by default because the full rebuild on an 8-CTA cluster is
@@ -251,6 +288,16 @@ int dctc_carver_batch_enlarge_width(dctc_carver_batch *batch, int n_seams, int *
  * dctc_carver_batch_enlarge_width apply (its buffers are reallocated when their size differs). */
 int dctc_carver_batch_resize_height(dctc_carver_batch *batch, int n_seams, int *seams_out);
 int dctc_carver_batch_enlarge_height(dctc_carver_batch *batch, int n_seams, int *seams_out);
+/* dctc_carver_resize for every frame: each frame gets exactly the seams, maps, image and energy map that
+ * dctc_carver_resize gives it alone on the same context.  Layout pass-major, then frame-major: pass p's block starts at
+ * n_frames * its offset, and inside it is what the per-axis batch call writes (n_frames * n_seams * len seams,
+ * n_frames * h * w map ints for the pass's start size).  The batch moves between frame sets: the transposed set is
+ * filled from the current frames, an enlarge pass reads the previous pass's enlarged frames, and a set is reallocated
+ * when its size differs (a batch that never calls this allocates nothing more).  Needs a loaded batch with no seam
+ * operation since the load; the errors are those of dctc_carver_resize.  Afterwards _images / _energy / _width /
+ * _height reflect the final frames; seam calls, another resize and _vmap return DCTC_ERR_STATE until
+ * dctc_carver_batch_load, which restarts the batch at its created size.  A CUDA failure leaves the batch unloaded. */
+int dctc_carver_batch_resize(dctc_carver_batch *batch, int new_w, int new_h, int *seams_out, int *vmaps_out);
 /* current width / height of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
 int dctc_carver_batch_height(const dctc_carver_batch *batch);
