@@ -31,6 +31,7 @@ ABI_SYMBOLS = [
     "dctc_carver_batch_enlarge_width", "dctc_carver_batch_width", "dctc_carver_batch_images", "dctc_carver_batch_energy",
     "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
     "dctc_resize_plan", "dctc_carver_resize", "dctc_carver_batch_resize",
+    "dctc_carver_set_bias", "dctc_carver_bias", "dctc_carver_batch_set_bias", "dctc_carver_batch_bias",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -140,6 +141,10 @@ def lib():
         "dctc_resize_plan": (i32, [i32, i32, i32, i32, vp, i32]),
         "dctc_carver_resize": (i32, [vp, i32, i32, vp, vp]),
         "dctc_carver_batch_resize": (i32, [vp, i32, i32, vp, vp]),
+        "dctc_carver_set_bias": (i32, [vp, vp, sz]),
+        "dctc_carver_bias": (i32, [vp, vp]),
+        "dctc_carver_batch_set_bias": (i32, [vp, vp, sz, sz]),
+        "dctc_carver_batch_bias": (i32, [vp, vp]),
         "dctc_pixel_energy": (f32, [i32, i32, i32, i32, vp, vp]),
         "dctc_synth_fill_dev": (i32, [vp, vp, i32, sz, i32, i32, i32, sz, u32, i32, i32, i32]),
         "dctc_synth_byte": (C.c_uint8, [u32, u32, u32, u32, u32, i32]),
@@ -245,6 +250,16 @@ def _resize(fn, handle, w, h, new_w, new_h, vmaps, n_frames):
             e["vmap"] = maps[vo:vo + nf * p["w"] * p["h"]].reshape(lead + (p["h"], p["w"]))
         out.append(e)
     return out
+
+
+def _bias_plane(bias, shape):
+    """bias as a C-contiguous float32 array of `shape`; ValueError for another shape or a non-finite value."""
+    b = np.asarray(bias, dtype=np.float32)
+    if b.shape != tuple(shape):
+        raise ValueError("bias must have shape %s, got %s" % (tuple(shape), b.shape))
+    if not np.isfinite(b).all():
+        raise ValueError("bias values must be finite")
+    return np.ascontiguousarray(b)
 
 
 def pinned_array(shape, dtype, write_combined=False):
@@ -456,6 +471,25 @@ class Context:
         w, h = self.carver_size()
         return _resize(lib().dctc_carver_resize, self._h, w, h, new_w, new_h, vmaps, None)
 
+    def carver_set_bias(self, bias):
+        """Per-pixel bias of the seam search (liblqr's lqr_carver_bias_add): float (h, w) at the current size, or None to
+        clear it.  Every seam operation then runs on energy + bias / ext, ext = the start width of the frame the seam
+        loop runs on (include/dctc.h); positive values preserve pixels, large negative values remove them first.  Needs
+        a freshly loaded session; carver_load clears the bias."""
+        if bias is None:
+            _check(lib().dctc_carver_set_bias(self._h, None, 0), "dctc_carver_set_bias")
+            return
+        w, h = self.carver_size()
+        b = _bias_plane(bias, (h, w))
+        _check(lib().dctc_carver_set_bias(self._h, _ptr(b), w * 4), "dctc_carver_set_bias")
+
+    def carver_bias(self):
+        """The current bias plane (h, w): carved, transposed back and inflated with the pixels."""
+        w, h = self.carver_size()
+        out = np.empty((h, w), np.float32)
+        _check(lib().dctc_carver_bias(self._h, _ptr(out)), "dctc_carver_bias")
+        return out
+
     def carver_set_incremental(self, on):
         """Device seam loop: update the cumulative map incrementally (liblqr's update_mmap) instead of rebuilding it."""
         _check(lib().dctc_carver_set_incremental(self._h, int(bool(on))), "dctc_carver_set_incremental")
@@ -631,6 +665,22 @@ class CarverBatch:
         [n, n_seams, len] and, with vmaps, "vmap" [n, h, w].  Needs a freshly loaded batch; afterwards no seam operation
         until the next load()."""
         return _resize(lib().dctc_carver_batch_resize, self._b, self.width, self.height, new_w, new_h, vmaps, self.n)
+
+    def set_bias(self, bias):
+        """Context.carver_set_bias for every frame: float (n, h, w0), or None to clear.  Needs a freshly loaded batch;
+        load() clears the bias."""
+        if bias is None:
+            _check(lib().dctc_carver_batch_set_bias(self._b, None, 0, 0), "dctc_carver_batch_set_bias")
+            return
+        b = _bias_plane(bias, (self.n, self.h, self.w0))
+        _check(lib().dctc_carver_batch_set_bias(self._b, _ptr(b), self.h * self.w0 * 4, self.w0 * 4),
+               "dctc_carver_batch_set_bias")
+
+    def bias(self):
+        """The current bias planes (n, height, width)."""
+        out = np.empty((self.n, self.height, self.width), np.float32)
+        _check(lib().dctc_carver_batch_bias(self._b, _ptr(out)), "dctc_carver_batch_bias")
+        return out
 
     def images(self):
         out = np.empty((self.n, self.height, self.width, self.ch), np.uint8)

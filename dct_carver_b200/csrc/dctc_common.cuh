@@ -39,6 +39,13 @@ struct DctcK1Args {
     int pdl;
 };
 
+// Band mode of a biased carver session (tile kernel only, a kernel argument of its own so that DctcK1Args and the other
+// kernels' parameters keep their layout): the stored value is e + bias[y][x] / ext, bias laid out like DctcK1Args::out.
+struct DctcK1Bias {
+    const float* bias;
+    float ext;
+};
+
 // Band limits of row y for a removed seam (seam[] in the coordinates before removal, w = width after removal).
 __host__ __device__ __forceinline__ void dctc_band_limits(const int* seam, int y, int h, int w, int r, int* xmin, int* xmax)
 {

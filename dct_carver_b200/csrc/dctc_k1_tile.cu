@@ -23,8 +23,9 @@
 #define DCTC_TILE16_P 4
 #endif
 
-template <int B, int TW, int TH, int P, bool UNIFORM>
-__global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Args a)
+// BIAS (band mode of a biased carver session): the band store writes the seam energy e + bias.bias / bias.ext
+template <int B, int TW, int TH, int P, bool UNIFORM, bool BIAS>
+__global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Args a, const DctcK1Bias bias)
 {
     DCTC_PDL_PROLOGUE();
     constexpr int NT = TW * TH / P;
@@ -132,6 +133,11 @@ __global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Ar
             if (!a.seam) {
                 out[(size_t) gy * a.out_pitch + gx] = e;
             } else if (gx >= s_xmin[y0 + p] && gx <= s_xmax[y0 + p]) {
+                if constexpr (BIAS) {
+                    const float b = bias.bias[(size_t) blockIdx.z * a.out_frame_stride + (size_t) gy * a.out_pitch + gx];
+                    out[(size_t) gy * a.out_pitch + gx] = __fadd_rn(e, __fdiv_rn(b, bias.ext));
+                    continue;   // (no band_vals: dctc_carve_and_update refuses biased sessions)
+                }
                 out[(size_t) gy * a.out_pitch + gx] = e;
                 if (a.band_vals) a.band_vals[(size_t) gy * a.band_stride + (gx - s_xmin[y0 + p])] = e;
             }
@@ -139,8 +145,8 @@ __global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Ar
     }
 }
 
-template <int B, int TW, int TH, int P>
-static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream)
+template <int B, int TW, int TH, int P, bool BIAS = false>
+static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, DctcK1Bias bias = {})
 {
     constexpr int LW = TW + B - 1, LH = TH + B - 1;
     constexpr size_t smem = sizeof(float) * (size_t) (LH * LW + B * LH * TW);
@@ -148,15 +154,23 @@ static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, 
     const int span = a.seam ? (TH + 4 * a.band_r) : a.w;
     dim3 grid((span + TW - 1) / TW, (a.h + TH - 1) / TH, n_frames), block(TW * TH / P);
     return dctc_dispatch<0>(uniform, 0, [&](auto U, auto) {   // one kernel for every channel count
-        const cudaError_t e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, U>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
+        const cudaError_t e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, U, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
         if (e != cudaSuccess) return e;
-        if (a.pdl) return dctc_launch_pdl(dctc_k1_tile_kernel<B, TW, TH, P, U>, grid, block, smem, stream, true, a);
-        dctc_k1_tile_kernel<B, TW, TH, P, U><<<grid, block, smem, stream>>>(a);
+        if (a.pdl) return dctc_launch_pdl(dctc_k1_tile_kernel<B, TW, TH, P, U, BIAS>, grid, block, smem, stream, true, a, bias);
+        dctc_k1_tile_kernel<B, TW, TH, P, U, BIAS><<<grid, block, smem, stream>>>(a, bias);
         return cudaGetLastError();
     });
 }
 
-cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream)
+// band configuration (32 x 16 tiles, two pixels per thread), with the bias store for biased carver sessions
+template <int B>
+static cudaError_t launch_band(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias)
+{
+    if (bias) return launch_tile<B, 32, 16, 2, true>(a, n_frames, uniform, stream, *bias);
+    return launch_tile<B, 32, 16, 2>(a, n_frames, uniform, stream);
+}
+
+cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
     if (n_frames > 65535 || (a.h + 31) / 32 > 65535) return cudaErrorInvalidConfiguration;
@@ -165,10 +179,10 @@ cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames
         // pixels per thread keep the per-thread chain short (8 k1 x 2 instead of 8 k1 x 8 transforms for b = 8); the
         // arithmetic per pixel is the same as in the full-map configuration (bit-identical energies)
         switch (blocksize) {
-        case 2: return launch_tile<2, 32, 16, 2>(a, n_frames, uniform, stream);
-        case 4: return launch_tile<4, 32, 16, 2>(a, n_frames, uniform, stream);
-        case 8: return launch_tile<8, 32, 16, 2>(a, n_frames, uniform, stream);
-        case 16: return launch_tile<16, 32, 16, 2>(a, n_frames, uniform, stream);
+        case 2: return launch_band<2>(a, n_frames, uniform, stream, bias);
+        case 4: return launch_band<4>(a, n_frames, uniform, stream, bias);
+        case 8: return launch_band<8>(a, n_frames, uniform, stream, bias);
+        case 16: return launch_band<16>(a, n_frames, uniform, stream, bias);
         default: return cudaErrorInvalidValue;
         }
     }

@@ -20,18 +20,36 @@
 // after the previous chunk's loads, so the one-element overlap between neighbouring chunks is safe.
 // Batch sessions: blockIdx.y = frame, whose planes start img_fs bytes / en_fs, m_fs floats after the previous frame's
 // and whose seam is seam[h * frame ...] (h = gridDim.x).
-template <int NT, int K>
+// BIAS: the bias plane of a biased session (laid out like the energy plane) is compacted too.
+template <int NT, int K, bool BIAS>
 __global__ void __launch_bounds__(NT) dctc_carve_rows_kernel(uint8_t* __restrict__ img, size_t pitch, int channels,
                                                              float* __restrict__ en, size_t en_pitch,
                                                              const int* __restrict__ seam, int w_old,
                                                              float* __restrict__ mplane, size_t m_pitch,
-                                                             size_t img_fs, size_t en_fs, size_t m_fs)
+                                                             size_t img_fs, size_t en_fs, size_t m_fs, float* __restrict__ bias)
 {
     DCTC_PDL_PROLOGUE();
     const int y = blockIdx.x, z = blockIdx.y;
     const int s = seam[(size_t) z * gridDim.x + y];
     uint8_t* row = img + z * img_fs + (size_t) y * pitch;
     float* erow = en + z * en_fs + (size_t) y * en_pitch;
+    if constexpr (BIAS) {
+        float* brow = bias + z * en_fs + (size_t) y * en_pitch;
+        for (int base = s; base < w_old - 1; base += NT * K) {
+            float v[K];
+#pragma unroll
+            for (int k = 0; k < K; k++) {
+                const int x = base + k * NT + threadIdx.x;
+                v[k] = x < w_old - 1 ? brow[x + 1] : 0.0f;
+            }
+            __syncthreads();
+#pragma unroll
+            for (int k = 0; k < K; k++) {
+                const int x = base + k * NT + threadIdx.x;
+                if (x < w_old - 1) brow[x] = v[k];
+            }
+        }
+    }
     // cumulative map of the seam DP (liblqr keeps it per pixel, so it moves with the pixels): dst x in [s, w_old-1)
     if (mplane) {
         float* mrow = mplane + z * m_fs + (size_t) y * m_pitch;
@@ -1030,9 +1048,14 @@ __global__ void __launch_bounds__(256) dctc_paint_seams_kernel(uint8_t* __restri
 // original row (a copy in column 0).  One CTA per row: block-wide prefix sum of the "seam pixel" flags gives every
 // original pixel its output column.  Batch sessions: blockIdx.y = frame, whose source image, visibility map and output
 // image start orig_fs bytes, vs_fs ints and out_fs bytes after the previous frame's.
+// BIAS: the bias planes of a biased session are inflated in the same pass with the copy rule (both copies of a doubled
+// pixel carry its bias): borig rows bpitch floats and frames bfs floats apart, bout rows bout_pitch and frames bout_fs.
+template <bool BIAS>
 __global__ void __launch_bounds__(256) dctc_inflate_rows_kernel(const uint8_t* __restrict__ orig, size_t pitch, int channels, int w0,
                                                                 const int* __restrict__ vs, int n, uint8_t* __restrict__ out, size_t out_pitch,
-                                                                size_t orig_fs, size_t vs_fs, size_t out_fs)
+                                                                size_t orig_fs, size_t vs_fs, size_t out_fs,
+                                                                const float* __restrict__ borig, size_t bpitch, size_t bfs,
+                                                                float* __restrict__ bout, size_t bout_pitch, size_t bout_fs)
 {
     __shared__ int wsum[8];
     __shared__ int running;
@@ -1065,11 +1088,30 @@ __global__ void __launch_bounds__(256) dctc_inflate_rows_kernel(const uint8_t* _
                 q += channels;
             }
             for (int c = 0; c < channels; c++) q[c] = p[c];
+            if constexpr (BIAS) {
+                const float b = borig[z * bfs + (size_t) y * bpitch + x];
+                float* bq = bout + z * bout_fs + (size_t) y * bout_pitch + pos;
+                bq[0] = b;
+                if (flag) bq[1] = b;
+            }
         }
         __syncthreads();
         if (tid == 255) running = before + inc;
         __syncthreads();
     }
+}
+
+// ---- bias (lqr_carver_bias_add: preserve / discard masks) ------------------------------------------------------------
+// The seam energy of a biased session, after a full K1 of its frames: en = fl(en + fl(bias / ext)), ext = the frames'
+// start width.  __fdiv_rn / __fadd_rn: IEEE division and add whatever the compiler flags (the band K1's bias store
+// computes the same).  blockIdx.y = row, blockIdx.z = frame (planes fs floats apart).
+__global__ void __launch_bounds__(256) dctc_bias_add_kernel(float* __restrict__ en, const float* __restrict__ bias, size_t pitch,
+                                                            size_t fs, int w, float ext)
+{
+    const int x = blockIdx.x * 256 + threadIdx.x;
+    if (x >= w) return;
+    const size_t i = blockIdx.z * fs + (size_t) blockIdx.y * pitch + x;
+    en[i] = __fadd_rn(en[i], __fdiv_rn(bias[i], ext));
 }
 
 // ---- carver sessions: host side -------------------------------------------------------------------------------------
@@ -1094,7 +1136,7 @@ static void frames_init(CarverFrames& f, int n, int w, int h, int ch)
 static void frames_free(CarverFrames& f)
 {
     cudaFree(f.img); cudaFree(f.en); cudaFree(f.m); cudaFree(f.dir); cudaFree(f.seam); cudaFree(f.xlast);
-    cudaFree(f.seam_log); cudaFree(f.raw); cudaFree(f.vs); cudaFree(f.scratch);
+    cudaFree(f.seam_log); cudaFree(f.raw); cudaFree(f.vs); cudaFree(f.scratch); cudaFree(f.bias); cudaFree(f.en_op);
     f = CarverFrames();
 }
 
@@ -1166,10 +1208,46 @@ static DctcK1Args frames_k1_args(const CarverFrames& f, const DctcK1Op& op, cons
     return a;
 }
 
+// The frames' energy planes from scratch: one K1 launch, and for biased frames one bias-add launch that turns the
+// operator map into the seam energy
 static int frames_full_energy(dctc_context* ctx, const CarverFrames& f, const DctcK1Op& op)
 {
     DctcK1Args a = frames_k1_args(f, op, nullptr);
-    return dctc_run_k1(ctx, op, a, f.n, ctx->stream);
+    const int rc = dctc_run_k1(ctx, op, a, f.n, ctx->stream);
+    if (rc || !f.bias) return rc;
+    dctc_bias_add_kernel<<<dim3((f.w + 255) / 256, f.h, f.n), 256, 0, ctx->stream>>>(f.en, f.bias, f.en_pitch, f.en_pitch * f.h, f.w,
+                                                                                     (float) f.w0);
+    CK(ctx, cudaGetLastError());
+    ctx->launches++;
+    return DCTC_OK;
+}
+
+// The operator energy maps of the frames: their energy planes, or for biased frames (whose planes hold the seam energy)
+// one full K1 of the current images into en_op.  Band updates equal a full recompute bit for bit, so this is the map the
+// frames would hold without a bias.
+static int frames_op_energy(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, const float** plane)
+{
+    *plane = f.en;
+    if (!f.bias) return DCTC_OK;
+    if (!f.en_op) CK(ctx, cudaMalloc((void**) &f.en_op, sizeof(float) * f.en_pitch * f.h * f.n));
+    DctcK1Args a = frames_k1_args(f, op, nullptr);
+    a.out = f.en_op;
+    const int rc = dctc_run_k1(ctx, op, a, f.n, ctx->stream);
+    if (rc) return rc;
+    *plane = f.en_op;
+    return DCTC_OK;
+}
+
+// Gives `to` a bias plane (laid out like its energy planes) when `from` has one, and none otherwise
+static int frames_bias_like(dctc_context* ctx, const CarverFrames& from, CarverFrames& to)
+{
+    if (!from.bias) {
+        cudaFree(to.bias);
+        to.bias = nullptr;
+    } else if (!to.bias) {
+        CK(ctx, cudaMalloc((void**) &to.bias, sizeof(float) * to.en_pitch * to.h * to.n));
+    }
+    return DCTC_OK;
 }
 
 // ---- the way out: everything the caller sees is in image orientation --------------------------------------------------
@@ -1201,13 +1279,20 @@ static int frames_oriented(dctc_context* ctx, CarverFrames& f, const void* plane
     return DCTC_OK;
 }
 
-// Images (w * ch bytes per row), energy planes (w floats per row) and visibility maps (vs_w ints per row) of all frames,
-// in image orientation, to the host
-static int frames_download(dctc_context* ctx, CarverFrames& f, uint8_t* img, float* en, int* vs)
+// Images (w * ch bytes per row), operator energy maps (w floats per row, frames_op_energy with op), visibility maps (vs_w
+// ints per row) and bias planes (w floats per row) of all frames, in image orientation, to the host
+static int frames_download(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, uint8_t* img, float* en, int* vs,
+                           float* bias = nullptr)
 {
     CK(ctx, cudaSetDevice(ctx->device));
-    struct { void* dst; const void* src; size_t pitch; int cols, esize; } planes[3] = {
-        {img, f.img, f.pitch, f.w, f.ch}, {en, f.en, sizeof(float) * f.en_pitch, f.w, 4}, {vs, f.vs, sizeof(int) * f.vs_w, f.vs_w, 4}};
+    const float* en_src = f.en;
+    if (en) {
+        const int rc = frames_op_energy(ctx, f, op, &en_src);
+        if (rc) return rc;
+    }
+    struct { void* dst; const void* src; size_t pitch; int cols, esize; } planes[4] = {
+        {img, f.img, f.pitch, f.w, f.ch}, {en, en_src, sizeof(float) * f.en_pitch, f.w, 4}, {vs, f.vs, sizeof(int) * f.vs_w, f.vs_w, 4},
+        {bias, f.bias, sizeof(float) * f.en_pitch, f.w, 4}};
     for (const auto& q : planes) {
         if (!q.dst) continue;
         Plane p;
@@ -1226,7 +1311,8 @@ static int frames_download(dctc_context* ctx, CarverFrames& f, uint8_t* img, flo
 // session's operator, not a transpose of f's maps: the operator's window is not symmetric) and, with vmaps, fresh visibility
 // maps.  The width seam loop then runs on t unchanged.  f may be carved or enlarged (dctc_carver_resize switches the
 // axis on the frame its width passes left).  t is allocated when it has no frames of f's transposed size yet (a batch
-// keeps it).
+// keeps it).  Biased frames: the bias planes are transposed too (one more launch) and t's seam energy uses ext = t.w0,
+// the image height (one bias-add launch after the K1).
 static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFrames& t, const DctcK1Op& op, bool vmaps)
 {
     if (!t.img || t.w0 != f.h || t.h != f.w) {
@@ -1239,7 +1325,14 @@ static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFram
     t.w = t.w0;
     CK(ctx, dctc_launch_transpose(f.img, f.pitch, f.img_fs, t.img, t.pitch, t.img_fs, f.w, f.h, f.n, f.ch, ctx->stream));
     ctx->launches++;
-    int rc = frames_full_energy(ctx, t, op);
+    int rc = frames_bias_like(ctx, f, t);
+    if (rc) return rc;
+    if (f.bias) {
+        const size_t fp = sizeof(float) * f.en_pitch, tp = sizeof(float) * t.en_pitch;
+        CK(ctx, dctc_launch_transpose(f.bias, fp, fp * f.h, t.bias, tp, tp * t.h, f.w, f.h, f.n, sizeof(float), ctx->stream));
+        ctx->launches++;
+    }
+    rc = frames_full_energy(ctx, t, op);
     if (rc == DCTC_OK && vmaps) rc = frames_vmaps(ctx, t);
     return rc;
 }
@@ -1412,8 +1505,9 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
             ctx->launches++;
         }
         // carve: compact image and energy rows (and the cumulative rows of the incremental map) over the seam
-        CK(ctx, dctc_launch_pdl(dctc_carve_rows_kernel<256, 4>, dim3(h, n), dim3(256), 0, ctx->stream, pdl, f.img, f.pitch, f.ch, f.en,
-                                f.en_pitch, f.seam, w_old, incr ? f.m : (float*) nullptr, f.m_pitch, f.img_fs, en_fs, m_fs));
+        CK(ctx, dctc_launch_pdl(f.bias ? dctc_carve_rows_kernel<256, 4, true> : dctc_carve_rows_kernel<256, 4, false>, dim3(h, n), dim3(256),
+                                0, ctx->stream, pdl, f.img, f.pitch, f.ch, f.en, f.en_pitch, f.seam, w_old, incr ? f.m : (float*) nullptr,
+                                f.m_pitch, f.img_fs, en_fs, m_fs, f.bias));
         ctx->launches += 2;
         f.w = w_old - 1;
         if (incr_valid) *incr_valid = incr;   // the plane now holds the map of the image before this removal, moved with the pixels
@@ -1423,7 +1517,8 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         // update_emap: K1 in band mode around every frame's removed seam
         DctcK1Args a = frames_k1_args(f, op, f.seam);
         a.pdl = pdl ? 1 : 0;
-        rc = dctc_run_k1(ctx, op, a, n, ctx->stream);
+        const DctcK1Bias bias{f.bias, (float) f.w0};   // biased frames: the band store writes the seam energy
+        rc = dctc_run_k1(ctx, op, a, n, ctx->stream, f.bias ? &bias : nullptr);
         if (rc) return rc;
 #ifdef DCTC_SYNC_DEBUG
         { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: band kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
@@ -1439,17 +1534,54 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
 // frames are copied to start_img, the seam loop removes n_seams seams and records their order in the visibility maps (as
 // frames_vmaps leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images
 // (w0 + n_seams wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
+// Biased frames: a copy of the start bias planes is inflated in the same launch (copy rule) into wide's bias planes, and
+// one bias-add launch gives wide's seam energy with ext = wide.w0.
 static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, bool* incr_valid,
                           uint8_t* start_img, CarverFrames& wide)
 {
     CK(ctx, cudaMemcpyAsync(start_img, f.img, f.img_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream));
-    int rc = seam_loop(ctx, f, op, n_seams, seams_out, true, incr_valid);
+    const size_t en_fs = f.en_pitch * f.h;
+    float* start_bias = nullptr;
+    int rc = frames_bias_like(ctx, f, wide);
+    if (rc == DCTC_OK && f.bias) {
+        cudaError_t e = cudaMalloc((void**) &start_bias, sizeof(float) * en_fs * f.n);
+        if (e == cudaSuccess) e = cudaMemcpyAsync(start_bias, f.bias, sizeof(float) * en_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream);
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+    }
+    if (rc == DCTC_OK) rc = seam_loop(ctx, f, op, n_seams, seams_out, true, incr_valid);
+    if (rc == DCTC_OK) {
+        auto inflate = f.bias ? dctc_inflate_rows_kernel<true> : dctc_inflate_rows_kernel<false>;
+        inflate<<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(start_img, f.pitch, f.ch, f.w0, f.vs, n_seams, wide.img, wide.pitch, f.img_fs,
+                                                         (size_t) f.w0 * f.h, wide.img_fs, start_bias, f.en_pitch, en_fs, wide.bias,
+                                                         wide.en_pitch, wide.en_pitch * wide.h);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+        ctx->launches++;
+    }
+    if (rc == DCTC_OK) rc = frames_full_energy(ctx, wide, op);
+    const cudaError_t es = cudaStreamSynchronize(ctx->stream);
+    cudaFree(start_bias);
     if (rc) return rc;
-    dctc_inflate_rows_kernel<<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(start_img, f.pitch, f.ch, f.w0, f.vs, n_seams, wide.img, wide.pitch,
-                                                                      f.img_fs, (size_t) f.w0 * f.h, wide.img_fs);
-    CK(ctx, cudaGetLastError());
-    ctx->launches++;
-    rc = frames_full_energy(ctx, wide, op);
+    if (es != cudaSuccess) return dctc_fail_cuda(ctx, es);
+    return DCTC_OK;
+}
+
+// dctc_carver_set_bias / dctc_carver_batch_set_bias on frames as loaded: the caller's planes (w x h floats per frame, rows
+// pitch bytes and frames fs bytes apart, any memory cudaMemcpyDefault reaches) become the bias planes and the energy
+// planes are rebuilt (frames_full_energy); null clears the bias (the planes are rebuilt when there was one).
+static int frames_set_bias(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, const float* bias, size_t fs, size_t pitch)
+{
+    if (!bias) {
+        if (!f.bias) return DCTC_OK;
+        cudaFree(f.bias);
+        f.bias = nullptr;
+    } else {
+        if (!f.bias) CK(ctx, cudaMalloc((void**) &f.bias, sizeof(float) * f.en_pitch * f.h * f.n));
+        for (int i = 0; i < f.n; i++)
+            CK(ctx, cudaMemcpy2DAsync(f.bias + (size_t) i * f.en_pitch * f.h, sizeof(float) * f.en_pitch, (const char*) bias + i * fs, pitch,
+                                      sizeof(float) * f.w, f.h, cudaMemcpyDefault, ctx->stream));
+    }
+    const int rc = frames_full_energy(ctx, f, op);
     if (rc) return rc;
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
@@ -1506,8 +1638,11 @@ static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h,
 int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pitch, int* w, int* h)
 {
     CarverFrames* f = ctx->carver;
+    const float* op_en;
+    int rc = frames_op_energy(ctx, *f, carver_op(ctx->op), &op_en);
+    if (rc) return rc;
     Plane p;
-    const int rc = frames_oriented(ctx, *f, f->en, sizeof(float) * f->en_pitch, f->w, sizeof(float), p);
+    rc = frames_oriented(ctx, *f, op_en, sizeof(float) * f->en_pitch, f->w, sizeof(float), p);
     if (rc) return rc;
     *en = (const float*) p.p;
     *en_pitch = p.pitch / sizeof(float);
@@ -1642,7 +1777,7 @@ static int carver_passes(dctc_context* ctx, const DctcResizePass* plan, int n, i
         int* seams = seams_out ? seams_out + p.seams_offset : nullptr;
         if (rc == DCTC_OK)
             rc = p.enlarge ? carver_enlarge(ctx, p.n_seams, seams) : carver_resize(ctx, p.n_seams, seams, vmaps_out != nullptr);
-        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *ctx->carver, nullptr, nullptr, vmaps_out + p.vmap_offset);
+        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, nullptr, vmaps_out + p.vmap_offset);
         if (rc) return rc;
     }
     return DCTC_OK;
@@ -1665,6 +1800,27 @@ int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int ch
     return rc;
 }
 
+int dctc_carver_set_bias(dctc_context* ctx, const float* bias, size_t pitch)
+{
+    if (!ctx) return DCTC_ERR_INVALID;
+    CarverFrames* f = ctx->carver;
+    if (!f || ctx->c_axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;   // loaded, no seam operation since
+    if (bias && pitch < sizeof(float) * f->w) return DCTC_ERR_INVALID;
+    CK(ctx, cudaSetDevice(ctx->device));
+    ctx->mirror_valid = false;
+    ctx->c_m_valid = false;
+    const int rc = frames_set_bias(ctx, *f, carver_op(ctx->op), bias, 0, pitch);
+    if (rc) dctc_carver_release(ctx);
+    return rc;
+}
+
+int dctc_carver_bias(dctc_context* ctx, float* out)
+{
+    if (!ctx || !out) return DCTC_ERR_INVALID;
+    if (!ctx->carver || !ctx->carver->bias) return DCTC_ERR_STATE;
+    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, nullptr, nullptr, out);
+}
+
 int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_w(*ctx->carver) : 0; }
 int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_h(*ctx->carver) : 0; }
 
@@ -1672,14 +1828,14 @@ int dctc_carver_energy(dctc_context* ctx, float* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
     if (!ctx->carver) return DCTC_ERR_STATE;
-    return frames_download(ctx, *ctx->carver, nullptr, out, nullptr);
+    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, out, nullptr);
 }
 
 int dctc_carver_image(dctc_context* ctx, uint8_t* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
     if (!ctx->carver) return DCTC_ERR_STATE;
-    return frames_download(ctx, *ctx->carver, out, nullptr, nullptr);
+    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), out, nullptr, nullptr);
 }
 
 int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out, int* xmin, int* xmax)
@@ -1688,6 +1844,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     CarverFrames* f = ctx->carver;
     if (!f || f->w <= 1 || ctx->c_axis == DCTC_AXIS_HEIGHT || ctx->c_axis == DCTC_AXIS_RESIZED)   // vertical seams only
         return DCTC_ERR_STATE;
+    if (f->bias) return DCTC_ERR_STATE;   // the caller's seam and the operator's band values: no place for a bias
     const DctcK1Op op = carver_op(ctx->op);
     const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
     int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * 32);
@@ -1700,8 +1857,8 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     ctx->c_axis = DCTC_AXIS_WIDTH;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpyAsync(f->seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
-    dctc_carve_rows_kernel<256, 4><<<h, 256, 0, ctx->stream>>>(f->img, f->pitch, f->ch, f->en, f->en_pitch, f->seam, w_old, nullptr,
-                                                               0, 0, 0, 0);
+    dctc_carve_rows_kernel<256, 4, false><<<h, 256, 0, ctx->stream>>>(f->img, f->pitch, f->ch, f->en, f->en_pitch, f->seam, w_old, nullptr,
+                                                                      0, 0, 0, 0, nullptr);
     CK(ctx, cudaGetLastError());
     ctx->launches++;
     f->w = w_old - 1;
@@ -1807,7 +1964,7 @@ int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
     if (!ctx) return DCTC_ERR_INVALID;
     CarverFrames* f = ctx->carver;
     if (!f || !f->vs || ctx->c_axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // dctc_carver_resize returned its maps
-    const int rc = frames_download(ctx, *f, nullptr, nullptr, vmap_out);
+    const int rc = frames_download(ctx, *f, carver_op(ctx->op), nullptr, nullptr, vmap_out);
     if (rc == DCTC_OK && depth_out) *depth_out = f->depth;
     return rc;
 }
@@ -2002,7 +2159,7 @@ int batch_passes(dctc_carver_batch* b, const DctcResizePass* plan, int n, int* s
             if (vmaps_out) rc = frames_fresh_vmaps(ctx, *src);
             if (rc == DCTC_OK) rc = seam_loop(ctx, *src, b->op, p.n_seams, seams, vmaps_out != nullptr, nullptr);
         }
-        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *src, nullptr, nullptr, vmaps_out + nf * p.vmap_offset);
+        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *src, b->op, nullptr, nullptr, vmaps_out + nf * p.vmap_offset);
         if (rc) return rc;
     }
     b->resized = cur;
@@ -2064,6 +2221,8 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     b->axis = DCTC_AXIS_NONE;
     b->op = carver_op(ctx->op);
     f.w = f.w0;
+    cudaFree(f.bias);   // a load clears the bias
+    f.bias = nullptr;
     for (int i = 0; i < f.n; i++)
         CK(ctx, cudaMemcpy2DAsync(f.img + (size_t) i * f.img_fs, f.pitch, imgs + (size_t) i * frame_stride, pitch, row, f.h,
                                   cudaMemcpyDefault, ctx->stream));
@@ -2073,6 +2232,28 @@ int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t fra
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     b->loaded = true;
     return DCTC_OK;
+}
+
+int dctc_carver_batch_set_bias(dctc_carver_batch* b, const float* bias, size_t frame_stride, size_t pitch)
+{
+    if (!b) return DCTC_ERR_INVALID;
+    if (!b->loaded || b->enlarged || b->resized || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
+    CarverFrames& f = b->f;
+    if (bias && (pitch < sizeof(float) * f.w0 || (f.n > 1 && frame_stride < pitch * f.h))) return DCTC_ERR_INVALID;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    b->loaded = false;
+    const int rc = frames_set_bias(ctx, f, b->op, bias, frame_stride, pitch);
+    if (rc) return rc;
+    b->loaded = true;
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_bias(dctc_carver_batch* b, float* out)
+{
+    if (!b || !out) return DCTC_ERR_INVALID;
+    if (!b->loaded || !batch_frames(b).bias) return DCTC_ERR_STATE;
+    return frames_download(b->ctx, batch_frames(b), b->op, nullptr, nullptr, nullptr, out);
 }
 
 int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? frames_image_w(batch_frames(b)) : 0; }
@@ -2119,14 +2300,14 @@ int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
     if (!b->loaded) return DCTC_ERR_STATE;
-    return frames_download(b->ctx, batch_frames(b), out, nullptr, nullptr);
+    return frames_download(b->ctx, batch_frames(b), b->op, out, nullptr, nullptr);
 }
 
 int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
     if (!b->loaded) return DCTC_ERR_STATE;
-    return frames_download(b->ctx, batch_frames(b), nullptr, out, nullptr);
+    return frames_download(b->ctx, batch_frames(b), b->op, nullptr, out, nullptr);
 }
 
 int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
@@ -2134,7 +2315,7 @@ int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
     if (!b) return DCTC_ERR_INVALID;
     if (!b->loaded || !b->dump_vmaps || b->resized) return DCTC_ERR_STATE;   // dctc_carver_batch_resize returned its maps
     CarverFrames& f = batch_src(b);
-    const int rc = frames_download(b->ctx, f, nullptr, nullptr, vmap_out);
+    const int rc = frames_download(b->ctx, f, b->op, nullptr, nullptr, vmap_out);
     if (rc == DCTC_OK && depth_out) *depth_out = f.depth;
     return rc;
 }

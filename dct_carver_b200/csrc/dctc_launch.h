@@ -8,6 +8,7 @@
 #include "../../include/dctc.h"
 
 struct DctcK1Args;
+struct DctcK1Bias;
 
 #define CK(ctx, call)                                             \
     do {                                                          \
@@ -78,7 +79,9 @@ static inline cudaError_t dctc_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
-cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream);
+// bias (band mode only, may be null): the band store of a biased carver session
+cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream,
+                                const DctcK1Bias* bias = nullptr);
 cudaError_t dctc_launch_k1_small(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, int sm_count, cudaStream_t stream);
 cudaError_t dctc_launch_k1_march8(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream);
 cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, int* counter, int sm_count, cudaStream_t stream);
@@ -129,6 +132,11 @@ struct CarverFrames {
     int vs_w = 0;                       // width of the frame the maps belong to (w0 when they were reset)
     void* scratch = nullptr;            // transposed frames: a plane in image orientation on its way out (4 * w0 * h bytes
                                         // per frame, allocated by the first use)
+    // bias (dctc_carver_set_bias): one float per pixel, laid out like en and carved, transposed and inflated with the
+    // pixels; null when the frames have none.  A biased set's en holds the seam energy en_op + bias / w0, and the
+    // getters compute the operator map into en_op (allocated by their first use).
+    float* bias = nullptr;
+    float* en_op = nullptr;
 };
 
 // The axis a carver session's seam operations work along since its load: the first one fixes it, a call for the other
@@ -170,12 +178,14 @@ struct dctc_context {
 };
 
 int dctc_fail_cuda(dctc_context* ctx, cudaError_t e);
-// Launches the one K1 kernel dctc_k1_select picks (dctc_k1_select.h)
-int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream);
+// Launches the one K1 kernel dctc_k1_select picks (dctc_k1_select.h); bias: band mode of a biased carver session (the
+// tile kernel's bias store)
+int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream,
+                const DctcK1Bias* bias = nullptr);
 // The layout the Small, Tc8 and Tc16 kernels (and the 1/3-channel variants of the march kernel) read: 1 or 3 channels,
 // image rows, frames and halo rows 16-byte aligned
 bool dctc_k1_fast_layout(const DctcK1Args& a);
 void dctc_carver_release(dctc_context* ctx);
 int dctc_carver_params_changed(dctc_context* ctx);   // rebuilds the resident energy map of a loaded carver session
-// The single session's energy plane in image orientation (K3 energy image): device pointer, row pitch in floats, w x h
+// The single session's operator energy plane in image orientation (K3 energy image): device pointer, row pitch in floats, w x h
 int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pitch, int* w, int* h);

@@ -228,6 +228,30 @@ int dctc_carver_set_incremental(dctc_context *ctx, int on);
 /* Number of full cumulative-map rebuilds the incremental mode fell back to since dctc_carver_load (-1 on error). */
 int dctc_carver_rebuild_count(dctc_context *ctx);
 
+/* ---- bias: preserve and discard masks (liblqr's lqr_carver_bias_add) ----------------------------------------
+ * A per-pixel float plane B that steers the seam search: every seam operation of the session (width and height resize
+ * and enlarge, split resizes, incremental mode, dctc_carver_resize) runs on
+ *     E_seam[y][x] = fl(en_op[y][x] + fl(B[y][x] / ext))      (FP32, IEEE division and add)
+ * with en_op the operator energy and ext the start width of the frame the seam loop runs on: the loaded width for width
+ * operations, the image height at the axis switch for height operations, the enlarged width for a pass after an enlarge
+ * (liblqr's en = nrg + bias / w_start, with w_start and h_start swapped by the transpose [from memory: parity unpinned]).
+ * The caller passes the value that is divided by ext.  Positive values keep pixels (a preserve mask), large negative
+ * values remove them first (a discard mask: object removal).  The plane moves with the pixels: it is carved with them,
+ * transposed at the axis switch, and an enlarge gives the inserted pixel the bias of the seam pixel it doubles.
+ * Everything that shows energy (dctc_carver_energy, _energy_image, dctc_pixel_energy, dctc_carver_batch_energy) keeps
+ * returning the operator map; on a biased session each such call computes it with one more K1 launch.
+ * Launches: a biased seam loop launches per seam exactly what an unbiased one does.  Fixed extras of a biased session:
+ * dctc_carver_set_bias one K1 and one bias-add launch; the axis switch one bias transpose and one bias add; an enlarge
+ * one bias add (its inflate launch carries the bias).  A session without a bias launches what it launched before.
+ * dctc_carver_set_bias: bias = w x h floats in image orientation, rows pitch_bytes apart, host or device memory (copied
+ * with cudaMemcpyDefault like the loads); NULL clears the bias.  The values must be finite: this call does not check
+ * them.  Needs a loaded session with no seam operation since the load (DCTC_ERR_STATE otherwise); dctc_carver_load clears
+ * the bias.  DCTC_ERR_INVALID for a pitch below w floats.  dctc_carve_and_update returns DCTC_ERR_STATE on a biased
+ * session.  A CUDA failure leaves the session unloaded. */
+int dctc_carver_set_bias(dctc_context *ctx, const float *bias, size_t pitch_bytes);
+/* The current bias plane (carved, transposed back, inflated): w * h floats, pitch w.  DCTC_ERR_STATE without a bias. */
+int dctc_carver_bias(dctc_context *ctx, float *out);
+
 /* ---- visibility map and seam display ------------------------------------------------------------------------
  * lqr_carver_set_dump_vmaps (src/render.c:374): ask the session to record, for every ORIGINAL pixel, the order in
  * which dctc_carver_resize_width removed it (1-based, 0 = still visible).  Call before the first seam is removed. */
@@ -298,6 +322,14 @@ int dctc_carver_batch_enlarge_height(dctc_carver_batch *batch, int n_seams, int 
  * _height reflect the final frames; seam calls, another resize and _vmap return DCTC_ERR_STATE until
  * dctc_carver_batch_load, which restarts the batch at its created size.  A CUDA failure leaves the batch unloaded. */
 int dctc_carver_batch_resize(dctc_carver_batch *batch, int new_w, int new_h, int *seams_out, int *vmaps_out);
+/* dctc_carver_set_bias for every frame: n_frames planes of w x h floats (the created size), frame_stride_bytes apart,
+ * rows pitch_bytes apart; NULL clears.  Every frame gets what dctc_carver_set_bias gives it on a single session.  Same
+ * state rules: a loaded batch with no seam operation since the load, dctc_carver_batch_load clears the bias.  A batch
+ * that never sets a bias allocates nothing more; its transposed and enlarged frame sets get bias planes only when the
+ * set they come from has them.  A CUDA failure leaves the batch unloaded. */
+int dctc_carver_batch_set_bias(dctc_carver_batch *batch, const float *bias, size_t frame_stride_bytes, size_t pitch_bytes);
+/* current bias planes of every frame (n_frames * h * w floats, image orientation); DCTC_ERR_STATE without a bias */
+int dctc_carver_batch_bias(dctc_carver_batch *batch, float *out);
 /* current width / height of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
 int dctc_carver_batch_height(const dctc_carver_batch *batch);
