@@ -1115,10 +1115,10 @@ __global__ void __launch_bounds__(256) dctc_bias_add_kernel(float* __restrict__ 
 }
 
 // ---- carver sessions: host side -------------------------------------------------------------------------------------
-// Both sessions keep their device state in a CarverFrames (dctc_launch.h): the context's single session one frame, a
-// batch session n equally sized frames.  The kernels above take the frame from a spare grid dimension, so one launch per
-// phase serves every frame and each frame's seam DP runs on its own cluster of DP_CL CTAs; a frame gets exactly the
-// seams, image, energy plane and visibility map whatever the number of frames around it.
+// A session keeps its device state in CarverFrames sets (dctc_launch.h) of n equally sized frames (one for the context's
+// single session).  The kernels above take the frame from a spare grid dimension, so one launch per phase serves every
+// frame and each frame's seam DP runs on its own cluster of DP_CL CTAs; a frame gets exactly the seams, image, energy
+// plane and visibility map whatever the number of frames around it.
 
 constexpr int DP_MAX_W = DP_CL * DP_MAXW * (512 - 2 * DP_R);   // widest frame the seam DP's strips cover
 
@@ -1154,9 +1154,8 @@ static int frames_alloc(dctc_context* ctx, CarverFrames& f)
     return DCTC_OK;
 }
 
-// Empty visibility maps (w0 x h ints per frame) and the identity column map raw[frame][y][x] = x.  Maps are allocated when
-// the frames have no raw map (a visibility map kept from before a single-session enlarge belongs to the narrower start
-// frame and is replaced).
+// Empty visibility maps (w0 x h ints per frame) and the identity column map raw[frame][y][x] = x, allocated when the frames
+// have none.
 static int frames_vmaps(dctc_context* ctx, CarverFrames& f)
 {
     const size_t nv = (size_t) f.w0 * f.h * f.n;
@@ -1310,8 +1309,8 @@ static int frames_download(dctc_context* ctx, CarverFrames& f, const DctcK1Op& o
 // transposes of f's frames (one launch), with the full energy maps of the transposed images (one K1 launch with the
 // session's operator, not a transpose of f's maps: the operator's window is not symmetric) and, with vmaps, fresh visibility
 // maps.  The width seam loop then runs on t unchanged.  f may be carved or enlarged (dctc_carver_resize switches the
-// axis on the frame its width passes left).  t is allocated when it has no frames of f's transposed size yet (a batch
-// keeps it).  Biased frames: the bias planes are transposed too (one more launch) and t's seam energy uses ext = t.w0,
+// axis on the frame its width passes left).  t is allocated when it has no frames of f's transposed size yet (the
+// session keeps it).  Biased frames: the bias planes are transposed too (one more launch) and t's seam energy uses ext = t.w0,
 // the image height (one bias-add launch after the K1).
 static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFrames& t, const DctcK1Op& op, bool vmaps)
 {
@@ -1440,15 +1439,22 @@ static int frames_loop_buffers(dctc_context* ctx, CarverFrames& f, const BtPlan&
     return DCTC_OK;
 }
 
+// What the caller of a seam operation brings besides the session: whether its seam loops record the visibility maps, and
+// the context's incremental cumulative map (dctc_carver_set_incremental), which only the single session has.
+struct SeamCall {
+    bool vmaps = false;
+    bool incremental = false;
+    bool* m_valid = nullptr;   // &ctx->c_m_valid (single session), null for a batch
+};
+
 // The device seam loop of every frame: removes n_seams seams from the images and energy planes (f.w shrinks by n_seams).
-// Per seam: build_mmap + build_vpath (seam DP, then jump + trace or the DP's serial walk), update_vsmap when vmaps (maps
+// Per seam: build_mmap + build_vpath (seam DP, then jump + trace or the DP's serial walk), update_vsmap when c.vmaps (maps
 // as frames_vmaps leaves them), the carve, and update_emap (band K1 around each removed seam).  The caller has checked the
 // width.
-// incr_valid, single session only: the incremental cumulative map of dctc_carver_set_incremental (its flag buffer is
-// ctx->c_band); *incr_valid says whether f.m holds the map of the image before the last removal, compacted over that seam.
-// The walk then replaces DP + jump + trace, the DP only runs when the walk gave up, and the carve also compacts f.m.
-static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, bool vmaps,
-                     bool* incr_valid)
+// c.incremental (one frame only, its flag buffer is ctx->c_band): *c.m_valid says whether f.m holds the map of the image
+// before the last removal, compacted over that seam.  The walk then replaces DP + jump + trace, the DP only runs when the
+// walk gave up, and the carve also compacts f.m.  A loop that does not keep the map up to date clears *c.m_valid.
+static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c)
 {
     const int n = f.n, h = f.h;
     const size_t log_fs = (size_t) n_seams * h, en_fs = f.en_pitch * h, m_fs = f.m_pitch * h;
@@ -1462,7 +1468,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
     int* const xlast = bt.par ? f.xlast : nullptr;
     // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
     const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
-    const bool incr = incr_valid && n == 1 && incr_smem <= 160 * 1024;
+    const bool incr = c.incremental && n == 1 && incr_smem <= 160 * 1024;
     if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
         CK(ctx, cudaFuncSetAttribute(dctc_seam_incr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
         if (!ctx->c_band) {
@@ -1474,7 +1480,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
     for (int s = 0; s < n_seams; s++) {
         const int w_old = f.w;
         int* log_s = f.seam_log + (size_t) s * h;
-        const bool walk = incr && *incr_valid;
+        const bool walk = incr && *c.m_valid;
         if (walk) {
             // update_mmap + build_vpath: walk the changed cells only; the DP below rebuilds the map only if the walk gave up
             dctc_seam_incr_kernel<<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2,
@@ -1499,7 +1505,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
 #ifdef DCTC_SYNC_DEBUG
         { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: dp kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
 #endif
-        if (vmaps) {   // update_vsmap
+        if (c.vmaps) {   // update_vsmap
             CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, f.raw, f.vs, f.w0, f.seam, w_old,
                                     ++f.depth));
             ctx->launches++;
@@ -1510,7 +1516,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
                                 f.m_pitch, f.img_fs, en_fs, m_fs, f.bias));
         ctx->launches += 2;
         f.w = w_old - 1;
-        if (incr_valid) *incr_valid = incr;   // the plane now holds the map of the image before this removal, moved with the pixels
+        if (c.m_valid) *c.m_valid = incr;   // the plane now holds the map of the image before this removal, moved with the pixels
 #ifdef DCTC_SYNC_DEBUG
         { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: carve kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
 #endif
@@ -1530,15 +1536,16 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
     return DCTC_OK;
 }
 
-// Enlarge core of both sessions (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): the start
-// frames are copied to start_img, the seam loop removes n_seams seams and records their order in the visibility maps (as
-// frames_vmaps leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images
-// (w0 + n_seams wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
+// Enlarge core (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): the start frames are copied
+// to start_img, the seam loop removes n_seams seams and records their order in the visibility maps (as frames_vmaps
+// leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images (w0 + n_seams
+// wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
 // Biased frames: a copy of the start bias planes is inflated in the same launch (copy rule) into wide's bias planes, and
 // one bias-add launch gives wide's seam energy with ext = wide.w0.
-static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, bool* incr_valid,
+static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, SeamCall c,
                           uint8_t* start_img, CarverFrames& wide)
 {
+    c.vmaps = true;
     CK(ctx, cudaMemcpyAsync(start_img, f.img, f.img_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream));
     const size_t en_fs = f.en_pitch * f.h;
     float* start_bias = nullptr;
@@ -1548,7 +1555,7 @@ static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op
         if (e == cudaSuccess) e = cudaMemcpyAsync(start_bias, f.bias, sizeof(float) * en_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream);
         if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
     }
-    if (rc == DCTC_OK) rc = seam_loop(ctx, f, op, n_seams, seams_out, true, incr_valid);
+    if (rc == DCTC_OK) rc = seam_loop(ctx, f, op, n_seams, seams_out, c);
     if (rc == DCTC_OK) {
         auto inflate = f.bias ? dctc_inflate_rows_kernel<true> : dctc_inflate_rows_kernel<false>;
         inflate<<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(start_img, f.pitch, f.ch, f.w0, f.vs, n_seams, wide.img, wide.pitch, f.img_fs,
@@ -1587,21 +1594,264 @@ static int frames_set_bias(dctc_context* ctx, CarverFrames& f, const DctcK1Op& o
     return DCTC_OK;
 }
 
-// ---- single session (the context's) --------------------------------------------------------------------------------
+// ---- the session: one type for the context's single session and for batch sessions ------------------------------------
+// A batch session (dctc_carver_batch_*) is a dctc_carver_batch of n frames, the context's single session (dctc_carver_*,
+// ctx->carver) one of one frame that each dctc_carver_load replaces.  The state machine below serves both.  The ways the
+// two APIs differ are fields set at create (dump_vmaps, ends_at_enlarge) or what a call passes (SeamCall); the single
+// session's wrappers also take the operator from the context at every call and release the session where a batch is
+// left unloaded.
+
+// The axis the seam operations work along since the load: the first one fixes it, a call for the other axis returns
+// DCTC_ERR_STATE until the next load.  RESIZED: a combined resize ran since the load, which fixes both axes.
+enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2, DCTC_AXIS_RESIZED = 3 };
+
+// Frame sets are allocated by their first use, reallocated when their size differs and freed with the session: the
+// loaded frames f next to their transposes t, and the start frames' copy next to the enlarged sets.
+struct dctc_carver_batch {
+    dctc_context* ctx = nullptr;        // device, stream and launch counter
+    DctcK1Op op;                        // the context's operator at load, with the carver's kernel rule (carver_op)
+    bool dump_vmaps = false;            // every seam loop records the visibility maps (a batch's create flag; the maps
+                                        // are reset at the load and at the axis switch).  The single session asks per call.
+    bool ends_at_enlarge = false;       // an enlarge or a combined resize is the last seam operation until the next load,
+                                        // n_seams = 0 included (a batch); otherwise the session continues on the enlarged frames
+    int axis = DCTC_AXIS_NONE;
+    CarverFrames* cur = nullptr;        // the frames the getters read and the next seam operation carves; null: not loaded
+    CarverFrames* maps = nullptr;       // the set whose visibility maps _vmap and _paint_seams read: the one the last
+                                        // map-recording seam loop ran on (null: none since the load or the axis switch)
+    CarverFrames f;                     // the loaded frames
+    CarverFrames t;                     // their transposes (height operations)
+    CarverFrames wide, wide2;           // enlarged frames: an enlarge writes into the one that is not cur
+    uint8_t* start_img = nullptr;       // an enlarge's copy of its start images
+    size_t start_bytes = 0;
+};
+
+namespace {
+
+void session_destroy(dctc_carver_batch* b)
+{
+    frames_free(b->f);
+    frames_free(b->t);
+    frames_free(b->wide);
+    frames_free(b->wide2);
+    cudaFree(b->start_img);
+    delete b;
+}
+
+int session_create(dctc_context* ctx, int n_frames, int w, int h, int channels, bool dump_vmaps, bool ends_at_enlarge,
+                   dctc_carver_batch** out)
+{
+    dctc_carver_batch* b = new (std::nothrow) dctc_carver_batch;
+    if (!b) return DCTC_ERR_NOMEM;
+    b->ctx = ctx;
+    b->dump_vmaps = dump_vmaps;
+    b->ends_at_enlarge = ends_at_enlarge;
+    frames_init(b->f, n_frames, w, h, channels);
+    int rc = frames_alloc(ctx, b->f);
+    if (rc == DCTC_OK) {
+        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+    }
+    if (rc) {
+        session_destroy(b);
+        return rc;
+    }
+    *out = b;
+    return DCTC_OK;
+}
+
+// The size the getters report: the current frames', or while unloaded the loaded frames'
+const CarverFrames& session_frames(const dctc_carver_batch* b) { return b->cur ? *b->cur : b->f; }
+
+// Host frames (frame_stride bytes apart, rows pitch bytes apart) into f, which becomes cur: no bias, the axis free, maps
+// reset with dump_vmaps, the full energy maps with the context's operator.  A failure leaves the session unloaded.
+int session_load(dctc_carver_batch* b, const uint8_t* imgs, size_t frame_stride, size_t pitch)
+{
+    dctc_context* ctx = b->ctx;
+    CarverFrames& f = b->f;
+    b->cur = b->maps = nullptr;
+    b->axis = DCTC_AXIS_NONE;
+    b->op = carver_op(ctx->op);
+    f.w = f.w0;
+    cudaFree(f.bias);
+    f.bias = nullptr;
+    for (int i = 0; i < f.n; i++)
+        CK(ctx, cudaMemcpy2DAsync(f.img + (size_t) i * f.img_fs, f.pitch, imgs + (size_t) i * frame_stride, pitch, (size_t) f.w0 * f.ch,
+                                  f.h, cudaMemcpyDefault, ctx->stream));
+    int rc = b->dump_vmaps ? frames_vmaps(ctx, f) : DCTC_OK;
+    if (rc == DCTC_OK) rc = frames_full_energy(ctx, f, b->op);
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    b->cur = &f;
+    b->maps = b->dump_vmaps ? &f : nullptr;
+    return DCTC_OK;
+}
+
+// frames_set_bias on the loaded frames, before any seam operation.  A failure leaves the session unloaded.
+int session_set_bias(dctc_carver_batch* b, const float* bias, size_t frame_stride, size_t pitch)
+{
+    if (!b->cur || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;   // loaded, no seam operation since
+    CarverFrames& f = b->f;
+    if (bias && (pitch < sizeof(float) * f.w0 || (f.n > 1 && frame_stride < pitch * f.h))) return DCTC_ERR_INVALID;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    b->cur = nullptr;
+    const int rc = frames_set_bias(ctx, f, b->op, bias, frame_stride, pitch);
+    if (rc) return rc;
+    b->cur = &f;
+    return DCTC_OK;
+}
+
+// The axis switch: cur becomes its transposes in t (frames_transpose), with fresh maps when vmaps.  A failure leaves the
+// session unloaded.
+int session_transpose(dctc_carver_batch* b, bool vmaps, const SeamCall& c)
+{
+    CarverFrames* src = b->cur;
+    b->cur = nullptr;
+    if (c.m_valid) *c.m_valid = false;
+    const int rc = frames_transpose(b->ctx, *src, b->t, b->op, vmaps);
+    if (rc) return rc;
+    b->cur = &b->t;
+    b->maps = vmaps ? &b->t : nullptr;
+    return DCTC_OK;
+}
+
+// A resize: the seam loop on cur.  Maps a call asks for start at its first recording loop on these frames (the caller
+// checked that no seam was removed from them before).
+int session_carve(dctc_carver_batch* b, int n_seams, int* seams_out, const SeamCall& c)
+{
+    CarverFrames& f = *b->cur;
+    if (c.vmaps && b->maps != &f) {
+        const int rc = frames_fresh_vmaps(b->ctx, f);
+        if (rc) return rc;
+        b->maps = &f;
+    }
+    return seam_loop(b->ctx, f, b->op, n_seams, seams_out, c);
+}
+
+// An enlarge: frames_enlarge from cur (as loaded or enlarged) into the enlarged set that is not cur, which becomes cur;
+// the maps stay those of the start frames.  cur is carved in place, so a failure leaves the session unloaded.
+int session_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out, const SeamCall& c)
+{
+    dctc_context* ctx = b->ctx;
+    CarverFrames& f = *b->cur;
+    CarverFrames& wide = b->cur == &b->wide ? b->wide2 : b->wide;
+    b->cur = nullptr;
+    const int w1 = f.w0 + n_seams;
+    if (b->start_bytes != f.img_fs * f.n) {
+        cudaFree(b->start_img);
+        b->start_img = nullptr; b->start_bytes = 0;
+        CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
+        b->start_bytes = f.img_fs * f.n;
+    }
+    if (wide.w0 != w1 || wide.h != f.h) {
+        frames_free(wide);
+        frames_init(wide, f.n, w1, f.h, f.ch);
+        const int rc = frames_alloc(ctx, wide);
+        if (rc) {
+            frames_free(wide);
+            return rc;
+        }
+    }
+    wide.w = wide.w0;   // (a set an earlier pass carved)
+    wide.transposed = f.transposed;
+    int rc = frames_fresh_vmaps(ctx, f);
+    if (rc == DCTC_OK) rc = frames_enlarge(ctx, f, b->op, n_seams, seams_out, c, b->start_img, wide);
+    if (rc) return rc;
+    b->cur = &wide;
+    b->maps = &f;
+    if (c.m_valid) {   // as after a load: no incremental map, its rebuild count from zero
+        *c.m_valid = false;
+        cudaFree(ctx->c_band);
+        ctx->c_band = nullptr;
+    }
+    return DCTC_OK;
+}
+
+// dctc_carver_resize_width / _height, dctc_carver_enlarge_width / _height and the batch's: the checks (the axis fixed
+// since the load, n_seams >= the image's extent along the axis, an extent wider than the seam DP covers), then the first
+// height operation since the load switches the axis.
+int session_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out, const SeamCall& c)
+{
+    const bool enlarged = b->cur == &b->wide || b->cur == &b->wide2;
+    if (!b->cur || (b->ends_at_enlarge && (enlarged || b->axis == DCTC_AXIS_RESIZED))) return DCTC_ERR_STATE;
+    if (n_seams == 0) return DCTC_OK;
+    const CarverFrames& f = *b->cur;
+    if (enlarge && f.w != f.w0) return DCTC_ERR_STATE;   // an enlarge starts from frames as loaded (or enlarged)
+    if (b->axis != DCTC_AXIS_NONE && b->axis != axis) return DCTC_ERR_STATE;
+    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(f) : frames_image_h(f);
+    if (n_seams >= extent) return DCTC_ERR_STATE;
+    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
+    if (!enlarge && c.vmaps && b->maps != &f && f.w != f.w0) return DCTC_ERR_STATE;   // maps: before the first seam
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    if (axis == DCTC_AXIS_HEIGHT && b->axis == DCTC_AXIS_NONE) {
+        const int rc = session_transpose(b, c.vmaps, c);
+        if (rc) return rc;
+    }
+    b->axis = axis;
+    return enlarge ? session_enlarge(b, n_seams, seams_out, c) : session_carve(b, n_seams, seams_out, c);
+}
+
+// dctc_carver_resize / dctc_carver_batch_resize: the plan (checked against the seam DP's reach before any work) as its
+// per-axis calls run it, maps recorded whenever vmaps_out is given and each pass's map read back before the next pass
+// reuses its set.  A failure leaves the session unloaded.
+int session_resize(dctc_carver_batch* b, int new_w, int new_h, int* seams_out, int* vmaps_out, const SeamCall& c)
+{
+    if (!b->cur || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
+    DctcResizePass plan[DCTC_RESIZE_MAX_PASSES];
+    const int n = dctc_resize_passes(b->f.w, b->f.h, new_w, new_h, plan, DCTC_RESIZE_MAX_PASSES);
+    if (n <= 0) return n;
+    for (int i = 0; i < n; i++)
+        if ((plan[i].axis == DCTC_RESIZE_WIDTH ? plan[i].w : plan[i].h) > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    SeamCall pc = c;
+    pc.vmaps = vmaps_out != nullptr;
+    const size_t nf = (size_t) b->f.n;
+    for (int i = 0; i < n; i++) {
+        const DctcResizePass& p = plan[i];
+        int* seams = seams_out ? seams_out + nf * p.seams_offset : nullptr;
+        int rc = DCTC_OK;
+        if (p.axis == DCTC_RESIZE_HEIGHT && !b->cur->transposed) rc = session_transpose(b, false, c);
+        if (rc == DCTC_OK) rc = p.enlarge ? session_enlarge(b, p.n_seams, seams, pc) : session_carve(b, p.n_seams, seams, pc);
+        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *b->maps, b->op, nullptr, nullptr, vmaps_out + nf * p.vmap_offset);
+        if (rc) {
+            b->cur = nullptr;
+            return rc;
+        }
+    }
+    b->axis = DCTC_AXIS_RESIZED;
+    return DCTC_OK;
+}
+
+// Images, operator energy maps or bias planes of the current frames
+int session_download(dctc_carver_batch* b, uint8_t* img, float* en, float* bias)
+{
+    if (!b->cur || (bias && !b->cur->bias)) return DCTC_ERR_STATE;
+    return frames_download(b->ctx, *b->cur, b->op, img, en, nullptr, bias);
+}
+
+int session_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
+{
+    if (!b->cur || !b->maps || b->axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // a combined resize returned its maps
+    const int rc = frames_download(b->ctx, *b->maps, b->op, nullptr, nullptr, vmap_out);
+    if (rc == DCTC_OK && depth_out) *depth_out = b->maps->depth;
+    return rc;
+}
+
+}  // namespace
+
+// ---- the context's single session ----------------------------------------------------------------------------------------
 
 void dctc_carver_release(dctc_context* ctx)
 {
-    if (ctx->carver) {
-        frames_free(*ctx->carver);
-        delete ctx->carver;
-        ctx->carver = nullptr;
-    }
+    if (ctx->carver) session_destroy(ctx->carver);
+    ctx->carver = nullptr;
     cudaFree(ctx->c_band); cudaFree(ctx->c_band_vals);
     cudaFreeHost(ctx->h_mirror); cudaFreeHost(ctx->h_band);
     ctx->c_band = nullptr; ctx->c_band_vals = nullptr; ctx->h_mirror = nullptr; ctx->h_band = nullptr;
     ctx->c_m_valid = false;
     ctx->mirror_valid = false;
-    ctx->c_axis = DCTC_AXIS_NONE;
 }
 
 // dctc_set_params with a session loaded (liblqr: lqr_carver_set_energy_function invalidates the energy map): the
@@ -1612,24 +1862,9 @@ int dctc_carver_params_changed(dctc_context* ctx)
     CK(ctx, cudaSetDevice(ctx->device));
     ctx->mirror_valid = false;
     ctx->c_m_valid = false;
-    const int rc = frames_full_energy(ctx, *ctx->carver, carver_op(ctx->op));
-    if (rc) return rc;
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    return DCTC_OK;
-}
-
-static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
-{
-    CarverFrames* f = new (std::nothrow) CarverFrames;
-    if (!f) return DCTC_ERR_NOMEM;
-    ctx->carver = f;
-    frames_init(*f, 1, w, h, channels);
-    int rc = frames_alloc(ctx, *f);
-    if (rc) return rc;
-    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * 32));
-    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * 32 + sizeof(int) * h));
-    CK(ctx, cudaMemcpy2DAsync(f->img, f->pitch, img, pitch, (size_t) w * channels, h, cudaMemcpyDefault, ctx->stream));
-    rc = frames_full_energy(ctx, *f, carver_op(ctx->op));
+    dctc_carver_batch* b = ctx->carver;
+    b->op = carver_op(ctx->op);
+    const int rc = frames_full_energy(ctx, *b->cur, b->op);
     if (rc) return rc;
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
@@ -1637,12 +1872,14 @@ static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h,
 
 int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pitch, int* w, int* h)
 {
-    CarverFrames* f = ctx->carver;
+    dctc_carver_batch* b = ctx->carver;
+    CarverFrames& f = *b->cur;
+    b->op = carver_op(ctx->op);
     const float* op_en;
-    int rc = frames_op_energy(ctx, *f, carver_op(ctx->op), &op_en);
+    int rc = frames_op_energy(ctx, f, b->op, &op_en);
     if (rc) return rc;
     Plane p;
-    rc = frames_oriented(ctx, *f, op_en, sizeof(float) * f->en_pitch, f->w, sizeof(float), p);
+    rc = frames_oriented(ctx, f, op_en, sizeof(float) * f.en_pitch, f.w, sizeof(float), p);
     if (rc) return rc;
     *en = (const float*) p.p;
     *en_pitch = p.pitch / sizeof(float);
@@ -1651,136 +1888,54 @@ int dctc_carver_energy_plane(dctc_context* ctx, const float** en, size_t* en_pit
     return DCTC_OK;
 }
 
-// The single session's axis switch: its frame is replaced by its transpose (frames_transpose).  A failure leaves the
-// session unloaded.
-static int carver_transpose(dctc_context* ctx)
+// A call on the loaded single session with the context's operator, maps request and incremental map.  A call that leaves
+// the session unloaded releases it; frames that changed invalidate the dctc_pixel_energy mirror, and frames that grew
+// drop its allocation (sized by its first use).
+template <typename Op>
+static int carver_call(dctc_context* ctx, Op&& op)
 {
-    CarverFrames* t = new (std::nothrow) CarverFrames;
-    if (!t) return DCTC_ERR_NOMEM;
-    const int rc = frames_transpose(ctx, *ctx->carver, *t, carver_op(ctx->op), false);
-    frames_free(*ctx->carver);
-    delete ctx->carver;
-    ctx->carver = t;
-    ctx->mirror_valid = false;
-    ctx->c_m_valid = false;
-    if (rc) dctc_carver_release(ctx);
-    return rc;
-}
-
-// Checks of a single-session seam operation along `axis` (n_seams > 0, a session loaded): the other axis fixed since the
-// load, n_seams >= the image's extent along the axis, an extent wider than the seam DP covers.  Then the operation fixes
-// the axis, and the first height operation replaces the session's frame by its transpose.  A failed switch leaves the
-// session unloaded.
-static int carver_axis(dctc_context* ctx, int axis, int n_seams)
-{
-    if (ctx->c_axis != DCTC_AXIS_NONE && ctx->c_axis != axis) return DCTC_ERR_STATE;
-    const CarverFrames& f = *ctx->carver;
-    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(f) : frames_image_h(f);
-    if (n_seams >= extent) return DCTC_ERR_STATE;
-    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips: use the host seam loop
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (axis == DCTC_AXIS_HEIGHT && ctx->c_axis == DCTC_AXIS_NONE) {
-        const int rc = carver_transpose(ctx);
-        if (rc) return rc;
-    }
-    ctx->c_axis = axis;
-    return DCTC_OK;
-}
-
-// A resize after carver_axis: the seam loop on the session's current frame, recording the visibility map when vmaps
-static int carver_resize(dctc_context* ctx, int n_seams, int* seams_out, bool vmaps)
-{
-    CarverFrames* f = ctx->carver;
-    if (vmaps && !f->raw) {
-        if (f->w != f->w0) return DCTC_ERR_STATE;   // the map must be requested before the first seam is removed
-        const int rc = frames_vmaps(ctx, *f);
-        if (rc) return rc;
-    }
-    ctx->mirror_valid = false;
-    if (!ctx->c_incremental) ctx->c_m_valid = false;
-    return seam_loop(ctx, *f, carver_op(ctx->op), n_seams, seams_out, vmaps, ctx->c_incremental ? &ctx->c_m_valid : nullptr);
-}
-
-// An enlarge after carver_axis: frames_enlarge, after which the session continues on the
-// enlarged frame (its w0 is the new width, its energy map the one frames_enlarge computed); the visibility map of the
-// start frame stays readable through dctc_carver_vmap and dctc_carver_paint_seams.  A failure leaves the session unloaded.
-static int carver_enlarge(dctc_context* ctx, int n_seams, int* seams_out)
-{
-    CarverFrames* f = ctx->carver;
-    CarverFrames* wide = new (std::nothrow) CarverFrames;
-    if (!wide) return DCTC_ERR_NOMEM;
-    uint8_t* start = nullptr;
-    frames_init(*wide, 1, f->w0 + n_seams, f->h, f->ch);
-    wide->transposed = f->transposed;
-    int rc = frames_alloc(ctx, *wide);
-    if (rc == DCTC_OK) rc = frames_vmaps(ctx, *f);
-    if (rc == DCTC_OK) {
-        const cudaError_t e = cudaMalloc((void**) &start, f->img_fs);
-        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
-    }
-    if (rc == DCTC_OK)
-        rc = frames_enlarge(ctx, *f, carver_op(ctx->op), n_seams, seams_out, ctx->c_incremental ? &ctx->c_m_valid : nullptr, start, *wide);
-    cudaFree(start);
-    if (rc) {
-        frames_free(*wide);
-        delete wide;
+    dctc_carver_batch* b = ctx->carver;
+    if (!b) return DCTC_ERR_STATE;
+    b->op = carver_op(ctx->op);
+    const CarverFrames* f = b->cur;
+    const int w = f->w, iw = frames_image_w(*f), ih = frames_image_h(*f);
+    SeamCall c;
+    c.vmaps = ctx->c_dump_vmaps;
+    c.incremental = ctx->c_incremental;
+    c.m_valid = &ctx->c_m_valid;
+    const int rc = op(b, c);
+    if (!b->cur) {
         dctc_carver_release(ctx);
         return rc;
     }
-    std::swap(wide->vs, f->vs);
-    wide->depth = f->depth;
-    wide->vs_w = f->vs_w;
-    frames_free(*f);
-    delete f;
-    ctx->carver = wide;
-    // as after a load: no cumulative map, no host mirror (the frame is wider), rebuild count from zero
-    cudaFree(ctx->c_band); cudaFreeHost(ctx->h_mirror);
-    ctx->c_band = nullptr; ctx->h_mirror = nullptr;
-    ctx->c_m_valid = false;
-    ctx->mirror_valid = false;
-    return DCTC_OK;
+    if (b->cur != f || b->cur->w != w) ctx->mirror_valid = false;
+    if (frames_image_w(*b->cur) > iw || frames_image_h(*b->cur) > ih) {
+        cudaFreeHost(ctx->h_mirror);
+        ctx->h_mirror = nullptr;
+    }
+    return rc;
 }
 
-// dctc_carver_resize_width / _height, dctc_carver_enlarge_width / _height
+static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
+{
+    const int rc = session_create(ctx, 1, w, h, channels, false, false, &ctx->carver);
+    if (rc) return rc;
+    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * 32));
+    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * 32 + sizeof(int) * h));
+    return session_load(ctx->carver, img, 0, pitch);
+}
+
 static int carver_seams(dctc_context* ctx, int axis, bool enlarge, int n_seams, int* seams_out)
 {
     if (!ctx || n_seams < 0) return DCTC_ERR_INVALID;
-    const CarverFrames* f = ctx->carver;
-    if (!f) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (enlarge && f->w != f->w0) return DCTC_ERR_STATE;   // enlarge starts from a freshly loaded (or enlarged) frame
-    const int rc = carver_axis(ctx, axis, n_seams);
-    if (rc) return rc;
-    return enlarge ? carver_enlarge(ctx, n_seams, seams_out) : carver_resize(ctx, n_seams, seams_out, ctx->c_dump_vmaps);
+    return carver_call(ctx, [&](dctc_carver_batch* b, const SeamCall& c) { return session_seams(b, axis, enlarge, n_seams, seams_out, c); });
 }
 
-// The plan of dctc_carver_resize / dctc_carver_batch_resize from w x h (plan holds DCTC_RESIZE_MAX_PASSES), with every
-// pass's extent along its axis checked against the seam DP's reach before any work
-static int resize_plan(int w, int h, int new_w, int new_h, DctcResizePass* plan, int* n_passes)
+static int carver_download(dctc_context* ctx, uint8_t* img, float* en, float* bias)
 {
-    const int n = dctc_resize_passes(w, h, new_w, new_h, plan, DCTC_RESIZE_MAX_PASSES);
-    if (n < 0) return n;
-    for (int i = 0; i < n; i++)
-        if ((plan[i].axis == DCTC_RESIZE_WIDTH ? plan[i].w : plan[i].h) > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
-    *n_passes = n;
-    return DCTC_OK;
-}
-
-// The passes of dctc_carver_resize on the single session: the per-axis helpers, the axis switch on the current frame,
-// and each pass's map read back before the next pass replaces the frame
-static int carver_passes(dctc_context* ctx, const DctcResizePass* plan, int n, int* seams_out, int* vmaps_out)
-{
-    for (int i = 0; i < n; i++) {
-        const DctcResizePass& p = plan[i];
-        int rc = DCTC_OK;
-        if (p.axis == DCTC_RESIZE_HEIGHT && !ctx->carver->transposed) rc = carver_transpose(ctx);
-        int* seams = seams_out ? seams_out + p.seams_offset : nullptr;
-        if (rc == DCTC_OK)
-            rc = p.enlarge ? carver_enlarge(ctx, p.n_seams, seams) : carver_resize(ctx, p.n_seams, seams, vmaps_out != nullptr);
-        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, nullptr, vmaps_out + p.vmap_offset);
-        if (rc) return rc;
-    }
-    return DCTC_OK;
+    if (!ctx->carver) return DCTC_ERR_STATE;
+    ctx->carver->op = carver_op(ctx->op);
+    return session_download(ctx->carver, img, en, bias);
 }
 
 extern "C" {
@@ -1803,47 +1958,43 @@ int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int ch
 int dctc_carver_set_bias(dctc_context* ctx, const float* bias, size_t pitch)
 {
     if (!ctx) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f || ctx->c_axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;   // loaded, no seam operation since
-    if (bias && pitch < sizeof(float) * f->w) return DCTC_ERR_INVALID;
-    CK(ctx, cudaSetDevice(ctx->device));
-    ctx->mirror_valid = false;
-    ctx->c_m_valid = false;
-    const int rc = frames_set_bias(ctx, *f, carver_op(ctx->op), bias, 0, pitch);
-    if (rc) dctc_carver_release(ctx);
+    dctc_carver_batch* b = ctx->carver;
+    if (!b) return DCTC_ERR_STATE;
+    b->op = carver_op(ctx->op);
+    const int rc = session_set_bias(b, bias, 0, pitch);
+    if (!b->cur) dctc_carver_release(ctx);
+    else if (rc == DCTC_OK) ctx->mirror_valid = false;
     return rc;
 }
 
 int dctc_carver_bias(dctc_context* ctx, float* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->carver || !ctx->carver->bias) return DCTC_ERR_STATE;
-    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, nullptr, nullptr, out);
+    return carver_download(ctx, nullptr, nullptr, out);
 }
 
-int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_w(*ctx->carver) : 0; }
-int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_h(*ctx->carver) : 0; }
+int dctc_carver_width(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_w(session_frames(ctx->carver)) : 0; }
+int dctc_carver_height(const dctc_context* ctx) { return ctx && ctx->carver ? frames_image_h(session_frames(ctx->carver)) : 0; }
 
 int dctc_carver_energy(dctc_context* ctx, float* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->carver) return DCTC_ERR_STATE;
-    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), nullptr, out, nullptr);
+    return carver_download(ctx, nullptr, out, nullptr);
 }
 
 int dctc_carver_image(dctc_context* ctx, uint8_t* out)
 {
     if (!ctx || !out) return DCTC_ERR_INVALID;
-    if (!ctx->carver) return DCTC_ERR_STATE;
-    return frames_download(ctx, *ctx->carver, carver_op(ctx->op), out, nullptr, nullptr);
+    return carver_download(ctx, out, nullptr, nullptr);
 }
 
 int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out, int* xmin, int* xmax)
 {
     if (!ctx || !seam_x) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f || f->w <= 1 || ctx->c_axis == DCTC_AXIS_HEIGHT || ctx->c_axis == DCTC_AXIS_RESIZED)   // vertical seams only
-        return DCTC_ERR_STATE;
+    dctc_carver_batch* s = ctx->carver;
+    if (!s || s->axis == DCTC_AXIS_HEIGHT || s->axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // vertical seams only
+    CarverFrames* f = s->cur;
+    if (f->w <= 1) return DCTC_ERR_STATE;
     if (f->bias) return DCTC_ERR_STATE;   // the caller's seam and the operator's band values: no place for a bias
     const DctcK1Op op = carver_op(ctx->op);
     const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
@@ -1854,7 +2005,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
         if (y > 0 && (seam_x[y] - seam_x[y - 1] > 1 || seam_x[y - 1] - seam_x[y] > 1)) return DCTC_ERR_INVALID;
         h_seam[y] = seam_x[y];
     }
-    ctx->c_axis = DCTC_AXIS_WIDTH;
+    s->axis = DCTC_AXIS_WIDTH;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaMemcpyAsync(f->seam, h_seam, sizeof(int) * h, cudaMemcpyHostToDevice, ctx->stream));
     dctc_carve_rows_kernel<256, 4, false><<<h, 256, 0, ctx->stream>>>(f->img, f->pitch, f->ch, f->en, f->en_pitch, f->seam, w_old, nullptr,
@@ -1915,20 +2066,7 @@ int dctc_resize_plan(int w, int h, int new_w, int new_h, DctcResizePass* passes,
 int dctc_carver_resize(dctc_context* ctx, int new_w, int new_h, int* seams_out, int* vmaps_out)
 {
     if (!ctx || new_w <= 0 || new_h <= 0) return DCTC_ERR_INVALID;
-    const CarverFrames* f = ctx->carver;
-    if (!f || ctx->c_axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
-    DctcResizePass plan[DCTC_RESIZE_MAX_PASSES];
-    int n = 0;
-    int rc = resize_plan(f->w, f->h, new_w, new_h, plan, &n);
-    if (rc || n == 0) return rc;
-    CK(ctx, cudaSetDevice(ctx->device));
-    rc = carver_passes(ctx, plan, n, seams_out, vmaps_out);
-    if (rc) {
-        dctc_carver_release(ctx);
-        return rc;
-    }
-    ctx->c_axis = DCTC_AXIS_RESIZED;
-    return DCTC_OK;
+    return carver_call(ctx, [&](dctc_carver_batch* b, const SeamCall& c) { return session_resize(b, new_w, new_h, seams_out, vmaps_out, c); });
 }
 
 int dctc_carver_set_incremental(dctc_context* ctx, int on)
@@ -1962,18 +2100,17 @@ int dctc_carver_set_dump_vmaps(dctc_context* ctx, int on)
 int dctc_carver_vmap(dctc_context* ctx, int* vmap_out, int* depth_out)
 {
     if (!ctx) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f || !f->vs || ctx->c_axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // dctc_carver_resize returned its maps
-    const int rc = frames_download(ctx, *f, carver_op(ctx->op), nullptr, nullptr, vmap_out);
-    if (rc == DCTC_OK && depth_out) *depth_out = f->depth;
-    return rc;
+    if (!ctx->carver) return DCTC_ERR_STATE;
+    ctx->carver->op = carver_op(ctx->op);
+    return session_vmap(ctx->carver, vmap_out, depth_out);
 }
 
 int dctc_carver_paint_seams(dctc_context* ctx, uint8_t* img, int channels, size_t pitch)
 {
     if (!ctx || !img || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
-    CarverFrames* f = ctx->carver;
-    if (!f || !f->vs || f->depth <= 0 || ctx->c_axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;
+    const dctc_carver_batch* s = ctx->carver;
+    if (!s || !s->maps || s->maps->depth <= 0 || s->axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;
+    CarverFrames* f = s->maps;
     CK(ctx, cudaSetDevice(ctx->device));
     Plane vs;   // the map in image orientation, row pitch = its width
     const int rc = frames_oriented(ctx, *f, f->vs, sizeof(int) * f->vs_w, f->vs_w, sizeof(int), vs);
@@ -2021,152 +2158,15 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
 }  // extern "C"
 
 // ---- batch session: n equally sized frames through one device seam loop ---------------------------------------------
-// The batch owns its frames and never touches the context's single session; it uses the context's device, stream and
-// launch counter, and the operator / kernel selection the context had when the frames were loaded.  The cumulative map is
-// always rebuilt (incremental mode is a single-session option).
-struct dctc_carver_batch {
-    dctc_context* ctx = nullptr;
-    CarverFrames f;
-    CarverFrames t;                     // the height operations' frames: transposes of f (the first allocates, destroy frees)
-    DctcK1Op op;                        // the context's operator at load time, with the carver's kernel rule (carver_op)
-    bool dump_vmaps = false, loaded = false;
-    int axis = DCTC_AXIS_NONE;          // fixed by the first seam operation since the load
-    // dctc_carver_batch_enlarge_width / _height: a copy of the start frames and the enlarged frames (images and energy
-    // planes).  Allocated by the first enlarge and kept for the next (reallocated when their size differs), freed by the
-    // destroy.
-    bool enlarged = false;              // the current frames are the enlarged ones
-    uint8_t* start_img = nullptr;
-    size_t start_bytes = 0;
-    CarverFrames wide;
-    // dctc_carver_batch_resize: the second enlarged set (consecutive enlarge passes alternate between wide and wide2,
-    // each reading the previous pass's frames; allocated by the first such pair) and the frames the call left (null
-    // until then; no seam operation until the next load)
-    CarverFrames wide2;
-    CarverFrames* resized = nullptr;
-};
+// The batch never touches the context's single session; it uses the context's device, stream and launch counter.
 
-namespace {
-
-// the frames the seam operations carve: the loaded ones, or their transposes along the height
-CarverFrames& batch_src(dctc_carver_batch* b) { return b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f; }
-const CarverFrames& batch_frames(const dctc_carver_batch* b)
-{
-    if (b->resized) return *b->resized;
-    return b->enlarged ? b->wide : b->axis == DCTC_AXIS_HEIGHT ? b->t : b->f;
-}
-CarverFrames& batch_frames(dctc_carver_batch* b) { return const_cast<CarverFrames&>(batch_frames((const dctc_carver_batch*) b)); }
-
-void batch_free(dctc_carver_batch* b)
-{
-    frames_free(b->f);
-    frames_free(b->t);
-    frames_free(b->wide);
-    frames_free(b->wide2);
-    cudaFree(b->start_img);
-}
-
-// Checks of a batch seam operation along `axis` (n_seams > 0, loaded, not enlarged), as carver_axis does them for the
-// single session; the first height operation since the load fills the transposed frames (frames_transpose).  A failed
-// switch leaves the batch unloaded.
-int batch_axis(dctc_carver_batch* b, int axis, int n_seams)
-{
-    if (b->axis != DCTC_AXIS_NONE && b->axis != axis) return DCTC_ERR_STATE;
-    const CarverFrames& f = batch_src(b);
-    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(f) : frames_image_h(f);
-    if (n_seams >= extent) return DCTC_ERR_STATE;
-    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;   // wider than the cluster's strips
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    if (axis == DCTC_AXIS_HEIGHT && b->axis == DCTC_AXIS_NONE) {
-        b->loaded = false;
-        const int rc = frames_transpose(ctx, b->f, b->t, b->op, b->dump_vmaps);
-        if (rc) return rc;
-        b->loaded = true;
-    }
-    b->axis = axis;
-    return DCTC_OK;
-}
-
-// Device work of dctc_carver_batch_enlarge_width / _height and of an enlarge pass of dctc_carver_batch_resize: f's frames
-// enlarged into wide
-int batch_enlarge(dctc_carver_batch* b, CarverFrames& f, CarverFrames& wide, int n_seams, int* seams_out)
-{
-    dctc_context* ctx = b->ctx;
-    const int w1 = f.w0 + n_seams;
-    if (b->start_bytes != f.img_fs * f.n) {
-        cudaFree(b->start_img);
-        b->start_img = nullptr; b->start_bytes = 0;
-        CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
-        b->start_bytes = f.img_fs * f.n;
-    }
-    if (wide.w0 != w1 || wide.h != f.h) {
-        frames_free(wide);
-        frames_init(wide, f.n, w1, f.h, f.ch);
-        const int rc = frames_alloc(ctx, wide);
-        if (rc) {
-            frames_free(wide);
-            return rc;
-        }
-    }
-    wide.w = wide.w0;   // (a set a previous pass of dctc_carver_batch_resize carved)
-    wide.transposed = f.transposed;
-    // (a batch with dump_vmaps had its maps reset by the load or the axis switch, and no seam was removed since)
-    const int rc = frames_fresh_vmaps(ctx, f);
-    if (rc) return rc;
-    return frames_enlarge(ctx, f, b->op, n_seams, seams_out, nullptr, b->start_img, wide);
-}
-
-// The batch's resize and enlarge calls.  An enlarge carves the frames in place: until every frame is enlarged the batch is
-// not loaded, so that a failure leaves it unloaded rather than half-updated.
-int batch_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out)
+static int batch_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out)
 {
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged || b->resized) return DCTC_ERR_STATE;
-    if (n_seams == 0) return DCTC_OK;
-    if (enlarge && batch_src(b).w != batch_src(b).w0) return DCTC_ERR_STATE;   // enlarge starts from freshly loaded frames
-    int rc = batch_axis(b, axis, n_seams);
-    if (rc) return rc;
-    if (!enlarge) return seam_loop(b->ctx, batch_src(b), b->op, n_seams, seams_out, b->dump_vmaps, nullptr);
-    b->loaded = false;
-    rc = batch_enlarge(b, batch_src(b), b->wide, n_seams, seams_out);
-    if (rc) return rc;
-    b->enlarged = true;
-    b->loaded = true;
-    return DCTC_OK;
+    SeamCall c;
+    c.vmaps = b->dump_vmaps;
+    return session_seams(b, axis, enlarge, n_seams, seams_out, c);
 }
-
-// The passes of dctc_carver_batch_resize, moving between the batch's frame sets: the loaded frames, their transposes
-// (filled from the current frames at the axis switch) and the two enlarged sets; each pass's maps are read back before
-// the next pass reuses the set they live in.  Maps are recorded when vmaps_out is given, whatever dump_vmaps says.
-int batch_passes(dctc_carver_batch* b, const DctcResizePass* plan, int n, int* seams_out, int* vmaps_out)
-{
-    dctc_context* ctx = b->ctx;
-    const size_t nf = (size_t) b->f.n;
-    CarverFrames* cur = &b->f;
-    for (int i = 0; i < n; i++) {
-        const DctcResizePass& p = plan[i];
-        int rc = DCTC_OK;
-        if (p.axis == DCTC_RESIZE_HEIGHT && !cur->transposed) {
-            rc = frames_transpose(ctx, *cur, b->t, b->op, false);
-            cur = &b->t;
-        }
-        CarverFrames* src = cur;
-        int* seams = seams_out ? seams_out + nf * p.seams_offset : nullptr;
-        if (rc == DCTC_OK && p.enlarge) {
-            cur = cur == &b->wide ? &b->wide2 : &b->wide;
-            rc = batch_enlarge(b, *src, *cur, p.n_seams, seams);
-        } else if (rc == DCTC_OK) {
-            if (vmaps_out) rc = frames_fresh_vmaps(ctx, *src);
-            if (rc == DCTC_OK) rc = seam_loop(ctx, *src, b->op, p.n_seams, seams, vmaps_out != nullptr, nullptr);
-        }
-        if (rc == DCTC_OK && vmaps_out) rc = frames_download(ctx, *src, b->op, nullptr, nullptr, vmaps_out + nf * p.vmap_offset);
-        if (rc) return rc;
-    }
-    b->resized = cur;
-    return DCTC_OK;
-}
-
-}  // namespace
 
 extern "C" {
 
@@ -2177,87 +2177,42 @@ int dctc_carver_batch_create(dctc_context* ctx, int n_frames, int w, int h, int 
     if (n_frames <= 0 || w <= 0 || h <= 0 || channels < 1 || channels > 4) return DCTC_ERR_INVALID;
     if (n_frames > 65535) return DCTC_ERR_UNSUPPORTED;   // the frame is a grid dimension of every launch
     CK(ctx, cudaSetDevice(ctx->device));
-    dctc_carver_batch* b = new (std::nothrow) dctc_carver_batch;
-    if (!b) return DCTC_ERR_NOMEM;
-    b->ctx = ctx;
-    b->dump_vmaps = dump_vmaps != 0;
-    frames_init(b->f, n_frames, w, h, channels);
-    int rc = frames_alloc(ctx, b->f);
-    if (rc == DCTC_OK) {
-        const cudaError_t e = cudaStreamSynchronize(ctx->stream);
-        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
-    }
-    if (rc) {
-        batch_free(b);
-        delete b;
-        return rc;
-    }
-    *batch = b;
-    return DCTC_OK;
+    return session_create(ctx, n_frames, w, h, channels, dump_vmaps != 0, true, batch);
 }
 
 void dctc_carver_batch_destroy(dctc_carver_batch* b)
 {
     if (!b) return;
     if (cudaSetDevice(b->ctx->device) == cudaSuccess) cudaStreamSynchronize(b->ctx->stream);
-    batch_free(b);
-    delete b;
+    session_destroy(b);
 }
 
 int dctc_carver_batch_load(dctc_carver_batch* b, const uint8_t* imgs, size_t frame_stride, size_t pitch)
 {
     if (!b || !imgs) return DCTC_ERR_INVALID;
-    CarverFrames& f = b->f;
-    const size_t row = (size_t) f.w0 * f.ch;
-    if (pitch < row || (f.n > 1 && frame_stride < pitch * f.h)) return DCTC_ERR_INVALID;
+    const CarverFrames& f = b->f;
+    if (pitch < (size_t) f.w0 * f.ch || (f.n > 1 && frame_stride < pitch * f.h)) return DCTC_ERR_INVALID;
     dctc_context* ctx = b->ctx;
-    const int bs = ctx->op.blocksize;
-    if (!dctc_valid_blocksize(bs)) return DCTC_ERR_BLOCKSIZE;
+    if (!dctc_valid_blocksize(ctx->op.blocksize)) return DCTC_ERR_BLOCKSIZE;
     CK(ctx, cudaSetDevice(ctx->device));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
-    b->loaded = false;
-    b->enlarged = false;
-    b->resized = nullptr;
-    b->axis = DCTC_AXIS_NONE;
-    b->op = carver_op(ctx->op);
-    f.w = f.w0;
-    cudaFree(f.bias);   // a load clears the bias
-    f.bias = nullptr;
-    for (int i = 0; i < f.n; i++)
-        CK(ctx, cudaMemcpy2DAsync(f.img + (size_t) i * f.img_fs, f.pitch, imgs + (size_t) i * frame_stride, pitch, row, f.h,
-                                  cudaMemcpyDefault, ctx->stream));
-    int rc = b->dump_vmaps ? frames_vmaps(ctx, f) : DCTC_OK;
-    if (rc == DCTC_OK) rc = frames_full_energy(ctx, f, b->op);
-    if (rc) return rc;
-    CK(ctx, cudaStreamSynchronize(ctx->stream));
-    b->loaded = true;
-    return DCTC_OK;
+    return session_load(b, imgs, frame_stride, pitch);
 }
 
 int dctc_carver_batch_set_bias(dctc_carver_batch* b, const float* bias, size_t frame_stride, size_t pitch)
 {
     if (!b) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged || b->resized || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
-    CarverFrames& f = b->f;
-    if (bias && (pitch < sizeof(float) * f.w0 || (f.n > 1 && frame_stride < pitch * f.h))) return DCTC_ERR_INVALID;
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    b->loaded = false;
-    const int rc = frames_set_bias(ctx, f, b->op, bias, frame_stride, pitch);
-    if (rc) return rc;
-    b->loaded = true;
-    return DCTC_OK;
+    return session_set_bias(b, bias, frame_stride, pitch);
 }
 
 int dctc_carver_batch_bias(dctc_carver_batch* b, float* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
-    if (!b->loaded || !batch_frames(b).bias) return DCTC_ERR_STATE;
-    return frames_download(b->ctx, batch_frames(b), b->op, nullptr, nullptr, nullptr, out);
+    return session_download(b, nullptr, nullptr, out);
 }
 
-int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? frames_image_w(batch_frames(b)) : 0; }
-int dctc_carver_batch_height(const dctc_carver_batch* b) { return b ? frames_image_h(batch_frames(b)) : 0; }
+int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? frames_image_w(session_frames(b)) : 0; }
+int dctc_carver_batch_height(const dctc_carver_batch* b) { return b ? frames_image_h(session_frames(b)) : 0; }
 
 int dctc_carver_batch_resize_width(dctc_carver_batch* b, int n_seams, int* seams_out)
 {
@@ -2282,42 +2237,26 @@ int dctc_carver_batch_enlarge_height(dctc_carver_batch* b, int n_seams, int* sea
 int dctc_carver_batch_resize(dctc_carver_batch* b, int new_w, int new_h, int* seams_out, int* vmaps_out)
 {
     if (!b || new_w <= 0 || new_h <= 0) return DCTC_ERR_INVALID;
-    if (!b->loaded || b->enlarged || b->resized || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;
-    DctcResizePass plan[DCTC_RESIZE_MAX_PASSES];
-    int n = 0;
-    int rc = resize_plan(b->f.w, b->f.h, new_w, new_h, plan, &n);
-    if (rc || n == 0) return rc;
-    dctc_context* ctx = b->ctx;
-    CK(ctx, cudaSetDevice(ctx->device));
-    b->loaded = false;
-    rc = batch_passes(b, plan, n, seams_out, vmaps_out);
-    if (rc) return rc;
-    b->loaded = true;
-    return DCTC_OK;
+    return session_resize(b, new_w, new_h, seams_out, vmaps_out, SeamCall());
 }
 
 int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
-    if (!b->loaded) return DCTC_ERR_STATE;
-    return frames_download(b->ctx, batch_frames(b), b->op, out, nullptr, nullptr);
+    return session_download(b, out, nullptr, nullptr);
 }
 
 int dctc_carver_batch_energy(dctc_carver_batch* b, float* out)
 {
     if (!b || !out) return DCTC_ERR_INVALID;
-    if (!b->loaded) return DCTC_ERR_STATE;
-    return frames_download(b->ctx, batch_frames(b), b->op, nullptr, out, nullptr);
+    return session_download(b, nullptr, out, nullptr);
 }
 
 int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
 {
     if (!b) return DCTC_ERR_INVALID;
-    if (!b->loaded || !b->dump_vmaps || b->resized) return DCTC_ERR_STATE;   // dctc_carver_batch_resize returned its maps
-    CarverFrames& f = batch_src(b);
-    const int rc = frames_download(b->ctx, f, b->op, nullptr, nullptr, vmap_out);
-    if (rc == DCTC_OK && depth_out) *depth_out = f.depth;
-    return rc;
+    if (!b->dump_vmaps) return DCTC_ERR_STATE;   // maps were not asked for at create (an enlarge records them anyway)
+    return session_vmap(b, vmap_out, depth_out);
 }
 
 }  // extern "C"

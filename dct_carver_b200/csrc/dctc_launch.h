@@ -103,9 +103,9 @@ struct DctcK1Op {
     int kernel = DCTC_KERNEL_AUTO;
 };
 
-// Device state of a carver session: n frames of w x h pixels (w0 x h when loaded), frame f of every plane at f times the
-// plane's frame stride.  The context's single session is one of these with n = 1, a batch session (dctc_carver_batch)
-// holds one with n frames; both run the same seam loop over it (dctc_k2_carver.cu).
+// A frame set of a carver session (dctc_carver_batch, dctc_k2_carver.cu): n frames of w x h pixels (w0 x h when filled),
+// frame f of every plane at f times the plane's frame stride.  The session moves between its sets (the loaded frames,
+// their transposes, the enlarged frames); the context's single session is a session with n = 1.
 // transposed: the frames are the transposes of the images (a height operation runs the width seam loop on them), so w is
 // the image height and h the image width.  Only the axis switch that fills such frames and the way out to the caller
 // (frames_download, frames_oriented) look at the flag.
@@ -139,10 +139,6 @@ struct CarverFrames {
     float* en_op = nullptr;
 };
 
-// The axis a carver session's seam operations work along since its load: the first one fixes it, a call for the other
-// axis returns DCTC_ERR_STATE until the next load.  RESIZED: dctc_carver_resize ran since the load, which fixes both axes.
-enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2, DCTC_AXIS_RESIZED = 3 };
-
 struct dctc_context {
     int device = 0;
     cudaStream_t stream = nullptr;      // compute
@@ -160,9 +156,9 @@ struct dctc_context {
     uint8_t* d_in[DCTC_SLOTS] = {};
     float* d_out[DCTC_SLOTS] = {};
     size_t d_in_cap[DCTC_SLOTS] = {}, d_out_cap[DCTC_SLOTS] = {};
-    // carver session (K2): one frame, null when nothing is loaded; the single-session-only state follows
-    CarverFrames* carver = nullptr;
-    int c_axis = 0;                // DCTC_AXIS_* the first seam operation since the load fixed
+    // carver session (K2): a one-frame dctc_carver_batch, null when nothing is loaded; the state only the single session
+    // has follows
+    dctc_carver_batch* carver = nullptr;
     bool c_dump_vmaps = false;     // record the visibility map in the next seam loops (lqr_carver_set_dump_vmaps)
     int* c_band = nullptr;         // c_band[0]: 'rebuild the cumulative map from scratch' flag of the incremental seam DP, c_band[1]: rebuilds (device)
     bool c_incremental = false;    // device seam loop: update the cumulative map incrementally (dctc_carver_set_incremental)
