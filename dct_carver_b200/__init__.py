@@ -32,6 +32,8 @@ ABI_SYMBOLS = [
     "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
     "dctc_resize_plan", "dctc_carver_resize", "dctc_carver_batch_resize",
     "dctc_carver_set_bias", "dctc_carver_bias", "dctc_carver_batch_set_bias", "dctc_carver_batch_bias",
+    "dctc_carver_levels_width", "dctc_carver_levels_height", "dctc_carver_render_levels", "dctc_carver_batch_levels_width",
+    "dctc_carver_batch_levels_height", "dctc_carver_batch_render_levels", "dctc_carver_batch_render_levels_dev",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
     "dctc_dev_alloc", "dctc_dev_free", "dctc_host_alloc_pinned", "dctc_host_alloc_pinned_wc", "dctc_host_free_pinned", "dctc_memcpy_h2d",
     "dctc_memcpy_d2h", "dctc_memset_dev", "dctc_sync", "dctc_timer_begin", "dctc_timer_end",
@@ -145,6 +147,13 @@ def lib():
         "dctc_carver_bias": (i32, [vp, vp]),
         "dctc_carver_batch_set_bias": (i32, [vp, vp, sz, sz]),
         "dctc_carver_batch_bias": (i32, [vp, vp]),
+        "dctc_carver_levels_width": (i32, [vp, i32, vp]),
+        "dctc_carver_levels_height": (i32, [vp, i32, vp]),
+        "dctc_carver_render_levels": (i32, [vp, i32, vp, vp]),
+        "dctc_carver_batch_levels_width": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_levels_height": (i32, [vp, i32, vp]),
+        "dctc_carver_batch_render_levels": (i32, [vp, i32, vp, vp]),
+        "dctc_carver_batch_render_levels_dev": (i32, [vp, i32, vp, vp]),
         "dctc_pixel_energy": (f32, [i32, i32, i32, i32, vp, vp]),
         "dctc_synth_fill_dev": (i32, [vp, vp, i32, sz, i32, i32, i32, sz, u32, i32, i32, i32]),
         "dctc_synth_byte": (C.c_uint8, [u32, u32, u32, u32, u32, i32]),
@@ -250,6 +259,28 @@ def _resize(fn, handle, w, h, new_w, new_h, vmaps, n_frames):
             e["vmap"] = maps[vo:vo + nf * p["w"] * p["h"]].reshape(lead + (p["h"], p["w"]))
         out.append(e)
     return out
+
+
+def _render_levels(fn, handle, levels, extents, n_frames, ch, out=None):
+    """Runs dctc_carver_render_levels / dctc_carver_batch_render_levels (fn) after a build along levels = (axis, w, h),
+    the image size at the build (None: no build, fn reports the state), and splits its buffer into one uint8 array
+    ([n_frames,] H_i, W_i, ch) per extent."""
+    ext = np.ascontiguousarray([int(e) for e in extents], np.int32)
+    if levels is None:
+        shapes = [(0, 0)] * len(ext)
+    else:
+        axis, w, h = levels
+        shapes = [(h, max(int(e), 0)) if axis == "width" else (max(int(e), 0), w) for e in ext]
+    nf = n_frames or 1
+    sizes = [nf * H * W * ch for H, W in shapes]
+    buf = np.empty(max(sum(sizes), 1), np.uint8)
+    _check(fn(handle, len(ext), _ptr(ext) if len(ext) else None, _ptr(buf)), fn.__name__)
+    lead = (n_frames,) if n_frames else ()
+    res, o = [], 0
+    for (H, W), s in zip(shapes, sizes):
+        res.append(buf[o:o + s].reshape(lead + (H, W, ch)))
+        o += s
+    return res
 
 
 def _bias_plane(bias, shape):
@@ -408,6 +439,7 @@ class Context:
             img = img[:, :, None]
         img = np.ascontiguousarray(img, dtype=np.uint8)
         h, w, ch = img.shape
+        self._carver_levels = None
         _check(lib().dctc_carver_load(self._h, _ptr(img), w, h, ch, w * ch), "dctc_carver_load")
         self._carver_ch = ch
 
@@ -470,6 +502,30 @@ class Context:
         afterwards no seam operation until the next carver_load."""
         w, h = self.carver_size()
         return _resize(lib().dctc_carver_resize, self._h, w, h, new_w, new_h, vmaps, None)
+
+    def carver_levels_width(self, depth):
+        """The interactive dialog's build (dctc_carver_levels_width): one seam loop to depth with visibility maps and a
+        copy of the start image, after which carver_render_levels shows any width within depth of the start.  Returns the
+        seams as carver_resize_width does.  Needs a freshly loaded session; afterwards no seam operation until the next
+        carver_load, and the getters show the image carved by depth."""
+        return self._carver_levels_build(lib().dctc_carver_levels_width, "width", depth)
+
+    def carver_levels_height(self, depth):
+        """carver_levels_width along the other axis (dctc_carver_levels_height); seams as carver_resize_height."""
+        return self._carver_levels_build(lib().dctc_carver_levels_height, "height", depth)
+
+    def _carver_levels_build(self, fn, axis, depth):
+        w, h = self.carver_size()
+        seams = np.empty((depth, h if axis == "width" else w), np.int32)
+        _check(fn(self._h, int(depth), _ptr(seams) if depth else None), fn.__name__)
+        self._carver_levels = (axis, w, h)
+        return seams
+
+    def carver_render_levels(self, extents):
+        """dctc_carver_render_levels: one uint8 (H_i, W_i, ch) image per extent along the built axis, each bit for bit
+        what a fresh load and the resize (extent below the start) or enlarge (above) to that extent gives."""
+        return _render_levels(lib().dctc_carver_render_levels, self._h, getattr(self, "_carver_levels", None), extents,
+                              None, getattr(self, "_carver_ch", 1))
 
     def carver_set_bias(self, bias):
         """Per-pixel bias of the seam search (liblqr's lqr_carver_bias_add): float (h, w) at the current size, or None to
@@ -611,6 +667,7 @@ class CarverBatch:
         imgs = self._frames(imgs)
         if imgs.shape != (self.n, self.h, self.w0, self.ch):
             raise ValueError("frames must have the batch's shape %s" % ((self.n, self.h, self.w0, self.ch),))
+        self._levels = None
         _check(lib().dctc_carver_batch_load(self._b, _ptr(imgs), self.h * self.w0 * self.ch, self.w0 * self.ch),
                "dctc_carver_batch_load")
 
@@ -665,6 +722,34 @@ class CarverBatch:
         [n, n_seams, len] and, with vmaps, "vmap" [n, h, w].  Needs a freshly loaded batch; afterwards no seam operation
         until the next load()."""
         return _resize(lib().dctc_carver_batch_resize, self._b, self.width, self.height, new_w, new_h, vmaps, self.n)
+
+    def levels_width(self, depth):
+        """Context.carver_levels_width for every frame: returns int32 [n, depth, h]."""
+        return self._levels_build(lib().dctc_carver_batch_levels_width, "width", depth)
+
+    def levels_height(self, depth):
+        """Context.carver_levels_height for every frame: returns int32 [n, depth, w]."""
+        return self._levels_build(lib().dctc_carver_batch_levels_height, "height", depth)
+
+    def _levels_build(self, fn, axis, depth):
+        w, h = self.width, self.height
+        seams = np.empty((self.n, depth, h if axis == "width" else w), np.int32)
+        _check(fn(self._b, int(depth), _ptr(seams) if depth else None), fn.__name__)
+        self._levels = (axis, w, h)
+        return seams
+
+    def render_levels(self, extents):
+        """Context.carver_render_levels for every frame: one uint8 (n, H_i, W_i, ch) array per extent."""
+        return _render_levels(lib().dctc_carver_batch_render_levels, self._b, self._levels, extents, self.n, self.ch)
+
+    def render_levels_dev(self, extents, d_out):
+        """dctc_carver_batch_render_levels_dev into device memory at d_out (the layout of render_levels back to back);
+        returns the bytes written."""
+        ext = np.ascontiguousarray([int(e) for e in extents], np.int32)
+        _check(lib().dctc_carver_batch_render_levels_dev(self._b, len(ext), _ptr(ext) if len(ext) else None,
+                                                         C.c_void_p(d_out)), "dctc_carver_batch_render_levels_dev")
+        other = self.h if self._levels is None or self._levels[0] == "width" else self._levels[1]
+        return int(ext.sum()) * other * self.n * self.ch
 
     def set_bias(self, bias):
         """Context.carver_set_bias for every frame: float (n, h, w0), or None to clear.  Needs a freshly loaded batch;

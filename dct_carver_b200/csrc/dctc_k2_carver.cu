@@ -1101,6 +1101,80 @@ __global__ void __launch_bounds__(256) dctc_inflate_rows_kernel(const uint8_t* _
     }
 }
 
+// ---- levels: every extent within the depth of one seam loop (liblqr's interactive resize) ------------------------------
+// After a seam loop to depth n with visibility maps, the start image shrunk by k <= n seams is the row's pixels with
+// vs == 0 || vs > k in their original order.  One CTA per row reads the row's map and pixels once and writes that row of
+// every level of the table: a kept pixel's output column is x minus the pixels before it with 1 <= vs <= k, from one
+// ballot per warp and level and the warps' counts in shared memory.  Chunks of 256 columns with a running count per level,
+// as in dctc_inflate_rows_kernel, so any width the seam DP covers fits.  blockIdx.y = frame (source image, map orig_fs
+// bytes and vs_fs ints after the previous frame's).  Level l is w0 - k[l] wide; its frames start at out + off[l], rows
+// packed ((w0 - k) * channels bytes), frames h rows apart.
+constexpr int LV_MAX = 32;   // levels per launch (the 256 threads hold one (level, warp) prefix each)
+struct LevelTable {
+    int n;
+    int k[LV_MAX];
+    size_t off[LV_MAX];
+};
+
+__global__ void __launch_bounds__(256) dctc_levels_gather_kernel(const uint8_t* __restrict__ orig, size_t pitch, int channels, int w0,
+                                                                 const int* __restrict__ vs, size_t orig_fs, size_t vs_fs,
+                                                                 const LevelTable lv, uint8_t* __restrict__ out)
+{
+    __shared__ int wsum[LV_MAX][8];      // removed pixels of the chunk in each warp
+    __shared__ int wpre[LV_MAX][8];      // removed pixels of the row before each warp's part of the chunk
+    __shared__ int running[LV_MAX];
+    __shared__ int ks[LV_MAX];
+    __shared__ size_t offs[LV_MAX];
+    const int y = blockIdx.x, z = blockIdx.y, tid = threadIdx.x, lane = tid & 31, wid = tid >> 5, nl = lv.n;
+    const uint8_t* src = orig + z * orig_fs + (size_t) y * pitch;
+    const int* vrow = vs + z * vs_fs + (size_t) y * w0;
+    const size_t row0 = (size_t) z * gridDim.x + y;   // row index of this row in a level's frames
+    const unsigned below = (1u << lane) - 1u;
+    if (tid < nl) {
+        running[tid] = 0;
+        ks[tid] = lv.k[tid];
+        offs[tid] = lv.off[tid];
+    }
+    __syncthreads();
+    for (int base = 0; base < w0; base += 256) {
+        const int x = base + tid;
+        const bool in = x < w0;
+        const int v = in ? vrow[x] : 0;
+        uint8_t px[4];
+#pragma unroll
+        for (int c = 0; c < 4; c++)
+            if (c < channels && in) px[c] = src[(size_t) x * channels + c];
+        for (int l = 0; l < nl; l++) {
+            const unsigned m = __ballot_sync(0xffffffffu, v >= 1 && v <= ks[l]);
+            if (lane == 0) wsum[l][wid] = __popc(m);
+        }
+        __syncthreads();
+        {
+            const int l = tid >> 3, w = tid & 7;
+            if (l < nl) {
+                int s = running[l];
+                for (int j = 0; j < w; j++) s += wsum[l][j];
+                wpre[l][w] = s;
+            }
+        }
+        __syncthreads();
+        if (tid < nl) running[tid] = wpre[tid][7] + wsum[tid][7];
+        for (int l = 0; l < nl; l++) {
+            const int k = ks[l];
+            const bool gone = v >= 1 && v <= k;
+            const unsigned m = __ballot_sync(0xffffffffu, gone);
+            if (in && !gone) {
+                const int e = w0 - k, col = x - wpre[l][wid] - __popc(m & below);
+                uint8_t* q = out + offs[l] + (row0 * e + col) * channels;
+#pragma unroll
+                for (int c = 0; c < 4; c++)
+                    if (c < channels) q[c] = px[c];
+            }
+        }
+        __syncthreads();
+    }
+}
+
 // ---- bias (lqr_carver_bias_add: preserve / discard masks) ------------------------------------------------------------
 // The seam energy of a biased session, after a full K1 of its frames: en = fl(en + fl(bias / ext)), ext = the frames'
 // start width.  __fdiv_rn / __fadd_rn: IEEE division and add whatever the compiler flags (the band K1's bias store
@@ -1536,17 +1610,16 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
     return DCTC_OK;
 }
 
-// Enlarge core (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): the start frames are copied
-// to start_img, the seam loop removes n_seams seams and records their order in the visibility maps (as frames_vmaps
-// leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images (w0 + n_seams
-// wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
+// Enlarge core (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): start_img holds a copy of
+// f's images (session_copy_start), the seam loop removes n_seams seams and records their order in the visibility maps (as
+// frames_vmaps leaves them), one inflate launch doubles every pixel of those seams in all frames into wide's images
+// (w0 + n_seams wide) and one K1 launch computes their full energy maps.  f is left carved by n_seams.
 // Biased frames: a copy of the start bias planes is inflated in the same launch (copy rule) into wide's bias planes, and
 // one bias-add launch gives wide's seam energy with ext = wide.w0.
 static int frames_enlarge(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, SeamCall c,
-                          uint8_t* start_img, CarverFrames& wide)
+                          const uint8_t* start_img, CarverFrames& wide)
 {
     c.vmaps = true;
-    CK(ctx, cudaMemcpyAsync(start_img, f.img, f.img_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream));
     const size_t en_fs = f.en_pitch * f.h;
     float* start_bias = nullptr;
     int rc = frames_bias_like(ctx, f, wide);
@@ -1602,8 +1675,10 @@ static int frames_set_bias(dctc_context* ctx, CarverFrames& f, const DctcK1Op& o
 // left unloaded.
 
 // The axis the seam operations work along since the load: the first one fixes it, a call for the other axis returns
-// DCTC_ERR_STATE until the next load.  RESIZED: a combined resize ran since the load, which fixes both axes.
-enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2, DCTC_AXIS_RESIZED = 3 };
+// DCTC_ERR_STATE until the next load.  RESIZED: a combined resize ran since the load, which fixes both axes.  LEVELS: a
+// levels build ran since the load (session_levels); it ends the seam operations until the next load, and the renders
+// read cur's maps and the start frames' copy (cur->transposed: height levels).
+enum { DCTC_AXIS_NONE = 0, DCTC_AXIS_WIDTH = 1, DCTC_AXIS_HEIGHT = 2, DCTC_AXIS_RESIZED = 3, DCTC_AXIS_LEVELS = 4 };
 
 // Frame sets are allocated by their first use, reallocated when their size differs and freed with the session: the
 // loaded frames f next to their transposes t, and the start frames' copy next to the enlarged sets.
@@ -1621,8 +1696,10 @@ struct dctc_carver_batch {
     CarverFrames f;                     // the loaded frames
     CarverFrames t;                     // their transposes (height operations)
     CarverFrames wide, wide2;           // enlarged frames: an enlarge writes into the one that is not cur
-    uint8_t* start_img = nullptr;       // an enlarge's copy of its start images
+    uint8_t* start_img = nullptr;       // an enlarge's or a levels build's copy of its start images
     size_t start_bytes = 0;
+    uint8_t* lv_scratch = nullptr;      // height levels in the transposed orientation on their way out (session_render)
+    size_t lv_scratch_bytes = 0;
 };
 
 namespace {
@@ -1634,6 +1711,7 @@ void session_destroy(dctc_carver_batch* b)
     frames_free(b->wide);
     frames_free(b->wide2);
     cudaFree(b->start_img);
+    cudaFree(b->lv_scratch);
     delete b;
 }
 
@@ -1728,6 +1806,21 @@ int session_carve(dctc_carver_batch* b, int n_seams, int* seams_out, const SeamC
     return seam_loop(b->ctx, f, b->op, n_seams, seams_out, c);
 }
 
+// The start frames' copy of an enlarge or a levels build: f's images into start_img (reallocated when its size differs,
+// kept until the destroy), one device copy on the stream
+int session_copy_start(dctc_carver_batch* b, const CarverFrames& f)
+{
+    dctc_context* ctx = b->ctx;
+    if (b->start_bytes != f.img_fs * f.n) {
+        cudaFree(b->start_img);
+        b->start_img = nullptr; b->start_bytes = 0;
+        CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
+        b->start_bytes = f.img_fs * f.n;
+    }
+    CK(ctx, cudaMemcpyAsync(b->start_img, f.img, f.img_fs * f.n, cudaMemcpyDeviceToDevice, ctx->stream));
+    return DCTC_OK;
+}
+
 // An enlarge: frames_enlarge from cur (as loaded or enlarged) into the enlarged set that is not cur, which becomes cur;
 // the maps stay those of the start frames.  cur is carved in place, so a failure leaves the session unloaded.
 int session_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out, const SeamCall& c)
@@ -1737,12 +1830,8 @@ int session_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out, const Sea
     CarverFrames& wide = b->cur == &b->wide ? b->wide2 : b->wide;
     b->cur = nullptr;
     const int w1 = f.w0 + n_seams;
-    if (b->start_bytes != f.img_fs * f.n) {
-        cudaFree(b->start_img);
-        b->start_img = nullptr; b->start_bytes = 0;
-        CK(ctx, cudaMalloc((void**) &b->start_img, f.img_fs * f.n));
-        b->start_bytes = f.img_fs * f.n;
-    }
+    const int rs = session_copy_start(b, f);
+    if (rs) return rs;
     if (wide.w0 != w1 || wide.h != f.h) {
         frames_free(wide);
         frames_init(wide, f.n, w1, f.h, f.ch);
@@ -1773,7 +1862,8 @@ int session_enlarge(dctc_carver_batch* b, int n_seams, int* seams_out, const Sea
 int session_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out, const SeamCall& c)
 {
     const bool enlarged = b->cur == &b->wide || b->cur == &b->wide2;
-    if (!b->cur || (b->ends_at_enlarge && (enlarged || b->axis == DCTC_AXIS_RESIZED))) return DCTC_ERR_STATE;
+    if (!b->cur || b->axis == DCTC_AXIS_LEVELS || (b->ends_at_enlarge && (enlarged || b->axis == DCTC_AXIS_RESIZED)))
+        return DCTC_ERR_STATE;
     if (n_seams == 0) return DCTC_OK;
     const CarverFrames& f = *b->cur;
     if (enlarge && f.w != f.w0) return DCTC_ERR_STATE;   // an enlarge starts from frames as loaded (or enlarged)
@@ -1822,6 +1912,128 @@ int session_resize(dctc_carver_batch* b, int new_w, int new_h, int* seams_out, i
     }
     b->axis = DCTC_AXIS_RESIZED;
     return DCTC_OK;
+}
+
+// dctc_carver_levels_width / _height and the batch's (lqr_carver_resize to the extreme size of the interactive dialog):
+// on frames as loaded, the start frames' copy (session_copy_start) and what resize_width / resize_height with maps runs
+// (the axis switch for heights, fresh maps, the seam loop to depth).  cur is left carved by depth with its maps recorded,
+// and the axis becomes LEVELS.  A failure leaves the session unloaded.
+int session_levels(dctc_carver_batch* b, int axis, int depth, int* seams_out, const SeamCall& c)
+{
+    if (!b->cur || b->axis != DCTC_AXIS_NONE) return DCTC_ERR_STATE;   // loaded, no seam operation since
+    const int extent = axis == DCTC_AXIS_WIDTH ? frames_image_w(*b->cur) : frames_image_h(*b->cur);
+    if (depth >= extent) return DCTC_ERR_STATE;
+    if (extent > DP_MAX_W) return DCTC_ERR_UNSUPPORTED;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    SeamCall lc = c;
+    lc.vmaps = true;
+    if (axis == DCTC_AXIS_HEIGHT) {
+        const int rc = session_transpose(b, true, lc);
+        if (rc) return rc;
+    }
+    b->axis = DCTC_AXIS_LEVELS;
+    CarverFrames& f = *b->cur;
+    b->cur = nullptr;
+    int rc = session_copy_start(b, f);
+    if (rc == DCTC_OK && b->maps != &f) {
+        rc = frames_fresh_vmaps(ctx, f);
+        b->maps = &f;
+    }
+    if (rc == DCTC_OK && depth > 0) rc = seam_loop(ctx, f, b->op, depth, seams_out, lc);
+    if (rc) return rc;
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    b->cur = &f;
+    return DCTC_OK;
+}
+
+// dctc_carver_render_levels_dev / dctc_carver_batch_render_levels_dev: the levels of a build since the load into d_out
+// (device memory), level-major in the order of extents, each n frames of rows packed in image orientation.  Extents up
+// to the start extent e0 are shrinks (one gather launch per LV_MAX of them), wider ones enlarges (one inflate launch each,
+// level e - e0: what an enlarge by e - e0 writes).  Height levels are built in the transposed orientation in lv_scratch
+// and turned into image orientation by one transpose launch each.  The session does not change.
+int session_render(dctc_carver_batch* b, int n_levels, const int* extents, uint8_t* d_out)
+{
+    if (!b->cur || b->axis != DCTC_AXIS_LEVELS) return DCTC_ERR_STATE;
+    const CarverFrames& f = *b->cur;
+    const int e0 = f.w0;
+    for (int i = 0; i < n_levels; i++)
+        if (extents[i] < e0 - f.depth || extents[i] > e0 + f.depth) return DCTC_ERR_STATE;
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    const size_t unit = (size_t) f.n * f.h * f.ch;   // bytes of a level per column of extent (rows f.h in f's orientation)
+    size_t total = 0;
+    for (int i = 0; i < n_levels; i++) total += unit * extents[i];
+    uint8_t* dst = d_out;
+    if (f.transposed) {
+        if (b->lv_scratch_bytes < total) {
+            cudaFree(b->lv_scratch);
+            b->lv_scratch = nullptr; b->lv_scratch_bytes = 0;
+            CK(ctx, cudaMalloc((void**) &b->lv_scratch, total));
+            b->lv_scratch_bytes = total;
+        }
+        dst = b->lv_scratch;
+    }
+    const size_t vs_fs = (size_t) f.w0 * f.h;
+    LevelTable lt;
+    lt.n = 0;
+    auto gather = [&]() {
+        dctc_levels_gather_kernel<<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(b->start_img, f.pitch, f.ch, f.w0, f.vs, f.img_fs, vs_fs, lt, dst);
+        ctx->launches++;
+        lt.n = 0;
+        return cudaGetLastError();
+    };
+    size_t off = 0;
+    for (int i = 0; i < n_levels; i++) {
+        const int e = extents[i];
+        const size_t row = (size_t) e * f.ch;
+        if (e <= e0) {
+            lt.k[lt.n] = e0 - e;
+            lt.off[lt.n] = off;
+            if (++lt.n == LV_MAX) CK(ctx, gather());
+        } else {
+            dctc_inflate_rows_kernel<false><<<dim3(f.h, f.n), 256, 0, ctx->stream>>>(b->start_img, f.pitch, f.ch, f.w0, f.vs, e - e0,
+                                                                                    dst + off, row, f.img_fs, vs_fs, row * f.h, nullptr,
+                                                                                    0, 0, nullptr, 0, 0);
+            ctx->launches++;
+            CK(ctx, cudaGetLastError());
+        }
+        off += unit * e;
+    }
+    if (lt.n) CK(ctx, gather());
+    if (f.transposed) {
+        off = 0;
+        for (int i = 0; i < n_levels; i++) {
+            const int e = extents[i];
+            const size_t row = (size_t) e * f.ch, orow = (size_t) f.h * f.ch;
+            CK(ctx, dctc_launch_transpose(dst + off, row, row * f.h, d_out + off, orow, orow * e, e, f.h, f.n, f.ch, ctx->stream));
+            ctx->launches++;
+            off += unit * e;
+        }
+    }
+    CK(ctx, cudaStreamSynchronize(ctx->stream));
+    return DCTC_OK;
+}
+
+// session_render into a device buffer of the call's size, then to the host
+int session_render_host(dctc_carver_batch* b, int n_levels, const int* extents, uint8_t* out)
+{
+    if (!b->cur || b->axis != DCTC_AXIS_LEVELS) return DCTC_ERR_STATE;
+    const CarverFrames& f = *b->cur;
+    size_t total = 0;
+    for (int i = 0; i < n_levels; i++) total += (size_t) f.n * f.h * f.ch * (size_t) (extents[i] > 0 ? extents[i] : 0);
+    dctc_context* ctx = b->ctx;
+    CK(ctx, cudaSetDevice(ctx->device));
+    uint8_t* d = nullptr;
+    CK(ctx, cudaMalloc((void**) &d, total));
+    int rc = session_render(b, n_levels, extents, d);
+    if (rc == DCTC_OK) {
+        cudaError_t e = cudaMemcpyAsync(out, d, total, cudaMemcpyDeviceToHost, ctx->stream);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+        if (e != cudaSuccess) rc = dctc_fail_cuda(ctx, e);
+    }
+    cudaFree(d);
+    return rc;
 }
 
 // Images, operator energy maps or bias planes of the current frames
@@ -1938,6 +2150,21 @@ static int carver_download(dctc_context* ctx, uint8_t* img, float* en, float* bi
     return session_download(ctx->carver, img, en, bias);
 }
 
+static int carver_levels(dctc_context* ctx, int axis, int depth, int* seams_out)
+{
+    if (!ctx || depth < 0) return DCTC_ERR_INVALID;
+    return carver_call(ctx, [&](dctc_carver_batch* b, const SeamCall& c) { return session_levels(b, axis, depth, seams_out, c); });
+}
+
+// The argument checks of the render calls
+static bool levels_args(int n_levels, const int* extents, const void* out)
+{
+    if (n_levels <= 0 || !extents || !out) return false;
+    for (int i = 0; i < n_levels; i++)
+        if (extents[i] <= 0) return false;
+    return true;
+}
+
 extern "C" {
 
 int dctc_carver_load(dctc_context* ctx, const uint8_t* img, int w, int h, int channels, size_t pitch)
@@ -1992,7 +2219,7 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
 {
     if (!ctx || !seam_x) return DCTC_ERR_INVALID;
     dctc_carver_batch* s = ctx->carver;
-    if (!s || s->axis == DCTC_AXIS_HEIGHT || s->axis == DCTC_AXIS_RESIZED) return DCTC_ERR_STATE;   // vertical seams only
+    if (!s || (s->axis != DCTC_AXIS_NONE && s->axis != DCTC_AXIS_WIDTH)) return DCTC_ERR_STATE;   // vertical seams only
     CarverFrames* f = s->cur;
     if (f->w <= 1) return DCTC_ERR_STATE;
     if (f->bias) return DCTC_ERR_STATE;   // the caller's seam and the operator's band values: no place for a bias
@@ -2056,6 +2283,23 @@ int dctc_carver_enlarge_width(dctc_context* ctx, int n_seams, int* seams_out)
 int dctc_carver_enlarge_height(dctc_context* ctx, int n_seams, int* seams_out)
 {
     return carver_seams(ctx, DCTC_AXIS_HEIGHT, true, n_seams, seams_out);
+}
+
+int dctc_carver_levels_width(dctc_context* ctx, int depth, int* seams_out)
+{
+    return carver_levels(ctx, DCTC_AXIS_WIDTH, depth, seams_out);
+}
+
+int dctc_carver_levels_height(dctc_context* ctx, int depth, int* seams_out)
+{
+    return carver_levels(ctx, DCTC_AXIS_HEIGHT, depth, seams_out);
+}
+
+int dctc_carver_render_levels(dctc_context* ctx, int n_levels, const int* extents, uint8_t* out)
+{
+    if (!ctx || !levels_args(n_levels, extents, out)) return DCTC_ERR_INVALID;
+    if (!ctx->carver) return DCTC_ERR_STATE;
+    return session_render_host(ctx->carver, n_levels, extents, out);
 }
 
 int dctc_resize_plan(int w, int h, int new_w, int new_h, DctcResizePass* passes, int max_passes)
@@ -2257,6 +2501,30 @@ int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
     if (!b) return DCTC_ERR_INVALID;
     if (!b->dump_vmaps) return DCTC_ERR_STATE;   // maps were not asked for at create (an enlarge records them anyway)
     return session_vmap(b, vmap_out, depth_out);
+}
+
+int dctc_carver_batch_levels_width(dctc_carver_batch* b, int depth, int* seams_out)
+{
+    if (!b || depth < 0) return DCTC_ERR_INVALID;
+    return session_levels(b, DCTC_AXIS_WIDTH, depth, seams_out, SeamCall());
+}
+
+int dctc_carver_batch_levels_height(dctc_carver_batch* b, int depth, int* seams_out)
+{
+    if (!b || depth < 0) return DCTC_ERR_INVALID;
+    return session_levels(b, DCTC_AXIS_HEIGHT, depth, seams_out, SeamCall());
+}
+
+int dctc_carver_batch_render_levels(dctc_carver_batch* b, int n_levels, const int* extents, uint8_t* out)
+{
+    if (!b || !levels_args(n_levels, extents, out)) return DCTC_ERR_INVALID;
+    return session_render_host(b, n_levels, extents, out);
+}
+
+int dctc_carver_batch_render_levels_dev(dctc_carver_batch* b, int n_levels, const int* extents, uint8_t* d_out)
+{
+    if (!b || !levels_args(n_levels, extents, d_out)) return DCTC_ERR_INVALID;
+    return session_render(b, n_levels, extents, d_out);
 }
 
 }  // extern "C"

@@ -220,6 +220,28 @@ int dctc_resize_plan(int w, int h, int new_w, int new_h, DctcResizePass *passes,
  * dctc_carver_resize, dctc_carver_vmap and dctc_carver_paint_seams return DCTC_ERR_STATE until the next load.  A CUDA
  * failure leaves the session unloaded. */
 int dctc_carver_resize(dctc_context *ctx, int new_w, int new_h, int *seams_out, int *vmaps_out);
+/* ---- levels: interactive resizing (gui_interactive_dialog, src/interface.c:37-135, callback_resize_slider :647-670) --
+ * One seam loop to depth n, then any extent within n of the start, each a gather over the start image and the visibility
+ * map.  dctc_carver_levels_width / _height run what dctc_carver_resize_width / _height(depth) with visibility maps run
+ * (maps recorded whatever dctc_carver_set_dump_vmaps says; incremental mode and a bias apply) and keep a device copy of
+ * the start frame (for heights its transpose).  seams_out as for dctc_carver_resize_width / _height.  Needs a loaded
+ * session with no seam operation since the load (DCTC_ERR_STATE otherwise).  DCTC_ERR_INVALID: depth < 0.
+ * DCTC_ERR_STATE: depth >= the extent along the axis.  DCTC_ERR_UNSUPPORTED: an extent wider than the device seam DP
+ * covers (before any work: the session stays loaded).  depth == 0: DCTC_OK, and only the start extent renders.
+ * Afterwards dctc_carver_width / _height / _image / _energy / _energy_image and dctc_pixel_energy show the frame carved by
+ * depth; dctc_carver_vmap and _paint_seams the depth-n map; dctc_set_params rebuilds the energy map and keeps the levels.
+ * Seam operations, dctc_carver_resize, dctc_carver_set_bias and another build return DCTC_ERR_STATE until the next load,
+ * which drops the levels.  A CUDA failure leaves the session unloaded. */
+int dctc_carver_levels_width(dctc_context *ctx, int depth, int *seams_out);
+int dctc_carver_levels_height(dctc_context *ctx, int depth, int *seams_out);
+/* n_levels images along the built axis, level-major in the order of extents: level i is n_frames * H_i * W_i * channels
+ * bytes in image orientation, rows packed (W_i = extents[i] for width levels, H_i = extents[i] for height levels, the
+ * other side the start frame's).  With e0 the start extent, an extent e0 - k (k <= depth) is bit for bit the image that
+ * dctc_carver_load + the resize by k gives, e0 + m (m <= depth) the image that dctc_carver_load + the enlarge by m gives.
+ * Extents may come in any order and repeat; the session does not change.  DCTC_ERR_INVALID: n_levels <= 0, NULL extents
+ * or out, an extent <= 0.  DCTC_ERR_STATE: no build since the load, an extent outside [e0 - depth, e0 + depth]. */
+int dctc_carver_render_levels(dctc_context *ctx, int n_levels, const int *extents, uint8_t *out);
+
 /* Optional: let the device loop update its cumulative map incrementally after each seam, like liblqr's update_mmap
  * (only the cells the removed seam can have changed are recomputed; a row whose changed range gets too wide falls
  * back to the full rebuild).  Same seams bit for bit; off by default because the full rebuild on an 8-CTA cluster is
@@ -339,6 +361,15 @@ int dctc_carver_batch_energy(dctc_carver_batch *batch, float *out);
 /* visibility map of every frame over the loaded size (n_frames * h * w0 ints) and the common depth; needs dump_vmaps
  * at create time */
 int dctc_carver_batch_vmap(dctc_carver_batch *batch, int *vmap_out, int *depth_out);
+/* dctc_carver_levels_width / _height and dctc_carver_render_levels for every frame: seams_out as the batch's
+ * _resize_width / _resize_height; every frame's level is what the single session renders for it alone.  The rules are the
+ * single session's; _vmap after a build needs dump_vmaps, as after an enlarge.  A CUDA failure in a build leaves the batch
+ * unloaded. */
+int dctc_carver_batch_levels_width(dctc_carver_batch *batch, int depth, int *seams_out);
+int dctc_carver_batch_levels_height(dctc_carver_batch *batch, int depth, int *seams_out);
+int dctc_carver_batch_render_levels(dctc_carver_batch *batch, int n_levels, const int *extents, uint8_t *out);
+/* the same layout into device memory the caller owns (4-byte aligned), no host copy */
+int dctc_carver_batch_render_levels_dev(dctc_carver_batch *batch, int n_levels, const int *extents, uint8_t *d_out);
 
 /* ---- K3: energy-image export ------------------------------------------------------------------------------
  * Replaces lqr_carver_get_energy_image(carver, buf, orientation, LQR_COLDEPTH_8I, LQR_GREY_IMAGE) as called at
