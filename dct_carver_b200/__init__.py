@@ -32,6 +32,7 @@ ABI_SYMBOLS = [
     "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
     "dctc_resize_plan", "dctc_carver_resize", "dctc_carver_batch_resize",
     "dctc_carver_set_bias", "dctc_carver_bias", "dctc_carver_batch_set_bias", "dctc_carver_batch_bias",
+    "dctc_carver_set_rigidity", "dctc_carver_batch_set_rigidity",
     "dctc_carver_levels_width", "dctc_carver_levels_height", "dctc_carver_render_levels", "dctc_carver_batch_levels_width",
     "dctc_carver_batch_levels_height", "dctc_carver_batch_render_levels", "dctc_carver_batch_render_levels_dev",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
@@ -147,6 +148,8 @@ def lib():
         "dctc_carver_bias": (i32, [vp, vp]),
         "dctc_carver_batch_set_bias": (i32, [vp, vp, sz, sz]),
         "dctc_carver_batch_bias": (i32, [vp, vp]),
+        "dctc_carver_set_rigidity": (i32, [vp, f32]),
+        "dctc_carver_batch_set_rigidity": (i32, [vp, f32]),
         "dctc_carver_levels_width": (i32, [vp, i32, vp]),
         "dctc_carver_levels_height": (i32, [vp, i32, vp]),
         "dctc_carver_render_levels": (i32, [vp, i32, vp, vp]),
@@ -546,6 +549,12 @@ class Context:
         _check(lib().dctc_carver_bias(self._h, _ptr(out)), "dctc_carver_bias")
         return out
 
+    def carver_set_rigidity(self, rigidity):
+        """liblqr's rigidity (lqr_carver_init): a seam step to a neighbouring column costs rigidity / h more, h the seam
+        length, so larger values give straighter seams (include/dctc.h).  Applies from the next seam operation and
+        survives carver_load; 0 (the default) is the plain seam search.  Raises for a negative or non-finite value."""
+        _check(lib().dctc_carver_set_rigidity(self._h, float(rigidity)), "dctc_carver_set_rigidity")
+
     def carver_set_incremental(self, on):
         """Device seam loop: update the cumulative map incrementally (liblqr's update_mmap) instead of rebuilding it."""
         _check(lib().dctc_carver_set_incremental(self._h, int(bool(on))), "dctc_carver_set_incremental")
@@ -760,6 +769,11 @@ class CarverBatch:
         b = _bias_plane(bias, (self.n, self.h, self.w0))
         _check(lib().dctc_carver_batch_set_bias(self._b, _ptr(b), self.h * self.w0 * 4, self.w0 * 4),
                "dctc_carver_batch_set_bias")
+
+    def set_rigidity(self, rigidity):
+        """Context.carver_set_rigidity for every frame of the batch: applies from the next seam operation and survives
+        load()."""
+        _check(lib().dctc_carver_batch_set_rigidity(self._b, float(rigidity)), "dctc_carver_batch_set_rigidity")
 
     def bias(self):
         """The current bias planes (n, height, width)."""

@@ -5,6 +5,7 @@
 // within +-radius of the seam (radius = blocksize/2, registered at src/render.c:314-315).  Here the image and the
 // energy plane stay resident in HBM; one kernel compacts both over the seam, then the K1 tile kernel runs in band
 // mode over just the touched pixels, with arithmetic identical to a full recompute (bit-identical results).
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <type_traits>
@@ -103,10 +104,14 @@ __global__ void __launch_bounds__(NT) dctc_carve_rows_kernel(uint8_t* __restrict
 
 
 // ---- seam DP + back-track on the device (SURVEY section 8f rank 1) ---------------------------------------------
-// liblqr's build_mmap / build_vpath for delta_x = 1, rigidity = 0 (src/render.c:313,377; restated in
-// dct_carver_b200/host/dctc_lqr.c and oracle/oracle_carver.c):
+// liblqr's build_mmap / build_vpath for delta_x = 1 (src/render.c:313,377; restated in dct_carver_b200/host/dctc_lqr.c
+// and oracle/oracle_carver.c):
 //   m[0][x] = en[0][x];  m[y][x] = en[y][x] + min(m[y-1][x-1], m[y-1][x], m[y-1][x+1])   (FP32, range clipped)
 //   parent of (y, x) = FIRST strict minimum scanning x-1, x, x+1;  seam end = LEFTMOST minimum of the last row.
+// Rigidity (the RIG instantiations of the DP, jump, trace and incremental kernels): a diagonal step costs pen =
+// fl(rigidity / h) more, i.e. the candidates are fl(m[y-1][x-1] + pen), m[y-1][x], fl(m[y-1][x+1] + pen) in the map and
+// in the parent choice (liblqr's rigidity_map[1] = rigidity / h [from memory: parity unpinned]).  The host passes pen
+// as a trailing kernel argument; the false instantiations never read it and are the kernels of rigidity 0.
 // The map is rebuilt from scratch for every seam (same values as liblqr's incremental update_mmap).  Row y depends on
 // the whole row y-1: a chain of h steps.  Versions with one CTA-wide barrier per row cost ~600-950 clk per row
 // (shared-memory bandwidth, then the latency of a 16-warp barrier round); this one removes the per-row barrier with
@@ -171,9 +176,10 @@ constexpr int DP_WIN = 144;       // back-track window (floats); the cumulative 
 constexpr int DP_WINP = DP_WIN + 8;   // window row in shared memory: 3 pad floats, the left sentinel, DP_WIN columns, the right
                                       // sentinel (needed when the window ends exactly at column w) and 3 pad floats
 
+template <bool RIG>
 __device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, size_t m_pitch, int w, int h, int x,
                                              int* __restrict__ seam, int* __restrict__ seam_log,
-                                             float (*win)[32][DP_WINP], int lane)
+                                             float (*win)[32][DP_WINP], int lane, float pen)
 {
     const float INF = __int_as_float(0x7f800000);
     if (lane == 0) { seam[h - 1] = x; if (seam_log) seam_log[h - 1] = x; }
@@ -212,7 +218,7 @@ __device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, s
         int mine = 0;
         const float* wp = &win[buf][0][4] + (x - base);        // wp[0] = cumulative value at (window row, column x)
         auto walk = [&](int i) {
-            const float a = wp[-1], b = wp[0], c = wp[1];
+            const float a = RIG ? wp[-1] + pen : wp[-1], b = wp[0], c = RIG ? wp[1] + pen : wp[1];
             const bool p1 = b < a;
             const float best = p1 ? b : a;
             const bool p2 = c < best;
@@ -275,13 +281,15 @@ __device__ __forceinline__ void dp_unroll(F&& f)
 // One cluster per frame: blockIdx.y = frame of a batch session, whose energy / cumulative planes start en_fs / m_fs
 // floats after the previous frame's, whose seam is seam[h * frame ...], its log seam_log[log_fs * frame ...] and its
 // last-row column xlast[frame].  The tensor map is 3-D (columns, rows, frames) with a box depth of one frame.
-template <int DP_P, int DP_SR>
+// RIG: rigidity pen (see above), the trailing argument.
+template <int DP_P, int DP_SR, bool RIG>
 __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dctc_seam_dp_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                                     float* __restrict__ mplane, size_t m_pitch,
                                                                     int* __restrict__ seam, int* __restrict__ seam_log,
                                                                     int* __restrict__ run_flag, int nst,
                                                                     const __grid_constant__ CUtensorMap tmap, int use_tmap,
-                                                                    int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs)
+                                                                    int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs,
+                                                                    float pen)
 {
     DCTC_PDL_PROLOGUE();
     // (the frame's seam, log and xlast offsets are applied after the row loop, so they occupy no registers in it)
@@ -455,20 +463,25 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
                 asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(e[0][g].x), "=f"(e[0][g].y), "=f"(e[0][g].z), "=f"(e[0][g].w)
                              : "r"(stg_s + (uint32_t) (((kk % SRD) * STRIP + 4 * g) * 4)));   // base register + immediate
         }
+        // q: the previous row as a diagonal parent sees it (RIG: cur + pen, one add per cell; else cur itself)
+        float4 q[DP_P];
+#pragma unroll
+        for (int g = 0; g < DP_P; g++)
+            q[g] = RIG ? make_float4(cur[g].x + pen, cur[g].y + pen, cur[g].z + pen, cur[g].w + pen) : cur[g];
         // neighbours across lanes; the strip's outermost lanes see +inf (their cells are never published)
-        float l = __shfl_up_sync(0xffffffffu, cur[DP_P - 1].w, 1);
-        float r = __shfl_down_sync(0xffffffffu, cur[0].x, 1);
+        float l = __shfl_up_sync(0xffffffffu, q[DP_P - 1].w, 1);
+        float r = __shfl_down_sync(0xffffffffu, q[0].x, 1);
         if (lane == 0) l = INF;
         if (lane == 31) r = INF;
         float4 o[DP_P];
 #pragma unroll
         for (int g = 0; g < DP_P; g++) {
-            const float lg = g == 0 ? l : cur[g > 0 ? g - 1 : 0].w;
-            const float rg = g == DP_P - 1 ? r : cur[g < DP_P - 1 ? g + 1 : g].x;
-            o[g].x = e[k][g].x + fminf(fminf(lg, cur[g].x), cur[g].y);
-            o[g].y = e[k][g].y + fminf(fminf(cur[g].x, cur[g].y), cur[g].z);
-            o[g].z = e[k][g].z + fminf(fminf(cur[g].y, cur[g].z), cur[g].w);
-            o[g].w = e[k][g].w + fminf(fminf(cur[g].z, cur[g].w), rg);
+            const float lg = g == 0 ? l : q[g > 0 ? g - 1 : 0].w;
+            const float rg = g == DP_P - 1 ? r : q[g < DP_P - 1 ? g + 1 : g].x;
+            o[g].x = e[k][g].x + fminf(fminf(lg, cur[g].x), q[g].y);
+            o[g].y = e[k][g].y + fminf(fminf(q[g].x, cur[g].y), q[g].z);
+            o[g].z = e[k][g].z + fminf(fminf(q[g].y, cur[g].z), q[g].w);
+            o[g].w = e[k][g].w + fminf(fminf(q[g].z, cur[g].w), rg);
         }
         // register-ring variant: refill the slot just consumed with the row PF ahead (issued after the last use of the
         // slot, so the load targets the slot's registers directly; they are not touched again for PF rows)
@@ -612,7 +625,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             // parallel back-track: the jump and trace kernels below take over from the seam's last-row column
             if (lane == 0) { *xlast = bi; seam[h - 1] = bi; if (seam_log) seam_log[h - 1] = bi; }
         } else {
-            dp_backtrack(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane);   // serial walk by warp 0 of CTA 0
+            dp_backtrack<RIG>(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);   // serial walk by warp 0 of CTA 0
         }
 #ifdef DCTC_SYNC_DEBUG
         if (tid == 0) {
@@ -636,10 +649,11 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
 // into shared memory first), then walks its 32 rows like dp_backtrack does.  ~100 dependent steps instead of h.
 constexpr int JB = 32;
 
-// Batch sessions: blockIdx.z = frame (planes m_fs floats / j_fs bytes apart).
+// Batch sessions: blockIdx.z = frame (planes m_fs floats / j_fs bytes apart).  RIG: rigidity pen, as in the DP.
+template <bool RIG>
 __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
                                                              int8_t* __restrict__ jump, size_t j_pitch, int strips,
-                                                             size_t m_fs, size_t j_fs)
+                                                             size_t m_fs, size_t j_fs, float pen)
 {
     DCTC_PDL_PROLOGUE();
     const int lane = threadIdx.x & 31;
@@ -668,7 +682,8 @@ __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __rest
         int Q[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) {
-            const float a = j == 0 ? l : m[j - 1], b = m[j], c = j == 3 ? r : m[j + 1];
+            const float a0 = j == 0 ? l : m[j - 1], b = m[j], c0 = j == 3 ? r : m[j + 1];
+            const float a = RIG ? a0 + pen : a0, c = RIG ? c0 + pen : c0;
             const int pa = j == 0 ? pl : P[j - 1], pb = P[j], pc = j == 3 ? pr : P[j + 1];
             const bool p1 = b < a;                    // first strict minimum scanning x-1, x, x+1
             const float best = p1 ? b : a;
@@ -699,11 +714,13 @@ constexpr int TR_WIN = 72;                            // walk window: columns x-
 constexpr int TR_THREADS = 256;
 
 // Batch sessions: blockIdx.y = frame (planes m_fs floats / j_fs bytes apart, seam[h * frame ...],
-// seam_log[log_fs * frame ...], xlast[frame]).
+// seam_log[log_fs * frame ...], xlast[frame]).  RIG: rigidity pen, as in the DP.
+template <bool RIG>
 __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
                                                               const int8_t* __restrict__ jump, size_t j_pitch,
                                                               const int* __restrict__ xlast, int* __restrict__ seam,
-                                                              int* __restrict__ seam_log, size_t m_fs, size_t j_fs, size_t log_fs)
+                                                              int* __restrict__ seam_log, size_t m_fs, size_t j_fs, size_t log_fs,
+                                                              float pen)
 {
     extern __shared__ __align__(16) unsigned char tr_smem[];
     __shared__ __align__(16) float win[JB][TR_WIN + 8];
@@ -767,7 +784,7 @@ __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float
     int mine = 0;
     const float* wp = &win[0][4] + (x - base);
     for (int i = 0; i < steps; i++) {
-        const float a = wp[-1], b = wp[0], c = wp[1];
+        const float a = RIG ? wp[-1] + pen : wp[-1], b = wp[0], c = RIG ? wp[1] + pen : wp[1];
         const bool p1 = b < a;
         const float best = p1 ? b : a;
         const bool p2 = c < best;
@@ -807,10 +824,10 @@ constexpr int INCR_T = 8;                               // rows between two tigh
 constexpr int INCR_SW = INCR_CAP + 2 * INCR_D + 16;     // floats per staged row and plane
 
 // one row of the walk with NK columns per lane: every shared-memory load first, then the arithmetic and the stores
-template <int NK>
+template <int NK, bool RIG>
 __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w, int plo, const float* __restrict__ re,
                                          const float* __restrict__ rm, int xs, const float* __restrict__ prev,
-                                         float* __restrict__ next, float* __restrict__ mrow, int& clo, int& chi)
+                                         float* __restrict__ next, float* __restrict__ mrow, int& clo, int& chi, float pen)
 {
     const float INF = __int_as_float(0x7f800000);
     float e[NK], mo[NK], pl[NK], pc[NK], pr[NK];
@@ -829,7 +846,7 @@ __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w,
         const int x = lo + lane + 32 * k;
         if (x <= hi) {
             float mn = e[k];
-            if (y > 0) mn = e[k] + fminf(fminf(x > 0 ? pl[k] : INF, pc[k]), x < w - 1 ? pr[k] : INF);
+            if (y > 0) mn = e[k] + fminf(fminf(x > 0 ? (RIG ? pl[k] + pen : pl[k]) : INF, pc[k]), x < w - 1 ? (RIG ? pr[k] + pen : pr[k]) : INF);
             next[x - lo + 2] = mn;
             if (__float_as_uint(mn) != __float_as_uint(mo[k])) {
 #if DCTC_INCR_ABL != 1
@@ -842,10 +859,12 @@ __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w,
     }
 }
 
+// RIG: rigidity pen, as in the DP (the changed cells still spread by one column per row).
+template <bool RIG>
 __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                             float* __restrict__ mplane, size_t m_pitch, int r,
                                                             int* __restrict__ seam, int* __restrict__ seam_log,
-                                                            int* __restrict__ rebuild_flag)
+                                                            int* __restrict__ rebuild_flag, float pen)
 {
     extern __shared__ __align__(16) int incr_sm[];
     float* ring = reinterpret_cast<float*>(incr_sm);                       // INCR_D slots x (energy row, map row) x INCR_SW
@@ -922,11 +941,11 @@ __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restr
         const int xs = xsb[slot];
         float* mrow = mplane + (size_t) y * m_pitch;
         int clo = 0x7fffffff, chi = -1;
-        if (width <= 32) incr_row<1>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi);
-        else if (width <= 64) incr_row<2>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi);
-        else if (width <= 128) incr_row<4>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi);
-        else if (width <= 256) incr_row<8>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi);
-        else incr_row<16>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi);
+        if (width <= 32) incr_row<1, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
+        else if (width <= 64) incr_row<2, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
+        else if (width <= 128) incr_row<4, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
+        else if (width <= 256) incr_row<8, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
+        else incr_row<16, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
 #ifdef DCTC_INCR_STATS
         const long long c2 = clock64();
 #endif
@@ -990,8 +1009,20 @@ __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restr
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
         if (oi != 0x7fffffff && (bi == 0x7fffffff || ov < bv || (ov == bv && oi < bi))) { bv = ov; bi = oi; }
     }
-    dp_backtrack(mplane, m_pitch, w, h, bi, seam, seam_log, win, lane);
+    dp_backtrack<RIG>(mplane, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);
 }
+
+// Instantiated here, ahead of the DP kernels: the module then declares the dynamic shared arrays of the trace and
+// incremental kernels before the DP's 128-byte aligned one, which keeps the trace kernel's dynamic shared memory at the
+// 16-byte aligned offset its static arrays end at (the rigidity-0 kernels stay what they were before RIG existed).
+template __global__ void dctc_seam_jump_kernel<false>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
+template __global__ void dctc_seam_jump_kernel<true>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
+template __global__ void dctc_seam_trace_kernel<false>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*, int*,
+                                                       size_t, size_t, size_t, float);
+template __global__ void dctc_seam_trace_kernel<true>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*, int*,
+                                                      size_t, size_t, size_t, float);
+template __global__ void dctc_seam_incr_kernel<false>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
+template __global__ void dctc_seam_incr_kernel<true>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
 
 // ---- visibility map + seam display (SURVEY section 8f rank 4) ---------------------------------------------------
 // liblqr's update_vsmap: the pixel removed from row y by the k-th seam is original column raw[y][s]; its entry of the
@@ -1411,8 +1442,9 @@ static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFram
 }
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
-// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map.
-using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*, size_t, size_t, size_t);
+// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map; rig selects the RIG twin.
+using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*, size_t, size_t, size_t,
+                       float);
 struct DpPlan {
     dp_fn dp = nullptr;
     int wpc = 0, nst = 0, use_tmap = 0;
@@ -1420,7 +1452,7 @@ struct DpPlan {
     CUtensorMap tmap;
 };
 
-static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, DpPlan& p)
+static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, bool rig, DpPlan& p)
 {
     // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
     const int cap = DP_CL * DP_MAXW;
@@ -1449,10 +1481,14 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
     p.wpc = wpc;
     p.nst = nst;
     p.smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
-    static const dp_fn table[3][3] = {{dctc_seam_dp_kernel<1, 0>, dctc_seam_dp_kernel<1, 16>, dctc_seam_dp_kernel<1, 32>},
-                                      {dctc_seam_dp_kernel<2, 0>, dctc_seam_dp_kernel<2, 16>, dctc_seam_dp_kernel<2, 32>},
-                                      {dctc_seam_dp_kernel<4, 0>, dctc_seam_dp_kernel<4, 16>, dctc_seam_dp_kernel<4, 32>}};
-    p.dp = table[P == 1 ? 0 : P == 2 ? 1 : 2][sr / 16];
+    static const dp_fn table[2][3][3] = {
+        {{dctc_seam_dp_kernel<1, 0, false>, dctc_seam_dp_kernel<1, 16, false>, dctc_seam_dp_kernel<1, 32, false>},
+         {dctc_seam_dp_kernel<2, 0, false>, dctc_seam_dp_kernel<2, 16, false>, dctc_seam_dp_kernel<2, 32, false>},
+         {dctc_seam_dp_kernel<4, 0, false>, dctc_seam_dp_kernel<4, 16, false>, dctc_seam_dp_kernel<4, 32, false>}},
+        {{dctc_seam_dp_kernel<1, 0, true>, dctc_seam_dp_kernel<1, 16, true>, dctc_seam_dp_kernel<1, 32, true>},
+         {dctc_seam_dp_kernel<2, 0, true>, dctc_seam_dp_kernel<2, 16, true>, dctc_seam_dp_kernel<2, 32, true>},
+         {dctc_seam_dp_kernel<4, 0, true>, dctc_seam_dp_kernel<4, 16, true>, dctc_seam_dp_kernel<4, 32, true>}}};
+    p.dp = table[rig ? 1 : 0][P == 1 ? 0 : P == 2 ? 1 : 2][sr / 16];
     // tensor map of the energy planes for the staged variant (strips of up to 256 columns: the TMA box limit); frames
     // are its third dimension, so that a box never reaches into the next frame's rows
     memset(&p.tmap, 0, sizeof(p.tmap));
@@ -1513,10 +1549,12 @@ static int frames_loop_buffers(dctc_context* ctx, CarverFrames& f, const BtPlan&
     return DCTC_OK;
 }
 
-// What the caller of a seam operation brings besides the session: whether its seam loops record the visibility maps, and
-// the context's incremental cumulative map (dctc_carver_set_incremental), which only the single session has.
+// What the caller of a seam operation brings besides the session: whether its seam loops record the visibility maps, the
+// rigidity (dctc_carver_set_rigidity, dctc_carver_batch_set_rigidity) and the context's incremental cumulative map
+// (dctc_carver_set_incremental), which only the single session has.
 struct SeamCall {
     bool vmaps = false;
+    float rigidity = 0.0f;
     bool incremental = false;
     bool* m_valid = nullptr;   // &ctx->c_m_valid (single session), null for a batch
 };
@@ -1528,23 +1566,30 @@ struct SeamCall {
 // c.incremental (one frame only, its flag buffer is ctx->c_band): *c.m_valid says whether f.m holds the map of the image
 // before the last removal, compacted over that seam.  The walk then replaces DP + jump + trace, the DP only runs when the
 // walk gave up, and the carve also compacts f.m.  A loop that does not keep the map up to date clears *c.m_valid.
+// c.rigidity: the seams are f.h rows long (the image width at the axis switch for height operations), so every kernel of
+// the loop gets pen = fl(rigidity / f.h); pen == 0 launches the kernels of rigidity 0.
 static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c)
 {
     const int n = f.n, h = f.h;
     const size_t log_fs = (size_t) n_seams * h, en_fs = f.en_pitch * h, m_fs = f.m_pitch * h;
+    const float pen = c.rigidity / (float) h;
+    const bool rig = pen != 0.0f;
     const BtPlan bt = bt_plan(h, f.m_pitch);
     int rc = frames_loop_buffers(ctx, f, bt, log_fs);
     if (rc) return rc;
     DpPlan plan;
-    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, plan));
+    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, rig, plan));
+    const auto jump = rig ? dctc_seam_jump_kernel<true> : dctc_seam_jump_kernel<false>;
+    const auto trace = rig ? dctc_seam_trace_kernel<true> : dctc_seam_trace_kernel<false>;
+    const auto incr_walk = rig ? dctc_seam_incr_kernel<true> : dctc_seam_incr_kernel<false>;
     if (bt.par && bt.cone_smem > 40 * 1024)
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+        CK(ctx, cudaFuncSetAttribute(trace, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
     int* const xlast = bt.par ? f.xlast : nullptr;
     // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
     const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
     const bool incr = c.incremental && n == 1 && incr_smem <= 160 * 1024;
     if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_incr_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
+        CK(ctx, cudaFuncSetAttribute(incr_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
         if (!ctx->c_band) {
             CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 4));
             CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 4, ctx->stream));
@@ -1557,8 +1602,8 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         const bool walk = incr && *c.m_valid;
         if (walk) {
             // update_mmap + build_vpath: walk the changed cells only; the DP below rebuilds the map only if the walk gave up
-            dctc_seam_incr_kernel<<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2,
-                                                                     f.seam, log_s, ctx->c_band);
+            incr_walk<<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2, f.seam, log_s,
+                                                         ctx->c_band, pen);
             CK(ctx, cudaGetLastError());
             ctx->launches++;
         }
@@ -1567,13 +1612,13 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         // drains and blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
         CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl && !walk, f.en, f.en_pitch, w_old,
                                 h, f.m, f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
-                                plan.use_tmap, walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs));
+                                plan.use_tmap, walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, pen));
         if (bt.par && !walk) {
             const int js = (w_old + 63) / 64;
-            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, f.m, f.m_pitch,
-                                    w_old, h, f.dir, bt.j_pitch, js, m_fs, f.dir_fs));
-            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, f.m, f.m_pitch,
-                                    w_old, h, f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs));
+            CK(ctx, dctc_launch_pdl(jump, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, f.m, f.m_pitch, w_old, h, f.dir,
+                                    bt.j_pitch, js, m_fs, f.dir_fs, pen));
+            CK(ctx, dctc_launch_pdl(trace, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, f.m, f.m_pitch, w_old, h,
+                                    f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, pen));
             ctx->launches += 2;
         }
 #ifdef DCTC_SYNC_DEBUG
@@ -1700,6 +1745,7 @@ struct dctc_carver_batch {
     size_t start_bytes = 0;
     uint8_t* lv_scratch = nullptr;      // height levels in the transposed orientation on their way out (session_render)
     size_t lv_scratch_bytes = 0;
+    float rigidity = 0.0f;              // dctc_carver_batch_set_rigidity (the single session takes the context's instead)
 };
 
 namespace {
@@ -2113,6 +2159,7 @@ static int carver_call(dctc_context* ctx, Op&& op)
     const int w = f->w, iw = frames_image_w(*f), ih = frames_image_h(*f);
     SeamCall c;
     c.vmaps = ctx->c_dump_vmaps;
+    c.rigidity = ctx->c_rigidity;
     c.incremental = ctx->c_incremental;
     c.m_valid = &ctx->c_m_valid;
     const int rc = op(b, c);
@@ -2320,6 +2367,16 @@ int dctc_carver_set_incremental(dctc_context* ctx, int on)
     return DCTC_OK;
 }
 
+int dctc_carver_set_rigidity(dctc_context* ctx, float rigidity)
+{
+    if (!ctx || !(rigidity >= 0.0f) || !std::isfinite(rigidity)) return DCTC_ERR_INVALID;
+    if (rigidity != ctx->c_rigidity) {
+        ctx->c_rigidity = rigidity;
+        ctx->c_m_valid = false;   // the incremental map was built with the old pen
+    }
+    return DCTC_OK;
+}
+
 int dctc_carver_rebuild_count(dctc_context* ctx)
 {
     if (!ctx || !ctx->carver) return -1;
@@ -2404,10 +2461,18 @@ float dctc_pixel_energy(int x, int y, int w, int h, struct DctcLqrReadingWindow_
 // ---- batch session: n equally sized frames through one device seam loop ---------------------------------------------
 // The batch never touches the context's single session; it uses the context's device, stream and launch counter.
 
+// A batch call brings the batch's rigidity; the per-axis calls also its maps rule
+static SeamCall batch_call(const dctc_carver_batch* b)
+{
+    SeamCall c;
+    c.rigidity = b->rigidity;
+    return c;
+}
+
 static int batch_seams(dctc_carver_batch* b, int axis, bool enlarge, int n_seams, int* seams_out)
 {
     if (!b || n_seams < 0) return DCTC_ERR_INVALID;
-    SeamCall c;
+    SeamCall c = batch_call(b);
     c.vmaps = b->dump_vmaps;
     return session_seams(b, axis, enlarge, n_seams, seams_out, c);
 }
@@ -2455,6 +2520,13 @@ int dctc_carver_batch_bias(dctc_carver_batch* b, float* out)
     return session_download(b, nullptr, nullptr, out);
 }
 
+int dctc_carver_batch_set_rigidity(dctc_carver_batch* b, float rigidity)
+{
+    if (!b || !(rigidity >= 0.0f) || !std::isfinite(rigidity)) return DCTC_ERR_INVALID;
+    b->rigidity = rigidity;
+    return DCTC_OK;
+}
+
 int dctc_carver_batch_width(const dctc_carver_batch* b) { return b ? frames_image_w(session_frames(b)) : 0; }
 int dctc_carver_batch_height(const dctc_carver_batch* b) { return b ? frames_image_h(session_frames(b)) : 0; }
 
@@ -2481,7 +2553,7 @@ int dctc_carver_batch_enlarge_height(dctc_carver_batch* b, int n_seams, int* sea
 int dctc_carver_batch_resize(dctc_carver_batch* b, int new_w, int new_h, int* seams_out, int* vmaps_out)
 {
     if (!b || new_w <= 0 || new_h <= 0) return DCTC_ERR_INVALID;
-    return session_resize(b, new_w, new_h, seams_out, vmaps_out, SeamCall());
+    return session_resize(b, new_w, new_h, seams_out, vmaps_out, batch_call(b));
 }
 
 int dctc_carver_batch_images(dctc_carver_batch* b, uint8_t* out)
@@ -2506,13 +2578,13 @@ int dctc_carver_batch_vmap(dctc_carver_batch* b, int* vmap_out, int* depth_out)
 int dctc_carver_batch_levels_width(dctc_carver_batch* b, int depth, int* seams_out)
 {
     if (!b || depth < 0) return DCTC_ERR_INVALID;
-    return session_levels(b, DCTC_AXIS_WIDTH, depth, seams_out, SeamCall());
+    return session_levels(b, DCTC_AXIS_WIDTH, depth, seams_out, batch_call(b));
 }
 
 int dctc_carver_batch_levels_height(dctc_carver_batch* b, int depth, int* seams_out)
 {
     if (!b || depth < 0) return DCTC_ERR_INVALID;
-    return session_levels(b, DCTC_AXIS_HEIGHT, depth, seams_out, SeamCall());
+    return session_levels(b, DCTC_AXIS_HEIGHT, depth, seams_out, batch_call(b));
 }
 
 int dctc_carver_batch_render_levels(dctc_carver_batch* b, int n_levels, const int* extents, uint8_t* out)

@@ -163,6 +163,7 @@ struct dctc_context {
     int* c_band = nullptr;         // c_band[0]: 'rebuild the cumulative map from scratch' flag of the incremental seam DP, c_band[1]: rebuilds (device)
     bool c_incremental = false;    // device seam loop: update the cumulative map incrementally (dctc_carver_set_incremental)
     bool c_m_valid = false;        // the cumulative plane holds the map of the image before the last removal, compacted over that seam
+    float c_rigidity = 0.0f;       // rigidity of the single session's seam loops (dctc_carver_set_rigidity); survives loads
     float* c_band_vals = nullptr;  // packed band values of dctc_carve_and_update
     float* h_mirror = nullptr;     // host mirror of the energy map for dctc_pixel_energy (pinned, allocated by its first use)
     int* h_band = nullptr;         // pinned: band values and seam of dctc_carve_and_update

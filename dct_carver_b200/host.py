@@ -38,6 +38,9 @@ def hostlib():
         L.dctc_render.restype = C.c_int
         L.dctc_render.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(PlugInVals), C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.POINTER(RenderResult)]
+        L.dctc_render_ext.restype = C.c_int
+        L.dctc_render_ext.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(PlugInVals), C.c_int, C.c_float,
+                                      C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(RenderResult)]
         L.dctc_host_set_device_seam_loop.restype = None
         L.dctc_host_set_device_seam_loop.argtypes = [C.c_int]
         L.dctc_render_result_free.restype = None
@@ -47,11 +50,12 @@ def hostlib():
 
 
 def render(img, seams_number, blocksize=8, edges=0.5, textures=0.5, vertically=False, ctx=None, callback=None,
-           callback_extra=None, output_energy=False, output_seams=True, device_loop=True):
+           callback_extra=None, output_energy=False, output_seams=True, device_loop=True, delta_x=1, rigidity=0.0):
     """Retargets `img` by `seams_number` (negative = shrink, as PlugInVals.seams_number) along the width
     (vertically=False) or height.  Energy comes from the GPU context `ctx`, or from a per-pixel `callback`
     (address of an LqrEnergyFunc; checker use only).  device_loop=False keeps the cumulative map, seam search and
-    carve on the host (energy batches still on the GPU): the cross-check of the device-resident seam loop."""
+    carve on the host (energy batches still on the GPU): the cross-check of the device-resident seam loop.
+    delta_x, rigidity: lqr_carver_init's (dctc_render_ext); the defaults are the plug-in's."""
     img = np.ascontiguousarray(img, dtype=np.uint8)
     if img.ndim == 2:
         img = img[:, :, None]
@@ -59,8 +63,8 @@ def render(img, seams_number, blocksize=8, edges=0.5, textures=0.5, vertically=F
     hostlib().dctc_host_set_device_seam_loop(int(device_loop))
     vals = PlugInVals(edges, textures, blocksize, seams_number, 0, 1, int(output_energy), int(output_seams), int(vertically))
     res = RenderResult()
-    rc = hostlib().dctc_render(img.ctypes.data, w, h, ch, C.byref(vals), ctx.handle if ctx is not None else None,
-                               callback, callback_extra, C.byref(res))
+    rc = hostlib().dctc_render_ext(img.ctypes.data, w, h, ch, C.byref(vals), int(delta_x), float(rigidity),
+                                   ctx.handle if ctx is not None else None, callback, callback_extra, C.byref(res))
     if rc != 0:
         raise DctcError(rc, "dctc_render")
     out = dict(

@@ -164,40 +164,62 @@ static void band_limits(const int *seam, int y, int h, int w, int rad, int *xmin
     *xmax = hi > w - 1 ? w - 1 : hi;
 }
 
-/* m[y][x] = en[y][x] + min over parents x-dx..x+dx (clipped), first strict minimum scanning left to right */
-static float min_parent(const float *mrow_prev, int x, int w, int dx)
+/* m[y][x] = en[y][x] + min over parents x1 = x-dx..x+dx (clipped) of m[y-1][x1] + rig[|x1-x|], first strict minimum
+ * scanning left to right.  rig: liblqr's rigidity_map (rigidity_map_of), NULL for rigidity 0. */
+static float parent_cost(const float *mrow_prev, int x1, int x, const float *rig)
+{
+    return rig ? mrow_prev[x1] + rig[x1 < x ? x - x1 : x1 - x] : mrow_prev[x1];
+}
+
+static float min_parent(const float *mrow_prev, int x, int w, int dx, const float *rig)
 {
     int x1, lo = x - dx < 0 ? 0 : x - dx, hi = x + dx > w - 1 ? w - 1 : x + dx;
-    float best = mrow_prev[lo];
+    float best = parent_cost(mrow_prev, lo, x, rig);
     for (x1 = lo + 1; x1 <= hi; x1++)
-        if (mrow_prev[x1] < best) best = mrow_prev[x1];
+        if (parent_cost(mrow_prev, x1, x, rig) < best) best = parent_cost(mrow_prev, x1, x, rig);
     return best;
 }
 
-static int argmin_parent(const float *mrow_prev, int x, int w, int dx)
+static int argmin_parent(const float *mrow_prev, int x, int w, int dx, const float *rig)
 {
     int x1, lo = x - dx < 0 ? 0 : x - dx, hi = x + dx > w - 1 ? w - 1 : x + dx, arg = lo;
-    float best = mrow_prev[lo];
+    float best = parent_cost(mrow_prev, lo, x, rig);
     for (x1 = lo + 1; x1 <= hi; x1++)
-        if (mrow_prev[x1] < best) { best = mrow_prev[x1]; arg = x1; }
+        if (parent_cost(mrow_prev, x1, x, rig) < best) { best = parent_cost(mrow_prev, x1, x, rig); arg = x1; }
     return arg;
+}
+
+/* liblqr's rigidity_map for seams h rows long [from memory: parity unpinned]: rig[d] = fl(fl(rigidity * |d|^1.5) / h),
+ * d = 0..dx, with |d|^1.5 = fl(d * fl(sqrt(d))) (correctly rounded steps, so that other implementations can restate it
+ * exactly; d = 1 gives the device's pen = fl(rigidity / h)).  Returns NULL for rigidity 0 (the plain seam search) or
+ * when the allocation fails (*nomem is set). */
+static float *rigidity_map_of(float rigidity, int dx, int h, int *nomem)
+{
+    float *rig;
+    int d;
+    *nomem = 0;
+    if (rigidity == 0.0f) return NULL;
+    rig = (float *) malloc(sizeof(float) * (size_t) (dx + 1));
+    if (!rig) { *nomem = 1; return NULL; }
+    for (d = 0; d <= dx; d++) rig[d] = (rigidity * ((float) d * sqrtf((float) d))) / (float) h;
+    return rig;
 }
 
 /* removes k vertical seams from the current frame */
 static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
 {
     const int P = r->pitch, h = r->h, ch = r->ch, dx = r->delta_x;
-    float *en = NULL, *m = NULL, *band = NULL;
+    float *en = NULL, *m = NULL, *band = NULL, *rig = NULL;
     int *raw = NULL, *seam = NULL, *xmin = NULL, *xmax = NULL;
     double *luma = NULL;
     DctcLqrReadingWindow rw;
-    int x, y, s, rc = DCTC_LQR_NOMEM;
+    int x, y, s, rc = DCTC_LQR_NOMEM, rig_nomem;
     double t0;
 
     if (k <= 0) return DCTC_LQR_OK;
     if (k >= r->w) return DCTC_LQR_ERROR;
     if (!r->gpu && !r->nrg) return DCTC_LQR_ERROR;
-    if (r->gpu && g_device_seam_loop && r->delta_x == 1 && r->rigidity == 0.0f) {
+    if (r->gpu && g_device_seam_loop && r->delta_x == 1) {
         /* the whole lqr_carver_resize loop on the device: energy, seam DP, back-track, carve, band update */
         int drc, *dseams;
         t0 = now_s();
@@ -209,6 +231,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
             r->seams = ns; r->seams_cap = r->n_seams + k;
         }
         dseams = r->seams + (size_t) r->n_seams * h;
+        if (dctc_carver_set_rigidity(r->gpu, r->rigidity) != DCTC_OK) return DCTC_LQR_ERROR;
         if (dctc_carver_load(r->gpu, r->rgb, r->w, h, ch, (size_t) P * ch) != DCTC_OK) return DCTC_LQR_ERROR;
         r->timing[0] += now_s() - t0;
         t0 = now_s();
@@ -243,7 +266,8 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     xmax = (int *) malloc(sizeof(int) * h);
     band = (float *) malloc(sizeof(float) * (size_t) h * (4 * (r->radius > 0 ? r->radius : 1) + 2));
     if (!r->gpu) luma = (double *) malloc(sizeof(double) * (size_t) P * h);
-    if (!en || !m || !raw || !seam || !xmin || !xmax || !band || (!r->gpu && !luma)) goto done;
+    rig = rigidity_map_of(r->rigidity, dx, h, &rig_nomem);
+    if (!en || !m || !raw || !seam || !xmin || !xmax || !band || (!r->gpu && !luma) || rig_nomem) goto done;
     if (r->n_seams + k > r->seams_cap || r->seam_len != h) {
         int *ns;
         if (r->seam_len != h) { r->n_seams = 0; r->seam_len = h; }
@@ -286,7 +310,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     memcpy(m, en, sizeof(float) * r->w);
     for (y = 1; y < h; y++)
         for (x = 0; x < r->w; x++)
-            m[(size_t) y * P + x] = en[(size_t) y * P + x] + min_parent(m + (size_t) (y - 1) * P, x, r->w, dx);
+            m[(size_t) y * P + x] = en[(size_t) y * P + x] + min_parent(m + (size_t) (y - 1) * P, x, r->w, dx, rig);
     r->timing[1] += now_s() - t0;
 
     for (s = 0; s < k; s++) {
@@ -300,7 +324,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
             for (x = 1; x < w; x++)
                 if (last[x] < last[best]) best = x;
             seam[h - 1] = best;
-            for (y = h - 1; y > 0; y--) seam[y - 1] = argmin_parent(m + (size_t) (y - 1) * P, seam[y], w, dx);
+            for (y = h - 1; y > 0; y--) seam[y - 1] = argmin_parent(m + (size_t) (y - 1) * P, seam[y], w, dx, rig);
         }
         memcpy(r->seams + (size_t) r->n_seams * h, seam, sizeof(int) * h);
         r->n_seams++;
@@ -359,7 +383,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
             if (lo < 0) lo = 0;
             if (hi > w1 - 1) hi = w1 - 1;
             for (x = lo; x <= hi; x++) {
-                const float v = y == 0 ? erow[x] : erow[x] + min_parent(mrow - P, x, w1, dx);
+                const float v = y == 0 ? erow[x] : erow[x] + min_parent(mrow - P, x, w1, dx, rig);
                 if (v != mrow[x]) {
                     mrow[x] = v;
                     if (x < nlo) nlo = x;
@@ -374,7 +398,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     r->pitch = r->w;
     rc = DCTC_LQR_OK;
 done:
-    free(en); free(m); free(raw); free(seam); free(xmin); free(xmax); free(band); free(luma);
+    free(en); free(m); free(raw); free(seam); free(xmin); free(xmax); free(band); free(luma); free(rig);
     return rc;
 }
 
@@ -408,14 +432,15 @@ static int enlarge_vertical(DctcLqrCarver *r, int k, int record_vs)
     orig = (uint8_t *) malloc((size_t) w0 * h * ch);
     if (!orig) return DCTC_LQR_NOMEM;
     for (y = 0; y < h; y++) memcpy(orig + (size_t) y * w0 * ch, r->rgb + (size_t) y * r->pitch * ch, (size_t) w0 * ch);
-    if (r->gpu && g_device_seam_loop && r->delta_x == 1 && r->rigidity == 0.0f) {
+    if (r->gpu && g_device_seam_loop && r->delta_x == 1) {
         /* seams, visibility map and the pixel synthesis on the device */
         int *ns;
         if (r->seam_len != h) { r->n_seams = 0; r->seam_len = h; }
         ns = (int *) realloc(r->seams, sizeof(int) * (size_t) (r->n_seams + k) * h);
         if (!ns) { free(orig); return DCTC_LQR_NOMEM; }
         r->seams = ns; r->seams_cap = r->n_seams + k;
-        rc = dctc_carver_load(r->gpu, orig, w0, h, ch, (size_t) w0 * ch);
+        rc = dctc_carver_set_rigidity(r->gpu, r->rigidity);
+        if (rc == DCTC_OK) rc = dctc_carver_load(r->gpu, orig, w0, h, ch, (size_t) w0 * ch);
         if (rc == DCTC_OK) rc = dctc_carver_enlarge_width(r->gpu, k, r->seams + (size_t) r->n_seams * h);
         if (rc == DCTC_OK) {
             out = (uint8_t *) malloc((size_t) (w0 + k) * h * ch);
@@ -559,6 +584,12 @@ void dctc_render_result_free(DctcRenderResult *res)
 int dctc_render(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, dctc_context *gpu,
                 DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res)
 {
+    return dctc_render_ext(img, w, h, channels, vals, 1, 0.0f, gpu, cb, cb_extra, res);   /* src/render.c:313 */
+}
+
+int dctc_render_ext(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, int delta_x, float rigidity,
+                    dctc_context *gpu, DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res)
+{
     DctcCarverEnergyParams ep;       /* superset of EnergyParameters: prefix layout of src/render.h:9-18 */
     DctcLqrCarver *carver;
     uint8_t *rgb_buffer, *line;
@@ -567,7 +598,7 @@ int dctc_render(const uint8_t *img, int w, int h, int channels, const DctcPlugIn
     double t0 = now_s();
     const double *tm;
 
-    if (!img || !vals || !res || w <= 0 || h <= 0) return DCTC_ERR_INVALID;
+    if (!img || !vals || !res || w <= 0 || h <= 0 || delta_x < 1 || !(rigidity >= 0.0f) || !isfinite(rigidity)) return DCTC_ERR_INVALID;
     if (!gpu && !cb) return DCTC_ERR_NO_DEVICE;     /* no CPU fallback in the product */
     memset(res, 0, sizeof(*res));
 
@@ -586,7 +617,7 @@ int dctc_render(const uint8_t *img, int w, int h, int channels, const DctcPlugIn
     memcpy(rgb_buffer, img, (size_t) w * h * channels);
     carver = dctc_lqr_carver_new(rgb_buffer, w, h, channels);
     if (!carver) { free(rgb_buffer); return DCTC_ERR_INVALID; }
-    dctc_lqr_carver_init(carver, 1, 0);  /* delta_x, rigidity: src/render.c:313 */
+    dctc_lqr_carver_init(carver, delta_x, rigidity);
     if (gpu) {
         dctc_lqr_carver_set_energy_function(carver, (DctcLqrEnergyFunc) dctc_pixel_energy, vals->blocksize / 2,
                                             DCTC_LQR_ER_LUMA, (void *) &ep);

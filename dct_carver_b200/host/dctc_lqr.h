@@ -5,6 +5,7 @@
  * installed here, so this restates the behaviour the reference relies on [liblqr 0.4.x, from memory; SURVEY
  * Appendix A]: seams of width 1, delta_x = 1, rigidity 0 (src/render.c:313), cumulative map
  *   m[y][x] = en[y][x] + min(m[y-1][x-1], m[y-1][x], m[y-1][x+1])      (first strict minimum, left to right)
+ * (dctc_lqr_carver_init also takes other delta_x and a rigidity: see dctc_render_ext)
  * seam end = leftmost minimum of the last row, energy update after each seam only within +-radius of it.
  * Call sites mirrored: src/render.c:312-316 (new/init/set_energy_function), :377 (resize), :264-269 (scan_line),
  * :214-231 (vmap), :413 (destroy).
@@ -93,9 +94,16 @@ typedef struct DctcRenderResult_ {
 } DctcRenderResult;
 
 /* gpu == NULL is refused (no CPU fallback in the product); cb != NULL selects the per-pixel callback source
- * instead (checker use: plug in the reference's dct_pixel_energy). */
+ * instead (checker use: plug in the reference's dct_pixel_energy).  The plug-in's carver: delta_x 1, rigidity 0
+ * (src/render.c:313), i.e. dctc_render_ext(.., 1, 0, ..). */
 int dctc_render(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, dctc_context *gpu,
                 DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res);
+/* dctc_render with lqr_carver_init(carver, delta_x, rigidity): a seam step of |d| <= delta_x columns costs
+ * fl(fl(rigidity * |d|^1.5) / h) more, h the seam length.  With a GPU attached, delta_x = 1 runs the device seam loop
+ * (the context's dctc_carver_set_rigidity is set to rigidity before each load); other delta_x run the host loop.
+ * DCTC_ERR_INVALID also for delta_x < 1 and a negative or non-finite rigidity. */
+int dctc_render_ext(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, int delta_x, float rigidity,
+                    dctc_context *gpu, DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res);
 void dctc_render_result_free(DctcRenderResult *res);
 
 #ifdef DCTC_LQR_COMPAT_NAMES

@@ -158,7 +158,7 @@ int dctc_carver_image(dctc_context *ctx, uint8_t *out);
 /* Whole retarget loop on the device (energy -> seam DP -> back-track -> carve -> band update), `n_seams`
  * vertical seams; seams_out (may be NULL) receives n_seams*h removed columns in the coordinates of the image
  * at the time of removal.  Mirrors lqr_carver_resize(carver, w - n_seams, h) (src/render.c:377) with
- * delta_x = 1, rigidity = 0 (src/render.c:313). */
+ * delta_x = 1 and the rigidity of dctc_carver_set_rigidity (0, the plug-in's value, src/render.c:313, by default). */
 int dctc_carver_resize_width(dctc_context *ctx, int n_seams, int *seams_out);
 /* Enlarging: lqr_carver_resize(carver, w + n_seams, h) as the plug-in calls it for seams_number > 0
  * (src/render.c:357-363,377).  The n_seams seams a shrink would remove are computed on a freshly loaded session (same
@@ -274,6 +274,22 @@ int dctc_carver_set_bias(dctc_context *ctx, const float *bias, size_t pitch_byte
 /* The current bias plane (carved, transposed back, inflated): w * h floats, pitch w.  DCTC_ERR_STATE without a bias. */
 int dctc_carver_bias(dctc_context *ctx, float *out);
 
+/* ---- rigidity: straighter seams (liblqr's lqr_carver_init(carver, delta_x, rigidity)) -------------------------
+ * A seam step to the left or right neighbour costs pen = fl(rigidity / h) more, h the length of the seams: the image
+ * height for width operations, the image width at the axis switch for height operations (an enlarge uses the h of a
+ * shrink along its axis).  Every seam loop of the session (width and height resize and enlarge, split resizes,
+ * incremental mode, dctc_carver_resize, levels builds, with or without a bias) runs on
+ *     m[y][x] = fl(E[y][x] + min(fl(m[y-1][x-1] + pen), m[y-1][x], fl(m[y-1][x+1] + pen)))
+ * with the parent = the FIRST strict minimum of those three candidates scanning x-1, x, x+1, and the seam end the
+ * leftmost minimum of the last row (liblqr's rigidity_map[dx] = rigidity * |dx|^1.5 / h for delta_x = 1, no rigidity
+ * mask [from memory: parity unpinned]).  rigidity 0 (the default) gives the seams of a session that never set it, with
+ * the same kernels.  A rigid seam loop launches per seam exactly what a loop of rigidity 0 launches.
+ * dctc_carver_set_rigidity: an option of the context like dctc_carver_set_incremental; it survives loads and applies
+ * from the next seam loop (so a value changed between two split resizes applies to the second one).  A levels build
+ * that already ran and its renders are not affected.  A changed value drops the incremental map (the next seam rebuilds
+ * it).  DCTC_ERR_INVALID: a negative or non-finite value. */
+int dctc_carver_set_rigidity(dctc_context *ctx, float rigidity);
+
 /* ---- visibility map and seam display ------------------------------------------------------------------------
  * lqr_carver_set_dump_vmaps (src/render.c:374): ask the session to record, for every ORIGINAL pixel, the order in
  * which dctc_carver_resize_width removed it (1-based, 0 = still visible).  Call before the first seam is removed. */
@@ -352,6 +368,10 @@ int dctc_carver_batch_resize(dctc_carver_batch *batch, int new_w, int new_h, int
 int dctc_carver_batch_set_bias(dctc_carver_batch *batch, const float *bias, size_t frame_stride_bytes, size_t pitch_bytes);
 /* current bias planes of every frame (n_frames * h * w floats, image orientation); DCTC_ERR_STATE without a bias */
 int dctc_carver_batch_bias(dctc_carver_batch *batch, float *out);
+/* dctc_carver_set_rigidity for the batch: every frame gets what the single session gives it with that rigidity.  A
+ * setting of the batch, 0 at create; it survives loads and applies from the next seam loop.  DCTC_ERR_INVALID: NULL
+ * batch, a negative or non-finite value. */
+int dctc_carver_batch_set_rigidity(dctc_carver_batch *batch, float rigidity);
 /* current width / height of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
 int dctc_carver_batch_height(const dctc_carver_batch *batch);
