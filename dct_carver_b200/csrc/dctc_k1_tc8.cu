@@ -812,8 +812,7 @@ cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, 
         const DctcTensorMapEncodeFn encode = dctc_tensor_map_encoder();
         const size_t fstride = n_frames > 1 ? a.frame_stride : a.pitch * (size_t) a.h;
         const int row = a.channels == 3 ? RawGeom<3>::ROW : RawGeom<1>::ROW;
-        if (encode && a.h >= 8 && !getenv("DCTC_TC_NO_TENSORMAP") && (fstride & 15) == 0 && fstride >= a.pitch && a.pitch < (1ull << 40) &&
-            fstride < (1ull << 40)) {
+        if (encode && a.h >= 8 && (fstride & 15) == 0 && fstride >= a.pitch && a.pitch < (1ull << 40) && fstride < (1ull << 40)) {
             const cuuint64_t gdim[3] = {(cuuint64_t) (a.pitch / 4), (cuuint64_t) a.h, (cuuint64_t) n_frames};
             const cuuint64_t gstr[2] = {(cuuint64_t) a.pitch, (cuuint64_t) fstride};
             const cuuint32_t box[3] = {(cuuint32_t) (row / 4), 8u, 1u};

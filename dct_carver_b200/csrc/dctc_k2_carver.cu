@@ -7,7 +7,6 @@
 // mode over just the touched pixels, with arithmetic identical to a full recompute (bit-identical results).
 #include <cmath>
 #include <cstdio>
-#include <cstdlib>
 #include <type_traits>
 #include <cstring>
 #include <new>
@@ -120,12 +119,9 @@ __global__ void __launch_bounds__(NT) dctc_carve_rows_kernel(uint8_t* __restrict
 // cannot see contaminates one more column per row, so after DP_R rows the outer DP_R columns on each side are
 // garbage and the warp publishes only its central 128*P - 2*DP_R columns; every DP_R rows the warps exchange the
 // last row through shared memory (one barrier per DP_R rows) and restart with fresh halos.  Energies are staged
-// three blocks ahead by bulk async copies (TMA variant) or prefetched into a register ring; the cumulative rows go to a global float plane from which warp 0 re-derives
+// a few chunks ahead by tensor copies (TMA variants) or prefetched into a register ring; the cumulative rows go to a global float plane from which warp 0 re-derives
 // the parent choices during the back-track (dp_backtrack: 32-row batches through double-buffered shared-memory windows).
 // Cells outside the image hold +inf, which reproduces the range clipping.
-#ifndef DP_EXP
-#define DP_EXP 0   // timing experiments only
-#endif
 constexpr int DP_R = 32;          // rows between two exchanges = halo columns on each side of a strip
 constexpr int DP_MAXW = 8;        // warps per CTA of the DP cluster (256 threads: room for a deep register prefetch ring)
 
@@ -241,9 +237,9 @@ __device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, s
     asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
-// TMA = true: the energies of a strip are staged nst chunks of DP_SR rows ahead into shared memory with 1-D bulk
-// async copies (cp.async.bulk, completion on an mbarrier per warp and stage) instead of a register ring of plain
-// loads: nothing the cluster barrier's memory fence has to wait for, and 48 rows in flight per warp.
+// TMA = true: the energies of a strip are staged nst chunks of DP_SR rows ahead into shared memory, one tensor copy per
+// chunk (cp.async.bulk.tensor.3d, completion on an mbarrier per warp and stage) instead of a register ring of plain
+// loads: nothing the cluster barrier's memory fence has to wait for, and up to 64 rows in flight per warp.
 constexpr int DP_NST_MAX = 4;     // stages per warp: as many (2..4) as fit into shared memory, chosen by the host
 
 __device__ __forceinline__ uint32_t dp_smem_u32(const void* p) { return (uint32_t) __cvta_generic_to_shared(p); }
@@ -277,7 +273,8 @@ __device__ __forceinline__ void dp_unroll(F&& f)
 }
 
 // DP_P float4 groups per lane: strip = 128 * DP_P columns, 128 * DP_P - 2 * DP_R of them published.
-// DP_SR: rows per staged chunk of the bulk-copy variant (32 when two stages per warp fit, else 16), 0 = register ring.
+// DP_SR: rows per staged chunk (32 when two stages per warp fit, else 16), 0 = register ring.  dp_plan instantiates the
+// (DP_P, DP_SR) pairs a width can select: (1, 32), (1, 16), (2, 16), (2, 0), (4, 0).
 // One cluster per frame: blockIdx.y = frame of a batch session, whose energy / cumulative planes start en_fs / m_fs
 // floats after the previous frame's, whose seam is seam[h * frame ...], its log seam_log[log_fs * frame ...] and its
 // last-row column xlast[frame].  The tensor map is 3-D (columns, rows, frames) with a box depth of one frame.
@@ -287,7 +284,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
                                                                     float* __restrict__ mplane, size_t m_pitch,
                                                                     int* __restrict__ seam, int* __restrict__ seam_log,
                                                                     int* __restrict__ run_flag, int nst,
-                                                                    const __grid_constant__ CUtensorMap tmap, int use_tmap,
+                                                                    const __grid_constant__ CUtensorMap tmap,
                                                                     int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs,
                                                                     float pen)
 {
@@ -350,37 +347,20 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
     float* const mframe = mplane + blockIdx.y * m_fs;
     const int hm1 = h - 1;
 
-    // TMA staging of this warp's strip: columns [cs, cs + STRIP) clipped to the row, DP_R rows per stage
+    // TMA staging of this warp's strip: columns [cs, cs + STRIP), DP_SR rows per stage
     const int cs = warp * WOUT - DP_R;
-    const int tx0 = max(cs, 0), tx1 = min(cs + STRIP, (int) en_pitch);
-    const int tbytes = tx1 > tx0 ? (tx1 - tx0) * 4 : 0;
     float* estage = xrow + 2 * xlen + (size_t) (tid >> 5) * nst * SRD * STRIP;
     const int nchunks = (h - 1 + SRD - 1) / SRD;
-    auto issue_chunk = [&](int ch, int st) {   // rows 1 + ch * DP_SR .. (clamped to h - 1) -> stage st = ch % nst
+    auto issue_chunk = [&](int ch, int st) {   // rows [1 + ch * DP_SR, 1 + (ch + 1) * DP_SR) -> stage st = ch % nst
+        // one tensor copy: box = STRIP columns x DP_SR rows x 1 frame; columns left of the image and rows below it are
+        // zero-filled by the TMA unit, never read from the next frame
         const uint32_t bar = dp_smem_u32(&ebar[tid >> 5][st]);
-        if (use_tmap) {
-            // one tensor copy (box = STRIP columns x DP_SR rows x 1 frame; columns left of the image and rows below it
-            // are zero-filled by the TMA unit, never read from the next frame) instead of DP_SR row copies, which the hardware issues one elected lane at a time
-            if (lane == 0) {
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t) (SRD * STRIP * 4)) : "memory");
-                asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
-                             ::"r"(dp_smem_u32(estage + (size_t) st * SRD * STRIP)), "l"(&tmap), "r"(cs), "r"(1 + ch * SRD), "r"(blockIdx.y), "r"(bar) : "memory");
-            }
-            __syncwarp();
-            return;
-        }
         if (lane == 0) {
-            if (tbytes > 0) asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t) (tbytes * SRD)) : "memory");
-            else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"((uint32_t) (SRD * STRIP * 4)) : "memory");
+            asm volatile("cp.async.bulk.tensor.3d.shared::cluster.global.tile.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3, %4}], [%5];"
+                         ::"r"(dp_smem_u32(estage + st * SRD * STRIP)), "l"(&tmap), "r"(cs), "r"(1 + ch * SRD), "r"(blockIdx.y), "r"(bar) : "memory");
         }
         __syncwarp();
-        if (lane < SRD && tbytes > 0) {
-            const int y = min(1 + ch * SRD + lane, hm1);
-            const float* src = en + (size_t) y * en_pitch + tx0;
-            const uint32_t dst = dp_smem_u32(estage + ((size_t) st * SRD + lane) * STRIP + (tx0 - cs));
-            asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                         ::"r"(dst), "l"(src), "r"((uint32_t) tbytes), "r"(bar) : "memory");
-        }
     };
     if (lane == 0) {
         if (TMA) {
@@ -485,18 +465,13 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         }
         // register-ring variant: refill the slot just consumed with the row PF ahead (issued after the last use of the
         // slot, so the load targets the slot's registers directly; they are not touched again for PF rows)
-#if !(DP_EXP & 1)
         if (!TMA) {
 #pragma unroll
             for (int g = 0; g < DP_P; g++)
                 e[k][g] = __ldg(reinterpret_cast<const float4*>(en_g[g] + (size_t) min(y + PF, hm1) * en_pitch));
         }
-#endif
 #pragma unroll
         for (int g = 0; g < DP_P; g++) {
-#if DP_EXP & 2
-            if (o[g].x == 12345.678f)
-#endif
             if (central && ld_ok[g]) *reinterpret_cast<float4*>(mptr + 4 * g) = o[g];
             if (!TMA) patch(o[g], inf_mask[g]);      // cells outside the image stay +inf (TMA: their staged energy is +inf)
             cur[g] = o[g];
@@ -526,7 +501,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         // memory fence: the release/acquire cluster barrier used before carried MEMBAR.ALL.GPU + CCTL.IVALL, i.e. it also
         // waited for the block's global stores of the cumulative plane (40 % of the kernel's stall samples).
         // Slot = block parity: a neighbour can be at most one block ahead, it needs this warp's row to go further.
-        if (yb + DP_R < h && !(DP_EXP & 4)) {
+        if (yb + DP_R < h) {
             const int wl = tid >> 5;                          // warp inside the CTA
             float* halo = xrow + (wl * 2 + xb) * 64;          // [0,32): cells left of the published range, [32,64): right
             const uint32_t my_bar = dp_smem_u32(&hbar[wl][xb]);
@@ -1443,11 +1418,11 @@ static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFram
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
 // en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map; rig selects the RIG twin.
-using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int, int*, size_t, size_t, size_t,
+using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int*, size_t, size_t, size_t,
                        float);
 struct DpPlan {
     dp_fn dp = nullptr;
-    int wpc = 0, nst = 0, use_tmap = 0;
+    int wpc = 0, nst = 0;
     size_t smem = 0;
     CUtensorMap tmap;
 };
@@ -1456,52 +1431,50 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
 {
     // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
     const int cap = DP_CL * DP_MAXW;
-    int P = wcur <= cap * (128 - 2 * DP_R) ? 1 : wcur <= cap * (256 - 2 * DP_R) ? 2 : 4;
-    if (const char* ep = getenv("DCTC_DP_P")) {   // timing experiments: wider strips than the width needs
-        const int want = atoi(ep);
-        if ((want == 2 || want == 4) && want > P) P = want;
-    }
+    const int P = wcur <= cap * (128 - 2 * DP_R) ? 1 : wcur <= cap * (256 - 2 * DP_R) ? 2 : 4;
     const int wout = 128 * P - 2 * DP_R;
     const int strips = (wcur + wout - 1) / wout;
     const int wpc = (strips + DP_CL - 1) / DP_CL;
-    // energies staged by bulk async copies when at least two stages (DP_SR rows each) per warp fit into shared memory
+    // energies staged by tensor copies when at least two stages (DP_SR rows each) per warp fit into shared memory
     // (the kernel also has ~38 KB of static shared memory: back-track windows, reduction scratch, mbarriers)
     const size_t xrow_smem = sizeof(float) * 2 * (size_t) wpc * wout;
-    int nst = 0, sr = 0;
-    if (!getenv("DCTC_DP_NO_TMA")) {
-        const size_t row_smem = sizeof(float) * ((size_t) wpc * 128 * P);      // one staged row of every warp
-        const size_t budget = 180 * 1024 - xrow_smem;
-        if (2 * 32 * row_smem <= budget) { sr = 32; nst = 2; }                 // whole 32-row blocks, two in flight
-        else {
-            sr = 16;
-            for (nst = DP_NST_MAX; nst >= 2 && (size_t) nst * 16 * row_smem > budget; nst--) {}
-            if (nst < 2) { sr = 0; nst = 0; }
-        }
+    const size_t row_smem = sizeof(float) * ((size_t) wpc * 128 * P);      // one staged row of every warp
+    const size_t budget = 180 * 1024 - xrow_smem;
+    int nst, sr;
+    if (2 * 32 * row_smem <= budget) { sr = 32; nst = 2; }                 // whole 32-row blocks, two in flight
+    else {
+        sr = 16;
+        for (nst = DP_NST_MAX; nst >= 2 && (size_t) nst * 16 * row_smem > budget; nst--) {}
+        if (nst < 2) { sr = 0; nst = 0; }
     }
     p.wpc = wpc;
     p.nst = nst;
     p.smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
-    static const dp_fn table[2][3][3] = {
-        {{dctc_seam_dp_kernel<1, 0, false>, dctc_seam_dp_kernel<1, 16, false>, dctc_seam_dp_kernel<1, 32, false>},
-         {dctc_seam_dp_kernel<2, 0, false>, dctc_seam_dp_kernel<2, 16, false>, dctc_seam_dp_kernel<2, 32, false>},
-         {dctc_seam_dp_kernel<4, 0, false>, dctc_seam_dp_kernel<4, 16, false>, dctc_seam_dp_kernel<4, 32, false>}},
-        {{dctc_seam_dp_kernel<1, 0, true>, dctc_seam_dp_kernel<1, 16, true>, dctc_seam_dp_kernel<1, 32, true>},
-         {dctc_seam_dp_kernel<2, 0, true>, dctc_seam_dp_kernel<2, 16, true>, dctc_seam_dp_kernel<2, 32, true>},
-         {dctc_seam_dp_kernel<4, 0, true>, dctc_seam_dp_kernel<4, 16, true>, dctc_seam_dp_kernel<4, 32, true>}}};
-    p.dp = table[rig ? 1 : 0][P == 1 ? 0 : P == 2 ? 1 : 2][sr / 16];
-    // tensor map of the energy planes for the staged variant (strips of up to 256 columns: the TMA box limit); frames
+    // the (P, SR) pairs the lines above select for widths 1 .. DP_MAX_W, and their RIG twins:
+    //   1-2560: (1, 32)   2561-4096: (1, 16)   4097-7680: (2, 16)   7681-12288: (2, 0)   12289-DP_MAX_W: (4, 0)
+    static const struct { int P, sr; dp_fn fn[2]; } variants[] = {
+        {1, 32, {dctc_seam_dp_kernel<1, 32, false>, dctc_seam_dp_kernel<1, 32, true>}},
+        {1, 16, {dctc_seam_dp_kernel<1, 16, false>, dctc_seam_dp_kernel<1, 16, true>}},
+        {2, 16, {dctc_seam_dp_kernel<2, 16, false>, dctc_seam_dp_kernel<2, 16, true>}},
+        {2, 0, {dctc_seam_dp_kernel<2, 0, false>, dctc_seam_dp_kernel<2, 0, true>}},
+        {4, 0, {dctc_seam_dp_kernel<4, 0, false>, dctc_seam_dp_kernel<4, 0, true>}}};
+    p.dp = nullptr;
+    for (const auto& v : variants)
+        if (v.P == P && v.sr == sr) p.dp = v.fn[rig ? 1 : 0];
+    if (!p.dp) return cudaErrorInvalidConfiguration;   // a pair without a kernel: the table and the plan disagree
+    // tensor map of the energy planes for the staged variants (strips of up to 256 columns: the TMA box limit); frames
     // are its third dimension, so that a box never reaches into the next frame's rows
     memset(&p.tmap, 0, sizeof(p.tmap));
-    p.use_tmap = 0;
-    const DctcTensorMapEncodeFn encode = dctc_tensor_map_encoder();
-    if (encode && sr > 0 && 128 * P <= 256 && !getenv("DCTC_DP_NO_TENSORMAP")) {
+    if (sr > 0) {
+        const DctcTensorMapEncodeFn encode = dctc_tensor_map_encoder();
+        if (!encode) return cudaErrorNotSupported;
         const cuuint64_t gdim[3] = {(cuuint64_t) en_pitch, (cuuint64_t) h, (cuuint64_t) n_frames};
         const cuuint64_t gstr[2] = {(cuuint64_t) en_pitch * sizeof(float), (cuuint64_t) en_pitch * h * sizeof(float)};
         const cuuint32_t box[3] = {(cuuint32_t) (128 * P), (cuuint32_t) sr, 1};
         const cuuint32_t estr[3] = {1, 1, 1};
         if (encode(&p.tmap, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, (void*) en, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS)
-            p.use_tmap = 1;
+                   CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+            return cudaErrorInvalidValue;
     }
     // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
     return cudaFuncSetAttribute(p.dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
@@ -1523,7 +1496,7 @@ static BtPlan bt_plan(int h, size_t m_pitch)
     b.nb = (h - 1 + JB - 1) / JB;
     b.cone_smem = b.nb > 0 ? (size_t) 32 * (b.nb - 1) * (b.nb - 1) + 16 * (size_t) (b.nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
     b.j_pitch = (m_pitch + 15) & ~(size_t) 15;    // jump rows start 16-byte aligned (staged in 16-byte chunks)
-    b.par = b.nb > 0 && b.cone_smem <= 200 * 1024 && !getenv("DCTC_SERIAL_BACKTRACK");
+    b.par = b.nb > 0 && b.cone_smem <= 200 * 1024;
     return b;
 }
 
@@ -1595,7 +1568,6 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
             CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 4, ctx->stream));
         }
     }
-    const bool pdl = !getenv("DCTC_NO_PDL");
     for (int s = 0; s < n_seams; s++) {
         const int w_old = f.w;
         int* log_s = f.seam_log + (size_t) s * h;
@@ -1610,14 +1582,14 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         // build_mmap, one cluster per frame, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per
         // block and frame (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor
         // drains and blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
-        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, pdl && !walk, f.en, f.en_pitch, w_old,
+        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, !walk, f.en, f.en_pitch, w_old,
                                 h, f.m, f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
-                                plan.use_tmap, walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, pen));
+                                walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, pen));
         if (bt.par && !walk) {
             const int js = (w_old + 63) / 64;
-            CK(ctx, dctc_launch_pdl(jump, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, pdl, f.m, f.m_pitch, w_old, h, f.dir,
+            CK(ctx, dctc_launch_pdl(jump, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m, f.m_pitch, w_old, h, f.dir,
                                     bt.j_pitch, js, m_fs, f.dir_fs, pen));
-            CK(ctx, dctc_launch_pdl(trace, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, pdl, f.m, f.m_pitch, w_old, h,
+            CK(ctx, dctc_launch_pdl(trace, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, true, f.m, f.m_pitch, w_old, h,
                                     f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, pen));
             ctx->launches += 2;
         }
@@ -1625,13 +1597,13 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: dp kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
 #endif
         if (c.vmaps) {   // update_vsmap
-            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, pdl, f.raw, f.vs, f.w0, f.seam, w_old,
+            CK(ctx, dctc_launch_pdl(dctc_vs_update_kernel, dim3(h, n), dim3(256), 0, ctx->stream, true, f.raw, f.vs, f.w0, f.seam, w_old,
                                     ++f.depth));
             ctx->launches++;
         }
         // carve: compact image and energy rows (and the cumulative rows of the incremental map) over the seam
         CK(ctx, dctc_launch_pdl(f.bias ? dctc_carve_rows_kernel<256, 4, true> : dctc_carve_rows_kernel<256, 4, false>, dim3(h, n), dim3(256),
-                                0, ctx->stream, pdl, f.img, f.pitch, f.ch, f.en, f.en_pitch, f.seam, w_old, incr ? f.m : (float*) nullptr,
+                                0, ctx->stream, true, f.img, f.pitch, f.ch, f.en, f.en_pitch, f.seam, w_old, incr ? f.m : (float*) nullptr,
                                 f.m_pitch, f.img_fs, en_fs, m_fs, f.bias));
         ctx->launches += 2;
         f.w = w_old - 1;
@@ -1641,7 +1613,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
 #endif
         // update_emap: K1 in band mode around every frame's removed seam
         DctcK1Args a = frames_k1_args(f, op, f.seam);
-        a.pdl = pdl ? 1 : 0;
+        a.pdl = 1;
         const DctcK1Bias bias{f.bias, (float) f.w0};   // biased frames: the band store writes the seam energy
         rc = dctc_run_k1(ctx, op, a, n, ctx->stream, f.bias ? &bias : nullptr);
         if (rc) return rc;

@@ -9,6 +9,7 @@ import pytest
 
 import dct_carver_b200 as dc
 import oracle_lib as ol
+from test_carver_batch_gpu import DP_VARIANT_SIZES
 from test_carver_cpu import inflate_from_vmap
 
 pytestmark = pytest.mark.gpu
@@ -87,13 +88,9 @@ def test_non_uniform_weights_equal_single_sessions(ctx):
         ctx.set_params(8, 0.5, 0.5)
 
 
-# the seam DP's strip widths and energy staging variants, as in test_carver_batch_gpu.py
-@pytest.mark.parametrize("w,h,env", [(300, 40, {}), (4000, 24, {}), (5000, 24, {}), (13000, 12, {}),
-                                     (300, 40, {"DCTC_DP_P": "4"}), (5000, 24, {"DCTC_DP_NO_TENSORMAP": "1"}),
-                                     (300, 40, {"DCTC_DP_NO_TMA": "1"})])
-def test_strip_widths_and_staging_variants(ctx, monkeypatch, w, h, env):
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+# the seam DP's strip widths and energy staging variants (the width map of test_carver_batch_gpu.py)
+@pytest.mark.parametrize("w,h", DP_VARIANT_SIZES)
+def test_strip_widths_and_staging_variants(ctx, w, h):
     frames = frames_of(w, h, 1, [w + 11, w + 12, w + 13], patterns=(0, 2, 0))
     ctx.set_params(8, 0.5, 0.5)
     assert_matches_single(ctx, frames, 3, run_batch(ctx, frames, 3))

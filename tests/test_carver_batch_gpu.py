@@ -79,16 +79,22 @@ def test_non_uniform_weights_equal_single_sessions(ctx):
         ctx.set_params(8, 0.5, 0.5)
 
 
-# strip width P of the seam DP and its energy staging, per width (see dp_plan in csrc/dctc_k2_carver.cu):
-#   300: P = 1, 32-row stages (tensor map)     4000: P = 1, 16-row stages     5000: P = 2, 16-row stages
-#   13000: P = 4, no staging (register ring); DCTC_DP_P=4 at 300: P = 4 with 32-row stages, 128 * P > 256 -> no tensor
-#   map (row-wise bulk copies); DCTC_DP_NO_TENSORMAP / DCTC_DP_NO_TMA: row-wise bulk copies / register ring at P = 2 / 1
-@pytest.mark.parametrize("w,h,env", [(300, 40, {}), (4000, 24, {}), (5000, 24, {}), (13000, 12, {}),
-                                     (300, 40, {"DCTC_DP_P": "4"}), (5000, 24, {"DCTC_DP_NO_TENSORMAP": "1"}),
-                                     (300, 40, {"DCTC_DP_NO_TMA": "1"})])
-def test_strip_widths_and_staging_variants(ctx, monkeypatch, w, h, env):
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+# The seam DP's variant per frame width (dp_plan in csrc/dctc_k2_carver.cu): P float4 groups per lane (strips of
+# 128 * P columns), energies staged in nst stages of SR rows by tensor copies, or SR = 0: a register ring.
+#   width             P  SR  nst    test width
+#   1 - 2560          1  32   2     300
+#   2561 - 3584       1  16   3     3000
+#   3585 - 4096       1  16   2     4000
+#   4097 - 4608       2  16   3     4500
+#   4609 - 7680       2  16   2     5000
+#   7681 - 12288      2   0   -     9000
+#   12289 - 28672     4   0   -     13000
+# The 16-row cases are tall enough to have more chunks than stages, so each of them refills a stage.
+DP_VARIANT_SIZES = [(300, 40), (3000, 56), (4000, 40), (4500, 56), (5000, 40), (9000, 16), (13000, 12)]
+
+
+@pytest.mark.parametrize("w,h", DP_VARIANT_SIZES)
+def test_strip_widths_and_staging_variants(ctx, w, h):
     frames = frames_of(w, h, 1, [w + 1, w + 2, w + 3], patterns=(0, 2, 0))
     ctx.set_params(8, 0.5, 0.5)
     assert_matches_single(ctx, frames, 3, run_batch(ctx, frames, 3))

@@ -194,9 +194,9 @@ def test_wide_image_takes_the_serial_backtrack(ctx):
     assert_same(device(ctx, img, 5, vmaps=True), reference(ctx, img, 5, vmaps=True))
 
 
-def test_dp_staging_variant(ctx, monkeypatch):
-    monkeypatch.setenv("DCTC_DP_NO_TMA", "1")
-    img = image(300, 200, 3, 101)
+def test_tall_narrow_image_takes_the_register_ring(ctx):
+    """16 x 9000: the transposed frame is 9000 wide, where the seam DP keeps its energies in a register ring (P = 2)."""
+    img = image(16, 9000, 3, 101)
     ctx.set_params(8, 0.5, 0.5)
     assert_same(device(ctx, img, 7), reference(ctx, img, 7))
 

@@ -9,6 +9,7 @@ import pytest
 
 import dct_carver_b200 as dc
 import oracle_lib as ol
+from test_carver_batch_gpu import DP_VARIANT_SIZES
 
 pytestmark = pytest.mark.gpu
 
@@ -157,13 +158,9 @@ def test_1080p_prefix(ctx, ectx):
     check_width(ctx, ectx, img, rigidity_for(ectx, img, 1.0), 3)
 
 
-# strip width P of the seam DP and its energy staging (the geometry matrix of test_carver_batch_gpu.py)
-@pytest.mark.parametrize("w,h,env", [(300, 40, {}), (4000, 24, {}), (5000, 24, {}), (13000, 12, {}),
-                                     (300, 40, {"DCTC_DP_P": "4"}), (5000, 24, {"DCTC_DP_NO_TENSORMAP": "1"}),
-                                     (300, 40, {"DCTC_DP_NO_TMA": "1"})])
-def test_dp_variants(ctx, ectx, monkeypatch, w, h, env):
-    for k, v in env.items():
-        monkeypatch.setenv(k, v)
+# strip width P of the seam DP and its energy staging (the width map of test_carver_batch_gpu.py)
+@pytest.mark.parametrize("w,h", DP_VARIANT_SIZES)
+def test_dp_variants(ctx, ectx, w, h):
     img = image(w, h, 1, w + 8300, pattern=2)
     check_width(ctx, ectx, img, rigidity_for(ectx, img, 1.0), 3)
 
