@@ -16,6 +16,7 @@ LIB_PATH = os.environ.get("DCTC_LIB") or os.path.join(_HERE, "libdctc.so")   # D
 OK = 0
 ERR_INVALID, ERR_BLOCKSIZE, ERR_NOMEM, ERR_CUDA, ERR_NO_DEVICE, ERR_STATE, ERR_UNSUPPORTED = -1, -2, -3, -4, -5, -6, -7
 KERNEL_AUTO, KERNEL_FP32_TILE, KERNEL_FP32_MARCH, KERNEL_TC_SPLIT, KERNEL_FP32_STREAM = 0, 1, 2, 3, 4
+MAX_DELTA_X = 4   # DCTC_MAX_DELTA_X: the widest seam step the device seam loop takes
 
 # every symbol include/dctc.h declares (tests check that the library exports exactly these)
 ABI_SYMBOLS = [
@@ -32,7 +33,7 @@ ABI_SYMBOLS = [
     "dctc_carver_batch_vmap", "dctc_carver_batch_resize_height", "dctc_carver_batch_enlarge_height", "dctc_carver_batch_height",
     "dctc_resize_plan", "dctc_carver_resize", "dctc_carver_batch_resize",
     "dctc_carver_set_bias", "dctc_carver_bias", "dctc_carver_batch_set_bias", "dctc_carver_batch_bias",
-    "dctc_carver_set_rigidity", "dctc_carver_batch_set_rigidity",
+    "dctc_carver_set_rigidity", "dctc_carver_batch_set_rigidity", "dctc_carver_set_delta_x", "dctc_carver_batch_set_delta_x",
     "dctc_carver_levels_width", "dctc_carver_levels_height", "dctc_carver_render_levels", "dctc_carver_batch_levels_width",
     "dctc_carver_batch_levels_height", "dctc_carver_batch_render_levels", "dctc_carver_batch_render_levels_dev",
     "dctc_synth_fill_dev", "dctc_synth_byte", "dctc_ipc_export", "dctc_ipc_open", "dctc_ipc_close",
@@ -150,6 +151,8 @@ def lib():
         "dctc_carver_batch_bias": (i32, [vp, vp]),
         "dctc_carver_set_rigidity": (i32, [vp, f32]),
         "dctc_carver_batch_set_rigidity": (i32, [vp, f32]),
+        "dctc_carver_set_delta_x": (i32, [vp, i32]),
+        "dctc_carver_batch_set_delta_x": (i32, [vp, i32]),
         "dctc_carver_levels_width": (i32, [vp, i32, vp]),
         "dctc_carver_levels_height": (i32, [vp, i32, vp]),
         "dctc_carver_render_levels": (i32, [vp, i32, vp, vp]),
@@ -555,6 +558,12 @@ class Context:
         survives carver_load; 0 (the default) is the plain seam search.  Raises for a negative or non-finite value."""
         _check(lib().dctc_carver_set_rigidity(self._h, float(rigidity)), "dctc_carver_set_rigidity")
 
+    def carver_set_delta_x(self, delta_x):
+        """liblqr's delta_x (lqr_carver_init): the largest number of columns a seam may move from one row to the next,
+        1 .. MAX_DELTA_X (include/dctc.h).  Applies from the next seam operation and survives carver_load; 1 (the
+        default) is the plug-in's value.  Raises for delta_x < 1 or above MAX_DELTA_X."""
+        _check(lib().dctc_carver_set_delta_x(self._h, int(delta_x)), "dctc_carver_set_delta_x")
+
     def carver_set_incremental(self, on):
         """Device seam loop: update the cumulative map incrementally (liblqr's update_mmap) instead of rebuilding it."""
         _check(lib().dctc_carver_set_incremental(self._h, int(bool(on))), "dctc_carver_set_incremental")
@@ -626,7 +635,8 @@ class Context:
             raise ValueError("seam must have one column per row")
         xmin = np.empty(h, np.int32)
         xmax = np.empty(h, np.int32)
-        band = np.empty(h * 4 * (self.blocksize // 2), np.float32) if want_band else None
+        # at most 2 r (delta_x + 1) values per row (include/dctc.h), r = blocksize / 2
+        band = np.empty(h * 2 * (self.blocksize // 2) * (MAX_DELTA_X + 1), np.float32) if want_band else None
         _check(lib().dctc_carve_and_update(self._h, _ptr(seam), _ptr(band) if want_band else None, _ptr(xmin),
                                            _ptr(xmax)), "dctc_carve_and_update")
         if want_band:
@@ -774,6 +784,11 @@ class CarverBatch:
         """Context.carver_set_rigidity for every frame of the batch: applies from the next seam operation and survives
         load()."""
         _check(lib().dctc_carver_batch_set_rigidity(self._b, float(rigidity)), "dctc_carver_batch_set_rigidity")
+
+    def set_delta_x(self, delta_x):
+        """Context.carver_set_delta_x for every frame of the batch: applies from the next seam operation and survives
+        load()."""
+        _check(lib().dctc_carver_batch_set_delta_x(self._b, int(delta_x)), "dctc_carver_batch_set_delta_x")
 
     def bias(self):
         """The current bias planes (n, height, width)."""

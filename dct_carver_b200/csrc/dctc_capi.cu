@@ -150,7 +150,8 @@ bool dctc_k1_fast_layout(const DctcK1Args& a)
 }
 
 // The context supplies the device, the tensor-core counters and the launch counter; op the operator and kernel selection.
-int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream, const DctcK1Bias* bias)
+int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream, const DctcK1Bias* bias,
+                int delta_x)
 {
     // E = max|T| * weight; the kernels keep luma in 0..255 units, so the 1/255 of liblqr's reader folds in here.
     a.w_edges = (float) ((double) op.edges / 255.0);
@@ -160,7 +161,7 @@ int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_fram
     auto counter = [ctx] { return ctx->tc_counters + (ctx->tc_next++ % DCTC_TC_COUNTERS); };
     cudaError_t e = cudaSuccess;
     switch (dctc_k1_select(op.kernel, op.blocksize, a.seam != nullptr, a.preview != 0, dctc_k1_fast_layout(a))) {
-    case DctcK1Variant::Tile: e = dctc_launch_k1_tile(a, op.blocksize, n_frames, uniform, stream, bias); break;
+    case DctcK1Variant::Tile: e = dctc_launch_k1_tile(a, op.blocksize, n_frames, uniform, stream, bias, delta_x); break;
     case DctcK1Variant::Small: e = dctc_launch_k1_small(a, op.blocksize, n_frames, uniform, ctx->sm_count, stream); break;
     case DctcK1Variant::March8: e = dctc_launch_k1_march8(a, n_frames, uniform, stream); break;
     case DctcK1Variant::Tc8: e = dctc_launch_k1_tc8(a, n_frames, uniform, counter(), ctx->sm_count, stream); break;

@@ -146,12 +146,13 @@ __global__ void __launch_bounds__(TW* TH / P) dctc_k1_tile_kernel(const DctcK1Ar
 }
 
 template <int B, int TW, int TH, int P, bool BIAS = false>
-static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, DctcK1Bias bias = {})
+static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, DctcK1Bias bias = {}, int dx = 1)
 {
     constexpr int LW = TW + B - 1, LH = TH + B - 1;
     constexpr size_t smem = sizeof(float) * (size_t) (LH * LW + B * LH * TW);
-    // band mode: a tile row spans at most (TH-1) + 4*band_r + 1 columns (seam drift over TH+2r rows plus 2r)
-    const int span = a.seam ? (TH + 4 * a.band_r) : a.w;
+    // band mode: a tile row spans at most dx * (TH-1 + 2*band_r) + 2*band_r + 1 columns (seam drift of dx per row over
+    // TH+2r rows plus 2r; TH + 4*band_r for connected seams)
+    const int span = a.seam ? dx * (TH - 1 + 2 * a.band_r) + 2 * a.band_r + 1 : a.w;
     dim3 grid((span + TW - 1) / TW, (a.h + TH - 1) / TH, n_frames), block(TW * TH / P);
     return dctc_dispatch<0>(uniform, 0, [&](auto U, auto) {   // one kernel for every channel count
         const cudaError_t e = cudaFuncSetAttribute(dctc_k1_tile_kernel<B, TW, TH, P, U, BIAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) smem);
@@ -164,13 +165,14 @@ static cudaError_t launch_tile(const DctcK1Args& a, int n_frames, bool uniform, 
 
 // band configuration (32 x 16 tiles, two pixels per thread), with the bias store for biased carver sessions
 template <int B>
-static cudaError_t launch_band(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias)
+static cudaError_t launch_band(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias, int dx)
 {
-    if (bias) return launch_tile<B, 32, 16, 2, true>(a, n_frames, uniform, stream, *bias);
-    return launch_tile<B, 32, 16, 2>(a, n_frames, uniform, stream);
+    if (bias) return launch_tile<B, 32, 16, 2, true>(a, n_frames, uniform, stream, *bias, dx);
+    return launch_tile<B, 32, 16, 2>(a, n_frames, uniform, stream, {}, dx);
 }
 
-cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias)
+cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream, const DctcK1Bias* bias,
+                                int delta_x)
 {
     if (a.w <= 0 || a.h <= 0 || n_frames <= 0) return cudaSuccess;
     if (n_frames > 65535 || (a.h + 31) / 32 > 65535) return cudaErrorInvalidConfiguration;
@@ -179,10 +181,10 @@ cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames
         // pixels per thread keep the per-thread chain short (8 k1 x 2 instead of 8 k1 x 8 transforms for b = 8); the
         // arithmetic per pixel is the same as in the full-map configuration (bit-identical energies)
         switch (blocksize) {
-        case 2: return launch_band<2>(a, n_frames, uniform, stream, bias);
-        case 4: return launch_band<4>(a, n_frames, uniform, stream, bias);
-        case 8: return launch_band<8>(a, n_frames, uniform, stream, bias);
-        case 16: return launch_band<16>(a, n_frames, uniform, stream, bias);
+        case 2: return launch_band<2>(a, n_frames, uniform, stream, bias, delta_x);
+        case 4: return launch_band<4>(a, n_frames, uniform, stream, bias, delta_x);
+        case 8: return launch_band<8>(a, n_frames, uniform, stream, bias, delta_x);
+        case 16: return launch_band<16>(a, n_frames, uniform, stream, bias, delta_x);
         default: return cudaErrorInvalidValue;
         }
     }

@@ -237,6 +237,81 @@ __device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, s
     asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
+// ---- seam step width (liblqr's delta_x) ----------------------------------------------------------------------------
+// With delta_x = dx in 2 .. DCTC_MAX_DELTA_X a seam may move up to dx columns from one row to the next:
+//   m[y][x] = en[y][x] + min_{|d| <= dx} fl(m[y-1][x+d] + pen[|d|]),   parent = FIRST strict minimum scanning x-dx .. x+dx,
+// pen[0] = 0, pen[d] = fl(fl(rigidity * fl(d * fl(sqrt(d)))) / h) (liblqr's rigidity_map [from memory: parity unpinned]).
+// The WIDE instantiations of the seam DP and the wide serial walk take the table with pen[d] = +inf for dx < d <= 4, so
+// one kernel serves every dx: a candidate beyond the step bound costs +inf and never wins (the d = 0 candidate is finite).
+struct DpSteps {
+    float pen[DCTC_MAX_DELTA_X + 1];
+    int dx;
+};
+
+// dp_backtrack for dx > 1: the same double-buffered windows, but batches of wb rows with 2 * wb * dx + dx <= 66, so that
+// the next batch's window (staged around the column the current batch starts at) still holds every candidate it reads.
+// The four floats left of the window hold the +inf sentinels of column 0, and the four columns from w on those of the
+// right edge.  best starts at +inf, so a candidate that is not a real one (+inf pen) never wins.
+__device__ __forceinline__ void dp_backtrack_wide(const float* __restrict__ mplane, size_t m_pitch, int w, int h, int x,
+                                                  int* __restrict__ seam, int* __restrict__ seam_log,
+                                                  float (*win)[32][DP_WINP], int lane, const DpSteps& st)
+{
+    const float INF = __int_as_float(0x7f800000);
+    const int wb = (66 - st.dx) / (2 * st.dx);
+    if (lane == 0) { seam[h - 1] = x; if (seam_log) seam_log[h - 1] = x; }
+    const int max_base = (int) m_pitch - DP_WIN;
+    auto stage = [&](int ytop, int xs, int buf) -> int {
+        int base = (xs - 66) & ~3;
+        base = base < 0 ? 0 : (base > max_base ? max_base : base);
+        if (ytop >= 1) {
+            for (int idx = lane; idx < wb * (DP_WIN / 4); idx += 32) {
+                const int i = idx / (DP_WIN / 4), c = idx - i * (DP_WIN / 4);
+                const int yy = ytop - 1 - i;
+                if (yy >= 0) {
+                    const float* src = mplane + (size_t) yy * m_pitch + base + 4 * c;
+                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t) __cvta_generic_to_shared(&win[buf][i][4 + 4 * c])), "l"(src) : "memory");
+                }
+            }
+        }
+        asm volatile("cp.async.commit_group;" ::: "memory");
+        return base;
+    };
+    int buf = 0;
+    int base = stage(h - 1, x, 0);
+    for (int ytop = h - 1; ytop >= 1; ytop -= wb) {
+        const int base_next = stage(ytop - wb, x, buf ^ 1);
+        asm volatile("cp.async.wait_group 1;" ::: "memory");
+        __syncwarp();
+        if (lane < wb) {
+            if (base == 0)
+                for (int j = 0; j < 4; j++) win[buf][lane][j] = INF;
+            if (w - base >= 0 && w - base <= DP_WIN)
+                for (int j = 0; j < 4; j++) win[buf][lane][4 + w - base + j] = INF;
+        }
+        __syncwarp();
+        const int steps = ytop < wb ? ytop : wb;
+        int mine = 0;
+        const float* wp = &win[buf][0][4] + (x - base);
+        for (int i = 0; i < steps; i++) {
+            float best = INF;
+            int dbest = 0;
+#pragma unroll
+            for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
+                const float v = d == 0 ? wp[0] : wp[d] + st.pen[d < 0 ? -d : d];
+                if (v < best) { best = v; dbest = d; }
+            }
+            x += dbest;
+            wp += DP_WINP + dbest;
+            if (lane == i) mine = x;
+        }
+        if (lane < steps) { seam[ytop - 1 - lane] = mine; if (seam_log) seam_log[ytop - 1 - lane] = mine; }
+        __syncwarp();
+        base = base_next;
+        buf ^= 1;
+    }
+    asm volatile("cp.async.wait_group 0;" ::: "memory");
+}
+
 // TMA = true: the energies of a strip are staged nst chunks of DP_SR rows ahead into shared memory, one tensor copy per
 // chunk (cp.async.bulk.tensor.3d, completion on an mbarrier per warp and stage) instead of a register ring of plain
 // loads: nothing the cluster barrier's memory fence has to wait for, and up to 64 rows in flight per warp.
@@ -279,14 +354,19 @@ __device__ __forceinline__ void dp_unroll(F&& f)
 // floats after the previous frame's, whose seam is seam[h * frame ...], its log seam_log[log_fs * frame ...] and its
 // last-row column xlast[frame].  The tensor map is 3-D (columns, rows, frames) with a box depth of one frame.
 // RIG: rigidity pen (see above), the trailing argument.
-template <int DP_P, int DP_SR, bool RIG>
+// WIDE (seam step width, see DpSteps): the trailing argument is the step table instead, every cell takes the minimum over
+// the 2 * 4 + 1 candidates of the table, and the warps exchange halos every DP_R / dx rows instead of every DP_R (a strip's
+// edge then contaminates dx columns per row, still at most DP_R after a block).  With at least 4 cells per lane every
+// candidate comes from the lane or its two neighbours.  No incremental map (run_flag is null); without xlast warp 0 of
+// CTA 0 walks back with dp_backtrack_wide, with it the wide jump and trace kernels follow.  RIG is false.
+template <int DP_P, int DP_SR, bool RIG, bool WIDE>
 __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dctc_seam_dp_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                                     float* __restrict__ mplane, size_t m_pitch,
                                                                     int* __restrict__ seam, int* __restrict__ seam_log,
                                                                     int* __restrict__ run_flag, int nst,
                                                                     const __grid_constant__ CUtensorMap tmap,
                                                                     int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs,
-                                                                    float pen)
+                                                                    std::conditional_t<WIDE, DpSteps, float> pen)
 {
     DCTC_PDL_PROLOGUE();
     // (the frame's seam, log and xlast offsets are applied after the row loop, so they occupy no registers in it)
@@ -443,6 +523,54 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
                 asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(e[0][g].x), "=f"(e[0][g].y), "=f"(e[0][g].z), "=f"(e[0][g].w)
                              : "r"(stg_s + (uint32_t) (((kk % SRD) * STRIP + 4 * g) * 4)));   // base register + immediate
         }
+        if constexpr (WIDE) {
+            // the 4 cells on each side of the lane's cells (neighbour lanes; +inf beyond the strip), then per cell the
+            // minimum of cur and fl(neighbour + pen[|d|]) over d = -4 .. 4 (min is exact: the order does not matter)
+            constexpr int CW = 4 * DP_P;
+            float c[CW + 8];
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) {
+                c[4 + 4 * g] = cur[g].x; c[5 + 4 * g] = cur[g].y; c[6 + 4 * g] = cur[g].z; c[7 + 4 * g] = cur[g].w;
+            }
+            const float lsrc[4] = {cur[DP_P - 1].x, cur[DP_P - 1].y, cur[DP_P - 1].z, cur[DP_P - 1].w};
+            const float rsrc[4] = {cur[0].x, cur[0].y, cur[0].z, cur[0].w};
+#pragma unroll
+            for (int j = 0; j < 4; j++) {
+                const float lv = __shfl_up_sync(0xffffffffu, lsrc[j], 1), rv = __shfl_down_sync(0xffffffffu, rsrc[j], 1);
+                c[j] = lane == 0 ? INF : lv;
+                c[CW + 4 + j] = lane == 31 ? INF : rv;
+            }
+            float mn[CW];
+#pragma unroll
+            for (int i = 0; i < CW; i++) mn[i] = c[4 + i];
+#pragma unroll
+            for (int d = 1; d <= 4; d++) {
+                const float pd = pen.pen[d];
+                float qd[CW + 8];
+#pragma unroll
+                for (int i = 4 - d; i < CW + 4 + d; i++) qd[i] = c[i] + pd;
+#pragma unroll
+                for (int i = 0; i < CW; i++) mn[i] = fminf(mn[i], fminf(qd[4 + i - d], qd[4 + i + d]));
+            }
+            float4 o[DP_P];
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) {
+                o[g].x = e[k][g].x + mn[4 * g]; o[g].y = e[k][g].y + mn[4 * g + 1];
+                o[g].z = e[k][g].z + mn[4 * g + 2]; o[g].w = e[k][g].w + mn[4 * g + 3];
+            }
+            if (!TMA) {
+#pragma unroll
+                for (int g = 0; g < DP_P; g++)
+                    e[k][g] = __ldg(reinterpret_cast<const float4*>(en_g[g] + (size_t) min(y + PF, hm1) * en_pitch));
+            }
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) {
+                if (central && ld_ok[g]) *reinterpret_cast<float4*>(mptr + 4 * g) = o[g];
+                if (!TMA) patch(o[g], inf_mask[g]);
+                cur[g] = o[g];
+            }
+            mptr += m_pitch;
+        } else {
         // q: the previous row as a diagonal parent sees it (RIG: cur + pen, one add per cell; else cur itself)
         float4 q[DP_P];
 #pragma unroll
@@ -477,7 +605,66 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             cur[g] = o[g];
         }
         mptr += m_pitch;
+        }
     };
+    if constexpr (WIDE) {
+        // the halo exchange of the block loop below (as there), after every DP_R / dx rows counted from row 0 and never
+        // after the last row
+        auto exchange = [&]() {
+            const int wl = tid >> 5;                          // warp inside the CTA
+            float* halo = xrow + (wl * 2 + xb) * 64;          // [0,32): cells left of the published range, [32,64): right
+            const uint32_t my_bar = dp_smem_u32(&hbar[wl][xb]);
+            if (lane == 0) {
+                const uint32_t expect = (warp > 0 ? 128u : 0u) + (warp < nwarps - 1 ? 128u : 0u);
+                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar), "r"(expect) : "memory");
+            }
+            if (lane >= HL && lane < 2 * HL && warp > 0) {                        // my leftmost 32 published cells
+                const int nw = warp - 1;
+                const uint32_t nrank = (uint32_t) (nw / wpc);
+                const int nwl = nw - (int) nrank * wpc;
+                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + 32 + (lane - HL) * CPL, nrank);
+                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
+    #pragma unroll
+                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+            }
+            if (lane >= 32 - 2 * HL && lane < 32 - HL && warp < nwarps - 1) {     // my rightmost 32 published cells
+                const int nw = warp + 1;
+                const uint32_t nrank = (uint32_t) (nw / wpc);
+                const int nwl = nw - (int) nrank * wpc;
+                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + (lane - (32 - 2 * HL)) * CPL, nrank);
+                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
+    #pragma unroll
+                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+            }
+            dp_mbar_wait(my_bar, (uint32_t) ((hround >> 1) & 1));
+            hround++;
+            if (!central) {
+                const float* hp = halo + (lane < HL ? lane * CPL : 32 + (lane - (32 - HL)) * CPL);
+    #pragma unroll
+                for (int g = 0; g < DP_P; g++) {
+                    const int x = c0 + 4 * g;
+                    if (x >= 0 && x < w) cur[g] = *reinterpret_cast<const float4*>(hp + 4 * g);   // cells right of the image arrive as +inf
+                    else cur[g] = make_float4(INF, INF, INF, INF);
+                }
+            }
+            xb ^= 1;
+        };
+        const int rb = DP_R / pen.dx;
+        int since = 0;
+        for (int yb = 1; yb < h; yb += DP_R) {
+            dp_unroll<DP_R>([&](auto kk_c) {
+                constexpr int kk = decltype(kk_c)::value;
+                const int y = yb + kk;
+                if (TMA && kk % SRD == 0 && y < h) chunk_begin();
+                if (y < h) row(kk_c, y);
+                if (++since == rb && y + 1 < h) {
+                    exchange();
+                    since = 0;
+                }
+                if (TMA && kk % SRD == SRD - 1) chunk_end();
+            });
+        }
+    } else {
     for (int yb = 1; yb < h; yb += DP_R) {
         if (yb + DP_R <= h) {                         // whole block: no per-row bounds checks
             dp_unroll<DP_R>([&](auto kk_c) {
@@ -541,6 +728,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             xb ^= 1;
         }
     }
+    }
 #ifdef DCTC_SYNC_DEBUG
     const long long dbg_t1 = clock64();
 #endif
@@ -599,6 +787,8 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         if (xlast) {
             // parallel back-track: the jump and trace kernels below take over from the seam's last-row column
             if (lane == 0) { *xlast = bi; seam[h - 1] = bi; if (seam_log) seam_log[h - 1] = bi; }
+        } else if constexpr (WIDE) {
+            dp_backtrack_wide(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);
         } else {
             dp_backtrack<RIG>(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);   // serial walk by warp 0 of CTA 0
         }
@@ -998,6 +1188,174 @@ template __global__ void dctc_seam_trace_kernel<true>(const float*, size_t, int,
                                                       size_t, size_t, size_t, float);
 template __global__ void dctc_seam_incr_kernel<false>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
 template __global__ void dctc_seam_incr_kernel<true>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
+
+// ---- parallel back-track for delta_x > 1 -----------------------------------------------------------------------------
+// The jump and trace kernels above with the step table of the WIDE seam DP (DpSteps: 9 candidates, +inf pen beyond dx,
+// best = +inf and a strict < = the first strict minimum of the real candidates).  A path moves up to dx columns per row,
+// so the jump blocks are JBW = 31 rows (offsets of up to 31 * 4 = 124 columns fit int8), a jump warp's lanes hold 16
+// columns each (strip of 512, 128 contaminated on each side after a block, 256 published) and a trace CTA walks its block
+// through a window of TRW_WIN columns.  The cone of block j spans x0 +- R j, R = JBW * dx: its rows are staged in
+// (R8 / 8) j + 3 chunks of 16 bytes, R8 = R rounded up to 8 (R8 = 32 and JBW = 32 give the layout of dx = 1).
+constexpr int JBW = 31;
+constexpr int TRW_WIN = 264;                          // walk window: columns x-132 .. x+131 around the block's bottom column
+
+__global__ void __launch_bounds__(128) dctc_seam_jump_wide_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
+                                                                  int8_t* __restrict__ jump, size_t j_pitch, int strips,
+                                                                  size_t m_fs, size_t j_fs, DpSteps st)
+{
+    DCTC_PDL_PROLOGUE();
+    const int lane = threadIdx.x & 31;
+    const int strip = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (strip >= strips) return;
+    const int k = blockIdx.y;
+    mplane += blockIdx.z * m_fs;
+    jump += blockIdx.z * j_fs;
+    const int yb = h - 1 - JBW * k;
+    const int yt = max(yb - JBW, 0);
+    const int steps = yb - yt;
+    const float INF = __int_as_float(0x7f800000);
+    const int c0 = strip * 256 - 128 + 16 * lane;     // this lane's 16 columns
+    bool ok[4];
+    const float* src[4];
+#pragma unroll
+    for (int g = 0; g < 4; g++) {
+        ok[g] = c0 + 4 * g >= 0 && c0 + 4 * g < w;     // (multiples of 4: the pitch covers round_up(w, 4))
+        src[g] = mplane + (size_t) yt * m_pitch + (ok[g] ? c0 + 4 * g : 0);
+    }
+    int P[16];
+#pragma unroll
+    for (int i = 0; i < 16; i++) P[i] = c0 + i;
+    auto row = [&](const float4 (&v)[4]) {            // cumulative values of row y-1 -> P of row y
+        float e[24];
+        int pe[24];
+#pragma unroll
+        for (int g = 0; g < 4; g++) {
+            const float c4[4] = {v[g].x, v[g].y, v[g].z, v[g].w};
+#pragma unroll
+            for (int j = 0; j < 4; j++) e[4 + 4 * g + j] = ok[g] && c0 + 4 * g + j < w ? c4[j] : INF;   // range clipping
+        }
+#pragma unroll
+        for (int i = 0; i < 16; i++) pe[4 + i] = P[i];
+#pragma unroll
+        for (int j = 0; j < 4; j++) {
+            const float l = __shfl_up_sync(0xffffffffu, e[16 + j], 1), r = __shfl_down_sync(0xffffffffu, e[4 + j], 1);
+            pe[j] = __shfl_up_sync(0xffffffffu, P[12 + j], 1);
+            pe[20 + j] = __shfl_down_sync(0xffffffffu, P[j], 1);
+            e[j] = lane == 0 ? INF : l;
+            e[20 + j] = lane == 31 ? INF : r;
+        }
+#pragma unroll
+        for (int i = 0; i < 16; i++) {
+            float best = INF;
+            int q = pe[4 + i];
+#pragma unroll
+            for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
+                const float v = d == 0 ? e[4 + i] : e[4 + i + d] + st.pen[d < 0 ? -d : d];
+                if (v < best) { best = v; q = pe[4 + i + d]; }
+            }
+            P[i] = q;
+        }
+    };
+    for (int i0 = 0; i0 < steps; i0 += 4) {           // four rows of loads in flight, then four dependent steps
+        float4 pv[4][4];
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+#pragma unroll
+            for (int g = 0; g < 4; g++)
+                pv[j][g] = __ldcg(reinterpret_cast<const float4*>(src[g] + (size_t) min(i0 + j, steps - 1) * m_pitch));
+#pragma unroll
+        for (int j = 0; j < 4; j++)
+            if (i0 + j < steps) row(pv[j]);
+    }
+    if (lane >= 8 && lane < 24) {
+        int8_t* dst = jump + (size_t) k * j_pitch;
+#pragma unroll
+        for (int i = 0; i < 16; i++)
+            if (c0 + i >= 0 && c0 + i < w) dst[c0 + i] = (int8_t) (P[i] - (c0 + i));
+    }
+}
+
+__global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_wide_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
+                                                                          const int8_t* __restrict__ jump, size_t j_pitch,
+                                                                          const int* __restrict__ xlast, int* __restrict__ seam,
+                                                                          int* __restrict__ seam_log, size_t m_fs, size_t j_fs,
+                                                                          size_t log_fs, DpSteps st)
+{
+    extern __shared__ __align__(16) unsigned char trw_smem[];
+    __shared__ __align__(16) float win[JBW][TRW_WIN + 8];
+    __shared__ int xb_s;
+    DCTC_PDL_PROLOGUE();
+    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const int k = blockIdx.x, fz = blockIdx.y;
+    mplane += fz * m_fs;
+    jump += fz * j_fs;
+    seam += (size_t) fz * h;
+    if (seam_log) seam_log += fz * log_fs;
+    const int x0 = xlast[fz];
+    const int R = JBW * st.dx, R8 = (R + 7) & ~7;
+    auto row_off = [&](int j) { return R8 * j * (j - 1) + 48 * j; };   // bytes of the cone rows before row j
+    for (int j = wid; j < k; j += TR_THREADS / 32) {
+        const int a0 = max(0, x0 - R * j) & ~15;
+        const int last = min(w - 1, x0 + R * j);
+        const int nchunk = ((last - a0) >> 4) + 1;                          // <= (R8 / 8) j + 3
+        const uint4* srcj = reinterpret_cast<const uint4*>(jump + (size_t) j * j_pitch + a0);
+        uint4* dstj = reinterpret_cast<uint4*>(trw_smem + row_off(j));
+        for (int c0 = 0; c0 < nchunk; c0 += 160) {
+            uint4 v[5];
+#pragma unroll
+            for (int i = 0; i < 5; i++)
+                if (c0 + lane + 32 * i < nchunk) v[i] = __ldcg(srcj + c0 + lane + 32 * i);
+#pragma unroll
+            for (int i = 0; i < 5; i++)
+                if (c0 + lane + 32 * i < nchunk) dstj[c0 + lane + 32 * i] = v[i];
+        }
+    }
+    __syncthreads();
+    if (tid == 0) {
+        const int8_t* cone = reinterpret_cast<const int8_t*>(trw_smem);
+        int x = x0;
+        for (int j = 0; j < k; j++) x += cone[row_off(j) + (x - (max(0, x0 - R * j) & ~15))];
+        xb_s = x;
+    }
+    __syncthreads();
+    int x = xb_s;
+    const int yb = h - 1 - JBW * k, yt = max(yb - JBW, 0), steps = yb - yt;
+    // window rows: win[i] = cumulative row yb-1-i, columns base .. base+TRW_WIN-1 at win[i][4 + c - base]
+    const int max_base = (int) m_pitch - TRW_WIN;                 // >= 0: bt_plan asks for m_pitch >= TRW_WIN
+    int base = (x - 132) & ~3;
+    base = base < 0 ? 0 : (base > max_base ? max_base : base);
+    for (int idx = tid; idx < steps * (TRW_WIN / 4); idx += TR_THREADS) {
+        const int i = idx / (TRW_WIN / 4), c = idx - i * (TRW_WIN / 4);
+        const float* src = mplane + (size_t) (yb - 1 - i) * m_pitch + base + 4 * c;
+        *reinterpret_cast<float4*>(&win[i][4 + 4 * c]) = __ldcg(reinterpret_cast<const float4*>(src));
+    }
+    __syncthreads();
+    if (tid >= 32) return;
+    const float INF = __int_as_float(0x7f800000);
+    // four +inf sentinels left of column 0 and from column w on (range clipping)
+    if (lane < steps) {
+        if (base == 0)
+            for (int j = 0; j < 4; j++) win[lane][j] = INF;
+        if (w - base >= 0 && w - base <= TRW_WIN)
+            for (int j = 0; j < 4; j++) win[lane][4 + w - base + j] = INF;
+    }
+    __syncwarp();
+    int mine = 0;
+    const float* wp = &win[0][4] + (x - base);
+    for (int i = 0; i < steps; i++) {
+        float best = INF;
+        int dbest = 0;
+#pragma unroll
+        for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
+            const float v = d == 0 ? wp[0] : wp[d] + st.pen[d < 0 ? -d : d];
+            if (v < best) { best = v; dbest = d; }
+        }
+        x += dbest;
+        wp += TRW_WIN + 8 + dbest;
+        if (lane == i) mine = x;
+    }
+    if (lane < steps) { seam[yb - 1 - lane] = mine; if (seam_log) seam_log[yb - 1 - lane] = mine; }
+}
 
 // ---- visibility map + seam display (SURVEY section 8f rank 4) ---------------------------------------------------
 // liblqr's update_vsmap: the pixel removed from row y by the k-th seam is original column raw[y][s]; its entry of the
@@ -1417,17 +1775,21 @@ static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFram
 }
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
-// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map; rig selects the RIG twin.
+// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map; rig selects the RIG twin, wide the
+// WIDE kernel of delta_x > 1 (p.dpw instead of p.dp).
 using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int*, size_t, size_t, size_t,
                        float);
+using dp_wide_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int*, size_t, size_t,
+                            size_t, DpSteps);
 struct DpPlan {
-    dp_fn dp = nullptr;
+    dp_fn dp = nullptr;          // delta_x = 1
+    dp_wide_fn dpw = nullptr;    // delta_x > 1
     int wpc = 0, nst = 0;
     size_t smem = 0;
     CUtensorMap tmap;
 };
 
-static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, bool rig, DpPlan& p)
+static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, bool rig, bool wide, DpPlan& p)
 {
     // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
     const int cap = DP_CL * DP_MAXW;
@@ -1450,18 +1812,23 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
     p.wpc = wpc;
     p.nst = nst;
     p.smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
-    // the (P, SR) pairs the lines above select for widths 1 .. DP_MAX_W, and their RIG twins:
+    // the (P, SR) pairs the lines above select for widths 1 .. DP_MAX_W, their RIG twins and their WIDE kernels:
     //   1-2560: (1, 32)   2561-4096: (1, 16)   4097-7680: (2, 16)   7681-12288: (2, 0)   12289-DP_MAX_W: (4, 0)
-    static const struct { int P, sr; dp_fn fn[2]; } variants[] = {
-        {1, 32, {dctc_seam_dp_kernel<1, 32, false>, dctc_seam_dp_kernel<1, 32, true>}},
-        {1, 16, {dctc_seam_dp_kernel<1, 16, false>, dctc_seam_dp_kernel<1, 16, true>}},
-        {2, 16, {dctc_seam_dp_kernel<2, 16, false>, dctc_seam_dp_kernel<2, 16, true>}},
-        {2, 0, {dctc_seam_dp_kernel<2, 0, false>, dctc_seam_dp_kernel<2, 0, true>}},
-        {4, 0, {dctc_seam_dp_kernel<4, 0, false>, dctc_seam_dp_kernel<4, 0, true>}}};
+    static const struct { int P, sr; dp_fn fn[2]; dp_wide_fn wide; } variants[] = {
+        {1, 32, {dctc_seam_dp_kernel<1, 32, false, false>, dctc_seam_dp_kernel<1, 32, true, false>}, dctc_seam_dp_kernel<1, 32, false, true>},
+        {1, 16, {dctc_seam_dp_kernel<1, 16, false, false>, dctc_seam_dp_kernel<1, 16, true, false>}, dctc_seam_dp_kernel<1, 16, false, true>},
+        {2, 16, {dctc_seam_dp_kernel<2, 16, false, false>, dctc_seam_dp_kernel<2, 16, true, false>}, dctc_seam_dp_kernel<2, 16, false, true>},
+        {2, 0, {dctc_seam_dp_kernel<2, 0, false, false>, dctc_seam_dp_kernel<2, 0, true, false>}, dctc_seam_dp_kernel<2, 0, false, true>},
+        {4, 0, {dctc_seam_dp_kernel<4, 0, false, false>, dctc_seam_dp_kernel<4, 0, true, false>}, dctc_seam_dp_kernel<4, 0, false, true>}};
     p.dp = nullptr;
+    p.dpw = nullptr;
     for (const auto& v : variants)
-        if (v.P == P && v.sr == sr) p.dp = v.fn[rig ? 1 : 0];
-    if (!p.dp) return cudaErrorInvalidConfiguration;   // a pair without a kernel: the table and the plan disagree
+        if (v.P == P && v.sr == sr) {
+            if (wide) p.dpw = v.wide;
+            else p.dp = v.fn[rig ? 1 : 0];
+        }
+    const void* fn = wide ? (const void*) p.dpw : (const void*) p.dp;
+    if (!fn) return cudaErrorInvalidConfiguration;   // a pair without a kernel: the table and the plan disagree
     // tensor map of the energy planes for the staged variants (strips of up to 256 columns: the TMA box limit); frames
     // are its third dimension, so that a box never reaches into the next frame's rows
     memset(&p.tmap, 0, sizeof(p.tmap));
@@ -1477,26 +1844,33 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
             return cudaErrorInvalidValue;
     }
     // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
-    return cudaFuncSetAttribute(p.dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
+    return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
 }
 
 // Back-track plan for frames of h rows.  The parallel back-track (jump + trace kernels) needs the jump plane and a cone
-// of jump entries in shared memory that grows with the square of the number of 32-row blocks; very tall frames keep the
-// serial walk of the DP kernel.
+// of jump entries in shared memory that grows with the square of the number of row blocks; very tall frames keep the
+// serial walk of the DP kernel.  delta_x > 1: blocks of JBW rows, a cone dx times as wide (next to the 34 KB of the
+// wide trace kernel's window, hence the lower limit), and the window needs cumulative rows of at least TRW_WIN floats.
 struct BtPlan {
-    int nb;             // 32-row blocks
+    int nb;             // row blocks (JB rows, JBW for delta_x > 1)
     size_t cone_smem;   // trace kernel's dynamic shared memory
     size_t j_pitch;     // bytes per row of the jump plane (nb rows per frame)
     bool par;           // parallel back-track
 };
 
-static BtPlan bt_plan(int h, size_t m_pitch)
+static BtPlan bt_plan(int h, size_t m_pitch, int dx)
 {
     BtPlan b;
-    b.nb = (h - 1 + JB - 1) / JB;
-    b.cone_smem = b.nb > 0 ? (size_t) 32 * (b.nb - 1) * (b.nb - 1) + 16 * (size_t) (b.nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
+    const int jb = dx == 1 ? JB : JBW;
+    b.nb = (h - 1 + jb - 1) / jb;
+    if (dx == 1) {
+        b.cone_smem = b.nb > 0 ? (size_t) 32 * (b.nb - 1) * (b.nb - 1) + 16 * (size_t) (b.nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
+    } else {
+        const size_t r8 = (size_t) ((JBW * dx + 7) & ~7), j = b.nb > 0 ? (size_t) (b.nb - 1) : 0;
+        b.cone_smem = r8 * j * (j > 0 ? j - 1 : 0) + 48 * j + 16;   // rows j < nb-1: 16 ((R8 / 8) j + 3) bytes each
+    }
     b.j_pitch = (m_pitch + 15) & ~(size_t) 15;    // jump rows start 16-byte aligned (staged in 16-byte chunks)
-    b.par = b.nb > 0 && b.cone_smem <= 200 * 1024;
+    b.par = b.nb > 0 && (dx == 1 ? b.cone_smem <= 200 * 1024 : b.cone_smem <= 180 * 1024 && m_pitch >= (size_t) TRW_WIN);
     return b;
 }
 
@@ -1509,7 +1883,9 @@ static int frames_loop_buffers(dctc_context* ctx, CarverFrames& f, const BtPlan&
         CK(ctx, cudaMalloc((void**) &f.m, sizeof(float) * f.m_pitch * f.h * n));
         CK(ctx, cudaMemsetAsync(f.m, 0, sizeof(float) * f.m_pitch * f.h * n, ctx->stream));
     }
-    if (bt.par && !f.dir) {
+    if (bt.par && (!f.dir || f.dir_fs < (size_t) bt.nb * bt.j_pitch)) {   // (delta_x > 1 has more, shorter blocks)
+        cudaFree(f.dir);
+        f.dir = nullptr;
         f.dir_fs = (size_t) bt.nb * bt.j_pitch;
         CK(ctx, cudaMalloc((void**) &f.dir, f.dir_fs * n));
     }
@@ -1523,11 +1899,13 @@ static int frames_loop_buffers(dctc_context* ctx, CarverFrames& f, const BtPlan&
 }
 
 // What the caller of a seam operation brings besides the session: whether its seam loops record the visibility maps, the
-// rigidity (dctc_carver_set_rigidity, dctc_carver_batch_set_rigidity) and the context's incremental cumulative map
-// (dctc_carver_set_incremental), which only the single session has.
+// rigidity (dctc_carver_set_rigidity, dctc_carver_batch_set_rigidity), the seam step width (dctc_carver_set_delta_x,
+// dctc_carver_batch_set_delta_x) and the context's incremental cumulative map (dctc_carver_set_incremental), which only
+// the single session has.
 struct SeamCall {
     bool vmaps = false;
     float rigidity = 0.0f;
+    int delta_x = 1;
     bool incremental = false;
     bool* m_valid = nullptr;   // &ctx->c_m_valid (single session), null for a batch
 };
@@ -1541,26 +1919,34 @@ struct SeamCall {
 // walk gave up, and the carve also compacts f.m.  A loop that does not keep the map up to date clears *c.m_valid.
 // c.rigidity: the seams are f.h rows long (the image width at the axis switch for height operations), so every kernel of
 // the loop gets pen = fl(rigidity / f.h); pen == 0 launches the kernels of rigidity 0.
+// c.delta_x > 1: the WIDE seam DP, jump and trace kernels with the step table (DpSteps), the incremental walk is off (the
+// DP rebuilds the map every seam) and the band K1 covers a seam drift of delta_x per row.
 static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c)
 {
-    const int n = f.n, h = f.h;
+    const int n = f.n, h = f.h, dx = c.delta_x;
     const size_t log_fs = (size_t) n_seams * h, en_fs = f.en_pitch * h, m_fs = f.m_pitch * h;
     const float pen = c.rigidity / (float) h;
-    const bool rig = pen != 0.0f;
-    const BtPlan bt = bt_plan(h, f.m_pitch);
+    const bool rig = pen != 0.0f, wide = dx > 1;
+    DpSteps steps;
+    steps.dx = dx;
+    for (int d = 0; d <= DCTC_MAX_DELTA_X; d++)   // the host carver's rigidity_map_of, +inf beyond the step bound
+        steps.pen[d] = d > dx ? INFINITY : (c.rigidity * ((float) d * sqrtf((float) d))) / (float) h;
+    const BtPlan bt = bt_plan(h, f.m_pitch, dx);
     int rc = frames_loop_buffers(ctx, f, bt, log_fs);
     if (rc) return rc;
     DpPlan plan;
-    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, rig, plan));
+    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, rig, wide, plan));
     const auto jump = rig ? dctc_seam_jump_kernel<true> : dctc_seam_jump_kernel<false>;
     const auto trace = rig ? dctc_seam_trace_kernel<true> : dctc_seam_trace_kernel<false>;
     const auto incr_walk = rig ? dctc_seam_incr_kernel<true> : dctc_seam_incr_kernel<false>;
-    if (bt.par && bt.cone_smem > 40 * 1024)
+    if (bt.par && !wide && bt.cone_smem > 40 * 1024)
         CK(ctx, cudaFuncSetAttribute(trace, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+    if (bt.par && wide)   // the window's 34 KB of static shared memory plus the cone
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
     int* const xlast = bt.par ? f.xlast : nullptr;
     // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
     const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
-    const bool incr = c.incremental && n == 1 && incr_smem <= 160 * 1024;
+    const bool incr = c.incremental && n == 1 && !wide && incr_smem <= 160 * 1024;
     if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
         CK(ctx, cudaFuncSetAttribute(incr_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
         if (!ctx->c_band) {
@@ -1582,10 +1968,20 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         // build_mmap, one cluster per frame, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per
         // block and frame (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor
         // drains and blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
-        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, !walk, f.en, f.en_pitch, w_old,
-                                h, f.m, f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
-                                walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, pen));
-        if (bt.par && !walk) {
+        auto launch_dp = [&](auto fn, auto last) {
+            return dctc_launch_pdl(fn, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, !walk, f.en, f.en_pitch, w_old, h, f.m,
+                                   f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
+                                   walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, last);
+        };
+        CK(ctx, wide ? launch_dp(plan.dpw, steps) : launch_dp(plan.dp, pen));
+        if (bt.par && !walk && wide) {   // strips of 256 published columns, JBW-row blocks
+            const int js = (w_old + 255) / 256;
+            CK(ctx, dctc_launch_pdl(dctc_seam_jump_wide_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m,
+                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, js, m_fs, f.dir_fs, steps));
+            CK(ctx, dctc_launch_pdl(dctc_seam_trace_wide_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, true, f.m,
+                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, steps));
+            ctx->launches += 2;
+        } else if (bt.par && !walk) {
             const int js = (w_old + 63) / 64;
             CK(ctx, dctc_launch_pdl(jump, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m, f.m_pitch, w_old, h, f.dir,
                                     bt.j_pitch, js, m_fs, f.dir_fs, pen));
@@ -1615,7 +2011,7 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         DctcK1Args a = frames_k1_args(f, op, f.seam);
         a.pdl = 1;
         const DctcK1Bias bias{f.bias, (float) f.w0};   // biased frames: the band store writes the seam energy
-        rc = dctc_run_k1(ctx, op, a, n, ctx->stream, f.bias ? &bias : nullptr);
+        rc = dctc_run_k1(ctx, op, a, n, ctx->stream, f.bias ? &bias : nullptr, dx);
         if (rc) return rc;
 #ifdef DCTC_SYNC_DEBUG
         { cudaError_t e_ = cudaStreamSynchronize(ctx->stream); if (e_ != cudaSuccess) { printf("seam %d: band kernel failed: %s (w %d)\n", s, cudaGetErrorString(e_), w_old); return dctc_fail_cuda(ctx, e_); } }
@@ -1718,6 +2114,7 @@ struct dctc_carver_batch {
     uint8_t* lv_scratch = nullptr;      // height levels in the transposed orientation on their way out (session_render)
     size_t lv_scratch_bytes = 0;
     float rigidity = 0.0f;              // dctc_carver_batch_set_rigidity (the single session takes the context's instead)
+    int delta_x = 1;                    // dctc_carver_batch_set_delta_x (likewise)
 };
 
 namespace {
@@ -2132,6 +2529,7 @@ static int carver_call(dctc_context* ctx, Op&& op)
     SeamCall c;
     c.vmaps = ctx->c_dump_vmaps;
     c.rigidity = ctx->c_rigidity;
+    c.delta_x = ctx->c_delta_x;
     c.incremental = ctx->c_incremental;
     c.m_valid = &ctx->c_m_valid;
     const int rc = op(b, c);
@@ -2151,8 +2549,8 @@ static int carver_load_impl(dctc_context* ctx, const uint8_t* img, int w, int h,
 {
     const int rc = session_create(ctx, 1, w, h, channels, false, false, &ctx->carver);
     if (rc) return rc;
-    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * 32));
-    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * 32 + sizeof(int) * h));
+    CK(ctx, cudaMalloc((void**) &ctx->c_band_vals, sizeof(float) * (size_t) h * DCTC_BAND_ROW));
+    CK(ctx, cudaMallocHost((void**) &ctx->h_band, sizeof(float) * (size_t) h * DCTC_BAND_ROW + sizeof(int) * h));
     return session_load(ctx->carver, img, 0, pitch);
 }
 
@@ -2243,12 +2641,12 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     if (f->w <= 1) return DCTC_ERR_STATE;
     if (f->bias) return DCTC_ERR_STATE;   // the caller's seam and the operator's band values: no place for a bias
     const DctcK1Op op = carver_op(ctx->op);
-    const int h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 4 * r;
-    int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * 32);
+    const int dx = ctx->c_delta_x, h = f->h, w_old = f->w, r = op.blocksize / 2, bs = 2 * r * (dx + 1);
+    int* h_seam = (int*) ((char*) ctx->h_band + sizeof(float) * (size_t) h * DCTC_BAND_ROW);
     for (int y = 0; y < h; y++) {
         if (seam_x[y] < 0 || seam_x[y] >= w_old) return DCTC_ERR_STATE;
-        // connected seams only (delta_x = 1, src/render.c:313): the band width 4*(b/2) and the band tiles rely on it
-        if (y > 0 && (seam_x[y] - seam_x[y - 1] > 1 || seam_x[y - 1] - seam_x[y] > 1)) return DCTC_ERR_INVALID;
+        // steps of at most delta_x (1 in the plug-in, src/render.c:313): the band width 2r(dx+1) and the band tiles rely on it
+        if (y > 0 && (seam_x[y] - seam_x[y - 1] > dx || seam_x[y - 1] - seam_x[y] > dx)) return DCTC_ERR_INVALID;
         h_seam[y] = seam_x[y];
     }
     s->axis = DCTC_AXIS_WIDTH;
@@ -2263,7 +2661,8 @@ int dctc_carve_and_update(dctc_context* ctx, const int* seam_x, float* band_out,
     ctx->c_m_valid = false;     // the host picked this seam: the device's cumulative plane no longer matches
     DctcK1Args a = frames_k1_args(*f, op, f->seam);
     a.band_vals = ctx->c_band_vals;
-    int rc = dctc_run_k1(ctx, op, a, 1, ctx->stream);
+    a.band_stride = bs;
+    int rc = dctc_run_k1(ctx, op, a, 1, ctx->stream, nullptr, dx);
     if (rc) return rc;
     if (band_out) {
         CK(ctx, cudaMemcpyAsync(ctx->h_band, ctx->c_band_vals, sizeof(float) * (size_t) h * bs, cudaMemcpyDeviceToHost,
@@ -2345,6 +2744,17 @@ int dctc_carver_set_rigidity(dctc_context* ctx, float rigidity)
     if (rigidity != ctx->c_rigidity) {
         ctx->c_rigidity = rigidity;
         ctx->c_m_valid = false;   // the incremental map was built with the old pen
+    }
+    return DCTC_OK;
+}
+
+int dctc_carver_set_delta_x(dctc_context* ctx, int delta_x)
+{
+    if (!ctx || delta_x < 1) return DCTC_ERR_INVALID;
+    if (delta_x > DCTC_MAX_DELTA_X) return DCTC_ERR_UNSUPPORTED;
+    if (delta_x != ctx->c_delta_x) {
+        ctx->c_delta_x = delta_x;
+        ctx->c_m_valid = false;   // the incremental map was built for the old step width
     }
     return DCTC_OK;
 }
@@ -2438,6 +2848,7 @@ static SeamCall batch_call(const dctc_carver_batch* b)
 {
     SeamCall c;
     c.rigidity = b->rigidity;
+    c.delta_x = b->delta_x;
     return c;
 }
 
@@ -2496,6 +2907,14 @@ int dctc_carver_batch_set_rigidity(dctc_carver_batch* b, float rigidity)
 {
     if (!b || !(rigidity >= 0.0f) || !std::isfinite(rigidity)) return DCTC_ERR_INVALID;
     b->rigidity = rigidity;
+    return DCTC_OK;
+}
+
+int dctc_carver_batch_set_delta_x(dctc_carver_batch* b, int delta_x)
+{
+    if (!b || delta_x < 1) return DCTC_ERR_INVALID;
+    if (delta_x > DCTC_MAX_DELTA_X) return DCTC_ERR_UNSUPPORTED;
+    b->delta_x = delta_x;
     return DCTC_OK;
 }
 

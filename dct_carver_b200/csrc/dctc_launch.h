@@ -79,9 +79,10 @@ static inline cudaError_t dctc_launch_pdl(void (*kern)(KArgs...), dim3 grid, dim
     return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
 }
 
-// bias (band mode only, may be null): the band store of a biased carver session
+// bias (band mode only, may be null): the band store of a biased carver session.  delta_x (band mode only): the seam's
+// largest step between two rows, which sets how many columns a tile row of the band can span.
 cudaError_t dctc_launch_k1_tile(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, cudaStream_t stream,
-                                const DctcK1Bias* bias = nullptr);
+                                const DctcK1Bias* bias = nullptr, int delta_x = 1);
 cudaError_t dctc_launch_k1_small(const DctcK1Args& a, int blocksize, int n_frames, bool uniform, int sm_count, cudaStream_t stream);
 cudaError_t dctc_launch_k1_march8(const DctcK1Args& a, int n_frames, bool uniform, cudaStream_t stream);
 cudaError_t dctc_launch_k1_tc8(const DctcK1Args& a, int n_frames, bool uniform, int* counter, int sm_count, cudaStream_t stream);
@@ -95,6 +96,8 @@ cudaError_t dctc_launch_transpose(const void* src, size_t src_pitch, size_t src_
 
 constexpr int DCTC_SLOTS = 4;   // device staging slots of the host-buffer batch call (H2D, kernel and D2H of different frames overlap)
 constexpr int DCTC_TC_COUNTERS = 64;
+// Floats per row of dctc_carve_and_update's band buffers: the widest band, 2 r (delta_x + 1) with r = 16 / 2
+constexpr int DCTC_BAND_ROW = 2 * 8 * (DCTC_MAX_DELTA_X + 1);
 
 // The energy operator and the K1 kernel selection of a K1 launch (dctc_run_k1)
 struct DctcK1Op {
@@ -164,9 +167,10 @@ struct dctc_context {
     bool c_incremental = false;    // device seam loop: update the cumulative map incrementally (dctc_carver_set_incremental)
     bool c_m_valid = false;        // the cumulative plane holds the map of the image before the last removal, compacted over that seam
     float c_rigidity = 0.0f;       // rigidity of the single session's seam loops (dctc_carver_set_rigidity); survives loads
+    int c_delta_x = 1;             // seam step width of the single session's seam loops (dctc_carver_set_delta_x); survives loads
     float* c_band_vals = nullptr;  // packed band values of dctc_carve_and_update
     float* h_mirror = nullptr;     // host mirror of the energy map for dctc_pixel_energy (pinned, allocated by its first use)
-    int* h_band = nullptr;         // pinned: band values and seam of dctc_carve_and_update
+    int* h_band = nullptr;         // pinned: band values (DCTC_BAND_ROW floats per row) and seam of dctc_carve_and_update
     bool mirror_valid = false;
     // K3 energy-image export
     unsigned int* k3_lohi = nullptr;   // device (min, max) of the compressed energies, as float bit patterns
@@ -176,9 +180,9 @@ struct dctc_context {
 
 int dctc_fail_cuda(dctc_context* ctx, cudaError_t e);
 // Launches the one K1 kernel dctc_k1_select picks (dctc_k1_select.h); bias: band mode of a biased carver session (the
-// tile kernel's bias store)
+// tile kernel's bias store); delta_x: band mode, the seam's largest step (dctc_launch_k1_tile)
 int dctc_run_k1(dctc_context* ctx, const DctcK1Op& op, DctcK1Args& a, int n_frames, cudaStream_t stream,
-                const DctcK1Bias* bias = nullptr);
+                const DctcK1Bias* bias = nullptr, int delta_x = 1);
 // The layout the Small, Tc8 and Tc16 kernels (and the 1/3-channel variants of the march kernel) read: 1 or 3 channels,
 // image rows, frames and halo rows 16-byte aligned
 bool dctc_k1_fast_layout(const DctcK1Args& a);

@@ -219,7 +219,7 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     if (k <= 0) return DCTC_LQR_OK;
     if (k >= r->w) return DCTC_LQR_ERROR;
     if (!r->gpu && !r->nrg) return DCTC_LQR_ERROR;
-    if (r->gpu && g_device_seam_loop && r->delta_x == 1) {
+    if (r->gpu && g_device_seam_loop && dx >= 1 && dx <= DCTC_MAX_DELTA_X) {
         /* the whole lqr_carver_resize loop on the device: energy, seam DP, back-track, carve, band update */
         int drc, *dseams;
         t0 = now_s();
@@ -231,7 +231,8 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
             r->seams = ns; r->seams_cap = r->n_seams + k;
         }
         dseams = r->seams + (size_t) r->n_seams * h;
-        if (dctc_carver_set_rigidity(r->gpu, r->rigidity) != DCTC_OK) return DCTC_LQR_ERROR;
+        if (dctc_carver_set_rigidity(r->gpu, r->rigidity) != DCTC_OK || dctc_carver_set_delta_x(r->gpu, dx) != DCTC_OK)
+            return DCTC_LQR_ERROR;
         if (dctc_carver_load(r->gpu, r->rgb, r->w, h, ch, (size_t) P * ch) != DCTC_OK) return DCTC_LQR_ERROR;
         r->timing[0] += now_s() - t0;
         t0 = now_s();
@@ -264,7 +265,8 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     seam = (int *) malloc(sizeof(int) * h);
     xmin = (int *) malloc(sizeof(int) * h);
     xmax = (int *) malloc(sizeof(int) * h);
-    band = (float *) malloc(sizeof(float) * (size_t) h * (4 * (r->radius > 0 ? r->radius : 1) + 2));
+    /* dctc_carve_and_update's band: at most 2 r (delta_x + 1) values per row */
+    band = (float *) malloc(sizeof(float) * (size_t) h * (2 * (r->radius > 0 ? r->radius : 1) * (dx + 1) + 2));
     if (!r->gpu) luma = (double *) malloc(sizeof(double) * (size_t) P * h);
     rig = rigidity_map_of(r->rigidity, dx, h, &rig_nomem);
     if (!en || !m || !raw || !seam || !xmin || !xmax || !band || (!r->gpu && !luma) || rig_nomem) goto done;
@@ -290,7 +292,9 @@ static int carve_vertical(DctcLqrCarver *r, int k, int record_vs)
     if (r->gpu) {
         float *tmp = (float *) malloc(sizeof(float) * (size_t) r->w * h);
         if (!tmp) { rc = DCTC_LQR_NOMEM; goto done; }
-        if (dctc_carver_load(r->gpu, r->rgb, r->w, h, ch, (size_t) P * ch) != DCTC_OK ||
+        /* dctc_carve_and_update takes steps up to the context's delta_x (1 above the device's bound: as before it existed) */
+        if (dctc_carver_set_delta_x(r->gpu, dx >= 1 && dx <= DCTC_MAX_DELTA_X ? dx : 1) != DCTC_OK ||
+            dctc_carver_load(r->gpu, r->rgb, r->w, h, ch, (size_t) P * ch) != DCTC_OK ||
             dctc_carver_energy(r->gpu, tmp) != DCTC_OK) { free(tmp); goto done; }
         for (y = 0; y < h; y++) memcpy(en + (size_t) y * P, tmp + (size_t) y * r->w, sizeof(float) * r->w);
         free(tmp);
@@ -432,7 +436,7 @@ static int enlarge_vertical(DctcLqrCarver *r, int k, int record_vs)
     orig = (uint8_t *) malloc((size_t) w0 * h * ch);
     if (!orig) return DCTC_LQR_NOMEM;
     for (y = 0; y < h; y++) memcpy(orig + (size_t) y * w0 * ch, r->rgb + (size_t) y * r->pitch * ch, (size_t) w0 * ch);
-    if (r->gpu && g_device_seam_loop && r->delta_x == 1) {
+    if (r->gpu && g_device_seam_loop && r->delta_x >= 1 && r->delta_x <= DCTC_MAX_DELTA_X) {
         /* seams, visibility map and the pixel synthesis on the device */
         int *ns;
         if (r->seam_len != h) { r->n_seams = 0; r->seam_len = h; }
@@ -440,6 +444,7 @@ static int enlarge_vertical(DctcLqrCarver *r, int k, int record_vs)
         if (!ns) { free(orig); return DCTC_LQR_NOMEM; }
         r->seams = ns; r->seams_cap = r->n_seams + k;
         rc = dctc_carver_set_rigidity(r->gpu, r->rigidity);
+        if (rc == DCTC_OK) rc = dctc_carver_set_delta_x(r->gpu, r->delta_x);
         if (rc == DCTC_OK) rc = dctc_carver_load(r->gpu, orig, w0, h, ch, (size_t) w0 * ch);
         if (rc == DCTC_OK) rc = dctc_carver_enlarge_width(r->gpu, k, r->seams + (size_t) r->n_seams * h);
         if (rc == DCTC_OK) {

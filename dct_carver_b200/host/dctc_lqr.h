@@ -99,8 +99,11 @@ typedef struct DctcRenderResult_ {
 int dctc_render(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, dctc_context *gpu,
                 DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res);
 /* dctc_render with lqr_carver_init(carver, delta_x, rigidity): a seam step of |d| <= delta_x columns costs
- * fl(fl(rigidity * |d|^1.5) / h) more, h the seam length.  With a GPU attached, delta_x = 1 runs the device seam loop
- * (the context's dctc_carver_set_rigidity is set to rigidity before each load); other delta_x run the host loop.
+ * fl(fl(rigidity * |d|^1.5) / h) more, h the seam length.  With a GPU attached, delta_x 1 .. DCTC_MAX_DELTA_X runs the
+ * device seam loop (the context's dctc_carver_set_rigidity and dctc_carver_set_delta_x are set before each load); larger
+ * delta_x run the host loop, whose band updates (dctc_carve_and_update) then refuse steps wider than 1.  Both context
+ * options keep the render's values after it returns (delta_x 1 above DCTC_MAX_DELTA_X): a caller that shares the context
+ * and relies on other values sets them again.
  * DCTC_ERR_INVALID also for delta_x < 1 and a negative or non-finite rigidity. */
 int dctc_render_ext(const uint8_t *img, int w, int h, int channels, const DctcPlugInVals *vals, int delta_x, float rigidity,
                     dctc_context *gpu, DctcLqrEnergyFunc cb, void *cb_extra, DctcRenderResult *res);

@@ -148,17 +148,20 @@ int dctc_carver_energy(dctc_context *ctx, float *out);
  * energy planes and recomputes the energy only in the band the seam touched:
  *   row y: x in [min_{|y'-y|<=r} seam_x[y'] - r, max_{|y'-y|<=r} seam_x[y'] + r - 1] clipped to [0, w-2].
  * On return *xmin / *xmax (h entries each, may be NULL) hold that band and band_out (may be NULL) receives, row
- * by row, the xmax[y]-xmin[y]+1 recomputed values packed back to back (at most 4*(blocksize/2) per row: band_out needs
- * room for h*4*(blocksize/2) floats).  The seam must be connected, |seam_x[y]-seam_x[y-1]| <= 1, as liblqr's are with
- * delta_x = 1 (src/render.c:313); anything else returns DCTC_ERR_INVALID, a column outside [0, w) DCTC_ERR_STATE.
+ * by row, the xmax[y]-xmin[y]+1 recomputed values packed back to back (at most 2*(blocksize/2)*(delta_x+1) per row,
+ * delta_x the context's dctc_carver_set_delta_x: band_out needs room for h*2*(blocksize/2)*(delta_x+1) floats, which
+ * is h*4*(blocksize/2) for the default delta_x = 1).  A seam step must stay within the context's delta_x,
+ * |seam_x[y]-seam_x[y-1]| <= delta_x, as liblqr's are (1 in the plug-in, src/render.c:313); anything else returns
+ * DCTC_ERR_INVALID, a column outside [0, w) DCTC_ERR_STATE.
  * A vertical-seam call: DCTC_ERR_STATE after a height call since the load. */
 int dctc_carve_and_update(dctc_context *ctx, const int *seam_x, float *band_out, int *xmin, int *xmax);
 /* Copies the current (carved) interleaved image back to the host, pitch = w*channels. */
 int dctc_carver_image(dctc_context *ctx, uint8_t *out);
 /* Whole retarget loop on the device (energy -> seam DP -> back-track -> carve -> band update), `n_seams`
  * vertical seams; seams_out (may be NULL) receives n_seams*h removed columns in the coordinates of the image
- * at the time of removal.  Mirrors lqr_carver_resize(carver, w - n_seams, h) (src/render.c:377) with
- * delta_x = 1 and the rigidity of dctc_carver_set_rigidity (0, the plug-in's value, src/render.c:313, by default). */
+ * at the time of removal.  Mirrors lqr_carver_resize(carver, w - n_seams, h) (src/render.c:377) with the delta_x of
+ * dctc_carver_set_delta_x and the rigidity of dctc_carver_set_rigidity (1 and 0, the plug-in's values,
+ * src/render.c:313, by default). */
 int dctc_carver_resize_width(dctc_context *ctx, int n_seams, int *seams_out);
 /* Enlarging: lqr_carver_resize(carver, w + n_seams, h) as the plug-in calls it for seams_number > 0
  * (src/render.c:357-363,377).  The n_seams seams a shrink would remove are computed on a freshly loaded session (same
@@ -290,6 +293,23 @@ int dctc_carver_bias(dctc_context *ctx, float *out);
  * it).  DCTC_ERR_INVALID: a negative or non-finite value. */
 int dctc_carver_set_rigidity(dctc_context *ctx, float rigidity);
 
+/* ---- seam step width (liblqr's lqr_carver_init(carver, delta_x, rigidity)) ----------------------------------
+ * delta_x = dx, 1 .. DCTC_MAX_DELTA_X: a seam may move up to dx columns from one row to the next.  Every seam loop of the
+ * session (the same list as for the rigidity) runs on
+ *     pen[0] = 0,  pen[d] = fl(fl(rigidity * fl(d * fl(sqrt(d)))) / h)    d = 1 .. dx   (pen[1] is the rigidity's pen)
+ *     m[y][x] = fl(E[y][x] + min over |d| <= dx of fl(m[y-1][x+d] + pen[|d|]))    (+inf outside the frame)
+ * with the parent = the FIRST strict minimum scanning x-dx .. x+dx and the seam end the leftmost minimum of the last row
+ * (liblqr's build_mmap with its rigidity_map [from memory: parity unpinned]).  delta_x = 1 (the default) is the plug-in's
+ * value and runs exactly the kernels and launches of a session that never set it.  delta_x > 1 launches per seam what
+ * delta_x = 1 launches, except for frames narrower than 261 columns or too tall for the parallel back-track's shared
+ * memory at that delta_x, which walk the seam back inside the seam DP kernel (two launches fewer per seam); incremental
+ * mode rebuilds the cumulative map for every seam (same seams: the incremental update is for delta_x = 1 only).  dctc_carve_and_update accepts steps up to delta_x.
+ * dctc_carver_set_delta_x: an option of the context like dctc_carver_set_rigidity; it survives loads and applies from the
+ * next seam loop, and a changed value drops the incremental map.  DCTC_ERR_INVALID: delta_x < 1.  DCTC_ERR_UNSUPPORTED:
+ * delta_x > DCTC_MAX_DELTA_X. */
+#define DCTC_MAX_DELTA_X 4
+int dctc_carver_set_delta_x(dctc_context *ctx, int delta_x);
+
 /* ---- visibility map and seam display ------------------------------------------------------------------------
  * lqr_carver_set_dump_vmaps (src/render.c:374): ask the session to record, for every ORIGINAL pixel, the order in
  * which dctc_carver_resize_width removed it (1-based, 0 = still visible).  Call before the first seam is removed. */
@@ -372,6 +392,9 @@ int dctc_carver_batch_bias(dctc_carver_batch *batch, float *out);
  * setting of the batch, 0 at create; it survives loads and applies from the next seam loop.  DCTC_ERR_INVALID: NULL
  * batch, a negative or non-finite value. */
 int dctc_carver_batch_set_rigidity(dctc_carver_batch *batch, float rigidity);
+/* dctc_carver_set_delta_x for the batch: a setting of the batch, 1 at create; it survives loads and applies from the
+ * next seam loop.  DCTC_ERR_INVALID: NULL batch, delta_x < 1.  DCTC_ERR_UNSUPPORTED: delta_x > DCTC_MAX_DELTA_X. */
+int dctc_carver_batch_set_delta_x(dctc_carver_batch *batch, int delta_x);
 /* current width / height of every frame */
 int dctc_carver_batch_width(const dctc_carver_batch *batch);
 int dctc_carver_batch_height(const dctc_carver_batch *batch);
