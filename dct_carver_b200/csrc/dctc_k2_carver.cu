@@ -107,10 +107,11 @@ __global__ void __launch_bounds__(NT) dctc_carve_rows_kernel(uint8_t* __restrict
 // and oracle/oracle_carver.c):
 //   m[0][x] = en[0][x];  m[y][x] = en[y][x] + min(m[y-1][x-1], m[y-1][x], m[y-1][x+1])   (FP32, range clipped)
 //   parent of (y, x) = FIRST strict minimum scanning x-1, x, x+1;  seam end = LEFTMOST minimum of the last row.
-// Rigidity (the RIG instantiations of the DP, jump, trace and incremental kernels): a diagonal step costs pen =
-// fl(rigidity / h) more, i.e. the candidates are fl(m[y-1][x-1] + pen), m[y-1][x], fl(m[y-1][x+1] + pen) in the map and
-// in the parent choice (liblqr's rigidity_map[1] = rigidity / h [from memory: parity unpinned]).  The host passes pen
-// as a trailing kernel argument; the false instantiations never read it and are the kernels of rigidity 0.
+// Rigidity (the DpStep1<true> instantiations of the DP, jump, trace and incremental kernels): a diagonal step costs
+// pen = fl(rigidity / h) more, i.e. the candidates are fl(m[y-1][x-1] + pen), m[y-1][x], fl(m[y-1][x+1] + pen) in the
+// map and in the parent choice (liblqr's rigidity_map[1] = rigidity / h [from memory: parity unpinned]).  The host
+// passes pen as the trailing kernel argument; DpStep1<false> never reads it and makes the kernels of rigidity 0.  Wider
+// steps (delta_x > 1) take the DpSteps rule below.
 // The map is rebuilt from scratch for every seam (same values as liblqr's incremental update_mmap).  Row y depends on
 // the whole row y-1: a chain of h steps.  Versions with one CTA-wide barrier per row cost ~600-950 clk per row
 // (shared-memory bandwidth, then the latency of a 16-warp barrier round); this one removes the per-row barrier with
@@ -161,105 +162,74 @@ __device__ __forceinline__ void dp_st_async_v4(uint32_t remote_addr, float4 v, u
 __device__ __forceinline__ void dp_st_cluster_f32(uint32_t ra, float v) { asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(ra), "f"(v) : "memory"); }
 __device__ __forceinline__ void dp_st_cluster_s32(uint32_t ra, int v) { asm volatile("st.shared::cluster.s32 [%0], %1;" ::"r"(ra), "r"(v) : "memory"); }
 
-// ---- back-track (build_vpath) ------------------------------------------------------------------------------------
-// One warp walks up from the last row: parent of (y, x) = FIRST strict minimum of m[y-1][x-1], m[y-1][x], m[y-1][x+1].
-// Every lane follows the same path, lane 0 records it.  The cumulative rows are read in batches of 32 rows through
-// shared-memory windows of DP_WIN columns, double buffered: the path moves at most one column per row, so the window
-// of the NEXT batch (columns xs-66 .. xs+66 around the column xs at which the current batch starts) is known before
-// the current batch is walked, and its cp.async copies land while the walk (a chain of dependent shared-memory reads)
-// is running.
-constexpr int DP_WIN = 144;       // back-track window (floats); the cumulative plane's pitch is at least this
-constexpr int DP_WINP = DP_WIN + 8;   // window row in shared memory: 3 pad floats, the left sentinel, DP_WIN columns, the right
-                                      // sentinel (needed when the window ends exactly at column w) and 3 pad floats
-
-template <bool RIG>
-__device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, size_t m_pitch, int w, int h, int x,
-                                             int* __restrict__ seam, int* __restrict__ seam_log,
-                                             float (*win)[32][DP_WINP], int lane, float pen)
-{
-    const float INF = __int_as_float(0x7f800000);
-    if (lane == 0) { seam[h - 1] = x; if (seam_log) seam_log[h - 1] = x; }
-    const int max_base = (int) m_pitch - DP_WIN;
-    // window rows of the batch that starts below image row ytop: window row i = image row ytop-1-i, column c of the
-    // plane at win[buf][i][4 + c - base]
-    auto stage = [&](int ytop, int xs, int buf) -> int {
-        int base = (xs - 66) & ~3;
-        base = base < 0 ? 0 : (base > max_base ? max_base : base);
-        if (ytop >= 1) {
-            for (int idx = lane; idx < 32 * (DP_WIN / 4); idx += 32) {
-                const int i = idx / (DP_WIN / 4), c = idx - i * (DP_WIN / 4);
-                const int yy = ytop - 1 - i;
-                if (yy >= 0) {
-                    const float* src = mplane + (size_t) yy * m_pitch + base + 4 * c;
-                    asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t) __cvta_generic_to_shared(&win[buf][i][4 + 4 * c])), "l"(src) : "memory");
-                }
-            }
-        }
-        asm volatile("cp.async.commit_group;" ::: "memory");
-        return base;
-    };
-    int buf = 0;
-    int base = stage(h - 1, x, 0);
-    for (int ytop = h - 1; ytop >= 1; ytop -= 32) {
-        const int base_next = stage(ytop - 32, x, buf ^ 1);     // lands while this batch is walked
-        asm volatile("cp.async.wait_group 1;" ::: "memory");
-        __syncwarp();
-        // +inf sentinels left of column 0 and at column w (range clipping), so that the walk needs no bounds checks
-        if (base == 0) win[buf][lane][3] = INF;
-        if (w - base >= 0 && w - base <= DP_WIN) win[buf][lane][4 + w - base] = INF;   // <=: w == base + DP_WIN lands in the row's tail pad
-        __syncwarp();
-        const int steps = ytop < 32 ? ytop : 32;
-        // the walk: three shared-memory reads at immediate offsets, two compares, a few selects per row; lane i remembers
-        // the column of step i and the 32 columns are written with one coalesced store at the end of the batch
-        int mine = 0;
-        const float* wp = &win[buf][0][4] + (x - base);        // wp[0] = cumulative value at (window row, column x)
-        auto walk = [&](int i) {
-            const float a = RIG ? wp[-1] + pen : wp[-1], b = wp[0], c = RIG ? wp[1] + pen : wp[1];
-            const bool p1 = b < a;
-            const float best = p1 ? b : a;
-            const bool p2 = c < best;
-            const int d = p2 ? 1 : (p1 ? 0 : -1);
-            x += d;
-            wp += DP_WINP + d;
-            if (lane == i) mine = x;
-        };
-        if (steps == 32) {
-#pragma unroll
-            for (int i = 0; i < 32; i++) walk(i);
-        } else {
-            for (int i = 0; i < steps; i++) walk(i);
-        }
-        if (lane < steps) { seam[ytop - 1 - lane] = mine; if (seam_log) seam_log[ytop - 1 - lane] = mine; }
-        __syncwarp();
-        base = base_next;
-        buf ^= 1;
-    }
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-}
-
-// ---- seam step width (liblqr's delta_x) ----------------------------------------------------------------------------
+// ---- seam step rules ------------------------------------------------------------------------------------------------
 // With delta_x = dx in 2 .. DCTC_MAX_DELTA_X a seam may move up to dx columns from one row to the next:
 //   m[y][x] = en[y][x] + min_{|d| <= dx} fl(m[y-1][x+d] + pen[|d|]),   parent = FIRST strict minimum scanning x-dx .. x+dx,
 // pen[0] = 0, pen[d] = fl(fl(rigidity * fl(d * fl(sqrt(d)))) / h) (liblqr's rigidity_map [from memory: parity unpinned]).
-// The WIDE instantiations of the seam DP and the wide serial walk take the table with pen[d] = +inf for dx < d <= 4, so
-// one kernel serves every dx: a candidate beyond the step bound costs +inf and never wins (the d = 0 candidate is finite).
+// Every seam-search kernel takes its step rule as a template parameter, and the rule's Arg as its trailing argument (a
+// float for DpStep1, so that the dx = 1 kernels keep the parameter a plain float has; the table for DpSteps); the kernel
+// rebuilds the rule from it.  A rule has D, the largest step it can take at compile time, dx, its step width, and
+// pick(v, q): q(d) of the parent, the first strict minimum of the candidates d = -D .. D, where v(d) is the cumulative
+// value at column x+d of the row above (+inf outside the image).  The serial walk, the jump and the trace kernels all
+// choose the parent through pick; the seam DP needs only the minimum and forms it in its own row arithmetic.
+template <bool RIG>
+struct DpStep1 {                  // dx = 1; RIG: rigidity pen on the two diagonal candidates, else pen is never read
+    using Arg = float;            // the kernel argument: pen
+    static constexpr int D = 1, dx = 1;
+    float pen;
+    __device__ __forceinline__ float diag(float v) const { return RIG ? v + pen : v; }   // a diagonal candidate's cost
+    template <typename V, typename Q>
+    __device__ __forceinline__ auto pick(V v, Q q) const
+    {
+        const float a = diag(v(-1)), b = v(0), c = diag(v(1));
+        const bool p1 = b < a;
+        const float best = p1 ? b : a;
+        const bool p2 = c < best;
+        return p2 ? q(1) : (p1 ? q(0) : q(-1));
+    }
+};
+// dx = 2 .. DCTC_MAX_DELTA_X at run time: pen[d] = +inf for dx < d <= D, so one kernel serves every dx: a candidate
+// beyond the step bound costs +inf and never wins (best starts at +inf and the d = 0 candidate is finite).
 struct DpSteps {
-    float pen[DCTC_MAX_DELTA_X + 1];
+    using Arg = DpSteps;
+    static constexpr int D = DCTC_MAX_DELTA_X;
+    float pen[D + 1];
     int dx;
+    template <typename V, typename Q>
+    __device__ __forceinline__ auto pick(V v, Q q) const
+    {
+        float best = __int_as_float(0x7f800000);
+        auto qb = q(0);
+#pragma unroll
+        for (int d = -D; d <= D; d++) {
+            const float c = d == 0 ? v(0) : v(d) + pen[d < 0 ? -d : d];
+            if (c < best) { best = c; qb = q(d); }
+        }
+        return qb;
+    }
 };
 
-// dp_backtrack for dx > 1: the same double-buffered windows, but batches of wb rows with 2 * wb * dx + dx <= 66, so that
-// the next batch's window (staged around the column the current batch starts at) still holds every candidate it reads.
-// The four floats left of the window hold the +inf sentinels of column 0, and the four columns from w on those of the
-// right edge.  best starts at +inf, so a candidate that is not a real one (+inf pen) never wins.
-__device__ __forceinline__ void dp_backtrack_wide(const float* __restrict__ mplane, size_t m_pitch, int w, int h, int x,
-                                                  int* __restrict__ seam, int* __restrict__ seam_log,
-                                                  float (*win)[32][DP_WINP], int lane, const DpSteps& st)
+// ---- back-track (build_vpath) ------------------------------------------------------------------------------------
+// One warp walks up from the last row: parent of (y, x) = the step rule's pick.  Every lane follows the same path,
+// lane 0 records it.  The cumulative rows are read in batches of wb rows through shared-memory windows of DP_WIN
+// columns, double buffered: with 2 wb dx + dx <= 66 (wb = 32 for dx = 1) the window of the NEXT batch (columns
+// xs-66 .. xs+66 around the column xs at which the current batch starts) is known before the current batch is walked,
+// and its cp.async copies land while the walk (a chain of dependent shared-memory reads) is running.
+constexpr int DP_WIN = 144;       // back-track window (floats); the cumulative plane's pitch is at least this
+constexpr int DP_WINP = DP_WIN + 8;   // window row in shared memory: 4 - D pad floats, D left sentinels, DP_WIN columns,
+                                      // D right sentinels (needed when the window ends at column w) and 4 - D pad floats
+
+template <typename Step>
+__device__ __forceinline__ void dp_backtrack(const float* __restrict__ mplane, size_t m_pitch, int w, int h, int x,
+                                             int* __restrict__ seam, int* __restrict__ seam_log,
+                                             float (*win)[32][DP_WINP], int lane, const Step& st)
 {
     const float INF = __int_as_float(0x7f800000);
     const int wb = (66 - st.dx) / (2 * st.dx);
     if (lane == 0) { seam[h - 1] = x; if (seam_log) seam_log[h - 1] = x; }
     const int max_base = (int) m_pitch - DP_WIN;
+    // window rows of the batch that starts below image row ytop: window row i = image row ytop-1-i, column c of the
+    // plane at win[buf][i][4 + c - base]
     auto stage = [&](int ytop, int xs, int buf) -> int {
         int base = (xs - 66) & ~3;
         base = base < 0 ? 0 : (base > max_base ? max_base : base);
@@ -279,30 +249,33 @@ __device__ __forceinline__ void dp_backtrack_wide(const float* __restrict__ mpla
     int buf = 0;
     int base = stage(h - 1, x, 0);
     for (int ytop = h - 1; ytop >= 1; ytop -= wb) {
-        const int base_next = stage(ytop - wb, x, buf ^ 1);
+        const int base_next = stage(ytop - wb, x, buf ^ 1);     // lands while this batch is walked
         asm volatile("cp.async.wait_group 1;" ::: "memory");
         __syncwarp();
+        // D +inf sentinels left of column 0 and from column w on (range clipping), so that the walk needs no bounds checks
         if (lane < wb) {
             if (base == 0)
-                for (int j = 0; j < 4; j++) win[buf][lane][j] = INF;
-            if (w - base >= 0 && w - base <= DP_WIN)
-                for (int j = 0; j < 4; j++) win[buf][lane][4 + w - base + j] = INF;
+                for (int j = 0; j < Step::D; j++) win[buf][lane][4 - Step::D + j] = INF;
+            if (w - base >= 0 && w - base <= DP_WIN)   // <=: w == base + DP_WIN lands in the row's tail pad
+                for (int j = 0; j < Step::D; j++) win[buf][lane][4 + w - base + j] = INF;
         }
         __syncwarp();
         const int steps = ytop < wb ? ytop : wb;
+        // the walk: a chain of shared-memory reads at immediate offsets and the pick per row; lane i remembers the column
+        // of step i and the batch's columns are written with one coalesced store at its end
         int mine = 0;
-        const float* wp = &win[buf][0][4] + (x - base);
-        for (int i = 0; i < steps; i++) {
-            float best = INF;
-            int dbest = 0;
-#pragma unroll
-            for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
-                const float v = d == 0 ? wp[0] : wp[d] + st.pen[d < 0 ? -d : d];
-                if (v < best) { best = v; dbest = d; }
-            }
-            x += dbest;
-            wp += DP_WINP + dbest;
+        const float* wp = &win[buf][0][4] + (x - base);        // wp[0] = cumulative value at (window row, column x)
+        auto walk = [&](int i) {
+            const int d = st.pick([&](int c) { return wp[c]; }, [](int c) { return c; });
+            x += d;
+            wp += DP_WINP + d;
             if (lane == i) mine = x;
+        };
+        if (Step::D == 1 && steps == 32) {
+#pragma unroll
+            for (int i = 0; i < 32; i++) walk(i);
+        } else {
+            for (int i = 0; i < steps; i++) walk(i);
         }
         if (lane < steps) { seam[ytop - 1 - lane] = mine; if (seam_log) seam_log[ytop - 1 - lane] = mine; }
         __syncwarp();
@@ -353,21 +326,21 @@ __device__ __forceinline__ void dp_unroll(F&& f)
 // One cluster per frame: blockIdx.y = frame of a batch session, whose energy / cumulative planes start en_fs / m_fs
 // floats after the previous frame's, whose seam is seam[h * frame ...], its log seam_log[log_fs * frame ...] and its
 // last-row column xlast[frame].  The tensor map is 3-D (columns, rows, frames) with a box depth of one frame.
-// RIG: rigidity pen (see above), the trailing argument.
-// WIDE (seam step width, see DpSteps): the trailing argument is the step table instead, every cell takes the minimum over
-// the 2 * 4 + 1 candidates of the table, and the warps exchange halos every DP_R / dx rows instead of every DP_R (a strip's
-// edge then contaminates dx columns per row, still at most DP_R after a block).  With at least 4 cells per lane every
-// candidate comes from the lane or its two neighbours.  No incremental map (run_flag is null); without xlast warp 0 of
-// CTA 0 walks back with dp_backtrack_wide, with it the wide jump and trace kernels follow.  RIG is false.
-template <int DP_P, int DP_SR, bool RIG, bool WIDE>
+// Step: the step rule (see DpStep1, DpSteps), the trailing argument.  Every cell takes the minimum over the rule's
+// candidates.  A DpSteps strip exchanges halos every DP_R / dx rows instead of every DP_R (its edge contaminates dx
+// columns per row, still at most DP_R after a block); with at least 4 cells per lane every candidate comes from the lane
+// or its two neighbours.  The incremental map (run_flag) is DpStep1 only.  Without xlast warp 0 of CTA 0 walks the seam
+// back itself (dp_backtrack), with it the jump and trace kernels follow.
+template <int DP_P, int DP_SR, typename Step>
 __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dctc_seam_dp_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                                     float* __restrict__ mplane, size_t m_pitch,
                                                                     int* __restrict__ seam, int* __restrict__ seam_log,
                                                                     int* __restrict__ run_flag, int nst,
                                                                     const __grid_constant__ CUtensorMap tmap,
                                                                     int* __restrict__ xlast, size_t en_fs, size_t m_fs, size_t log_fs,
-                                                                    std::conditional_t<WIDE, DpSteps, float> pen)
+                                                                    typename Step::Arg arg)
 {
+    const Step st{arg};
     DCTC_PDL_PROLOGUE();
     // (the frame's seam, log and xlast offsets are applied after the row loop, so they occupy no registers in it)
     en += blockIdx.y * en_fs;
@@ -523,7 +496,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
                 asm volatile("ld.shared.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(e[0][g].x), "=f"(e[0][g].y), "=f"(e[0][g].z), "=f"(e[0][g].w)
                              : "r"(stg_s + (uint32_t) (((kk % SRD) * STRIP + 4 * g) * 4)));   // base register + immediate
         }
-        if constexpr (WIDE) {
+        if constexpr (Step::D > 1) {
             // the 4 cells on each side of the lane's cells (neighbour lanes; +inf beyond the strip), then per cell the
             // minimum of cur and fl(neighbour + pen[|d|]) over d = -4 .. 4 (min is exact: the order does not matter)
             constexpr int CW = 4 * DP_P;
@@ -545,7 +518,7 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             for (int i = 0; i < CW; i++) mn[i] = c[4 + i];
 #pragma unroll
             for (int d = 1; d <= 4; d++) {
-                const float pd = pen.pen[d];
+                const float pd = st.pen[d];
                 float qd[CW + 8];
 #pragma unroll
                 for (int i = 4 - d; i < CW + 4 + d; i++) qd[i] = c[i] + pd;
@@ -571,11 +544,11 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
             }
             mptr += m_pitch;
         } else {
-        // q: the previous row as a diagonal parent sees it (RIG: cur + pen, one add per cell; else cur itself)
+        // q: the previous row as a diagonal parent sees it (rigidity: cur + pen, one add per cell; else cur itself)
         float4 q[DP_P];
 #pragma unroll
         for (int g = 0; g < DP_P; g++)
-            q[g] = RIG ? make_float4(cur[g].x + pen, cur[g].y + pen, cur[g].z + pen, cur[g].w + pen) : cur[g];
+            q[g] = make_float4(st.diag(cur[g].x), st.diag(cur[g].y), st.diag(cur[g].z), st.diag(cur[g].w));
         // neighbours across lanes; the strip's outermost lanes see +inf (their cells are never published)
         float l = __shfl_up_sync(0xffffffffu, q[DP_P - 1].w, 1);
         float r = __shfl_down_sync(0xffffffffu, q[0].x, 1);
@@ -607,49 +580,78 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         mptr += m_pitch;
         }
     };
-    if constexpr (WIDE) {
-        // the halo exchange of the block loop below (as there), after every DP_R / dx rows counted from row 0 and never
-        // after the last row
-        auto exchange = [&]() {
-            const int wl = tid >> 5;                          // warp inside the CTA
-            float* halo = xrow + (wl * 2 + xb) * 64;          // [0,32): cells left of the published range, [32,64): right
-            const uint32_t my_bar = dp_smem_u32(&hbar[wl][xb]);
-            if (lane == 0) {
-                const uint32_t expect = (warp > 0 ? 128u : 0u) + (warp < nwarps - 1 ? 128u : 0u);
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar), "r"(expect) : "memory");
+    // Exchange the last row of a block with the two neighbouring strips only: the outer 32 published cells on each side
+    // go straight into the neighbour warp's halo slot (st.async into its CTA's shared memory, completion counted on ITS
+    // mbarrier), then this warp waits for the 2 x 128 bytes it expects itself.  No cluster-wide barrier and no memory
+    // fence: the release/acquire cluster barrier used before carried MEMBAR.ALL.GPU + CCTL.IVALL, i.e. it also waited
+    // for the block's global stores of the cumulative plane (40 % of the kernel's stall samples).
+    // Slot xb = block parity: a neighbour can be at most one block ahead, it needs this warp's row to go further.  The
+    // slot and the exchange count hround (mbarrier parity (hround >> 1) & 1) are advanced by the caller.
+    auto exchange = [&](int xb, int hround) {
+        const int wl = tid >> 5;                          // warp inside the CTA
+        float* halo = xrow + (wl * 2 + xb) * 64;          // [0,32): cells left of the published range, [32,64): right
+        const uint32_t my_bar = dp_smem_u32(&hbar[wl][xb]);
+        if (lane == 0) {
+            const uint32_t expect = (warp > 0 ? 128u : 0u) + (warp < nwarps - 1 ? 128u : 0u);
+            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar), "r"(expect) : "memory");
+        }
+        if (lane >= HL && lane < 2 * HL && warp > 0) {                        // my leftmost 32 published cells
+            const int nw = warp - 1;
+            const uint32_t nrank = (uint32_t) (nw / wpc);
+            const int nwl = nw - (int) nrank * wpc;
+            const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + 32 + (lane - HL) * CPL, nrank);
+            const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+        }
+        if (lane >= 32 - 2 * HL && lane < 32 - HL && warp < nwarps - 1) {     // my rightmost 32 published cells
+            const int nw = warp + 1;
+            const uint32_t nrank = (uint32_t) (nw / wpc);
+            const int nwl = nw - (int) nrank * wpc;
+            const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + (lane - (32 - 2 * HL)) * CPL, nrank);
+            const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+        }
+        dp_mbar_wait(my_bar, (uint32_t) ((hround >> 1) & 1));
+        if (!central) {
+            const float* hp = halo + (lane < HL ? lane * CPL : 32 + (lane - (32 - HL)) * CPL);
+#pragma unroll
+            for (int g = 0; g < DP_P; g++) {
+                const int x = c0 + 4 * g;
+                if (x >= 0 && x < w) cur[g] = *reinterpret_cast<const float4*>(hp + 4 * g);   // cells right of the image arrive as +inf
+                else cur[g] = make_float4(INF, INF, INF, INF);
             }
-            if (lane >= HL && lane < 2 * HL && warp > 0) {                        // my leftmost 32 published cells
-                const int nw = warp - 1;
-                const uint32_t nrank = (uint32_t) (nw / wpc);
-                const int nwl = nw - (int) nrank * wpc;
-                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + 32 + (lane - HL) * CPL, nrank);
-                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
-    #pragma unroll
-                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+        }
+    };
+    // Two block loops: one for DpStep1 (exchange after every DP_R rows) and one for DpSteps (after every DP_R / dx rows
+    // counted from row 0); merged into one, the DpStep1 kernels got another register allocation.  Never after the last row.
+    if constexpr (Step::D == 1) {
+        for (int yb = 1; yb < h; yb += DP_R) {
+            if (yb + DP_R <= h) {                         // whole block: no per-row bounds checks
+                dp_unroll<DP_R>([&](auto kk_c) {
+                    constexpr int kk = decltype(kk_c)::value;
+                    if (TMA && kk % SRD == 0) chunk_begin();
+                    row(kk_c, yb + kk);
+                    if (TMA && kk % SRD == SRD - 1) chunk_end();
+                });
+            } else {
+                dp_unroll<DP_R>([&](auto kk_c) {
+                    constexpr int kk = decltype(kk_c)::value;
+                    const int y = yb + kk;
+                    if (TMA && kk % SRD == 0 && y < h) chunk_begin();
+                    if (y < h) row(kk_c, y);              // uniform across the CTA
+                    if (TMA && kk % SRD == SRD - 1) chunk_end();
+                });
             }
-            if (lane >= 32 - 2 * HL && lane < 32 - HL && warp < nwarps - 1) {     // my rightmost 32 published cells
-                const int nw = warp + 1;
-                const uint32_t nrank = (uint32_t) (nw / wpc);
-                const int nwl = nw - (int) nrank * wpc;
-                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + (lane - (32 - 2 * HL)) * CPL, nrank);
-                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
-    #pragma unroll
-                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
+            if (yb + DP_R < h) {
+                exchange(xb, hround);
+                xb ^= 1;
+                hround++;
             }
-            dp_mbar_wait(my_bar, (uint32_t) ((hround >> 1) & 1));
-            hround++;
-            if (!central) {
-                const float* hp = halo + (lane < HL ? lane * CPL : 32 + (lane - (32 - HL)) * CPL);
-    #pragma unroll
-                for (int g = 0; g < DP_P; g++) {
-                    const int x = c0 + 4 * g;
-                    if (x >= 0 && x < w) cur[g] = *reinterpret_cast<const float4*>(hp + 4 * g);   // cells right of the image arrive as +inf
-                    else cur[g] = make_float4(INF, INF, INF, INF);
-                }
-            }
-            xb ^= 1;
-        };
-        const int rb = DP_R / pen.dx;
+        }
+    } else {
+        const int rb = DP_R / st.dx;
         int since = 0;
         for (int yb = 1; yb < h; yb += DP_R) {
             dp_unroll<DP_R>([&](auto kk_c) {
@@ -658,76 +660,14 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
                 if (TMA && kk % SRD == 0 && y < h) chunk_begin();
                 if (y < h) row(kk_c, y);
                 if (++since == rb && y + 1 < h) {
-                    exchange();
+                    exchange(xb, hround);
+                    xb ^= 1;
+                    hround++;
                     since = 0;
                 }
                 if (TMA && kk % SRD == SRD - 1) chunk_end();
             });
         }
-    } else {
-    for (int yb = 1; yb < h; yb += DP_R) {
-        if (yb + DP_R <= h) {                         // whole block: no per-row bounds checks
-            dp_unroll<DP_R>([&](auto kk_c) {
-                constexpr int kk = decltype(kk_c)::value;
-                if (TMA && kk % SRD == 0) chunk_begin();
-                row(kk_c, yb + kk);
-                if (TMA && kk % SRD == SRD - 1) chunk_end();
-            });
-        } else {
-            dp_unroll<DP_R>([&](auto kk_c) {
-                constexpr int kk = decltype(kk_c)::value;
-                const int y = yb + kk;
-                if (TMA && kk % SRD == 0 && y < h) chunk_begin();
-                if (y < h) row(kk_c, y);              // uniform across the CTA
-                if (TMA && kk % SRD == SRD - 1) chunk_end();
-            });
-        }
-        // Exchange the last row of the block with the two neighbouring strips only: the outer 32 published cells on each
-        // side go straight into the neighbour warp's halo slot (st.async into its CTA's shared memory, completion counted
-        // on ITS mbarrier), then this warp waits for the 2 x 128 bytes it expects itself.  No cluster-wide barrier and no
-        // memory fence: the release/acquire cluster barrier used before carried MEMBAR.ALL.GPU + CCTL.IVALL, i.e. it also
-        // waited for the block's global stores of the cumulative plane (40 % of the kernel's stall samples).
-        // Slot = block parity: a neighbour can be at most one block ahead, it needs this warp's row to go further.
-        if (yb + DP_R < h) {
-            const int wl = tid >> 5;                          // warp inside the CTA
-            float* halo = xrow + (wl * 2 + xb) * 64;          // [0,32): cells left of the published range, [32,64): right
-            const uint32_t my_bar = dp_smem_u32(&hbar[wl][xb]);
-            if (lane == 0) {
-                const uint32_t expect = (warp > 0 ? 128u : 0u) + (warp < nwarps - 1 ? 128u : 0u);
-                asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(my_bar), "r"(expect) : "memory");
-            }
-            if (lane >= HL && lane < 2 * HL && warp > 0) {                        // my leftmost 32 published cells
-                const int nw = warp - 1;
-                const uint32_t nrank = (uint32_t) (nw / wpc);
-                const int nwl = nw - (int) nrank * wpc;
-                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + 32 + (lane - HL) * CPL, nrank);
-                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
-#pragma unroll
-                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
-            }
-            if (lane >= 32 - 2 * HL && lane < 32 - HL && warp < nwarps - 1) {     // my rightmost 32 published cells
-                const int nw = warp + 1;
-                const uint32_t nrank = (uint32_t) (nw / wpc);
-                const int nwl = nw - (int) nrank * wpc;
-                const uint32_t dst = dp_map(xrow + (nwl * 2 + xb) * 64 + (lane - (32 - 2 * HL)) * CPL, nrank);
-                const uint32_t bar = dp_map(&hbar[nwl][xb], nrank);
-#pragma unroll
-                for (int g = 0; g < DP_P; g++) dp_st_async_v4(dst + 16u * g, cur[g], bar);
-            }
-            dp_mbar_wait(my_bar, (uint32_t) ((hround >> 1) & 1));
-            hround++;
-            if (!central) {
-                const float* hp = halo + (lane < HL ? lane * CPL : 32 + (lane - (32 - HL)) * CPL);
-#pragma unroll
-                for (int g = 0; g < DP_P; g++) {
-                    const int x = c0 + 4 * g;
-                    if (x >= 0 && x < w) cur[g] = *reinterpret_cast<const float4*>(hp + 4 * g);   // cells right of the image arrive as +inf
-                    else cur[g] = make_float4(INF, INF, INF, INF);
-                }
-            }
-            xb ^= 1;
-        }
-    }
     }
 #ifdef DCTC_SYNC_DEBUG
     const long long dbg_t1 = clock64();
@@ -787,10 +727,8 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
         if (xlast) {
             // parallel back-track: the jump and trace kernels below take over from the seam's last-row column
             if (lane == 0) { *xlast = bi; seam[h - 1] = bi; if (seam_log) seam_log[h - 1] = bi; }
-        } else if constexpr (WIDE) {
-            dp_backtrack_wide(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);
         } else {
-            dp_backtrack<RIG>(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);   // serial walk by warp 0 of CTA 0
+            dp_backtrack(mplane + fz * m_fs, m_pitch, w, h, bi, seam, seam_log, win, lane, st);   // serial walk by warp 0 of CTA 0
         }
 #ifdef DCTC_SYNC_DEBUG
         if (tid == 0) {
@@ -803,23 +741,41 @@ __global__ void __cluster_dims__(DP_CL, 1, 1) __launch_bounds__(DP_MAXW * 32) dc
 
 // ---- parallel back-track (build_vpath without the h-step dependent chain) ---------------------------------------
 // The serial walk above is a chain of h dependent shared-memory reads (133 clk per row: 73 us of a 1080-row seam).  The
-// parent choice of a cell depends only on the cumulative map, not on the path, so the rows are cut into blocks of JB
+// parent choice of a cell depends only on the cumulative map, not on the path, so the rows are cut into blocks of jb
 // rows (counted upwards from the last row) and, for EVERY column x of a block's bottom row, the column its path has at
 // the block's top row is computed in parallel: top-down, P_top[x] = x, P_y[x] = P_{y-1}[x + d_y(x)] with d_y(x) the
-// parent direction of (y, x) -- neighbours only, so a warp keeps a strip of 128 columns in registers and exchanges
-// the outer cells by shuffles, exactly like the seam DP (JB = 32 contaminated columns on each side, 64 published).
+// parent step of (y, x) -- at most D columns, so a warp keeps a strip of 32 jc columns in registers and exchanges the
+// outer cells by shuffles, like the seam DP (jb * D <= 8 jc contaminated columns on each side, 16 jc published).
 // dctc_seam_jump_kernel: one warp per (strip, block), the whole grid busy for ~1 us; it stores the jump as an int8
-// offset.  dctc_seam_trace_kernel: one CTA per block; it follows the ceil((h-1)/32) jumps from the seam's last-row
-// column down to its own block (the jump entries a path can reach form a cone of 64*j+1 columns in block j, staged
-// into shared memory first), then walks its 32 rows like dp_backtrack does.  ~100 dependent steps instead of h.
-constexpr int JB = 32;
+// offset (at most jb * D = 124 columns).  dctc_seam_trace_kernel: one CTA per block; it follows the ceil((h-1)/jb)
+// jumps from the seam's last-row column down to its own block (the jump entries a path can reach form a cone of
+// 2 jb dx j + 1 columns in block j, staged into shared memory first), then walks its jb rows like dp_backtrack does.
+// ~100 dependent steps instead of h.
+// The geometry of a rule whose steps reach D columns (DpStep1: D = 1, DpSteps: D = DCTC_MAX_DELTA_X), in one place:
+//   jb        jump block rows
+//   jc        jump cells per lane: strips of 32 jc columns, the central 16 jc published
+//   jr        jump rows of loads in flight
+//   win, wl   trace window: columns, of which wl lie left of the block's bottom column
+//   cone_max  largest cone (bytes of the trace kernel's dynamic shared memory) of the parallel back-track: D > 1 has less
+//             room next to its window's 34 KB of static shared memory
+template <int D>
+struct BtGeom;
+template <>
+struct BtGeom<1> { static constexpr int jb = 32, jc = 4, jr = 8, win = 72, wl = 34, cone_max = 200 * 1024; };
+template <>
+struct BtGeom<DCTC_MAX_DELTA_X> { static constexpr int jb = 31, jc = 16, jr = 4, win = 264, wl = 132, cone_max = 180 * 1024; };
+constexpr int JH = 8;             // jump halo lanes on each side of a strip (8 jc >= jb * D)
 
-// Batch sessions: blockIdx.z = frame (planes m_fs floats / j_fs bytes apart).  RIG: rigidity pen, as in the DP.
-template <bool RIG>
+// Batch sessions: blockIdx.z = frame (planes m_fs floats / j_fs bytes apart).
+template <typename Step>
 __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
                                                              int8_t* __restrict__ jump, size_t j_pitch, int strips,
-                                                             size_t m_fs, size_t j_fs, float pen)
+                                                             size_t m_fs, size_t j_fs, typename Step::Arg arg)
 {
+    constexpr int D = Step::D;
+    using G = BtGeom<D>;
+    constexpr int JC = G::jc, NG = JC / 4;         // cells and float4 groups per lane
+    const Step st{arg};
     DCTC_PDL_PROLOGUE();
     const int lane = threadIdx.x & 31;
     const int strip = blockIdx.x * 4 + (threadIdx.x >> 5);
@@ -827,68 +783,78 @@ __global__ void __launch_bounds__(128) dctc_seam_jump_kernel(const float* __rest
     const int k = blockIdx.y;
     mplane += blockIdx.z * m_fs;
     jump += blockIdx.z * j_fs;
-    const int yb = h - 1 - JB * k;                    // bottom row of the block
-    const int yt = max(yb - JB, 0);                   // top row
+    const int yb = h - 1 - G::jb * k;                  // bottom row of the block
+    const int yt = max(yb - G::jb, 0);                 // top row
     const int steps = yb - yt;
     const float INF = __int_as_float(0x7f800000);
-    const int c0 = strip * 64 - JB + 4 * lane;        // this lane's four columns
-    const bool in_row = c0 >= 0 && c0 < w;            // (c0 is a multiple of 4 and the pitch covers round_up(w, 4))
-    const float* src = mplane + (size_t) yt * m_pitch + (in_row ? c0 : 0);
-    int P[4] = {c0, c0 + 1, c0 + 2, c0 + 3};
-    auto row = [&](float4 v) {                        // v = cumulative values of row y-1 -> P of row y
-        float m[4] = {v.x, v.y, v.z, v.w};
+    const int c0 = strip * 16 * JC - JH * JC + JC * lane;   // this lane's JC columns
+    bool ok[NG];
 #pragma unroll
-        for (int j = 0; j < 4; j++)
-            if (!in_row || c0 + j >= w) m[j] = INF;   // outside the image: never a parent (range clipping)
-        float l = __shfl_up_sync(0xffffffffu, m[3], 1), r = __shfl_down_sync(0xffffffffu, m[0], 1);
-        int pl = __shfl_up_sync(0xffffffffu, P[3], 1), pr = __shfl_down_sync(0xffffffffu, P[0], 1);
-        if (lane == 0) l = INF;
-        if (lane == 31) r = INF;
-        int Q[4];
+    for (int g = 0; g < NG; g++) ok[g] = c0 + 4 * g >= 0 && c0 + 4 * g < w;     // (multiples of 4: the pitch covers round_up(w, 4))
+    const float* const src = mplane + (size_t) yt * m_pitch;
+    int P[JC];
 #pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const float a0 = j == 0 ? l : m[j - 1], b = m[j], c0 = j == 3 ? r : m[j + 1];
-            const float a = RIG ? a0 + pen : a0, c = RIG ? c0 + pen : c0;
-            const int pa = j == 0 ? pl : P[j - 1], pb = P[j], pc = j == 3 ? pr : P[j + 1];
-            const bool p1 = b < a;                    // first strict minimum scanning x-1, x, x+1
-            const float best = p1 ? b : a;
-            const bool p2 = c < best;
-            Q[j] = p2 ? pc : (p1 ? pb : pa);
+    for (int i = 0; i < JC; i++) P[i] = c0 + i;
+    auto row = [&](const float4 (&v)[NG]) {           // cumulative values of row y-1 -> P of row y
+        float e[JC + 2 * D];                          // e[D + i]: column c0 + i, D neighbour cells on each side
+        int pe[JC + 2 * D];
+#pragma unroll
+        for (int g = 0; g < NG; g++) {
+            const float c4[4] = {v[g].x, v[g].y, v[g].z, v[g].w};
+#pragma unroll
+            for (int j = 0; j < 4; j++) e[D + 4 * g + j] = ok[g] && c0 + 4 * g + j < w ? c4[j] : INF;   // range clipping
         }
 #pragma unroll
-        for (int j = 0; j < 4; j++) P[j] = Q[j];
+        for (int i = 0; i < JC; i++) pe[D + i] = P[i];
+#pragma unroll
+        for (int j = 0; j < D; j++) {                 // neighbours across lanes; the strip's outermost lanes see +inf
+            const float l = __shfl_up_sync(0xffffffffu, e[JC + j], 1), r = __shfl_down_sync(0xffffffffu, e[D + j], 1);
+            pe[j] = __shfl_up_sync(0xffffffffu, P[JC - D + j], 1);
+            pe[JC + D + j] = __shfl_down_sync(0xffffffffu, P[j], 1);
+            e[j] = lane == 0 ? INF : l;
+            e[JC + D + j] = lane == 31 ? INF : r;
+        }
+#pragma unroll
+        for (int i = 0; i < JC; i++) P[i] = st.pick([&](int d) { return e[D + i + d]; }, [&](int d) { return pe[D + i + d]; });
     };
-    for (int i0 = 0; i0 < steps; i0 += 8) {           // eight independent loads in flight, then eight dependent steps
-        float4 pv[8];
+    for (int i0 = 0; i0 < steps; i0 += G::jr) {       // jr rows of independent loads in flight, then jr dependent steps
+        float4 pv[G::jr][NG];
 #pragma unroll
-        for (int j = 0; j < 8; j++)
-            pv[j] = __ldcg(reinterpret_cast<const float4*>(src + (size_t) min(i0 + j, steps - 1) * m_pitch));
+        for (int j = 0; j < G::jr; j++)
 #pragma unroll
-        for (int j = 0; j < 8; j++)
+            for (int g = 0; g < NG; g++)
+                pv[j][g] = __ldcg(reinterpret_cast<const float4*>(src + (ok[g] ? c0 + 4 * g : 0) + (size_t) min(i0 + j, steps - 1) * m_pitch));
+#pragma unroll
+        for (int j = 0; j < G::jr; j++)
             if (i0 + j < steps) row(pv[j]);
     }
-    if (lane >= JB / 4 && lane < 32 - JB / 4 && in_row) {
-        int8_t* dst = jump + (size_t) k * j_pitch + c0;
+    dp_unroll<NG>([&](auto g_c) {                    // (expanded at compile time: as an unrolled loop, D > 1 takes one register more)
+        constexpr int g = decltype(g_c)::value;
+        if (lane >= JH && lane < 32 - JH && ok[g]) {
+            int8_t* dst = jump + (size_t) k * j_pitch + c0 + 4 * g;
 #pragma unroll
-        for (int j = 0; j < 4; j++)
-            if (c0 + j < w) dst[j] = (int8_t) (P[j] - (c0 + j));
-    }
+            for (int j = 0; j < 4; j++)
+                if (c0 + 4 * g + j < w) dst[j] = (int8_t) (P[4 * g + j] - (c0 + 4 * g + j));
+        }
+    });
 }
 
-constexpr int TR_WIN = 72;                            // walk window: columns x-34 .. x+37 around the block's bottom column
 constexpr int TR_THREADS = 256;
 
 // Batch sessions: blockIdx.y = frame (planes m_fs floats / j_fs bytes apart, seam[h * frame ...],
-// seam_log[log_fs * frame ...], xlast[frame]).  RIG: rigidity pen, as in the DP.
-template <bool RIG>
+// seam_log[log_fs * frame ...], xlast[frame]).
+template <typename Step>
 __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
                                                               const int8_t* __restrict__ jump, size_t j_pitch,
                                                               const int* __restrict__ xlast, int* __restrict__ seam,
                                                               int* __restrict__ seam_log, size_t m_fs, size_t j_fs, size_t log_fs,
-                                                              float pen)
+                                                              typename Step::Arg arg)
 {
+    constexpr int D = Step::D;
+    using G = BtGeom<D>;
+    const Step st{arg};
     extern __shared__ __align__(16) unsigned char tr_smem[];
-    __shared__ __align__(16) float win[JB][TR_WIN + 8];
+    __shared__ __align__(16) float win[G::jb][G::win + 8];
     __shared__ int xb_s;
     DCTC_PDL_PROLOGUE();
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
@@ -898,17 +864,19 @@ __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float
     seam += (size_t) fz * h;
     if (seam_log) seam_log += fz * log_fs;
     const int x0 = xlast[fz];
-    // Cone of block j: its bottom column can be x0 - 32 j .. x0 + 32 j.  The entries are staged as aligned 16-byte
-    // chunks (at most 4 j + 3 per row, at byte offset 32 j^2 + 16 j of the cone buffer); warp w takes the rows
-    // j = w, w + 8, ... and issues all chunks of a row before it stores any of them, so the loads of a row (and of the
-    // other warps' rows) are in flight together instead of one L2 round trip per iteration.
+    // Cone of block j: its bottom column can be x0 - R j .. x0 + R j, R = jb dx.  The entries are staged as aligned
+    // 16-byte chunks (at most (R8 / 8) j + 3 per row, R8 = R rounded up to 8, at byte offset R8 j (j - 1) + 48 j of the
+    // cone buffer); warp w takes the rows j = w, w + 8, ... and issues all chunks of a row before it stores any of them,
+    // so the loads of a row (and of the other warps' rows) are in flight together instead of one L2 round trip per
+    // iteration.
+    const int R = G::jb * st.dx, R8 = (R + 7) & ~7;
     for (int j = wid; j < k; j += TR_THREADS / 32) {
-        const int a0 = max(0, x0 - JB * j) & ~15;
-        const int last = min(w - 1, x0 + JB * j);
-        const int nchunk = ((last - a0) >> 4) + 1;                          // <= 4 j + 3
+        const int a0 = max(0, x0 - R * j) & ~15;
+        const int last = min(w - 1, x0 + R * j);
+        const int nchunk = ((last - a0) >> 4) + 1;                          // <= (R8 / 8) j + 3
         const uint4* srcj = reinterpret_cast<const uint4*>(jump + (size_t) j * j_pitch + a0);
-        uint4* dstj = reinterpret_cast<uint4*>(tr_smem + 32 * j * j + 16 * j);
-        for (int c0 = 0; c0 < nchunk; c0 += 160) {                          // (one pass up to 1080 rows, two beyond)
+        uint4* dstj = reinterpret_cast<uint4*>(tr_smem + R8 * j * j + (48 - R8) * j);
+        for (int c0 = 0; c0 < nchunk; c0 += 160) {                          // (one pass up to 1080 rows at dx = 1, two beyond)
             uint4 v[5];
 #pragma unroll
             for (int i = 0; i < 5; i++)
@@ -922,40 +890,38 @@ __global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_kernel(const float
     if (tid == 0) {
         const int8_t* cone = reinterpret_cast<const int8_t*>(tr_smem);
         int x = x0;
-        for (int j = 0; j < k; j++) x += cone[32 * j * j + 16 * j + (x - (max(0, x0 - JB * j) & ~15))];
+        for (int j = 0; j < k; j++) x += cone[R8 * j * j + (48 - R8) * j + (x - (max(0, x0 - R * j) & ~15))];
         xb_s = x;
     }
     __syncthreads();
     int x = xb_s;
-    const int yb = h - 1 - JB * k, yt = max(yb - JB, 0), steps = yb - yt;
-    // window rows: win[i] = cumulative row yb-1-i, columns base .. base+TR_WIN-1 at win[i][4 + c - base]
-    const int max_base = (int) m_pitch - TR_WIN;
-    int base = (x - 34) & ~3;
+    const int yb = h - 1 - G::jb * k, yt = max(yb - G::jb, 0), steps = yb - yt;
+    // window rows: win[i] = cumulative row yb-1-i, columns base .. base+win-1 at win[i][4 + c - base]
+    const int max_base = (int) m_pitch - G::win;                   // >= 0: bt_plan asks for m_pitch >= win
+    int base = (x - G::wl) & ~3;
     base = base < 0 ? 0 : (base > max_base ? max_base : base);
-    for (int idx = tid; idx < steps * (TR_WIN / 4); idx += TR_THREADS) {
-        const int i = idx / (TR_WIN / 4), c = idx - i * (TR_WIN / 4);
+    for (int idx = tid; idx < steps * (G::win / 4); idx += TR_THREADS) {
+        const int i = idx / (G::win / 4), c = idx - i * (G::win / 4);
         const float* src = mplane + (size_t) (yb - 1 - i) * m_pitch + base + 4 * c;
         *reinterpret_cast<float4*>(&win[i][4 + 4 * c]) = __ldcg(reinterpret_cast<const float4*>(src));
     }
     __syncthreads();
     if (tid >= 32) return;
     const float INF = __int_as_float(0x7f800000);
-    // +inf sentinels left of column 0 and at column w (range clipping), so that the walk needs no bounds checks
+    // D +inf sentinels left of column 0 and from column w on (range clipping), so that the walk needs no bounds checks
     if (lane < steps) {
-        if (base == 0) win[lane][3] = INF;
-        if (w - base >= 0 && w - base <= TR_WIN) win[lane][4 + w - base] = INF;
+        if (base == 0)
+            for (int j = 0; j < D; j++) win[lane][4 - D + j] = INF;
+        if (w - base >= 0 && w - base <= G::win)
+            for (int j = 0; j < D; j++) win[lane][4 + w - base + j] = INF;
     }
     __syncwarp();
     int mine = 0;
     const float* wp = &win[0][4] + (x - base);
     for (int i = 0; i < steps; i++) {
-        const float a = RIG ? wp[-1] + pen : wp[-1], b = wp[0], c = RIG ? wp[1] + pen : wp[1];
-        const bool p1 = b < a;
-        const float best = p1 ? b : a;
-        const bool p2 = c < best;
-        const int d = p2 ? 1 : (p1 ? 0 : -1);
+        const int d = st.pick([&](int c) { return wp[c]; }, [](int c) { return c; });
         x += d;
-        wp += TR_WIN + 8 + d;
+        wp += G::win + 8 + d;
         if (lane == i) mine = x;
     }
     if (lane < steps) { seam[yb - 1 - lane] = mine; if (seam_log) seam_log[yb - 1 - lane] = mine; }
@@ -989,10 +955,10 @@ constexpr int INCR_T = 8;                               // rows between two tigh
 constexpr int INCR_SW = INCR_CAP + 2 * INCR_D + 16;     // floats per staged row and plane
 
 // one row of the walk with NK columns per lane: every shared-memory load first, then the arithmetic and the stores
-template <int NK, bool RIG>
+template <int NK, typename Step>
 __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w, int plo, const float* __restrict__ re,
                                          const float* __restrict__ rm, int xs, const float* __restrict__ prev,
-                                         float* __restrict__ next, float* __restrict__ mrow, int& clo, int& chi, float pen)
+                                         float* __restrict__ next, float* __restrict__ mrow, int& clo, int& chi, const Step& st)
 {
     const float INF = __int_as_float(0x7f800000);
     float e[NK], mo[NK], pl[NK], pc[NK], pr[NK];
@@ -1011,7 +977,7 @@ __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w,
         const int x = lo + lane + 32 * k;
         if (x <= hi) {
             float mn = e[k];
-            if (y > 0) mn = e[k] + fminf(fminf(x > 0 ? (RIG ? pl[k] + pen : pl[k]) : INF, pc[k]), x < w - 1 ? (RIG ? pr[k] + pen : pr[k]) : INF);
+            if (y > 0) mn = e[k] + fminf(fminf(x > 0 ? st.diag(pl[k]) : INF, pc[k]), x < w - 1 ? st.diag(pr[k]) : INF);
             next[x - lo + 2] = mn;
             if (__float_as_uint(mn) != __float_as_uint(mo[k])) {
 #if DCTC_INCR_ABL != 1
@@ -1024,13 +990,14 @@ __device__ __forceinline__ void incr_row(int y, int lane, int lo, int hi, int w,
     }
 }
 
-// RIG: rigidity pen, as in the DP (the changed cells still spread by one column per row).
-template <bool RIG>
+// Step: DpStep1, as in the DP (the changed cells spread by one column per row).
+template <typename Step>
 __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restrict__ en, size_t en_pitch, int w, int h,
                                                             float* __restrict__ mplane, size_t m_pitch, int r,
                                                             int* __restrict__ seam, int* __restrict__ seam_log,
-                                                            int* __restrict__ rebuild_flag, float pen)
+                                                            int* __restrict__ rebuild_flag, typename Step::Arg arg)
 {
+    const Step st{arg};
     extern __shared__ __align__(16) int incr_sm[];
     float* ring = reinterpret_cast<float*>(incr_sm);                       // INCR_D slots x (energy row, map row) x INCR_SW
     float* buf = ring + INCR_D * 2 * INCR_SW;                              // two hand-over rows of INCR_CAP + 4 cells
@@ -1106,11 +1073,11 @@ __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restr
         const int xs = xsb[slot];
         float* mrow = mplane + (size_t) y * m_pitch;
         int clo = 0x7fffffff, chi = -1;
-        if (width <= 32) incr_row<1, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
-        else if (width <= 64) incr_row<2, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
-        else if (width <= 128) incr_row<4, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
-        else if (width <= 256) incr_row<8, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
-        else incr_row<16, RIG>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, pen);
+        if (width <= 32) incr_row<1>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, st);
+        else if (width <= 64) incr_row<2>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, st);
+        else if (width <= 128) incr_row<4>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, st);
+        else if (width <= 256) incr_row<8>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, st);
+        else incr_row<16>(y, lane, lo, hi, w, plo, re, rm, xs, prev, next, mrow, clo, chi, st);
 #ifdef DCTC_INCR_STATS
         const long long c2 = clock64();
 #endif
@@ -1174,188 +1141,23 @@ __global__ void __launch_bounds__(32) dctc_seam_incr_kernel(const float* __restr
         const int oi = __shfl_xor_sync(0xffffffffu, bi, o);
         if (oi != 0x7fffffff && (bi == 0x7fffffff || ov < bv || (ov == bv && oi < bi))) { bv = ov; bi = oi; }
     }
-    dp_backtrack<RIG>(mplane, m_pitch, w, h, bi, seam, seam_log, win, lane, pen);
+    dp_backtrack(mplane, m_pitch, w, h, bi, seam, seam_log, win, lane, st);
 }
 
 // Instantiated here, ahead of the DP kernels: the module then declares the dynamic shared arrays of the trace and
 // incremental kernels before the DP's 128-byte aligned one, which keeps the trace kernel's dynamic shared memory at the
-// 16-byte aligned offset its static arrays end at (the rigidity-0 kernels stay what they were before RIG existed).
-template __global__ void dctc_seam_jump_kernel<false>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
-template __global__ void dctc_seam_jump_kernel<true>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
-template __global__ void dctc_seam_trace_kernel<false>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*, int*,
-                                                       size_t, size_t, size_t, float);
-template __global__ void dctc_seam_trace_kernel<true>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*, int*,
-                                                      size_t, size_t, size_t, float);
-template __global__ void dctc_seam_incr_kernel<false>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
-template __global__ void dctc_seam_incr_kernel<true>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
-
-// ---- parallel back-track for delta_x > 1 -----------------------------------------------------------------------------
-// The jump and trace kernels above with the step table of the WIDE seam DP (DpSteps: 9 candidates, +inf pen beyond dx,
-// best = +inf and a strict < = the first strict minimum of the real candidates).  A path moves up to dx columns per row,
-// so the jump blocks are JBW = 31 rows (offsets of up to 31 * 4 = 124 columns fit int8), a jump warp's lanes hold 16
-// columns each (strip of 512, 128 contaminated on each side after a block, 256 published) and a trace CTA walks its block
-// through a window of TRW_WIN columns.  The cone of block j spans x0 +- R j, R = JBW * dx: its rows are staged in
-// (R8 / 8) j + 3 chunks of 16 bytes, R8 = R rounded up to 8 (R8 = 32 and JBW = 32 give the layout of dx = 1).
-constexpr int JBW = 31;
-constexpr int TRW_WIN = 264;                          // walk window: columns x-132 .. x+131 around the block's bottom column
-
-__global__ void __launch_bounds__(128) dctc_seam_jump_wide_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
-                                                                  int8_t* __restrict__ jump, size_t j_pitch, int strips,
-                                                                  size_t m_fs, size_t j_fs, DpSteps st)
-{
-    DCTC_PDL_PROLOGUE();
-    const int lane = threadIdx.x & 31;
-    const int strip = blockIdx.x * 4 + (threadIdx.x >> 5);
-    if (strip >= strips) return;
-    const int k = blockIdx.y;
-    mplane += blockIdx.z * m_fs;
-    jump += blockIdx.z * j_fs;
-    const int yb = h - 1 - JBW * k;
-    const int yt = max(yb - JBW, 0);
-    const int steps = yb - yt;
-    const float INF = __int_as_float(0x7f800000);
-    const int c0 = strip * 256 - 128 + 16 * lane;     // this lane's 16 columns
-    bool ok[4];
-    const float* src[4];
-#pragma unroll
-    for (int g = 0; g < 4; g++) {
-        ok[g] = c0 + 4 * g >= 0 && c0 + 4 * g < w;     // (multiples of 4: the pitch covers round_up(w, 4))
-        src[g] = mplane + (size_t) yt * m_pitch + (ok[g] ? c0 + 4 * g : 0);
-    }
-    int P[16];
-#pragma unroll
-    for (int i = 0; i < 16; i++) P[i] = c0 + i;
-    auto row = [&](const float4 (&v)[4]) {            // cumulative values of row y-1 -> P of row y
-        float e[24];
-        int pe[24];
-#pragma unroll
-        for (int g = 0; g < 4; g++) {
-            const float c4[4] = {v[g].x, v[g].y, v[g].z, v[g].w};
-#pragma unroll
-            for (int j = 0; j < 4; j++) e[4 + 4 * g + j] = ok[g] && c0 + 4 * g + j < w ? c4[j] : INF;   // range clipping
-        }
-#pragma unroll
-        for (int i = 0; i < 16; i++) pe[4 + i] = P[i];
-#pragma unroll
-        for (int j = 0; j < 4; j++) {
-            const float l = __shfl_up_sync(0xffffffffu, e[16 + j], 1), r = __shfl_down_sync(0xffffffffu, e[4 + j], 1);
-            pe[j] = __shfl_up_sync(0xffffffffu, P[12 + j], 1);
-            pe[20 + j] = __shfl_down_sync(0xffffffffu, P[j], 1);
-            e[j] = lane == 0 ? INF : l;
-            e[20 + j] = lane == 31 ? INF : r;
-        }
-#pragma unroll
-        for (int i = 0; i < 16; i++) {
-            float best = INF;
-            int q = pe[4 + i];
-#pragma unroll
-            for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
-                const float v = d == 0 ? e[4 + i] : e[4 + i + d] + st.pen[d < 0 ? -d : d];
-                if (v < best) { best = v; q = pe[4 + i + d]; }
-            }
-            P[i] = q;
-        }
-    };
-    for (int i0 = 0; i0 < steps; i0 += 4) {           // four rows of loads in flight, then four dependent steps
-        float4 pv[4][4];
-#pragma unroll
-        for (int j = 0; j < 4; j++)
-#pragma unroll
-            for (int g = 0; g < 4; g++)
-                pv[j][g] = __ldcg(reinterpret_cast<const float4*>(src[g] + (size_t) min(i0 + j, steps - 1) * m_pitch));
-#pragma unroll
-        for (int j = 0; j < 4; j++)
-            if (i0 + j < steps) row(pv[j]);
-    }
-    if (lane >= 8 && lane < 24) {
-        int8_t* dst = jump + (size_t) k * j_pitch;
-#pragma unroll
-        for (int i = 0; i < 16; i++)
-            if (c0 + i >= 0 && c0 + i < w) dst[c0 + i] = (int8_t) (P[i] - (c0 + i));
-    }
-}
-
-__global__ void __launch_bounds__(TR_THREADS) dctc_seam_trace_wide_kernel(const float* __restrict__ mplane, size_t m_pitch, int w, int h,
-                                                                          const int8_t* __restrict__ jump, size_t j_pitch,
-                                                                          const int* __restrict__ xlast, int* __restrict__ seam,
-                                                                          int* __restrict__ seam_log, size_t m_fs, size_t j_fs,
-                                                                          size_t log_fs, DpSteps st)
-{
-    extern __shared__ __align__(16) unsigned char trw_smem[];
-    __shared__ __align__(16) float win[JBW][TRW_WIN + 8];
-    __shared__ int xb_s;
-    DCTC_PDL_PROLOGUE();
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const int k = blockIdx.x, fz = blockIdx.y;
-    mplane += fz * m_fs;
-    jump += fz * j_fs;
-    seam += (size_t) fz * h;
-    if (seam_log) seam_log += fz * log_fs;
-    const int x0 = xlast[fz];
-    const int R = JBW * st.dx, R8 = (R + 7) & ~7;
-    auto row_off = [&](int j) { return R8 * j * (j - 1) + 48 * j; };   // bytes of the cone rows before row j
-    for (int j = wid; j < k; j += TR_THREADS / 32) {
-        const int a0 = max(0, x0 - R * j) & ~15;
-        const int last = min(w - 1, x0 + R * j);
-        const int nchunk = ((last - a0) >> 4) + 1;                          // <= (R8 / 8) j + 3
-        const uint4* srcj = reinterpret_cast<const uint4*>(jump + (size_t) j * j_pitch + a0);
-        uint4* dstj = reinterpret_cast<uint4*>(trw_smem + row_off(j));
-        for (int c0 = 0; c0 < nchunk; c0 += 160) {
-            uint4 v[5];
-#pragma unroll
-            for (int i = 0; i < 5; i++)
-                if (c0 + lane + 32 * i < nchunk) v[i] = __ldcg(srcj + c0 + lane + 32 * i);
-#pragma unroll
-            for (int i = 0; i < 5; i++)
-                if (c0 + lane + 32 * i < nchunk) dstj[c0 + lane + 32 * i] = v[i];
-        }
-    }
-    __syncthreads();
-    if (tid == 0) {
-        const int8_t* cone = reinterpret_cast<const int8_t*>(trw_smem);
-        int x = x0;
-        for (int j = 0; j < k; j++) x += cone[row_off(j) + (x - (max(0, x0 - R * j) & ~15))];
-        xb_s = x;
-    }
-    __syncthreads();
-    int x = xb_s;
-    const int yb = h - 1 - JBW * k, yt = max(yb - JBW, 0), steps = yb - yt;
-    // window rows: win[i] = cumulative row yb-1-i, columns base .. base+TRW_WIN-1 at win[i][4 + c - base]
-    const int max_base = (int) m_pitch - TRW_WIN;                 // >= 0: bt_plan asks for m_pitch >= TRW_WIN
-    int base = (x - 132) & ~3;
-    base = base < 0 ? 0 : (base > max_base ? max_base : base);
-    for (int idx = tid; idx < steps * (TRW_WIN / 4); idx += TR_THREADS) {
-        const int i = idx / (TRW_WIN / 4), c = idx - i * (TRW_WIN / 4);
-        const float* src = mplane + (size_t) (yb - 1 - i) * m_pitch + base + 4 * c;
-        *reinterpret_cast<float4*>(&win[i][4 + 4 * c]) = __ldcg(reinterpret_cast<const float4*>(src));
-    }
-    __syncthreads();
-    if (tid >= 32) return;
-    const float INF = __int_as_float(0x7f800000);
-    // four +inf sentinels left of column 0 and from column w on (range clipping)
-    if (lane < steps) {
-        if (base == 0)
-            for (int j = 0; j < 4; j++) win[lane][j] = INF;
-        if (w - base >= 0 && w - base <= TRW_WIN)
-            for (int j = 0; j < 4; j++) win[lane][4 + w - base + j] = INF;
-    }
-    __syncwarp();
-    int mine = 0;
-    const float* wp = &win[0][4] + (x - base);
-    for (int i = 0; i < steps; i++) {
-        float best = INF;
-        int dbest = 0;
-#pragma unroll
-        for (int d = -DCTC_MAX_DELTA_X; d <= DCTC_MAX_DELTA_X; d++) {
-            const float v = d == 0 ? wp[0] : wp[d] + st.pen[d < 0 ? -d : d];
-            if (v < best) { best = v; dbest = d; }
-        }
-        x += dbest;
-        wp += TRW_WIN + 8 + dbest;
-        if (lane == i) mine = x;
-    }
-    if (lane < steps) { seam[yb - 1 - lane] = mine; if (seam_log) seam_log[yb - 1 - lane] = mine; }
-}
+// 16-byte aligned offset its static arrays end at.
+template __global__ void dctc_seam_jump_kernel<DpStep1<false>>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
+template __global__ void dctc_seam_jump_kernel<DpStep1<true>>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, float);
+template __global__ void dctc_seam_trace_kernel<DpStep1<false>>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*,
+                                                                int*, size_t, size_t, size_t, float);
+template __global__ void dctc_seam_trace_kernel<DpStep1<true>>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*,
+                                                               int*, size_t, size_t, size_t, float);
+template __global__ void dctc_seam_incr_kernel<DpStep1<false>>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
+template __global__ void dctc_seam_incr_kernel<DpStep1<true>>(const float*, size_t, int, int, float*, size_t, int, int*, int*, int*, float);
+template __global__ void dctc_seam_jump_kernel<DpSteps>(const float*, size_t, int, int, int8_t*, size_t, int, size_t, size_t, DpSteps);
+template __global__ void dctc_seam_trace_kernel<DpSteps>(const float*, size_t, int, int, const int8_t*, size_t, const int*, int*, int*,
+                                                         size_t, size_t, size_t, DpSteps);
 
 // ---- visibility map + seam display (SURVEY section 8f rank 4) ---------------------------------------------------
 // liblqr's update_vsmap: the pixel removed from row y by the k-th seam is original column raw[y][s]; its entry of the
@@ -1775,21 +1577,20 @@ static int frames_transpose(dctc_context* ctx, const CarverFrames& f, CarverFram
 }
 
 // Launch plan of the seam DP for frames of wcur x h (energy planes at en, row pitch en_pitch floats, n_frames of them
-// en_pitch * h floats apart): strip width, CTA size, energy staging and the tensor map; rig selects the RIG twin, wide the
-// WIDE kernel of delta_x > 1 (p.dpw instead of p.dp).
+// en_pitch * h floats apart) with the step rule Step: strip width, CTA size, energy staging and the tensor map.
+template <typename Step>
 using dp_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int*, size_t, size_t, size_t,
-                       float);
-using dp_wide_fn = void (*)(const float*, size_t, int, int, float*, size_t, int*, int*, int*, int, const CUtensorMap, int*, size_t, size_t,
-                            size_t, DpSteps);
+                       typename Step::Arg);
+template <typename Step>
 struct DpPlan {
-    dp_fn dp = nullptr;          // delta_x = 1
-    dp_wide_fn dpw = nullptr;    // delta_x > 1
+    dp_fn<Step> dp = nullptr;
     int wpc = 0, nst = 0;
     size_t smem = 0;
     CUtensorMap tmap;
 };
 
-static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, bool rig, bool wide, DpPlan& p)
+template <typename Step>
+static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, int n_frames, DpPlan<Step>& p)
 {
     // strip geometry: 128*P columns per warp, 128*P - 2*DP_R published; the strips are spread over a cluster of DP_CL CTAs
     const int cap = DP_CL * DP_MAXW;
@@ -1812,23 +1613,15 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
     p.wpc = wpc;
     p.nst = nst;
     p.smem = xrow_smem + sizeof(float) * ((size_t) nst * sr * wpc * 128 * P);
-    // the (P, SR) pairs the lines above select for widths 1 .. DP_MAX_W, their RIG twins and their WIDE kernels:
+    // the (P, SR) pairs the lines above select for widths 1 .. DP_MAX_W, for each of the three step rules:
     //   1-2560: (1, 32)   2561-4096: (1, 16)   4097-7680: (2, 16)   7681-12288: (2, 0)   12289-DP_MAX_W: (4, 0)
-    static const struct { int P, sr; dp_fn fn[2]; dp_wide_fn wide; } variants[] = {
-        {1, 32, {dctc_seam_dp_kernel<1, 32, false, false>, dctc_seam_dp_kernel<1, 32, true, false>}, dctc_seam_dp_kernel<1, 32, false, true>},
-        {1, 16, {dctc_seam_dp_kernel<1, 16, false, false>, dctc_seam_dp_kernel<1, 16, true, false>}, dctc_seam_dp_kernel<1, 16, false, true>},
-        {2, 16, {dctc_seam_dp_kernel<2, 16, false, false>, dctc_seam_dp_kernel<2, 16, true, false>}, dctc_seam_dp_kernel<2, 16, false, true>},
-        {2, 0, {dctc_seam_dp_kernel<2, 0, false, false>, dctc_seam_dp_kernel<2, 0, true, false>}, dctc_seam_dp_kernel<2, 0, false, true>},
-        {4, 0, {dctc_seam_dp_kernel<4, 0, false, false>, dctc_seam_dp_kernel<4, 0, true, false>}, dctc_seam_dp_kernel<4, 0, false, true>}};
+    static const struct { int P, sr; dp_fn<Step> fn; } variants[] = {
+        {1, 32, dctc_seam_dp_kernel<1, 32, Step>}, {1, 16, dctc_seam_dp_kernel<1, 16, Step>}, {2, 16, dctc_seam_dp_kernel<2, 16, Step>},
+        {2, 0, dctc_seam_dp_kernel<2, 0, Step>}, {4, 0, dctc_seam_dp_kernel<4, 0, Step>}};
     p.dp = nullptr;
-    p.dpw = nullptr;
     for (const auto& v : variants)
-        if (v.P == P && v.sr == sr) {
-            if (wide) p.dpw = v.wide;
-            else p.dp = v.fn[rig ? 1 : 0];
-        }
-    const void* fn = wide ? (const void*) p.dpw : (const void*) p.dp;
-    if (!fn) return cudaErrorInvalidConfiguration;   // a pair without a kernel: the table and the plan disagree
+        if (v.P == P && v.sr == sr) p.dp = v.fn;
+    if (!p.dp) return cudaErrorInvalidConfiguration;   // a pair without a kernel: the table and the plan disagree
     // tensor map of the energy planes for the staged variants (strips of up to 256 columns: the TMA box limit); frames
     // are its third dimension, so that a box never reaches into the next frame's rows
     memset(&p.tmap, 0, sizeof(p.tmap));
@@ -1844,33 +1637,30 @@ static cudaError_t dp_plan(int wcur, int h, const float* en, size_t en_pitch, in
             return cudaErrorInvalidValue;
     }
     // always opt in: the kernel's static shared memory (back-track windows) plus the dynamic part can exceed 48 KB
-    return cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
+    return cudaFuncSetAttribute(p.dp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) (p.smem > 1024 ? p.smem : 1024));
 }
 
-// Back-track plan for frames of h rows.  The parallel back-track (jump + trace kernels) needs the jump plane and a cone
-// of jump entries in shared memory that grows with the square of the number of row blocks; very tall frames keep the
-// serial walk of the DP kernel.  delta_x > 1: blocks of JBW rows, a cone dx times as wide (next to the 34 KB of the
-// wide trace kernel's window, hence the lower limit), and the window needs cumulative rows of at least TRW_WIN floats.
+// Back-track plan for frames of h rows and a step rule whose steps reach D columns, dx at most.  The parallel back-track
+// (jump + trace kernels) needs the jump plane and a cone of jump entries in shared memory that grows with the square of
+// the number of row blocks; very tall frames keep the serial walk of the DP kernel, and so do frames whose cumulative
+// rows are narrower than the trace window (only possible for D > 1: the rows are at least DP_WIN floats).
 struct BtPlan {
-    int nb;             // row blocks (JB rows, JBW for delta_x > 1)
+    int nb;             // row blocks of BtGeom<D>::jb rows
     size_t cone_smem;   // trace kernel's dynamic shared memory
     size_t j_pitch;     // bytes per row of the jump plane (nb rows per frame)
     bool par;           // parallel back-track
 };
 
+template <int D>
 static BtPlan bt_plan(int h, size_t m_pitch, int dx)
 {
+    using G = BtGeom<D>;
     BtPlan b;
-    const int jb = dx == 1 ? JB : JBW;
-    b.nb = (h - 1 + jb - 1) / jb;
-    if (dx == 1) {
-        b.cone_smem = b.nb > 0 ? (size_t) 32 * (b.nb - 1) * (b.nb - 1) + 16 * (size_t) (b.nb - 1) + 16 : 16;   // rows j < nb-1: 16 (4 j + 3) bytes each
-    } else {
-        const size_t r8 = (size_t) ((JBW * dx + 7) & ~7), j = b.nb > 0 ? (size_t) (b.nb - 1) : 0;
-        b.cone_smem = r8 * j * (j > 0 ? j - 1 : 0) + 48 * j + 16;   // rows j < nb-1: 16 ((R8 / 8) j + 3) bytes each
-    }
+    b.nb = (h - 1 + G::jb - 1) / G::jb;
+    const size_t r8 = (size_t) ((G::jb * dx + 7) & ~7), j = b.nb > 0 ? (size_t) (b.nb - 1) : 0;
+    b.cone_smem = r8 * j * (j > 0 ? j - 1 : 0) + 48 * j + 16;   // rows j < nb-1: 16 ((R8 / 8) j + 3) bytes each
     b.j_pitch = (m_pitch + 15) & ~(size_t) 15;    // jump rows start 16-byte aligned (staged in 16-byte chunks)
-    b.par = b.nb > 0 && (dx == 1 ? b.cone_smem <= 200 * 1024 : b.cone_smem <= 180 * 1024 && m_pitch >= (size_t) TRW_WIN);
+    b.par = b.nb > 0 && b.cone_smem <= (size_t) G::cone_max && m_pitch >= (size_t) G::win;
     return b;
 }
 
@@ -1917,76 +1707,60 @@ struct SeamCall {
 // c.incremental (one frame only, its flag buffer is ctx->c_band): *c.m_valid says whether f.m holds the map of the image
 // before the last removal, compacted over that seam.  The walk then replaces DP + jump + trace, the DP only runs when the
 // walk gave up, and the carve also compacts f.m.  A loop that does not keep the map up to date clears *c.m_valid.
-// c.rigidity: the seams are f.h rows long (the image width at the axis switch for height operations), so every kernel of
-// the loop gets pen = fl(rigidity / f.h); pen == 0 launches the kernels of rigidity 0.
-// c.delta_x > 1: the WIDE seam DP, jump and trace kernels with the step table (DpSteps), the incremental walk is off (the
-// DP rebuilds the map every seam) and the band K1 covers a seam drift of delta_x per row.
-static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c)
+// Step: the step rule (DpStep1 or DpSteps, chosen by seam_loop below) of every seam-search kernel of the loop, arg its
+// kernel argument.  The incremental walk is DpStep1 only: with DpSteps the DP rebuilds the map every seam.
+template <typename Step>
+static int seam_loop_rule(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c,
+                          const typename Step::Arg arg)
 {
-    const int n = f.n, h = f.h, dx = c.delta_x;
+    using G = BtGeom<Step::D>;
+    const int n = f.n, h = f.h, dx = Step{arg}.dx;
     const size_t log_fs = (size_t) n_seams * h, en_fs = f.en_pitch * h, m_fs = f.m_pitch * h;
-    const float pen = c.rigidity / (float) h;
-    const bool rig = pen != 0.0f, wide = dx > 1;
-    DpSteps steps;
-    steps.dx = dx;
-    for (int d = 0; d <= DCTC_MAX_DELTA_X; d++)   // the host carver's rigidity_map_of, +inf beyond the step bound
-        steps.pen[d] = d > dx ? INFINITY : (c.rigidity * ((float) d * sqrtf((float) d))) / (float) h;
-    const BtPlan bt = bt_plan(h, f.m_pitch, dx);
+    const BtPlan bt = bt_plan<Step::D>(h, f.m_pitch, dx);
     int rc = frames_loop_buffers(ctx, f, bt, log_fs);
     if (rc) return rc;
-    DpPlan plan;
-    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, rig, wide, plan));
-    const auto jump = rig ? dctc_seam_jump_kernel<true> : dctc_seam_jump_kernel<false>;
-    const auto trace = rig ? dctc_seam_trace_kernel<true> : dctc_seam_trace_kernel<false>;
-    const auto incr_walk = rig ? dctc_seam_incr_kernel<true> : dctc_seam_incr_kernel<false>;
-    if (bt.par && !wide && bt.cone_smem > 40 * 1024)
-        CK(ctx, cudaFuncSetAttribute(trace, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
-    if (bt.par && wide)   // the window's 34 KB of static shared memory plus the cone
-        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
+    DpPlan<Step> plan;
+    CK(ctx, dp_plan(f.w, h, f.en, f.en_pitch, n, plan));
+    if (bt.par)   // the window's static shared memory plus the cone can exceed the 48 KB default
+        CK(ctx, cudaFuncSetAttribute(dctc_seam_trace_kernel<Step>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) bt.cone_smem));
     int* const xlast = bt.par ? f.xlast : nullptr;
     // incremental update (update_mmap): one warp; needs the band table of h rows twice in shared memory
     const size_t incr_smem = sizeof(float) * (INCR_D * 2 * INCR_SW + 2 * (INCR_CAP + 4)) + sizeof(int) * (INCR_D + 2 * (size_t) h);
-    const bool incr = c.incremental && n == 1 && !wide && incr_smem <= 160 * 1024;
-    if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
-        CK(ctx, cudaFuncSetAttribute(incr_walk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
-        if (!ctx->c_band) {
-            CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 4));
-            CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 4, ctx->stream));
+    const bool incr = Step::D == 1 && c.incremental && n == 1 && incr_smem <= 160 * 1024;
+    if constexpr (Step::D == 1) {
+        if (incr) {   // dynamic + static shared memory can exceed the 48 KB default
+            CK(ctx, cudaFuncSetAttribute(dctc_seam_incr_kernel<Step>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int) incr_smem));
+            if (!ctx->c_band) {
+                CK(ctx, cudaMalloc((void**) &ctx->c_band, sizeof(int) * 4));
+                CK(ctx, cudaMemsetAsync(ctx->c_band, 0, sizeof(int) * 4, ctx->stream));
+            }
         }
     }
     for (int s = 0; s < n_seams; s++) {
         const int w_old = f.w;
         int* log_s = f.seam_log + (size_t) s * h;
         const bool walk = incr && *c.m_valid;
-        if (walk) {
-            // update_mmap + build_vpath: walk the changed cells only; the DP below rebuilds the map only if the walk gave up
-            incr_walk<<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2, f.seam, log_s,
-                                                         ctx->c_band, pen);
-            CK(ctx, cudaGetLastError());
-            ctx->launches++;
+        if constexpr (Step::D == 1) {
+            if (walk) {
+                // update_mmap + build_vpath: walk the changed cells only; the DP below rebuilds the map only if the walk gave up
+                dctc_seam_incr_kernel<Step><<<1, 32, incr_smem, ctx->stream>>>(f.en, f.en_pitch, w_old, h, f.m, f.m_pitch, op.blocksize / 2,
+                                                                               f.seam, log_s, ctx->c_band, arg);
+                CK(ctx, cudaGetLastError());
+                ctx->launches++;
+            }
         }
-        // build_mmap, one cluster per frame, then build_vpath: jump maps of all 32-row blocks in parallel, one trace CTA per
+        // build_mmap, one cluster per frame, then build_vpath: jump maps of all row blocks in parallel, one trace CTA per
         // block and frame (programmatic dependent launches: each kernel of the loop is scheduled while its predecessor
         // drains and blocks in DCTC_PDL_PROLOGUE until that one's results are visible)
-        auto launch_dp = [&](auto fn, auto last) {
-            return dctc_launch_pdl(fn, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, !walk, f.en, f.en_pitch, w_old, h, f.m,
-                                   f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
-                                   walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, last);
-        };
-        CK(ctx, wide ? launch_dp(plan.dpw, steps) : launch_dp(plan.dp, pen));
-        if (bt.par && !walk && wide) {   // strips of 256 published columns, JBW-row blocks
-            const int js = (w_old + 255) / 256;
-            CK(ctx, dctc_launch_pdl(dctc_seam_jump_wide_kernel, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m,
-                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, js, m_fs, f.dir_fs, steps));
-            CK(ctx, dctc_launch_pdl(dctc_seam_trace_wide_kernel, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, true, f.m,
-                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, steps));
-            ctx->launches += 2;
-        } else if (bt.par && !walk) {
-            const int js = (w_old + 63) / 64;
-            CK(ctx, dctc_launch_pdl(jump, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m, f.m_pitch, w_old, h, f.dir,
-                                    bt.j_pitch, js, m_fs, f.dir_fs, pen));
-            CK(ctx, dctc_launch_pdl(trace, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, true, f.m, f.m_pitch, w_old, h,
-                                    f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, pen));
+        CK(ctx, dctc_launch_pdl(plan.dp, dim3(DP_CL, n), dim3(plan.wpc * 32), plan.smem, ctx->stream, !walk, f.en, f.en_pitch, w_old, h,
+                                f.m, f.m_pitch, f.seam, log_s, walk ? ctx->c_band : (int*) nullptr, plan.nst, plan.tmap,
+                                walk ? (int*) nullptr : xlast, en_fs, m_fs, log_fs, arg));
+        if (bt.par && !walk) {   // strips of 16 jc published columns
+            const int js = (w_old + 16 * G::jc - 1) / (16 * G::jc);
+            CK(ctx, dctc_launch_pdl(dctc_seam_jump_kernel<Step>, dim3((js + 3) / 4, bt.nb, n), dim3(128), 0, ctx->stream, true, f.m,
+                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, js, m_fs, f.dir_fs, arg));
+            CK(ctx, dctc_launch_pdl(dctc_seam_trace_kernel<Step>, dim3(bt.nb, n), dim3(TR_THREADS), bt.cone_smem, ctx->stream, true, f.m,
+                                    f.m_pitch, w_old, h, f.dir, bt.j_pitch, f.xlast, f.seam, log_s, m_fs, f.dir_fs, log_fs, arg));
             ctx->launches += 2;
         }
 #ifdef DCTC_SYNC_DEBUG
@@ -2021,6 +1795,24 @@ static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int
         CK(ctx, cudaMemcpyAsync(seams_out, f.seam_log, sizeof(int) * log_fs * n, cudaMemcpyDeviceToHost, ctx->stream));
     CK(ctx, cudaStreamSynchronize(ctx->stream));
     return DCTC_OK;
+}
+
+// c.rigidity: the seams are f.h rows long (the image width at the axis switch for height operations), so the step rule
+// gets pen = fl(rigidity / f.h) (DpStep1<true>; pen == 0 runs the kernels of rigidity 0, DpStep1<false>) or, for
+// c.delta_x > 1, the table of pen[d] (DpSteps).  The band K1 covers a seam drift of delta_x per row.
+static int seam_loop(dctc_context* ctx, CarverFrames& f, const DctcK1Op& op, int n_seams, int* seams_out, const SeamCall& c)
+{
+    const int h = f.h, dx = c.delta_x;
+    if (dx > 1) {
+        DpSteps steps;
+        steps.dx = dx;
+        for (int d = 0; d <= DCTC_MAX_DELTA_X; d++)   // the host carver's rigidity_map_of, +inf beyond the step bound
+            steps.pen[d] = d > dx ? INFINITY : (c.rigidity * ((float) d * sqrtf((float) d))) / (float) h;
+        return seam_loop_rule<DpSteps>(ctx, f, op, n_seams, seams_out, c, steps);
+    }
+    const float pen = c.rigidity / (float) h;
+    return pen != 0.0f ? seam_loop_rule<DpStep1<true>>(ctx, f, op, n_seams, seams_out, c, pen)
+                       : seam_loop_rule<DpStep1<false>>(ctx, f, op, n_seams, seams_out, c, pen);
 }
 
 // Enlarge core (lqr_carver_resize to a larger width, seams_number > 0, src/render.c:357-363): start_img holds a copy of

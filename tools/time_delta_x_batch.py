@@ -2,8 +2,9 @@
 """Cost of the seam step width in the batch seam loop: N distinct 1920x1080 RGB frames (ol.synth_image, seeds
 0x1920108 + i) reduced to 1440 wide (480 vertical seams) with delta_x = 1, 2 and 4, rigidity 0.  Every shape and step
 width runs once untimed before it is timed.  For every N it runs, in the same process, REPS alternations of: for each
-delta_x, load (untimed), then CarverBatch.resize_width(480), device events around the call.  delta_x = 1 launches per
-seam the seam DP, jump and trace kernels; delta_x > 1 the WIDE seam DP, which walks the seam back itself.
+delta_x, load (untimed), then CarverBatch.resize_width(480), device events around the call.  Every delta_x launches
+per seam the seam DP, jump and trace kernels (at this size every step width takes the parallel back-track), with the
+step rule of delta_x = 1 or the step table of delta_x > 1.
 Reports the time per batch seam and the ratio to delta_x = 1.
 python tools/time_delta_x_batch.py [N ...]   (DCTC_LIB=<path> loads an alternative build)"""
 import json
